@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 3 --warmup 1        # the reference's CPU path on the host cores
+    python bench.py --steps 40 --dump-outputs OUT    # also write the last timed step's results as OUT/<name>.npy
 
 Workload (BASELINE.json configs[1]): NIGHTS-shaped 2AFC triplets (reference, left, right), SD-1.5 512^2,
 up_blocks layer 0 => Q/K/V of shape (2,8,256,160) fp16 per image, AAS + cosine.  One step scores T triplets
@@ -41,6 +42,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 SHAPE = (2, 8, 256, 160)  # SD-1.5 512^2 up_blocks layer 0 (SURVEY.md section 8)
 # dram__bytes_read.sum + dram__bytes_write.sum of K1 per triplet, from the ncu --set full capture named in TRAFFIC_SOURCE
@@ -128,6 +130,17 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": statistics.median(sm), "sm_min_mhz": min(sm), "sm_max_mhz": max(s[1] for s in self.samples),
                 "reasons": reasons, "samples": len(self.samples), "power_w_max": max(s[2] for s in self.samples),
                 "source": "nvml" if self.nvml else "nvidia-smi"}
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write each result tensor as out_dir/<name>.npy: floating results as float32, integer results as float64 (exact
+    for int32), so that the outputs of two builds can be compared array by array."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
 
 
 def physical_gpu_index(local_rank: int) -> int:
@@ -465,7 +478,12 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not bind ranks to their GPU's NUMA-local CPUs")
     ap.add_argument("--profiler-range", action="store_true",
                     help="bracket the timed device-resident steps with cudaProfilerStart/Stop (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's ab, ac, counts, flags of "
+                         "score_triplets) as DIR/<name>.npy; the inputs are seeded, so runs with the same arguments compare")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -539,6 +557,8 @@ def main():
     ms_per_step = ms_total / args.steps
     value = world * pairs_per_step * args.steps / (ms_total * 1e-3)
     correct = int(counts[0].item())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ab": ab, "ac": ac, "counts": counts, "flags": flags})
 
     # ---- roofline of the dominant kernel ---------------------------------------------------------------------
     peaks = load_peaks()

@@ -59,16 +59,52 @@ def dino_images():
     return md.image(based, 1.0, torch.float16, "sd", g), md.image(based, 0.6, torch.float16, "sd", g)
 
 
+def clip_images():
+    """The inputs of the clip_cross golden case (tests/golden/make_golden_metrics.py): (q,k,v) of two images as
+    (1,12,50,64) views of (1,50,768) fp16 memory, then the fp16 out_proj weight and bias."""
+    import torch
+
+    from diffsim_b200 import synth
+
+    g = torch.Generator().manual_seed(32)
+    H, S, D = 12, 50, 64
+    mc = synth.SynthModel(1, H, S, D, seed=77)
+    basec = mc.new_base(g)
+    a = mc.image(basec, 1.0, torch.float16, "sd", g)
+    b = mc.image(basec, 0.7, torch.float16, "sd", g)
+    weight = (torch.randn(H * D, H * D, generator=g) / (H * D) ** 0.5).half()
+    bias = (0.1 * torch.randn(H * D, generator=g)).half()
+    return a, b, weight, bias
+
+
+def diffeats_features():
+    """The fp16 feature maps of the diffeats_minmax_cosine golden case (tests/golden/make_golden.py)."""
+    import torch
+
+    g = torch.Generator().manual_seed(6)
+    fa = torch.randn(2, 256, 320, generator=g) * 1.3 + 0.4
+    fb = 0.7 * fa + 0.5 * torch.randn(2, 256, 320, generator=g)
+    return fa.half(), fb.half()
+
+
+def gram_features():
+    """The fp16 ReLU-like feature maps of the gram golden case (tests/golden/make_golden_metrics.py)."""
+    import torch
+
+    g = torch.Generator().manual_seed(34)
+    fa = torch.randn(1, 64, 16, 24, generator=g).abs().half()
+    fb = (0.6 * fa.float() + 0.4 * torch.randn(1, 64, 16, 24, generator=g).abs()).half()
+    return fa, fb
+
+
 def regenerate_case(case):
-    """Rebuild the (q,k,v) images of a golden case from its seed; small cases carry their tensors."""
+    """Rebuild the (q,k,v) images of a golden case from its seed."""
     import torch
 
     from diffsim_b200 import synth
 
     dtype = getattr(torch, case["dtype"].split(".")[-1])
     B, H, S, D = case["shape"]
-    if "inputs" in case:
-        return [tuple(t.permute(0, 2, 1, 3) for t in im) for im in case["inputs"]]
     m = synth.SynthModel(B, H, S, D, seed=2334)
     if case["alphas"] is None:
         images, pairs = synth.make_pairs(m, case["n_pairs"], dtype, seed=case["seed"], layout=case["layout"])

@@ -13,8 +13,8 @@ recorded scores are produced by the reference's lines 177-197 with torch's own S
 mse_loss.  Likewise metrics/dino.py:attention_calc and metrics/diffeats.py:min_max_normalize are called from
 the imported reference modules.
 
-Inputs come from diffsim_b200.synth (seeded); small cases store the tensors themselves, large ones store a
-checksum so that tests can verify they regenerated identical inputs.
+Inputs come from seeded generators (diffsim_b200.synth, torch.Generator); the file stores their checksums, not the
+tensors, so that it stays small and tests can verify they regenerated identical inputs.
 """
 import importlib
 import importlib.abc
@@ -167,7 +167,7 @@ def main():
     golden = {"torch_version": torch.__version__, "cases": []}
     torch.set_num_threads(8)
 
-    def add_case(name, shape, dtype, layout, n_pairs, seed, store_inputs, alphas=None):
+    def add_case(name, shape, dtype, layout, n_pairs, seed, alphas=None):
         B, H, S, D = shape
         m = synth.SynthModel(B, H, S, D, seed=2334)
         if alphas is None:
@@ -181,8 +181,6 @@ def main():
                 pairs.append((0, len(images) - 1))
         case = {"name": name, "shape": shape, "dtype": str(dtype), "layout": layout, "n_pairs": len(pairs), "seed": seed,
                 "alphas": alphas, "pairs": pairs, "scores": {}, "checksums": [[checksum(t) for t in im] for im in images]}
-        if store_inputs:
-            case["inputs"] = [[t.permute(0, 2, 1, 3).contiguous() for t in im] for im in images]  # (B,S,H,D) memory
         for sim in ("cosine", "mse"):
             native, f32 = [], []
             for a, b in pairs:
@@ -193,19 +191,19 @@ def main():
         golden["cases"].append(case)
         print(name, {k: [round(x, 5) for x in v["reference_fp32_math"][:4]] for k, v in case["scores"].items()})
 
-    # small, fully stored
-    add_case("small_f32", (2, 2, 64, 40), torch.float32, "sd", 3, 11, True)
-    add_case("small_f16", (2, 2, 64, 40), torch.float16, "sd", 3, 12, True)
-    add_case("small_bf16", (2, 2, 64, 40), torch.bfloat16, "sd", 3, 13, True)
-    add_case("ragged_f16", (1, 3, 50, 64), torch.float16, "sd", 2, 14, True)           # CLIP-like 50 tokens
-    # the benchmark shapes, regenerated from the seed at test time
-    add_case("sd15_up0_f16_cute16", (2, 8, 256, 160), torch.float16, "sd", 16, 2334, False)  # config 1
-    add_case("sd15_up0_bf16", (2, 8, 256, 160), torch.bfloat16, "sd", 4, 21, False)
-    add_case("sd15_up0_alpha_sweep", (2, 8, 256, 160), torch.float16, "sd", 0, 22, False,
+    # small
+    add_case("small_f32", (2, 2, 64, 40), torch.float32, "sd", 3, 11)
+    add_case("small_f16", (2, 2, 64, 40), torch.float16, "sd", 3, 12)
+    add_case("small_bf16", (2, 2, 64, 40), torch.bfloat16, "sd", 3, 13)
+    add_case("ragged_f16", (1, 3, 50, 64), torch.float16, "sd", 2, 14)           # CLIP-like 50 tokens
+    # the benchmark shapes
+    add_case("sd15_up0_f16_cute16", (2, 8, 256, 160), torch.float16, "sd", 16, 2334)  # config 1
+    add_case("sd15_up0_bf16", (2, 8, 256, 160), torch.bfloat16, "sd", 4, 21)
+    add_case("sd15_up0_alpha_sweep", (2, 8, 256, 160), torch.float16, "sd", 0, 22,
              alphas=[1.0, 0.95, 0.8, 0.5, 0.2, 0.0])
-    add_case("dit_xl2_f16_packed", (2, 16, 256, 72), torch.float16, "dit", 4, 23, False)  # config 5
-    add_case("sd15_mid_f16", (2, 8, 64, 160), torch.float16, "sd", 3, 24, False)
-    add_case("sdxl_like_f16", (2, 4, 320, 64), torch.float16, "sd", 2, 25, False)
+    add_case("dit_xl2_f16_packed", (2, 16, 256, 72), torch.float16, "dit", 4, 23)  # config 5
+    add_case("sd15_mid_f16", (2, 8, 64, 160), torch.float16, "sd", 3, 24)
+    add_case("sdxl_like_f16", (2, 4, 320, 64), torch.float16, "sd", 2, 25)
 
     # metrics helpers from the reference modules
     extra = {}
@@ -234,7 +232,8 @@ def main():
 
         na, nb = diffeats.min_max_normalize(fa), diffeats.min_max_normalize(fb)
         cos = F.cosine_similarity(na.reshape(-1).unsqueeze(0), nb.reshape(-1).unsqueeze(0))
-        extra["diffeats_minmax_cosine"] = {"fa": fa.half(), "fb": fb.half(), "score_fp32_inputs": float(cos),
+        # the features are regenerated from the seed at test time (conftest.diffeats_features)
+        extra["diffeats_minmax_cosine"] = {"checksums": [checksum(fa.half()), checksum(fb.half())], "score_fp32_inputs": float(cos),
                                            "score_f16_inputs": float(F.cosine_similarity(
                                                diffeats.min_max_normalize(fa.half().float()).reshape(1, -1),
                                                diffeats.min_max_normalize(fb.half().float()).reshape(1, -1)))}

@@ -4,7 +4,7 @@ of tests/golden/metrics_golden.pt and the CPU oracle."""
 import pytest
 import torch
 
-from conftest import dino_images, ip_images
+from conftest import checksum, clip_images, dino_images, gram_features, ip_images
 from oracle import aas_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -16,11 +16,6 @@ def _cuda():
     if not torch.cuda.is_available():
         pytest.skip("needs a CUDA device")
     return torch.device("cuda:0")
-
-
-def _dev_views(mems, dev):
-    """(B,S,H,D) memory -> (B,H,S,D) views on the device, layout kept."""
-    return [m.to(dev).permute(0, 2, 1, 3) for m in mems]
 
 
 def _keep(t, dev):
@@ -76,9 +71,11 @@ def test_clip_cross_score_matches_the_reference_run(metrics_golden):
     from diffsim_b200 import metrics
 
     c = metrics_golden["clip_cross"]
-    (qa, qb), (ka, kb), (va, vb) = _dev_views(c["q"], dev), _dev_views(c["k"], dev), _dev_views(c["v"], dev)
+    img_a, img_b, w_host, bias_host = clip_images()
+    assert [[checksum(t) for t in im] for im in (img_a, img_b, (w_host, bias_host))] == c["checksums"]
+    (qa, ka, va), (qb, kb, vb) = (tuple(_keep(t, dev) for t in im) for im in (img_a, img_b))
     shape = (1, qa.shape[2], qa.shape[1] * qa.shape[3])
-    w, b = c["out_proj_weight"].to(dev), c["out_proj_bias"].to(dev)
+    w, b = w_host.to(dev), bias_host.to(dev)
     a_on_b = metrics.attention_calc(qa, kb, vb, c["scale"], shape, w, b)
     assert a_on_b.shape == shape and a_on_b.dtype == torch.float16
     ref = c["attention_calc_a_on_b_fp32"].double()
@@ -87,9 +84,7 @@ def test_clip_cross_score_matches_the_reference_run(metrics_golden):
     assert got.shape == (1,)
     # two 16-bit roundings (attention output, projection output) sit between the kernel path and the fp32 reference
     assert float(got) == pytest.approx(c["score_fp32_math"], rel=REL_16BIT)
-    cpu = lambda ts: [t.cpu() for t in ts]  # noqa: E731
-    t1 = O.clip_cross_score(*cpu((qa, ka, va)), *cpu((qb, kb, vb)), c["scale"], shape, c["out_proj_weight"],
-                            c["out_proj_bias"], round_to=torch.float16)
+    t1 = O.clip_cross_score(*img_a, *img_b, c["scale"], shape, w_host, bias_host, round_to=torch.float16)
     assert float(got) == pytest.approx(t1, rel=2e-4)
 
 
@@ -98,18 +93,20 @@ def test_gram_and_flat_feature_scores(metrics_golden):
     from diffsim_b200 import metrics
 
     c = metrics_golden["gram"]
-    fa, fb = c["fa"].to(dev), c["fb"].to(dev)
+    fa_host, fb_host = gram_features()
+    assert [checksum(fa_host), checksum(fb_host)] == c["checksums"]
+    fa, fb = fa_host.to(dev), fb_host.to(dev)
     g = metrics.gram_matrix(fa)
     ref = c["gram_a_fp32"].double()
     assert g.shape == (64, 64) and (g.double().cpu() - ref).abs().max().item() <= 1e-3 * ref.abs().max().item()  # fp16 ulp
     got = metrics.gram_similarity(fa, fb, match_reference_dtype=False)
     assert float(got) == pytest.approx(c["score_fp32_math"], rel=REL_16BIT)
-    assert float(got) == pytest.approx(O.gram_similarity(c["fa"], c["fb"], round_to=torch.float16), rel=1e-5)
+    assert float(got) == pytest.approx(O.gram_similarity(fa_host, fb_host, round_to=torch.float16), rel=1e-5)
     # flat cosine / embedding score / masked mean
     x, y = fa.reshape(1, -1), fb.reshape(1, -1)
     assert float(metrics.feature_score(x, y, False)) == pytest.approx(O.flat_cosine(x.cpu(), y.cpu()), rel=2e-5)
     s, n = metrics.embedding_score(fa.reshape(64, -1), fb.reshape(64, -1))
-    want = sum(100.0 * O.flat_cosine(c["fa"].reshape(64, -1)[i], c["fb"].reshape(64, -1)[i]) for i in range(64))
+    want = sum(100.0 * O.flat_cosine(fa_host.reshape(64, -1)[i], fb_host.reshape(64, -1)[i]) for i in range(64))
     assert n == 64 and float(s) == pytest.approx(want, rel=2e-5)
     grid = torch.randn(2, 24, 24, 32, device=dev)
     masks = (torch.rand(2, 1, 24, 24, device=dev) > 0.5).float()

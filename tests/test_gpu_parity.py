@@ -8,7 +8,7 @@ and like the reference's SDPA outputs; tier T0 rounds nothing), 1e-5 for the fp3
 import pytest
 import torch
 
-from conftest import regenerate_case
+from conftest import checksum, diffeats_features, regenerate_case
 from oracle import aas_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -342,7 +342,9 @@ def test_minmax_cosine_matches_reference_helper(golden):
     from diffsim_b200 import ops
 
     ex = golden["extra"]["diffeats_minmax_cosine"]
-    got = ops.pair_reduce(ex["fa"].reshape(1, -1).to(dev), ex["fb"].reshape(1, -1).to(dev), "minmax_cosine")
+    fa, fb = diffeats_features()
+    assert [checksum(fa), checksum(fb)] == ex["checksums"]
+    got = ops.pair_reduce(fa.reshape(1, -1).to(dev), fb.reshape(1, -1).to(dev), "minmax_cosine")
     assert got.item() == pytest.approx(ex["score_f16_inputs"], rel=1e-5)
 
 

@@ -7,13 +7,8 @@ import zlib
 import pytest
 import torch
 
-from conftest import checksum, dino_images, ip_images
+from conftest import checksum, clip_images, dino_images, gram_features, ip_images
 from oracle import aas_oracle as O
-
-
-def _views(mems):
-    """(B,S,H,D) memory -> the hook's (B,H,S,D) views."""
-    return [m.permute(0, 2, 1, 3) for m in mems]
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -34,11 +29,12 @@ def test_oracle_ip_adapter_matches_reference_run(metrics_golden):
 
 def test_oracle_clip_cross_matches_reference_run(metrics_golden):
     c = metrics_golden["clip_cross"]
-    (qa, qb), (ka, kb), (va, vb) = _views(c["q"]), _views(c["k"]), _views(c["v"])
+    (qa, ka, va), (qb, kb, vb), w, b = clip_images()
+    assert [[checksum(t) for t in im] for im in ((qa, ka, va), (qb, kb, vb), (w, b))] == c["checksums"]
     shape = (1, qa.shape[2], qa.shape[1] * qa.shape[3])
-    got = O.clip_cross_score(qa, ka, va, qb, kb, vb, c["scale"], shape, c["out_proj_weight"], c["out_proj_bias"])
+    got = O.clip_cross_score(qa, ka, va, qb, kb, vb, c["scale"], shape, w, b)
     assert got == pytest.approx(c["score_fp32_math"], rel=5e-5)
-    a_on_b = O.clip_attention_calc(qa, kb, vb, c["scale"], shape, c["out_proj_weight"], c["out_proj_bias"])
+    a_on_b = O.clip_attention_calc(qa, kb, vb, c["scale"], shape, w, b)
     assert (a_on_b - c["attention_calc_a_on_b_fp32"].double()).abs().max().item() < 2e-5
 
 
@@ -52,8 +48,10 @@ def test_oracle_dino_cross_matches_reference_run(metrics_golden):
 
 def test_oracle_gram_matches_reference_run(metrics_golden):
     c = metrics_golden["gram"]
-    assert (O.gram_matrix(c["fa"]) - c["gram_a_fp32"].double()).abs().max().item() < 1e-2   # fp32 sums of 384 products ~ 600
-    assert O.gram_similarity(c["fa"], c["fb"]) == pytest.approx(c["score_fp32_math"], rel=2e-6)
+    fa, fb = gram_features()
+    assert [checksum(fa), checksum(fb)] == c["checksums"]
+    assert (O.gram_matrix(fa) - c["gram_a_fp32"].double()).abs().max().item() < 1e-2   # fp32 sums of 384 products ~ 600
+    assert O.gram_similarity(fa, fb) == pytest.approx(c["score_fp32_math"], rel=2e-6)
 
 
 # ------------------------------------------------------------------------------------------------------

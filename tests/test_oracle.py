@@ -5,7 +5,7 @@ import math
 import pytest
 import torch
 
-from conftest import checksum, regenerate_case
+from conftest import checksum, diffeats_features, regenerate_case
 from oracle import aas_oracle as O
 
 
@@ -106,7 +106,9 @@ def test_cosine_eps_semantics():
 
 def test_minmax_cosine_matches_reference_helper(golden):
     ex = golden["extra"]["diffeats_minmax_cosine"]
-    got = O.minmax_cosine(ex["fa"], ex["fb"])
+    fa, fb = diffeats_features()
+    assert [checksum(fa), checksum(fb)] == ex["checksums"]
+    got = O.minmax_cosine(fa, fb)
     assert got == pytest.approx(ex["score_f16_inputs"], rel=2e-6)
 
 
