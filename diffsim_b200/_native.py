@@ -60,6 +60,11 @@ PROTOTYPES = {
     "ds_debug_set_attn_l2_promotion": (_i, [_i]),
     "ds_attn_fwd": (_i, [Tensor4, Tensor4, Tensor4, _f, Tensor4, _vp, _sz, _vp]),
     "ds_attn_fwd_workspace_bytes": (_sz, [Tensor4, Tensor4]),
+    "ds_attn_bwd": (_i, [Tensor4, Tensor4, Tensor4, Tensor4, Tensor4, _f, Tensor4, Tensor4, Tensor4, _vp, _sz, _vp]),
+    "ds_attn_bwd_workspace_bytes": (_sz, [Tensor4, Tensor4]),
+    "ds_aas_dir_bwd": (_i, [Tensor4, Tensor4, Tensor4, Tensor4, Tensor4, _f, _i, _vp, Tensor4, Tensor4, Tensor4, Tensor4,
+                            Tensor4, _vp, _sz, _vp]),
+    "ds_aas_dir_bwd_workspace_bytes": (_sz, [Tensor4, Tensor4]),
     "ds_aas_groups": (_i, [Tensor5, Tensor5, Tensor5, Tensor5, Tensor5, _vp, _vp, _i64, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),
     "ds_aas_groups_workspace_bytes": (_sz, [Tensor5, _i64, _i64]),
     "ds_aas_pairs": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),

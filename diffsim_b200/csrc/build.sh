@@ -9,7 +9,7 @@ mkdir -p "${OUT}" "${OBJ}"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC
        --expt-relaxed-constexpr -cudart static ${DS_EXTRA_NVCC_FLAGS:-})
-SRCS=(ds_host.cu ds_reduce.cu ds_simmat.cu ds_qkv.cu ds_attn.cu)
+SRCS=(ds_host.cu ds_reduce.cu ds_simmat.cu ds_qkv.cu ds_attn.cu ds_attn_bwd.cu)
 pids=()
 for s in "${SRCS[@]}"; do
   [ -f "${HERE}/${s}" ] || continue

@@ -53,14 +53,12 @@ def aas_score(A: QKV, B: QKV, similarity: str = "cosine", scale: Optional[float]
     """The tail of DiffSim.diffsim (diffsim/diffsim.py:177-197) on captured (q,k,v) of two images.
 
     Two launches of the fused kernel, one per direction; each evaluates the query image's self attention and the
-    cross attention against the other image's K/V and reduces them on chip.  The q/k/v views are passed as they
+    cross attention against the other image's K/V and reduces them on chip.  Differentiable in all six inputs when one
+    of them requires grad (K5 backward, ops.aas_dir_bwd); the score is the same either way.  The q/k/v views are passed as they
     are (unsqueeze(0) adds the image axis without copying).  With match_reference_dtype the result has the
     reference's dtype and shape: input dtype, (1,) for cosine and () for MSE."""
     (qa, ka, va), (qb, kb, vb) = A, B
-    one = [0]
-    off = [0, 1]
-    d_ab = ops.aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, similarity, scale)
-    d_ba = ops.aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, similarity, scale)
+    d_ab, d_ba = ops.pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale)
     if not match_reference_dtype:
         return (d_ab + d_ba) * 0.5
     dt = qa.dtype
@@ -87,11 +85,9 @@ def aas_score_ip_adapter(A, B, similarity: str = "cosine", scale: Optional[float
                              "diffsim/diffsim.py:191-192, is not executable; only similarity='cosine' is defined)")
     if not (len(ka_l) == len(va_l) == len(kb_l) == len(vb_l)) or len(ka_l) == 0:
         raise RuntimeError("both images need the same, non-zero number of ip key/value tensors")
-    one, off = [0], [0, 1]
-    d_ab = [ops.aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, "cosine", scale)
-            for ka, va, kb, vb in zip(ka_l, va_l, kb_l, vb_l)]
-    d_ba = [ops.aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, "cosine", scale)
-            for ka, va, kb, vb in zip(ka_l, va_l, kb_l, vb_l)]
+    dirs = [ops.pair_dirs(qa, ka, va, qb, kb, vb, "cosine", scale) for ka, va, kb, vb in zip(ka_l, va_l, kb_l, vb_l)]
+    d_ab = [d[0] for d in dirs]
+    d_ba = [d[1] for d in dirs]
     if match_reference_dtype:
         dt = qa.dtype   # torch.mean(torch.stack([...], dim=0)) of (1,) fp16 tensors is a 0-d fp16 tensor
         m_ab = torch.mean(torch.stack([d.to(dt) for d in d_ab], dim=0))

@@ -99,11 +99,25 @@ def _i32(x, dev) -> torch.Tensor:
 # --------------------------------------------------------------------------------------
 # K1: attention
 # --------------------------------------------------------------------------------------
+def wants_grad(*ts: torch.Tensor) -> bool:
+    """True when autograd records this call: grad mode is on and some input requires grad."""
+    return torch.is_grad_enabled() and any(t.requires_grad for t in ts)
+
+
 def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Optional[float] = None,
              out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """softmax(q k^T * scale) v per (b,h) -- F.scaled_dot_product_attention(q,k,v,dropout_p=0.0,is_causal=False)
     (diffsim/hacked_attn.py:81-83, diffsim/diffsim.py:177-180).  Returns (B,H,Sq,D) in q's dtype, laid out like
-    the reference's head-split views: memory (B,Sq,H*D)."""
+    the reference's head-split views: memory (B,Sq,H*D).  Differentiable (attn_bwd) when an input requires grad;
+    `out` is not accepted then."""
+    if wants_grad(q, k, v):
+        if out is not None:
+            raise RuntimeError("attn_fwd: out= is not supported when an input requires grad")
+        return _AttnFn.apply(q, k, v, scale)
+    return _attn_fwd(q, k, v, scale, out)
+
+
+def _attn_fwd(q, k, v, scale=None, out=None) -> torch.Tensor:
     lib = N.load()
     dev = _need_cuda(q, k, v)
     B, H, Sq, D = q.shape
@@ -117,6 +131,117 @@ def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Optional[
                                 _stream(dev)))
     _count(2)  # meta + attention
     return out
+
+
+class _AttnFn(torch.autograd.Function):
+    """attn_fwd with the K5 backward; saves only the inputs and recomputes the output in backward."""
+
+    @staticmethod
+    def forward(ctx, q, k, v, scale):
+        ctx.save_for_backward(q, k, v)
+        ctx.scale = scale
+        return _attn_fwd(q, k, v, scale)
+
+    @staticmethod
+    def backward(ctx, dout):
+        q, k, v = ctx.saved_tensors
+        out = _attn_fwd(q, k, v, ctx.scale)
+        dq, dk, dv = attn_bwd(q, k, v, out, dout, ctx.scale)
+        return dq, dk, dv, None
+
+
+def _tma_ok(t: torch.Tensor) -> torch.Tensor:
+    # a 16-bit operand the library reads by TMA: unit innermost stride, 16-byte aligned base and rows (autograd hands
+    # out expanded or otherwise arbitrary gradients)
+    ok = t.stride(-1) == 1 and t.data_ptr() % 16 == 0 and all(
+        n == 1 or (s > 0 and s % 8 == 0) for n, s in zip(t.shape[:-1], t.stride()[:-1]))
+    return t if ok else t.contiguous()
+
+
+def _grads_like(ts, grads) -> Tuple[torch.Tensor, ...]:
+    if grads is None:
+        return tuple(torch.zeros(t.shape, dtype=torch.float32, device=t.device) for t in ts)
+    if len(grads) != len(ts) or any(g.dtype != torch.float32 or g.shape != t.shape for g, t in zip(grads, ts)):
+        raise RuntimeError("grads must be float32 tensors of the inputs' shapes")
+    return tuple(grads)
+
+
+def attn_bwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, out: torch.Tensor, dout: torch.Tensor,
+             scale: Optional[float] = None, grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
+    """Gradients (dq, dk, dv) of attn_fwd for the output gradient dout, in float32 (deterministic: no atomics).
+    out: the forward output attn_fwd(q, k, v, scale).  grads: optional float32 (dq, dk, dv) to add into."""
+    lib = N.load()
+    dev = _need_cuda(q, k, v, out, dout)
+    dout = _tma_ok(dout.to(q.dtype))
+    dq, dk, dv = _grads_like((q, k, v), grads)
+    q4, k4 = _t4(q), _t4(k)
+    ws = _workspace(dev, lib.ds_attn_bwd_workspace_bytes(q4, k4), "bwd")
+    with torch.cuda.device(dev):
+        N.check(lib.ds_attn_bwd(q4, k4, _t4(v), _t4(out), _t4(dout), float(scale) if scale else 0.0, _t4(dq), _t4(dk),
+                                _t4(dv), ws.data_ptr(), ws.numel(), _stream(dev)))
+    _count(2)  # dQ + dK/dV
+    return dq, dk, dv
+
+
+def aas_dir_bwd(q_i: torch.Tensor, k_i: torch.Tensor, v_i: torch.Tensor, k_j: torch.Tensor, v_j: torch.Tensor,
+                d_dir: torch.Tensor, similarity="cosine", scale: Optional[float] = None,
+                grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
+    """Gradients (dq_i, dk_i, dv_i, dk_j, dv_j) of dir = sim(Attn(q_i,k_j,v_j), Attn(q_i,k_i,v_i)) for dL/ddir = d_dir
+    (a one-element tensor on the device; no host sync), in float32.  (B,H,S,D) inputs as for attn_fwd.
+    grads: optional float32 tensors to add into (they may alias, e.g. dk_i is dk_j when image i is image j)."""
+    lib = N.load()
+    dev = _need_cuda(q_i, k_i, v_i, k_j, v_j, d_dir)
+    g = d_dir.detach().reshape(-1).to(torch.float32)
+    if g.numel() != 1:
+        raise RuntimeError("d_dir must have exactly one element")
+    out = _grads_like((q_i, k_i, v_i, k_j, v_j), grads)
+    q4, kj4 = _t4(q_i), _t4(k_j)
+    ws = _workspace(dev, lib.ds_aas_dir_bwd_workspace_bytes(q4, kj4), "bwd")
+    with torch.cuda.device(dev):
+        N.check(lib.ds_aas_dir_bwd(q4, _t4(k_i), _t4(v_i), kj4, _t4(v_j), float(scale) if scale else 0.0,
+                                   _mode(similarity), g.data_ptr(), *[_t4(t) for t in out], ws.data_ptr(), ws.numel(),
+                                   _stream(dev)))
+    _count(11)  # 2 x (meta + attention) recompute + partials + coefficients + factors + 2 x (dQ + dK/dV)
+    return out
+
+
+def _pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale):
+    one, off = [0], [0, 1]
+    d_ab = aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, similarity, scale)
+    d_ba = aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, similarity, scale)
+    return d_ab, d_ba
+
+
+def pair_dirs_bwd(qa, ka, va, qb, kb, vb, g_ab, g_ba, similarity="cosine", scale=None) -> Tuple[torch.Tensor, ...]:
+    """float32 gradients of (qa, ka, va, qb, kb, vb) for dL/d dir(a->b) = g_ab and dL/d dir(b->a) = g_ba (either may be
+    None), accumulated in float32 in a fixed order."""
+    grads = _grads_like((qa, ka, va, qb, kb, vb), None)
+    dqa, dka, dva, dqb, dkb, dvb = grads
+    if g_ab is not None:
+        aas_dir_bwd(qa, ka, va, kb, vb, g_ab, similarity, scale, grads=(dqa, dka, dva, dkb, dvb))
+    if g_ba is not None:
+        aas_dir_bwd(qb, kb, vb, ka, va, g_ba, similarity, scale, grads=(dqb, dkb, dvb, dka, dva))
+    return grads
+
+
+class _PairDirsFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, similarity, scale, qa, ka, va, qb, kb, vb):
+        ctx.save_for_backward(qa, ka, va, qb, kb, vb)
+        ctx.similarity, ctx.scale = similarity, scale
+        return _pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale)
+
+    @staticmethod
+    def backward(ctx, g_ab, g_ba):
+        return (None, None) + pair_dirs_bwd(*ctx.saved_tensors, g_ab, g_ba, ctx.similarity, ctx.scale)
+
+
+def pair_dirs(qa, ka, va, qb, kb, vb, similarity="cosine", scale: Optional[float] = None):
+    """(dir(a->b), dir(b->a)) of one image pair as float32 (1,) tensors -- two aas_groups launches.  Differentiable
+    (aas_dir_bwd) when an input requires grad; the values are the same either way."""
+    if wants_grad(qa, ka, va, qb, kb, vb):
+        return _PairDirsFn.apply(similarity, scale, qa, ka, va, qb, kb, vb)
+    return _pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale)
 
 
 def aas_groups(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,

@@ -10,6 +10,7 @@ strides), and this module registers its calls with the dispatcher so that refere
 
 There is no CPU (or any other) kernel behind these operators: called on CPU tensors the dispatcher raises
 NotImplementedError -- the loud failure the path requires.  `scale = 0.0` means the default 1/sqrt(D).
+attn_fwd and aas_score have autograd kernels (K5 backward); the other operators are forward-only.
 """
 from __future__ import annotations
 
@@ -78,5 +79,30 @@ for _name, _fn in (("attn_fwd", _attn_fwd), ("aas_score", _aas_score), ("aas_pai
                    ("aas_triplets", _aas_triplets), ("aas_matrix", _aas_matrix), ("pair_reduce", _pair_reduce),
                    ("simmat", _simmat), ("qkv_project", _qkv_project)):
     _lib.impl(_name, _fn, "CUDA")
+
+
+# Gradients (K5): attn_fwd and aas_score are differentiable in their tensor inputs.  Only the inputs are saved; the
+# backward recomputes what it needs.  The float32 gradients are cast to the input dtype by the autograd engine.
+def _setup_inputs(ctx, inputs, output):
+    ctx.save_for_backward(*[t for t in inputs if isinstance(t, torch.Tensor)])
+    ctx.rest = [x for x in inputs if not isinstance(x, torch.Tensor)]
+
+
+def _attn_fwd_bwd(ctx, dout):
+    q, k, v = ctx.saved_tensors
+    (scale,) = ctx.rest or [0.0]
+    out = ops.attn_fwd(q, k, v, _sc(scale))
+    return ops.attn_bwd(q, k, v, out, dout, _sc(scale)) + (None,)
+
+
+def _aas_score_bwd(ctx, grad):
+    similarity, scale = (ctx.rest + ["cosine", 0.0][len(ctx.rest):])[:2]
+    g = grad.reshape(1) * 0.5   # score = (dir(a->b) + dir(b->a)) / 2
+    return ops.pair_dirs_bwd(*ctx.saved_tensors, g, g, similarity, _sc(scale)) + (None, None)
+
+
+torch.library.register_autograd("diffsim_b200::attn_fwd", _attn_fwd_bwd, setup_context=_setup_inputs, lib=_lib)
+torch.library.register_autograd("diffsim_b200::aas_score", _aas_score_bwd, setup_context=_setup_inputs, lib=_lib)
+DIFFERENTIABLE = ("attn_fwd", "aas_score")
 
 OPERATORS = ("attn_fwd", "aas_score", "aas_pairs", "aas_triplets", "aas_matrix", "pair_reduce", "simmat", "qkv_project")

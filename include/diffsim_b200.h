@@ -198,6 +198,37 @@ int ds_aas_matrix(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self,
                   void* ws, size_t ws_bytes, void* stream);
 size_t ds_aas_matrix_workspace_bytes(ds_tensor5 q, ds_tensor5 k);
 
+/* ---- K5: gradients ------------------------------------------------------ */
+
+/*
+ * Backward of ds_attn_fwd (of F.scaled_dot_product_attention without mask or
+ * dropout): given out = ds_attn_fwd(q, k, v, scale) and dout = dL/dout,
+ *     dq += dL/dq,  dk += dL/dk,  dv += dL/dv.
+ * q, k, v, out, dout: 16-bit tensors as in ds_attn_fwd (any strides with a unit
+ * innermost one).  dq, dk, dv: FLOAT32 tensors of q's / k's / v's shape that the
+ * call ADDS INTO (so several calls accumulate in fp32 in a fixed order).  No
+ * float atomics: the result is bitwise reproducible.  Head dims 40, 64, 72,
+ * 80, 128, 160.
+ */
+int ds_attn_bwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, ds_tensor4 out, ds_tensor4 dout, float scale,
+                ds_tensor4 dq, ds_tensor4 dk, ds_tensor4 dv, void* ws, size_t ws_bytes, void* stream);
+size_t ds_attn_bwd_workspace_bytes(ds_tensor4 q, ds_tensor4 k);
+
+/*
+ * Backward of the directional similarity of ds_aas_groups,
+ *     dir = sim( Attn(q_i, k_j, v_j), Attn(q_i, k_i, v_i) )   (mode DS_SIM_COSINE | DS_SIM_MSE),
+ * with both attention outputs rounded to the input dtype as in the forward and
+ * the rounding passed straight through.  d_dir: ONE float on the device (dL/ddir;
+ * read there, no host synchronisation).  The five FLOAT32 gradients are added
+ * into; they may alias (dk_i = dk_j when image i is image j).  dq_i receives
+ * the cross term before the self term.
+ */
+int ds_aas_dir_bwd(ds_tensor4 q_i, ds_tensor4 k_i, ds_tensor4 v_i, ds_tensor4 k_j, ds_tensor4 v_j,
+                   float scale, int mode, const float* d_dir,
+                   ds_tensor4 dq_i, ds_tensor4 dk_i, ds_tensor4 dv_i, ds_tensor4 dk_j, ds_tensor4 dv_j,
+                   void* ws, size_t ws_bytes, void* stream);
+size_t ds_aas_dir_bwd_workspace_bytes(ds_tensor4 q_i, ds_tensor4 k_j);
+
 /* ---- K2: similarity reductions ----------------------------------------- */
 
 /*
