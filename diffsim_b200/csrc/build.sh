@@ -14,7 +14,7 @@ pids=()
 for s in "${SRCS[@]}"; do
   [ -f "${HERE}/${s}" ] || continue
   o="${OBJ}/${s%.cu}.o"
-  if [ ! -f "$o" ] || [ "${HERE}/${s}" -nt "$o" ] || [ "${HERE}/ds_ptx.cuh" -nt "$o" ] || [ "${HERE}/ds_gemm.cuh" -nt "$o" ] || [ "${HERE}/ds_host.h" -nt "$o" ] \
+  if [ ! -f "$o" ] || [ "${HERE}/${s}" -nt "$o" ] || [ "${HERE}/ds_ptx.cuh" -nt "$o" ] || [ "${HERE}/ds_attn_common.cuh" -nt "$o" ] || [ "${HERE}/ds_gemm.cuh" -nt "$o" ] || [ "${HERE}/ds_host.h" -nt "$o" ] \
      || [ "${HERE}/../../include/diffsim_b200.h" -nt "$o" ]; then
     "${NVCC}" "${FLAGS[@]}" -Xptxas -v -c "${HERE}/${s}" -o "$o" 2> "${OBJ}/${s%.cu}.ptxas.log" &
     pids+=($!)

@@ -41,8 +41,7 @@
 //
 // Replaces diffsim/diffsim.py:177-197 (diffsim_xl.py:135-155, diffsim_dit.py:130-142).
 // Algorithmic work per directional attention: 4*B*H*Sq*Skv*D flops.
-#include "ds_host.h"
-#include "ds_ptx.cuh"
+#include "ds_attn_common.cuh"
 
 namespace ds {
 
@@ -66,29 +65,24 @@ constexpr int kTmemOs = 416;     // O_self, packed 16-bit: [416, 416 + D_PAD/2)
 constexpr int kTmemL = 496;      // softmax denominators l = P . 1 (a 16-column MMA against a constant ones tile): [496,512)
 
 template <int D>
-struct AttnCfg {
-  static constexpr int D_PAD = (D + 15) / 16 * 16;
+struct AttnCfg : AttnTile<D> {
+  using Tile = AttnTile<D>;
   // Every POLY_STRIDE-th pair of exponentials is evaluated with a degree-3 polynomial on the FMA pipe instead of MUFU
   // (0: none).  With head dims <= 80 an item carries at most half the tensor work of D = 160 but the same 32 768
   // exponentials, and long-kv streams of such items are MUFU-bound: measured +13% on SDXL (2,20,1024,64) / (2,10,4096,64),
   // +6% on SD-1.5 up1 / up2, neutral on DiT-XL/2, and -4% at D = 160 (profiles/r1z_poly_shapes.txt).
   static constexpr int POLY_STRIDE = DS_POLY_STRIDE >= 0 ? DS_POLY_STRIDE : (D <= 80 ? 3 : 0);
-  static constexpr int SUBW = (D % 64 == 0) ? 64 : 32;           // elements per swizzle row
-  static constexpr int SUB_BYTES = SUBW * 2;                      // 128 or 64: TMA box row == swizzle span
-  static constexpr int NSUB = (D_PAD + SUBW - 1) / SUBW;
-  static constexpr uint32_t LAYOUT = (SUBW == 64) ? UMMA_SW128 : UMMA_SW64;
-  static constexpr int CPS = SUBW / 16;                           // 16-element K chunks per sub-tile
-  static constexpr int Q_SUB_BYTES = kBlockQ * SUB_BYTES;
-  static constexpr int Q_BYTES = NSUB * Q_SUB_BYTES;
-  static constexpr int KV_SUB_BYTES = kHalfKV * SUB_BYTES;
-  static constexpr int STAGE_BYTES = NSUB * KV_SUB_BYTES;
+  static constexpr int Q_SUB_BYTES = kBlockQ * Tile::SUB_BYTES;
+  static constexpr int Q_BYTES = Tile::NSUB * Q_SUB_BYTES;
+  static constexpr int KV_SUB_BYTES = kHalfKV * Tile::SUB_BYTES;
+  static constexpr int STAGE_BYTES = Tile::NSUB * KV_SUB_BYTES;
   static constexpr int MISC_BYTES = 2048 /*ones tile*/ + 4096 /*max exchange*/ + 128 /*epilogue reduce*/ + 512 /*barriers*/;
   static constexpr int kMaxSmem = 232448;
   static constexpr int STAGES_RAW = (kMaxSmem - Q_BYTES - MISC_BYTES) / STAGE_BYTES;
   static constexpr int STAGES = STAGES_RAW > 12 ? 12 : STAGES_RAW;
   static constexpr int SMEM_BYTES = Q_BYTES + STAGES * STAGE_BYTES + MISC_BYTES;
   static_assert(STAGES >= 4, "not enough shared memory for the K/V ring");
-  static_assert(kTmemO + D_PAD <= kTmemOs && kTmemOs + D_PAD / 2 <= kTmemL, "TMEM budget");
+  static_assert(kTmemO + Tile::D_PAD <= kTmemOs && kTmemOs + Tile::D_PAD / 2 <= kTmemL, "TMEM budget");
   static_assert(Q_BYTES % 1024 == 0 && STAGE_BYTES % 1024 == 0, "swizzle atoms need 1024-byte aligned tiles");
 };
 
@@ -966,37 +960,7 @@ __global__ void matrix_setup_kernel(int64_t n_rows, int64_t n_cols, int chunks, 
 // head's D elements (80-320 bytes) out of a (B, S, H*D) memory row whose other heads are needed much later (streams are
 // head-major): with 256-byte promotion every miss dragged the neighbouring heads' bytes in from DRAM -- 17.1 MB per triplet
 // against 11.8 MB algorithmic at D = 160, 2.9x at DiT's 144-byte rows.  64 bytes: +3% sustained, +5% DiT (gpurun_out/r2bc).
-static int g_attn_l2_promotion = 64;
-
-static int check_t5(const ds_tensor5& t, const char* name) {
-  if (!t.ptr) return fail(DS_ERR_INVALID, "%s: null pointer", name);
-  if (t.dtype != DS_F16 && t.dtype != DS_BF16) return fail(DS_ERR_UNSUPPORTED, "%s: dtype must be f16 or bf16", name);
-  for (int i = 0; i < 5; ++i)
-    if (t.size[i] <= 0) return fail(DS_ERR_INVALID, "%s: size[%d] = %lld", name, i, (long long)t.size[i]);
-  if (t.stride[4] != 1) return fail(DS_ERR_INVALID, "%s: innermost stride must be 1 (got %lld)", name, (long long)t.stride[4]);
-  if ((uintptr_t)t.ptr & 15) return fail(DS_ERR_INVALID, "%s: base pointer must be 16-byte aligned", name);
-  for (int i = 0; i < 4; ++i) {
-    if (t.size[i] > 1 && (t.stride[i] <= 0 || (t.stride[i] & 7)))
-      return fail(DS_ERR_INVALID, "%s: stride[%d] = %lld must be a positive multiple of 8 elements (16 bytes)", name, i,
-                  (long long)t.stride[i]);
-  }
-  if (t.size[0] > INT32_MAX || t.size[3] > INT32_MAX) return fail(DS_ERR_INVALID, "%s: too large", name);
-  return DS_OK;
-}
-
-static int make_map(CUtensorMap* m, const ds_tensor5& t, int subw, int rows) {
-  // TMA dims, fastest first: (d, s, h, b, n)
-  uint64_t dims[5] = {(uint64_t)t.size[4], (uint64_t)t.size[3], (uint64_t)t.size[2], (uint64_t)t.size[1],
-                      (uint64_t)t.size[0]};
-  auto st = [&](int i) -> uint64_t {
-    // a size-1 dimension may carry any stride; give it a harmless 16-byte one
-    int64_t s = t.size[i] > 1 ? t.stride[i] : 8;
-    return (uint64_t)s * 2;
-  };
-  uint64_t strides[4] = {st(3), st(2), st(1), st(0)};
-  uint32_t box[5] = {(uint32_t)subw, (uint32_t)rows, 1, 1, 1};
-  return encode_tensor_map(m, t.dtype, 5, t.ptr, dims, strides, box, subw * 2, g_attn_l2_promotion);
-}
+int g_attn_l2_promotion = 64;
 
 // ds_debug_set_attn_mc: -1 automatic (the N x N matrix only: +2-3% there, -1% sustained and +16% DRAM reads on pair / triplet
 // lists, profiles/r2_attn_experiments.txt section 8), 0 off, 1 on wherever the q tile count is even
@@ -1064,7 +1028,7 @@ static int launch_attn_mode(const AttnLaunch& a, int grid, const CUtensorMap& mq
 }
 
 template <int D>
-static int launch_attn_d(const AttnLaunch& a, cudaStream_t st) {
+static int launch_attn_d(AttnLaunch a, cudaStream_t st) {
   using C = AttnCfg<D>;
   CUtensorMap mq, mks, mvs, mk, mv;
   int rc;
@@ -1075,9 +1039,9 @@ static int launch_attn_d(const AttnLaunch& a, cudaStream_t st) {
   if ((rc = make_map(&mv, a.v, C::SUBW, kHalfKV)) != DS_OK) return rc;
   const int64_t n_streams = (int64_t)a.p.n_groups * a.p.B * a.p.H * a.p.n_qt;
   if (n_streams >= (int64_t)1 << 31) return fail(DS_ERR_INVALID, "too many (group, head, q-tile) streams in one call: split the work list");
-  const_cast<AttnLaunch&>(a).p.trace = g_trace_ptr;
-  const_cast<AttnLaunch&>(a).p.trace_cap = g_trace_cap;
-  const_cast<AttnLaunch&>(a).p.cycles = g_trace_ptr ? g_trace_ptr + (size_t)8 * g_trace_cap : nullptr;
+  a.p.trace = g_trace_ptr;
+  a.p.trace_cap = g_trace_cap;
+  a.p.cycles = g_trace_ptr ? g_trace_ptr + (size_t)8 * g_trace_cap : nullptr;
   int grid = sm_count();
   if (n_streams < grid) grid = (int)n_streams;
   if (g_attn_grid > 0 && g_attn_grid < grid) grid = g_attn_grid;
@@ -1085,40 +1049,31 @@ static int launch_attn_d(const AttnLaunch& a, cudaStream_t st) {
   // K/V multicast over CTA pairs needs the two q tiles of a pair to exist (q tile is the fastest stream index, so CTAs
   // 2c and 2c + 1 hold q tiles 2j and 2j + 1 of the same (group, b, h) when n_qt and the grid are even)
   const bool want_mc = g_attn_mc == 1 || (g_attn_mc < 0 && a.prefer_mc);
-  const_cast<AttnLaunch&>(a).p.mc = (want_mc && a.p.n_qt % 2 == 0 && grid >= 2) ? 1 : 0;
+  a.p.mc = (want_mc && a.p.n_qt % 2 == 0 && grid >= 2) ? 1 : 0;
   profile_begin(st);
-  int rc2 = DS_OK;
-  if (a.q.dtype == DS_BF16) rc2 = launch_attn_mode<D, true>(a, grid, mq, mks, mvs, mk, mv, st);
-  else rc2 = launch_attn_mode<D, false>(a, grid, mq, mks, mvs, mk, mv, st);
-  if (rc2 != DS_OK) return rc2;
+  rc = with_dtype(a.q.dtype, [&](auto bf) {
+    return launch_attn_mode<D, decltype(bf)::value>(a, grid, mq, mks, mvs, mk, mv, st);
+  });
+  if (rc != DS_OK) return rc;
   profile_end(st);
   DS_CUDA_TRY(cudaGetLastError());
   return DS_OK;
 }
 
-static int launch_attn(const AttnLaunch& a, cudaStream_t st) {
-  switch ((int)a.q.size[4]) {
-    case 40: return launch_attn_d<40>(a, st);
-    case 64: return launch_attn_d<64>(a, st);
-    case 72: return launch_attn_d<72>(a, st);
-    case 80: return launch_attn_d<80>(a, st);
-    case 128: return launch_attn_d<128>(a, st);
-    case 160: return launch_attn_d<160>(a, st);
-    default:
-      return fail(DS_ERR_UNSUPPORTED, "head dim %lld is not built (supported: 40, 64, 72, 80, 128, 160)",
-                  (long long)a.q.size[4]);
-  }
+static int launch_attn(const AttnLaunch& a, const char* who, cudaStream_t st) {
+  return with_head_dim(a.q.size[4], who, [&](auto d) { return launch_attn_d<decltype(d)::value>(a, st); });
 }
 
-// common validation of a (q, k_self, v_self, k, v) set; fills the shape part of AttnParams
+// common validation of a (q, k_self, v_self, k, v) set, before any device work; fills the shape part of AttnParams
 static int prepare(AttnLaunch& a, float scale, const char* who) {
-  int rc;
-  if ((rc = check_t5(a.q, "q")) != DS_OK) return rc;
-  if ((rc = check_t5(a.ks, "k_self")) != DS_OK) return rc;
-  if ((rc = check_t5(a.vs, "v_self")) != DS_OK) return rc;
-  if ((rc = check_t5(a.k, "k")) != DS_OK) return rc;
-  if ((rc = check_t5(a.v, "v")) != DS_OK) return rc;
   const ds_tensor5* all[5] = {&a.q, &a.ks, &a.vs, &a.k, &a.v};
+  const char* const names[5] = {"q", "k_self", "v_self", "k", "v"};
+  int rc;
+  for (int i = 0; i < 5; ++i) {
+    if ((rc = check_operand(*all[i], who, names[i])) != DS_OK) return rc;
+    if (all[i]->size[0] > INT32_MAX || all[i]->size[3] > INT32_MAX)
+      return fail(DS_ERR_INVALID, "%s: %s: too large", who, names[i]);
+  }
   for (int i = 1; i < 5; ++i) {
     if (all[i]->dtype != a.q.dtype) return fail(DS_ERR_INVALID, "%s: all tensors must share one dtype", who);
     if (all[i]->size[1] != a.q.size[1] || all[i]->size[2] != a.q.size[2] || all[i]->size[4] != a.q.size[4])
@@ -1132,6 +1087,7 @@ static int prepare(AttnLaunch& a, float scale, const char* who) {
   const int64_t Skv = a.k.size[3];
   if (Skv > INT32_MAX / 2) return fail(DS_ERR_INVALID, "%s: kv length too large", who);
   const int64_t D = a.q.size[4];
+  if ((rc = with_head_dim(D, who, [](auto) { return DS_OK; })) != DS_OK) return rc;
   a.p.B = (int)a.q.size[1];
   a.p.H = (int)a.q.size[2];
   a.p.Sq = (int)a.q.size[3];
@@ -1139,20 +1095,7 @@ static int prepare(AttnLaunch& a, float scale, const char* who) {
   a.p.n_qt = (int)((a.q.size[3] + kBlockQ - 1) / kBlockQ);
   const float sc = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
   a.p.scale_log2 = sc * 1.4426950408889634f;
-  return ds_device_ok();
-}
-
-static ds_tensor5 lift(const ds_tensor4& t) {
-  ds_tensor5 r;
-  r.ptr = t.ptr;
-  r.dtype = t.dtype;
-  r.size[0] = 1;
-  r.stride[0] = 8;
-  for (int i = 0; i < 4; ++i) {
-    r.size[i + 1] = t.size[i];
-    r.stride[i + 1] = t.stride[i];
-  }
-  return r;
+  return DS_OK;
 }
 
 }  // namespace ds
@@ -1192,6 +1135,7 @@ size_t ds_attn_fwd_workspace_bytes(ds_tensor4 q, ds_tensor4 k) {
 int ds_attn_fwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, float scale, ds_tensor4 out, void* ws, size_t ws_bytes,
                 void* stream) {
   using namespace ds;
+  const char* who = "ds_attn_fwd";
   AttnLaunch a;
   a.q = lift(q);
   a.k = lift(k);
@@ -1199,16 +1143,12 @@ int ds_attn_fwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, float scale, ds_tensor
   a.ks = a.k;
   a.vs = a.v;
   // k_self / v_self are unused in store mode, but must pass validation: give them q's image count
-  int rc = prepare(a, scale, "ds_attn_fwd");
-  if (rc != DS_OK) return rc;
-  if (!out.ptr || out.dtype != q.dtype) return fail(DS_ERR_INVALID, "ds_attn_fwd: out must have q's dtype");
-  for (int i = 0; i < 4; ++i)
-    if (out.size[i] != q.size[i]) return fail(DS_ERR_INVALID, "ds_attn_fwd: out must have q's shape");
-  if (out.stride[3] != 1 || ((uintptr_t)out.ptr & 15) || (out.stride[0] & 7) || (out.stride[1] & 7) || (out.stride[2] & 7))
-    return fail(DS_ERR_INVALID, "ds_attn_fwd: out needs a unit innermost stride and 16-byte aligned rows");
+  int rc;
+  if ((rc = prepare(a, scale, who)) != DS_OK || (rc = check_like(lift(out), a.q, who, "out")) != DS_OK) return rc;
   Workspace w(ws, ws_bytes);
   int32_t* meta = static_cast<int32_t*>(w.take(4 * sizeof(int32_t)));
   if (!meta) return fail(DS_ERR_WORKSPACE, "ds_attn_fwd: workspace too small (need %zu bytes)", (size_t)1024);
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // one group: query image 0, one entry: kv image 0
   single_meta_kernel<<<1, 32, 0, st>>>(meta);
@@ -1224,7 +1164,7 @@ int ds_attn_fwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, float scale, ds_tensor
   a.p.out_sb = out.stride[0];
   a.p.out_sh = out.stride[1];
   a.p.out_ss = out.stride[2];
-  return launch_attn(a, st);
+  return launch_attn(a, who, st);
 }
 
 size_t ds_aas_groups_workspace_bytes(ds_tensor5 q, int64_t n_groups, int64_t n_entries) {
@@ -1258,6 +1198,7 @@ int ds_aas_groups(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5
   if (!part || !bad)
     return fail(DS_ERR_WORKSPACE, "ds_aas_groups: workspace too small (%zu given, need %zu)", ws_bytes,
                 ds_aas_groups_workspace_bytes(q, n_groups, n_entries));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DS_CUDA_TRY(cudaMemsetAsync(bad, 0, sizeof(int32_t), st));
   {
@@ -1275,7 +1216,7 @@ int ds_aas_groups(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5
   a.p.part = part;
   a.p.out = nullptr;
   a.p.out_sb = a.p.out_sh = a.p.out_ss = 0;
-  rc = launch_attn(a, st);
+  rc = launch_attn(a, "ds_aas_groups", st);
   if (rc != DS_OK) return rc;
   const double E = (double)a.p.B * a.p.H * a.p.Sq * (double)q.size[4];
   aas_finish_kernel<<<(unsigned)((n_entries + 127) / 128), 128, 0, st>>>(part, n_entries, tiles, E, mode, dir, 0, 0, 0, 0, bad);
@@ -1429,6 +1370,7 @@ int ds_aas_matrix(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5
   if (!gq || !go || !kv || !part)
     return fail(DS_ERR_WORKSPACE, "ds_aas_matrix: workspace too small (%zu given, need %zu)", ws_bytes,
                 ds_aas_matrix_workspace_bytes(q, k));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t setup_n = (T > G + 1 ? T : G + 1);
   matrix_setup_kernel<<<(unsigned)((setup_n + 255) / 256), 256, 0, st>>>(nr, nc, chunks, cc, gq, go, kv);
@@ -1443,7 +1385,7 @@ int ds_aas_matrix(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5
   a.p.part = part;
   a.p.out = nullptr;
   a.p.out_sb = a.p.out_sh = a.p.out_ss = 0;
-  rc = launch_attn(a, st);
+  rc = launch_attn(a, "ds_aas_matrix", st);
   if (rc != DS_OK) return rc;
   const double E = (double)a.p.B * a.p.H * a.p.Sq * (double)q.size[4];
   aas_finish_kernel<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(part, T, tiles, E, mode, Dm, nc, ldd, nr, cc, nullptr);

@@ -27,8 +27,7 @@
 // issues 12 (the LSE pass recomputes QK^T once more).
 #include <algorithm>
 
-#include "ds_host.h"
-#include "ds_ptx.cuh"
+#include "ds_attn_common.cuh"
 
 namespace ds {
 namespace bwd {
@@ -37,22 +36,18 @@ constexpr int kThreads = 128;   // four warps = the four TMEM lane quadrants
 constexpr int kTile = 128;      // q rows of a dQ stream, kv rows of a dK/dV stream, kv rows per dQ step
 
 template <int D>
-struct Cfg {
-  static constexpr int D_PAD = (D + 15) / 16 * 16;
-  static constexpr int SUBW = (D % 64 == 0) ? 64 : 32;   // elements per swizzle row (as K1)
-  static constexpr int SUB_BYTES = SUBW * 2;
-  static constexpr int NSUB = (D_PAD + SUBW - 1) / SUBW;
-  static constexpr uint32_t LAYOUT = (SUBW == 64) ? UMMA_SW128 : UMMA_SW64;
-  static constexpr int CPS = SUBW / 16;                  // 16-element K chunks per sub-tile
-  static constexpr int BQ = (2 * 128 + 2 * D_PAD <= 512) ? 128 : 64;   // q rows per dK/dV step
-  static constexpr int TILE_BYTES = NSUB * kTile * SUB_BYTES;        // 128-row tile
-  static constexpr int QB_BYTES = NSUB * BQ * SUB_BYTES;             // BQ-row tile
-  static constexpr int DQ_SMEM = 4 * TILE_BYTES + 1024;              // Q, dO, K, V + barriers
+struct Cfg : AttnTile<D> {   // K1's operand tiles
+  using Tile = AttnTile<D>;
+  static constexpr int BQ = (2 * 128 + 2 * Tile::D_PAD <= 512) ? 128 : 64;   // q rows per dK/dV step
+  static constexpr int TILE_BYTES = Tile::NSUB * kTile * Tile::SUB_BYTES;      // 128-row tile
+  static constexpr int QB_BYTES = Tile::NSUB * BQ * Tile::SUB_BYTES;           // BQ-row tile
+  static constexpr int DQ_SMEM = 4 * TILE_BYTES + 1024;                        // Q, dO, K, V + barriers
   static constexpr int DKV_SMEM = 2 * TILE_BYTES + 2 * QB_BYTES + 2 * BQ * 4 + 1024;
-  static_assert(256 + D_PAD <= 512, "dQ TMEM budget");
-  static_assert(2 * BQ + 2 * D_PAD <= 512, "dK/dV TMEM budget");
+  static_assert(256 + Tile::D_PAD <= 512, "dQ TMEM budget");
+  static_assert(2 * BQ + 2 * Tile::D_PAD <= 512, "dK/dV TMEM budget");
   static_assert(DQ_SMEM <= 232448 && DKV_SMEM <= 232448, "shared memory");
-  static_assert((kTile * SUB_BYTES) % 1024 == 0 && (BQ * SUB_BYTES) % 1024 == 0, "swizzle atoms need 1024-byte tiles");
+  static_assert((kTile * Tile::SUB_BYTES) % 1024 == 0 && (BQ * Tile::SUB_BYTES) % 1024 == 0,
+                "swizzle atoms need 1024-byte tiles");
 };
 
 struct Params {
@@ -527,21 +522,6 @@ __global__ void sim_factor_kernel(const uint32_t* __restrict__ x, const uint32_t
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-static int check_in(const ds_tensor4& t, const char* who, const char* name) {
-  if (!t.ptr) return fail(DS_ERR_INVALID, "%s: %s: null pointer", who, name);
-  if (t.dtype != DS_F16 && t.dtype != DS_BF16) return fail(DS_ERR_UNSUPPORTED, "%s: %s: dtype must be f16 or bf16", who, name);
-  for (int i = 0; i < 4; ++i)
-    if (t.size[i] <= 0) return fail(DS_ERR_INVALID, "%s: %s: size[%d] = %lld", who, name, i, (long long)t.size[i]);
-  if (t.stride[3] != 1) return fail(DS_ERR_INVALID, "%s: %s: innermost stride must be 1 (got %lld)", who, name, (long long)t.stride[3]);
-  if ((uintptr_t)t.ptr & 15) return fail(DS_ERR_INVALID, "%s: %s: base pointer must be 16-byte aligned", who, name);
-  for (int i = 0; i < 3; ++i)
-    if (t.size[i] > 1 && (t.stride[i] <= 0 || (t.stride[i] & 7)))
-      return fail(DS_ERR_INVALID, "%s: %s: stride[%d] = %lld must be a positive multiple of 8 elements (16 bytes)", who, name,
-                  i, (long long)t.stride[i]);
-  if (t.size[2] > INT32_MAX / 2) return fail(DS_ERR_INVALID, "%s: %s: sequence too long", who, name);
-  return DS_OK;
-}
-
 static int check_grad(const ds_tensor4& g, const ds_tensor4& like, const char* who, const char* name) {
   if (!g.ptr) return fail(DS_ERR_INVALID, "%s: %s: null pointer", who, name);
   if (g.dtype != DS_F32) return fail(DS_ERR_INVALID, "%s: %s: gradients are float32", who, name);
@@ -554,39 +534,18 @@ static int check_grad(const ds_tensor4& g, const ds_tensor4& like, const char* w
   return DS_OK;
 }
 
-static bool head_dim_ok(int64_t d) { return d == 40 || d == 64 || d == 72 || d == 80 || d == 128 || d == 160; }
-
-// q, k, v, out, dout: shapes, dtypes and layouts of one attention backward
+// q, k, v: shapes, dtypes and layouts of one attention backward
 static int check_attn(const ds_tensor4& q, const ds_tensor4& k, const ds_tensor4& v, const char* who) {
   int rc;
-  if ((rc = check_in(q, who, "q")) != DS_OK || (rc = check_in(k, who, "k")) != DS_OK || (rc = check_in(v, who, "v")) != DS_OK)
+  if ((rc = check_operand(lift(q), who, "q")) != DS_OK || (rc = check_operand(lift(k), who, "k")) != DS_OK ||
+      (rc = check_operand(lift(v), who, "v")) != DS_OK)
     return rc;
   if (k.dtype != q.dtype || v.dtype != q.dtype) return fail(DS_ERR_INVALID, "%s: q, k and v must share one dtype", who);
   for (int i : {0, 1, 3})
     if (k.size[i] != q.size[i] || v.size[i] != q.size[i]) return fail(DS_ERR_INVALID, "%s: B, H and D must match across q, k, v", who);
   if (v.size[2] != k.size[2]) return fail(DS_ERR_INVALID, "%s: k and v must have the same length", who);
-  if (!head_dim_ok(q.size[3]))
-    return fail(DS_ERR_UNSUPPORTED, "%s: head dim %lld is not built (supported: 40, 64, 72, 80, 128, 160)", who,
-                (long long)q.size[3]);
-  return DS_OK;
-}
-
-static int check_like(const ds_tensor4& t, const ds_tensor4& q, const char* who, const char* name) {
-  int rc = check_in(t, who, name);
-  if (rc != DS_OK) return rc;
-  if (t.dtype != q.dtype) return fail(DS_ERR_INVALID, "%s: %s must have q's dtype", who, name);
-  for (int i = 0; i < 4; ++i)
-    if (t.size[i] != q.size[i]) return fail(DS_ERR_INVALID, "%s: %s must have q's shape", who, name);
-  return DS_OK;
-}
-
-static int make_map4(CUtensorMap* m, const ds_tensor4& t, int subw, int rows) {
-  // TMA dims, fastest first: (d, s, h, b, 1)
-  uint64_t dims[5] = {(uint64_t)t.size[3], (uint64_t)t.size[2], (uint64_t)t.size[1], (uint64_t)t.size[0], 1};
-  auto st = [&](int i) -> uint64_t { return (uint64_t)(t.size[i] > 1 ? t.stride[i] : 8) * 2; };
-  uint64_t strides[4] = {st(2), st(1), st(0), 16};
-  uint32_t box[5] = {(uint32_t)subw, (uint32_t)rows, 1, 1, 1};
-  return encode_tensor_map(m, t.dtype, 5, t.ptr, dims, strides, box, subw * 2, 64);
+  if (q.size[2] > INT32_MAX / 2 || k.size[2] > INT32_MAX / 2) return fail(DS_ERR_INVALID, "%s: sequence too long", who);
+  return with_head_dim(q.size[3], who, [](auto) { return DS_OK; });
 }
 
 static size_t stats_bytes(const ds_tensor4& q) {
@@ -607,9 +566,10 @@ static int launch_bwd_t(const BwdArgs& a, cudaStream_t st) {
   using C = Cfg<D>;
   CUtensorMap mq, mk, mv, mdo, mqb, mdob;
   int rc;
-  if ((rc = make_map4(&mq, a.q, C::SUBW, kTile)) != DS_OK || (rc = make_map4(&mk, a.k, C::SUBW, kTile)) != DS_OK ||
-      (rc = make_map4(&mv, a.v, C::SUBW, kTile)) != DS_OK || (rc = make_map4(&mdo, a.dout, C::SUBW, kTile)) != DS_OK ||
-      (rc = make_map4(&mqb, a.q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map4(&mdob, a.dout, C::SUBW, C::BQ)) != DS_OK)
+  const ds_tensor5 q = lift(a.q), dout = lift(a.dout);
+  if ((rc = make_map(&mq, q, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mk, lift(a.k), C::SUBW, kTile)) != DS_OK ||
+      (rc = make_map(&mv, lift(a.v), C::SUBW, kTile)) != DS_OK || (rc = make_map(&mdo, dout, C::SUBW, kTile)) != DS_OK ||
+      (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, dout, C::SUBW, C::BQ)) != DS_OK)
     return rc;
   Params p;
   p.B = (int)a.q.size[0];
@@ -644,20 +604,10 @@ static int launch_bwd_t(const BwdArgs& a, cudaStream_t st) {
   return DS_OK;
 }
 
-template <int D>
-static int launch_bwd_d(const BwdArgs& a, cudaStream_t st) {
-  return a.q.dtype == DS_BF16 ? launch_bwd_t<D, true>(a, st) : launch_bwd_t<D, false>(a, st);
-}
-
-static int launch_bwd(const BwdArgs& a, cudaStream_t st) {
-  switch ((int)a.q.size[3]) {
-    case 40: return launch_bwd_d<40>(a, st);
-    case 64: return launch_bwd_d<64>(a, st);
-    case 72: return launch_bwd_d<72>(a, st);
-    case 80: return launch_bwd_d<80>(a, st);
-    case 128: return launch_bwd_d<128>(a, st);
-    default: return launch_bwd_d<160>(a, st);
-  }
+static int launch_bwd(const BwdArgs& a, const char* who, cudaStream_t st) {
+  return with_head_dim(a.q.size[3], who, [&](auto d) {
+    return with_dtype(a.q.dtype, [&](auto bf) { return launch_bwd_t<decltype(d)::value, decltype(bf)::value>(a, st); });
+  });
 }
 
 static ds_tensor4 contiguous_like(const ds_tensor4& t, void* ptr) {
@@ -686,8 +636,8 @@ int ds_attn_bwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, ds_tensor4 out, ds_ten
   using namespace ds::bwd;
   const char* who = "ds_attn_bwd";
   int rc;
-  if ((rc = check_attn(q, k, v, who)) != DS_OK || (rc = check_like(out, q, who, "out")) != DS_OK ||
-      (rc = check_like(dout, q, who, "dout")) != DS_OK || (rc = check_grad(dq, q, who, "dq")) != DS_OK ||
+  if ((rc = check_attn(q, k, v, who)) != DS_OK || (rc = check_like(lift(out), lift(q), who, "out")) != DS_OK ||
+      (rc = check_like(lift(dout), lift(q), who, "dout")) != DS_OK || (rc = check_grad(dq, q, who, "dq")) != DS_OK ||
       (rc = check_grad(dk, k, who, "dk")) != DS_OK || (rc = check_grad(dv, v, who, "dv")) != DS_OK)
     return rc;
   Workspace w(ws, ws_bytes);
@@ -698,7 +648,7 @@ int ds_attn_bwd(ds_tensor4 q, ds_tensor4 k, ds_tensor4 v, ds_tensor4 out, ds_ten
     return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes, ds_attn_bwd_workspace_bytes(q, k));
   if ((rc = ds_device_ok()) != DS_OK) return rc;
   BwdArgs a{q, k, v, out, dout, dq, dk, dv, scale, nullptr, lse, delta};
-  return launch_bwd(a, static_cast<cudaStream_t>(stream));
+  return launch_bwd(a, who, static_cast<cudaStream_t>(stream));
 }
 
 size_t ds_aas_dir_bwd_workspace_bytes(ds_tensor4 q_i, ds_tensor4 k_j) {
@@ -759,9 +709,9 @@ int ds_aas_dir_bwd(ds_tensor4 q_i, ds_tensor4 k_i, ds_tensor4 v_i, ds_tensor4 k_
   DS_CUDA_TRY(cudaGetLastError());
   // cross term first, then the self term: dq_i receives its two contributions in this fixed order
   BwdArgs cross{q_i, k_j, v_j, X, contiguous_like(q_i, fx), dq_i, dk_j, dv_j, scale, coef + 0, lse, delta};
-  if ((rc = launch_bwd(cross, st)) != DS_OK) return rc;
+  if ((rc = launch_bwd(cross, who, st)) != DS_OK) return rc;
   BwdArgs self{q_i, k_i, v_i, Y, contiguous_like(q_i, fy), dq_i, dk_i, dv_i, scale, coef + 1, lse, delta};
-  return launch_bwd(self, st);
+  return launch_bwd(self, who, st);
 }
 
 }  // extern "C"

@@ -37,9 +37,7 @@ def dino_cross_score(A: QKV, B: QKV, attention_head_size: Optional[int] = None,
     two directions -- the AAS pair formula, so it runs on the fused attention kernel."""
     (qa, ka, va), (qb, kb, vb) = A, B
     scale = None if attention_head_size is None else float(attention_head_size) ** -0.5
-    one, off = [0], [0, 1]
-    d_ab = ops.aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, "cosine", scale)
-    d_ba = ops.aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, "cosine", scale)
+    d_ab, d_ba = ops._pair_dirs(qa, ka, va, qb, kb, vb, "cosine", scale)
     if match_reference_dtype:
         return (d_ab.to(qa.dtype) + d_ba.to(qa.dtype)) / 2
     return (d_ab + d_ba) * 0.5

@@ -25,11 +25,6 @@ _workspaces: dict = {}
 LAUNCHES = 0
 
 
-def _count(n: int) -> None:
-    global LAUNCHES
-    LAUNCHES += n
-
-
 def _mode(similarity) -> int:
     if isinstance(similarity, int):
         return similarity
@@ -57,10 +52,6 @@ def _workspace(dev: torch.device, nbytes: int, slot: str = "main") -> torch.Tens
     return buf
 
 
-def _stream(dev: torch.device) -> int:
-    return torch.cuda.current_stream(dev).cuda_stream
-
-
 def _dtype_code(t: torch.Tensor) -> int:
     try:
         return _DTYPES[t.dtype]
@@ -68,10 +59,15 @@ def _dtype_code(t: torch.Tensor) -> int:
         raise RuntimeError(f"unsupported dtype {t.dtype}") from None
 
 
-def _t4(t: torch.Tensor) -> N.Tensor4:
-    if t.dim() != 4:
-        raise RuntimeError(f"expected a (B,H,S,D) tensor, got shape {tuple(t.shape)}")
-    d = N.Tensor4()
+_DESCRIPTORS = {4: (N.Tensor4, "(B,H,S,D)"), 5: (N.Tensor5, "(N,B,H,S,D)")}
+
+
+def _desc(t: torch.Tensor, rank: int):
+    """The ds_tensor4 / ds_tensor5 descriptor of t (no copy: sizes and strides as they are)."""
+    cls, layout = _DESCRIPTORS[rank]
+    if t.dim() != rank:
+        raise RuntimeError(f"expected a {layout} tensor, got shape {tuple(t.shape)}")
+    d = cls()
     d.ptr = t.data_ptr()
     d.size[:] = list(t.shape)
     d.stride[:] = list(t.stride())
@@ -79,15 +75,25 @@ def _t4(t: torch.Tensor) -> N.Tensor4:
     return d
 
 
-def _t5(t: torch.Tensor) -> N.Tensor5:
-    if t.dim() != 5:
-        raise RuntimeError(f"expected a (N,B,H,S,D) tensor, got shape {tuple(t.shape)}")
-    d = N.Tensor5()
-    d.ptr = t.data_ptr()
-    d.size[:] = list(t.shape)
-    d.stride[:] = list(t.stride())
-    d.dtype = _dtype_code(t)
-    return d
+def _scale_arg(scale) -> float:
+    # the library's softmax scale argument: anything not positive (None, 0, < 0) selects the default 1/sqrt(D)
+    return 0.0 if scale is None or not scale > 0 else float(scale)
+
+
+def _call(name: str, dev: torch.device, *args, launches: int, ws_query: Optional[tuple] = None,
+          slot: str = "main") -> None:
+    """lib.<name>(*args, ws, ws_bytes, stream) on dev's current stream, with the workspace sized by
+    lib.<name>_workspace_bytes(*ws_query); without ws_query, lib.<name>(*args, stream).  An error status raises
+    DiffSimError; `launches` (the kernels the call issues) is added to LAUNCHES."""
+    global LAUNCHES
+    lib = N.load()
+    tail = ()
+    if ws_query is not None:
+        ws = _workspace(dev, getattr(lib, name + "_workspace_bytes")(*ws_query), slot)
+        tail = (ws.data_ptr(), ws.numel())
+    with torch.cuda.device(dev):
+        N.check(getattr(lib, name)(*args, *tail, torch.cuda.current_stream(dev).cuda_stream))
+    LAUNCHES += launches
 
 
 def _i32(x, dev) -> torch.Tensor:
@@ -118,18 +124,13 @@ def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: Optional[
 
 
 def _attn_fwd(q, k, v, scale=None, out=None) -> torch.Tensor:
-    lib = N.load()
     dev = _need_cuda(q, k, v)
     B, H, Sq, D = q.shape
     if out is None:
         out = torch.empty((B, Sq, H, D), dtype=q.dtype, device=dev).permute(0, 2, 1, 3)
-    q4, k4 = _t4(q), _t4(k)
-    nbytes = lib.ds_attn_fwd_workspace_bytes(q4, k4)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_attn_fwd(q4, k4, _t4(v), float(scale) if scale else 0.0, _t4(out), ws.data_ptr(), ws.numel(),
-                                _stream(dev)))
-    _count(2)  # meta + attention
+    q4, k4 = _desc(q, 4), _desc(k, 4)
+    _call("ds_attn_fwd", dev, q4, k4, _desc(v, 4), _scale_arg(scale), _desc(out, 4), ws_query=(q4, k4),
+          launches=2)  # meta + attention
     return out
 
 
@@ -170,16 +171,12 @@ def attn_bwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, out: torch.Tenso
              scale: Optional[float] = None, grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
     """Gradients (dq, dk, dv) of attn_fwd for the output gradient dout, in float32 (deterministic: no atomics).
     out: the forward output attn_fwd(q, k, v, scale).  grads: optional float32 (dq, dk, dv) to add into."""
-    lib = N.load()
     dev = _need_cuda(q, k, v, out, dout)
     dout = _tma_ok(dout.to(q.dtype))
     dq, dk, dv = _grads_like((q, k, v), grads)
-    q4, k4 = _t4(q), _t4(k)
-    ws = _workspace(dev, lib.ds_attn_bwd_workspace_bytes(q4, k4), "bwd")
-    with torch.cuda.device(dev):
-        N.check(lib.ds_attn_bwd(q4, k4, _t4(v), _t4(out), _t4(dout), float(scale) if scale else 0.0, _t4(dq), _t4(dk),
-                                _t4(dv), ws.data_ptr(), ws.numel(), _stream(dev)))
-    _count(2)  # dQ + dK/dV
+    q4, k4 = _desc(q, 4), _desc(k, 4)
+    _call("ds_attn_bwd", dev, q4, k4, _desc(v, 4), _desc(out, 4), _desc(dout, 4), _scale_arg(scale), _desc(dq, 4),
+          _desc(dk, 4), _desc(dv, 4), ws_query=(q4, k4), slot="bwd", launches=2)  # dQ + dK/dV
     return dq, dk, dv
 
 
@@ -189,23 +186,20 @@ def aas_dir_bwd(q_i: torch.Tensor, k_i: torch.Tensor, v_i: torch.Tensor, k_j: to
     """Gradients (dq_i, dk_i, dv_i, dk_j, dv_j) of dir = sim(Attn(q_i,k_j,v_j), Attn(q_i,k_i,v_i)) for dL/ddir = d_dir
     (a one-element tensor on the device; no host sync), in float32.  (B,H,S,D) inputs as for attn_fwd.
     grads: optional float32 tensors to add into (they may alias, e.g. dk_i is dk_j when image i is image j)."""
-    lib = N.load()
     dev = _need_cuda(q_i, k_i, v_i, k_j, v_j, d_dir)
     g = d_dir.detach().reshape(-1).to(torch.float32)
     if g.numel() != 1:
         raise RuntimeError("d_dir must have exactly one element")
     out = _grads_like((q_i, k_i, v_i, k_j, v_j), grads)
-    q4, kj4 = _t4(q_i), _t4(k_j)
-    ws = _workspace(dev, lib.ds_aas_dir_bwd_workspace_bytes(q4, kj4), "bwd")
-    with torch.cuda.device(dev):
-        N.check(lib.ds_aas_dir_bwd(q4, _t4(k_i), _t4(v_i), kj4, _t4(v_j), float(scale) if scale else 0.0,
-                                   _mode(similarity), g.data_ptr(), *[_t4(t) for t in out], ws.data_ptr(), ws.numel(),
-                                   _stream(dev)))
-    _count(11)  # 2 x (meta + attention) recompute + partials + coefficients + factors + 2 x (dQ + dK/dV)
+    q4, kj4 = _desc(q_i, 4), _desc(k_j, 4)
+    _call("ds_aas_dir_bwd", dev, q4, _desc(k_i, 4), _desc(v_i, 4), kj4, _desc(v_j, 4), _scale_arg(scale),
+          _mode(similarity), g.data_ptr(), *[_desc(t, 4) for t in out], ws_query=(q4, kj4), slot="bwd",
+          launches=11)  # 2 x (meta + attention) recompute + partials + coefficients + factors + 2 x (dQ + dK/dV)
     return out
 
 
 def _pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale):
+    """(dir(a->b), dir(b->a)) of one image pair: two aas_groups calls, forward only."""
     one, off = [0], [0, 1]
     d_ab = aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, similarity, scale)
     d_ba = aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, similarity, scale)
@@ -248,21 +242,16 @@ def aas_groups(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: t
                group_q, group_off, kv_idx, similarity="cosine", scale: Optional[float] = None) -> torch.Tensor:
     """Directional AAS similarities for grouped (query image, kv image list) work -- see ds_aas_groups.
     q/k_self/v_self: (Nq,B,H,S,D); k/v: (Nk,B,H,S,D).  Returns float32 [n_entries]."""
-    lib = N.load()
     dev = _need_cuda(q, k_self, v_self, k, v)
     gq, go, kv = _i32(group_q, dev), _i32(group_off, dev), _i32(kv_idx, dev)
     n_groups, n_entries = gq.numel(), kv.numel()
     if go.numel() != n_groups + 1:
         raise RuntimeError("group_off must have n_groups + 1 entries")
     dirs = torch.empty(n_entries, dtype=torch.float32, device=dev)
-    q5 = _t5(q)
-    nbytes = lib.ds_aas_groups_workspace_bytes(q5, n_groups, n_entries)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_aas_groups(q5, _t5(k_self), _t5(v_self), _t5(k), _t5(v), gq.data_ptr(), go.data_ptr(), n_groups,
-                                  kv.data_ptr(), n_entries, float(scale) if scale else 0.0, _mode(similarity),
-                                  dirs.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
-    _count(3)  # index validation + attention + finish
+    q5 = _desc(q, 5)
+    _call("ds_aas_groups", dev, q5, _desc(k_self, 5), _desc(v_self, 5), _desc(k, 5), _desc(v, 5), gq.data_ptr(),
+          go.data_ptr(), n_groups, kv.data_ptr(), n_entries, _scale_arg(scale), _mode(similarity), dirs.data_ptr(),
+          ws_query=(q5, n_groups, n_entries), launches=3)  # index validation + attention + finish
     return dirs
 
 
@@ -270,18 +259,13 @@ def aas_pairs(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, pair_idx, simil
               scale: Optional[float] = None) -> torch.Tensor:
     """score[p] = (dir(a->b) + dir(b->a)) / 2 for pair_idx[p] = (a, b): the value DiffSim.diffsim returns
     (diffsim/diffsim.py:177-197).  q,k,v: (N,B,H,S,D) caches.  Returns float32 [P]."""
-    lib = N.load()
     dev = _need_cuda(q, k, v)
     pairs = _i32(pair_idx, dev).reshape(-1, 2)
     P = pairs.shape[0]
     scores = torch.empty(P, dtype=torch.float32, device=dev)
-    q5 = _t5(q)
-    nbytes = lib.ds_aas_pairs_workspace_bytes(q5, P)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_aas_pairs(q5, _t5(k), _t5(v), pairs.data_ptr(), P, float(scale) if scale else 0.0,
-                                 _mode(similarity), scores.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
-    _count(5)  # setup + index validation + attention + finish + pair combine
+    q5 = _desc(q, 5)
+    _call("ds_aas_pairs", dev, q5, _desc(k, 5), _desc(v, 5), pairs.data_ptr(), P, _scale_arg(scale), _mode(similarity),
+          scores.data_ptr(), ws_query=(q5, P), launches=5)  # setup + index validation + attention + finish + combine
     return scores
 
 
@@ -290,7 +274,6 @@ def aas_triplets(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, trip_idx, si
     """2AFC triplets (ref, left, right) as the benchmark drivers score them (cute_main.py:111-132,196-205):
     returns (ab, ac, counts, flags) on the device: ab = diffsim(ref,left), ac = diffsim(ref,right) (float32 [T]),
     counts int32[2] = {correct, correct_2x}, flags uint8[T].  One library call, no host sync."""
-    lib = N.load()
     dev = _need_cuda(q, k, v)
     trips = _i32(trip_idx, dev).reshape(-1, 3)
     T = trips.shape[0]
@@ -298,15 +281,11 @@ def aas_triplets(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, trip_idx, si
     ac = torch.empty(T, dtype=torch.float32, device=dev)
     counts = torch.empty(2, dtype=torch.int32, device=dev)
     flags = torch.empty(T, dtype=torch.uint8, device=dev) if want_flags else None
-    q5 = _t5(q)
-    nbytes = lib.ds_aas_triplets_workspace_bytes(q5, T)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_aas_triplets(q5, _t5(k), _t5(v), trips.data_ptr(), T, float(scale) if scale else 0.0,
-                                    _mode(similarity), N.DS_OPT_ROUND_SCORES if round_scores else 0, ab.data_ptr(),
-                                    ac.data_ptr(), counts.data_ptr(), flags.data_ptr() if want_flags else None,
-                                    ws.data_ptr(), ws.numel(), _stream(dev)))
-    _count(5)  # setup + index validation + attention + finish + combine/decide
+    q5 = _desc(q, 5)
+    _call("ds_aas_triplets", dev, q5, _desc(k, 5), _desc(v, 5), trips.data_ptr(), T, _scale_arg(scale),
+          _mode(similarity), N.DS_OPT_ROUND_SCORES if round_scores else 0, ab.data_ptr(), ac.data_ptr(),
+          counts.data_ptr(), flags.data_ptr() if want_flags else None, ws_query=(q5, T),
+          launches=5)  # setup + index validation + attention + finish + combine/decide
     return ab, ac, counts, flags
 
 
@@ -314,19 +293,13 @@ def aas_matrix(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: t
                similarity="cosine", scale: Optional[float] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Directional matrix Dm[r,c] = dir(row image r -> column image c); rows (q,k_self,v_self): (Nr,...),
     columns (k,v): (Nc,...).  Returns float32 [Nr,Nc]."""
-    lib = N.load()
     dev = _need_cuda(q, k_self, v_self, k, v)
     nr, nc = q.shape[0], k.shape[0]
     if out is None:
         out = torch.empty((nr, nc), dtype=torch.float32, device=dev)
-    q5, k5 = _t5(q), _t5(k)
-    nbytes = lib.ds_aas_matrix_workspace_bytes(q5, k5)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_aas_matrix(q5, _t5(k_self), _t5(v_self), k5, _t5(v), float(scale) if scale else 0.0,
-                                  _mode(similarity), out.data_ptr(), out.stride(0), ws.data_ptr(), ws.numel(),
-                                  _stream(dev)))
-    _count(3)  # setup + attention + finish
+    q5, k5 = _desc(q, 5), _desc(k, 5)
+    _call("ds_aas_matrix", dev, q5, _desc(k_self, 5), _desc(v_self, 5), k5, _desc(v, 5), _scale_arg(scale),
+          _mode(similarity), out.data_ptr(), out.stride(0), ws_query=(q5, k5), launches=3)  # setup + attention + finish
     return out
 
 
@@ -337,7 +310,6 @@ def pair_reduce(x: torch.Tensor, y: torch.Tensor, similarity="cosine") -> torch.
     """sim(x[p], y[p]) over the flattened trailing dims, for every leading row p.  x, y: (P, ...) tensors whose rows
     are contiguous.  Replaces F.cosine_similarity on flattened tensors / F.mse_loss / min-max + cosine
     (diffsim/diffsim.py:182-195, metrics/diffeats.py:136-140,202-205).  Returns float32 [P]."""
-    lib = N.load()
     dev = _need_cuda(x, y)
     if x.shape != y.shape or x.dtype != y.dtype:
         raise RuntimeError("x and y must have the same shape and dtype")
@@ -351,13 +323,8 @@ def pair_reduce(x: torch.Tensor, y: torch.Tensor, similarity="cosine") -> torch.
         y2 = y2.contiguous()
     E = x2.shape[1]
     out = torch.empty(P, dtype=torch.float32, device=dev)
-    nbytes = lib.ds_pair_reduce_workspace_bytes(P, E)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_pair_reduce(x2.data_ptr(), y2.data_ptr(), P, E, x2.stride(0) if P > 1 else E,
-                                   y2.stride(0) if P > 1 else E, _dtype_code(x2), _mode(similarity), out.data_ptr(),
-                                   ws.data_ptr(), ws.numel(), _stream(dev)))
-    _count(1)
+    _call("ds_pair_reduce", dev, x2.data_ptr(), y2.data_ptr(), P, E, x2.stride(0) if P > 1 else E,
+          y2.stride(0) if P > 1 else E, _dtype_code(x2), _mode(similarity), out.data_ptr(), ws_query=(P, E), launches=1)
     return out
 
 
@@ -367,7 +334,6 @@ def pair_reduce(x: torch.Tensor, y: torch.Tensor, similarity="cosine") -> torch.
 def simmat(rows: torch.Tensor, cols: Optional[torch.Tensor] = None, similarity="cosine",
            out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """C[r,c] = sim(rows[r], cols[c]) for 16-bit feature matrices rows (Nr,L), cols (Nc,L) (default cols = rows)."""
-    lib = N.load()
     if cols is None:
         cols = rows
     dev = _need_cuda(rows, cols)
@@ -379,14 +345,11 @@ def simmat(rows: torch.Tensor, cols: Optional[torch.Tensor] = None, similarity="
     nc = cols.shape[0]
     if out is None:
         out = torch.empty((nr, nc), dtype=torch.float32, device=dev)
-    nbytes = lib.ds_simmat_workspace_bytes(nr, nc, L)
-    ws = _workspace(dev, nbytes)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_simmat(rows.data_ptr(), nr, rows.stride(0), cols.data_ptr(), nc, cols.stride(0), L,
-                              _dtype_code(rows), _mode(similarity), out.data_ptr(), out.stride(0), ws.data_ptr(),
-                              ws.numel(), _stream(dev)))
     # statistics pass + its finish per operand (one operand when rows is cols: the symmetric call), GEMM, normalise
-    _count(4 if (cols.data_ptr() == rows.data_ptr() and nr == nc and cols.stride(0) == rows.stride(0)) else 6)
+    symmetric = cols.data_ptr() == rows.data_ptr() and nr == nc and cols.stride(0) == rows.stride(0)
+    _call("ds_simmat", dev, rows.data_ptr(), nr, rows.stride(0), cols.data_ptr(), nc, cols.stride(0), L,
+          _dtype_code(rows), _mode(similarity), out.data_ptr(), out.stride(0), ws_query=(nr, nc, L),
+          launches=4 if symmetric else 6)
     return out
 
 
@@ -403,7 +366,6 @@ def qkv_project(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch
     `out`: optional pre-allocated outputs (row stride may exceed the column count, e.g. slices of a cache)."""
     import ctypes as C
 
-    lib = N.load()
     dev = _need_cuda(hidden, weight)
     if hidden.dtype != weight.dtype or (bias is not None and bias.dtype != hidden.dtype):
         raise RuntimeError("hidden, weight and bias must share one 16-bit dtype")
@@ -430,11 +392,8 @@ def qkv_project(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch
         o2.append(o_rows)
     ptrs = (C.c_void_p * n_outputs)(*[o.data_ptr() for o in o2])
     lds = (C.c_int64 * n_outputs)(*[o.stride(0) for o in o2])
-    with torch.cuda.device(dev):
-        N.check(lib.ds_qkv_project(h2.data_ptr(), rows, h2.stride(0), c_in, weight.data_ptr(), weight.stride(0),
-                                   bias.data_ptr() if bias is not None else None, n_out, cols, ptrs, lds,
-                                   _dtype_code(hidden), _stream(dev)))
-    _count(1)
+    _call("ds_qkv_project", dev, h2.data_ptr(), rows, h2.stride(0), c_in, weight.data_ptr(), weight.stride(0),
+          bias.data_ptr() if bias is not None else None, n_out, cols, ptrs, lds, _dtype_code(hidden), launches=1)
     return tuple(out)
 
 
@@ -444,17 +403,14 @@ def qkv_project(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch
 def twoafc(ab: torch.Tensor, ac: torch.Tensor, similarity="cosine") -> Tuple[torch.Tensor, torch.Tensor]:
     """2AFC counts of the benchmark drivers (cute_main.py:196-205).  Returns (counts int32[2] = {correct,
     correct_2x}, flags uint8[n]) on the device -- one launch, no host sync."""
-    lib = N.load()
     dev = _need_cuda(ab, ac)
     ab = ab.to(torch.float32).contiguous()
     ac = ac.to(torch.float32).contiguous()
     n = ab.numel()
     counts = torch.empty(2, dtype=torch.int32, device=dev)
     flags = torch.empty(n, dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        N.check(lib.ds_twoafc(ab.data_ptr(), ac.data_ptr(), n, _mode(similarity), counts.data_ptr(), flags.data_ptr(),
-                              _stream(dev)))
-    _count(1)
+    _call("ds_twoafc", dev, ab.data_ptr(), ac.data_ptr(), n, _mode(similarity), counts.data_ptr(), flags.data_ptr(),
+          launches=1)
     return counts, flags
 
 

@@ -14,7 +14,7 @@ attn_fwd and aas_score have autograd kernels (K5 backward); the other operators 
 """
 from __future__ import annotations
 
-from typing import List, Optional
+from typing import List
 
 import torch
 from torch.library import Library
@@ -36,31 +36,25 @@ _lib.define("simmat(Tensor rows, Tensor? cols=None, str similarity='cosine') -> 
 _lib.define("qkv_project(Tensor hidden, Tensor weight, Tensor? bias=None, int n_outputs=3) -> Tensor[]")
 
 
-def _sc(scale: float) -> Optional[float]:
-    return float(scale) if scale and scale > 0 else None
-
-
 def _attn_fwd(q, k, v, scale=0.0):
-    return ops.attn_fwd(q, k, v, _sc(scale))
+    return ops.attn_fwd(q, k, v, scale)
 
 
 def _aas_score(qa, ka, va, qb, kb, vb, similarity="cosine", scale=0.0):
-    one, off = [0], [0, 1]
-    d_ab = ops.aas_groups(qa[None], ka[None], va[None], kb[None], vb[None], one, off, one, similarity, _sc(scale))
-    d_ba = ops.aas_groups(qb[None], kb[None], vb[None], ka[None], va[None], one, off, one, similarity, _sc(scale))
+    d_ab, d_ba = ops._pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale)
     return (d_ab + d_ba) * 0.5
 
 
 def _aas_pairs(q, k, v, pair_idx, similarity="cosine", scale=0.0):
-    return ops.aas_pairs(q, k, v, pair_idx, similarity, _sc(scale))
+    return ops.aas_pairs(q, k, v, pair_idx, similarity, scale)
 
 
 def _aas_triplets(q, k, v, trip_idx, similarity="cosine", scale=0.0, round_scores=False):
-    return ops.aas_triplets(q, k, v, trip_idx, similarity, _sc(scale), round_scores)
+    return ops.aas_triplets(q, k, v, trip_idx, similarity, scale, round_scores)
 
 
 def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=0.0):
-    return ops.aas_matrix(q, k_self, v_self, k, v, similarity, _sc(scale))
+    return ops.aas_matrix(q, k_self, v_self, k, v, similarity, scale)
 
 
 def _pair_reduce(x, y, similarity="cosine"):
@@ -91,14 +85,14 @@ def _setup_inputs(ctx, inputs, output):
 def _attn_fwd_bwd(ctx, dout):
     q, k, v = ctx.saved_tensors
     (scale,) = ctx.rest or [0.0]
-    out = ops.attn_fwd(q, k, v, _sc(scale))
-    return ops.attn_bwd(q, k, v, out, dout, _sc(scale)) + (None,)
+    out = ops.attn_fwd(q, k, v, scale)
+    return ops.attn_bwd(q, k, v, out, dout, scale) + (None,)
 
 
 def _aas_score_bwd(ctx, grad):
     similarity, scale = (ctx.rest + ["cosine", 0.0][len(ctx.rest):])[:2]
     g = grad.reshape(1) * 0.5   # score = (dir(a->b) + dir(b->a)) / 2
-    return ops.pair_dirs_bwd(*ctx.saved_tensors, g, g, similarity, _sc(scale)) + (None, None)
+    return ops.pair_dirs_bwd(*ctx.saved_tensors, g, g, similarity, scale) + (None, None)
 
 
 torch.library.register_autograd("diffsim_b200::attn_fwd", _attn_fwd_bwd, setup_context=_setup_inputs, lib=_lib)

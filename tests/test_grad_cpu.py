@@ -1,6 +1,7 @@
 """K5 backward without a GPU: the float64 gradient oracle, the autograd registration of the differentiable operators,
 argument validation of the backward ABI and its loud failure without a device."""
 import ctypes as C
+import math
 
 import pytest
 import torch
@@ -64,12 +65,12 @@ def test_autograd_is_registered_on_the_differentiable_ops():
         torch.ops.diffsim_b200.attn_fwd(x, x, x)
 
 
-def _t4(shape, dtype, ptr=16, strides=None):
-    t = N.Tensor4()
+def _desc(shape, dtype, ptr=16, strides=None):
+    t = (N.Tensor4 if len(shape) == 4 else N.Tensor5)()
     t.ptr = ptr
     t.size[:] = list(shape)
     if strides is None:
-        strides = [shape[1] * shape[2] * shape[3], shape[2] * shape[3], shape[3], 1]
+        strides = [math.prod(shape[i + 1:]) for i in range(len(shape))]
     t.stride[:] = strides
     t.dtype = dtype
     return t
@@ -78,7 +79,7 @@ def _t4(shape, dtype, ptr=16, strides=None):
 def test_backward_abi_validates_before_touching_the_device():
     lib = N.load()
     s = (1, 2, 128, 64)
-    h, f = _t4(s, N.DS_F16), _t4(s, N.DS_F32)
+    h, f = _desc(s, N.DS_F16), _desc(s, N.DS_F32)
     ws = (C.c_uint8 * 4096)()
     assert lib.ds_attn_bwd_workspace_bytes(h, h) >= 2 * 2 * 128 * 4
     assert lib.ds_aas_dir_bwd_workspace_bytes(h, h) >= 4 * 2 * 128 * 64 * 2
@@ -86,15 +87,15 @@ def test_backward_abi_validates_before_touching_the_device():
     def attn(q=h, out=h, dq=f, dk=f):
         return lib.ds_attn_bwd(q, h, h, out, h, 0.0, dq, dk, f, ws, 4096, None)
 
-    assert attn(q=_t4(s, N.DS_F16, ptr=0)) == N.DS_ERR_INVALID and "null" in N.last_error()
-    assert attn(dq=_t4(s, N.DS_F16)) == N.DS_ERR_INVALID and "float32" in N.last_error()
-    assert attn(dk=_t4((1, 2, 64, 64), N.DS_F32)) == N.DS_ERR_INVALID
-    assert attn(out=_t4(s, N.DS_BF16)) == N.DS_ERR_INVALID
-    assert attn(q=_t4(s, N.DS_F16, ptr=24)) == N.DS_ERR_INVALID and "aligned" in N.last_error()
-    assert attn(q=_t4(s, N.DS_F16, strides=[16384, 8192, 60, 1])) == N.DS_ERR_INVALID
-    d96 = _t4((1, 2, 128, 96), N.DS_F16)
-    assert lib.ds_attn_bwd(d96, d96, d96, d96, d96, 0.0, _t4((1, 2, 128, 96), N.DS_F32), _t4((1, 2, 128, 96), N.DS_F32),
-                           _t4((1, 2, 128, 96), N.DS_F32), ws, 4096, None) == N.DS_ERR_UNSUPPORTED
+    assert attn(q=_desc(s, N.DS_F16, ptr=0)) == N.DS_ERR_INVALID and "null" in N.last_error()
+    assert attn(dq=_desc(s, N.DS_F16)) == N.DS_ERR_INVALID and "float32" in N.last_error()
+    assert attn(dk=_desc((1, 2, 64, 64), N.DS_F32)) == N.DS_ERR_INVALID
+    assert attn(out=_desc(s, N.DS_BF16)) == N.DS_ERR_INVALID
+    assert attn(q=_desc(s, N.DS_F16, ptr=24)) == N.DS_ERR_INVALID and "aligned" in N.last_error()
+    assert attn(q=_desc(s, N.DS_F16, strides=[16384, 8192, 60, 1])) == N.DS_ERR_INVALID
+    d96 = _desc((1, 2, 128, 96), N.DS_F16)
+    assert lib.ds_attn_bwd(d96, d96, d96, d96, d96, 0.0, _desc((1, 2, 128, 96), N.DS_F32), _desc((1, 2, 128, 96), N.DS_F32),
+                           _desc((1, 2, 128, 96), N.DS_F32), ws, 4096, None) == N.DS_ERR_UNSUPPORTED
     assert lib.ds_attn_bwd(h, h, h, h, h, 0.0, f, f, f, ws, 8, None) == N.DS_ERR_WORKSPACE
     g = (C.c_float * 1)()
 
@@ -103,8 +104,35 @@ def test_backward_abi_validates_before_touching_the_device():
 
     assert dirb(mode=N.DS_SIM_MINMAX_COSINE) == N.DS_ERR_INVALID and "mode" in N.last_error()
     assert dirb(d_dir=None) == N.DS_ERR_INVALID and "d_dir" in N.last_error()
-    assert dirb(dkj=_t4(s, N.DS_BF16)) == N.DS_ERR_INVALID
+    assert dirb(dkj=_desc(s, N.DS_BF16)) == N.DS_ERR_INVALID
     assert dirb() == N.DS_ERR_WORKSPACE
+
+
+def test_forward_abi_validates_before_touching_the_device():
+    lib = N.load()
+    ws = (C.c_uint8 * 4096)()
+    idx = (C.c_int32 * 2)(0, 1)
+    dirs = (C.c_float * 1)()
+    entry_points = {
+        "ds_attn_fwd": ((), lambda q, t: lib.ds_attn_fwd(q, t, t, 0.0, t, ws, 4096, None)),
+        "ds_aas_groups": ((1,), lambda q, t: lib.ds_aas_groups(q, t, t, t, t, idx, idx, 1, idx, 1, 0.0, N.DS_SIM_COSINE,
+                                                               dirs, ws, 4096, None)),
+        "ds_aas_matrix": ((1,), lambda q, t: lib.ds_aas_matrix(q, t, t, t, t, 0.0, N.DS_SIM_COSINE, dirs, 1, ws, 4096,
+                                                               None)),
+    }
+    for name, (lead, call) in entry_points.items():
+        s = lead + (1, 2, 128, 64)
+        h = _desc(s, N.DS_F16)
+        misaligned_rows = _desc(s, N.DS_F16)
+        misaligned_rows.stride[len(s) - 2] = 60
+        d96 = _desc(lead + (1, 2, 128, 96), N.DS_F16)
+        for q, t, code, text in ((_desc(s, N.DS_F16, ptr=0), h, N.DS_ERR_INVALID, "null"),
+                                 (_desc(s, N.DS_F16, ptr=24), h, N.DS_ERR_INVALID, "aligned"),
+                                 (misaligned_rows, h, N.DS_ERR_INVALID, "multiple of 8"),
+                                 (d96, d96, N.DS_ERR_UNSUPPORTED, "head dim 96 is not built")):
+            assert call(q, t) == code, (name, text)
+            msg = N.last_error()
+            assert msg.startswith(name + ": ") and text in msg, msg
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the behaviour on a machine without a GPU")
@@ -113,8 +141,8 @@ def test_backward_without_gpu_fails_loudly():
     s = (1, 2, 128, 64)
     x = torch.zeros(s, dtype=torch.float16)
     g32 = torch.zeros(s, dtype=torch.float32)
-    h = _t4(s, N.DS_F16, ptr=x.data_ptr())
-    f = _t4(s, N.DS_F32, ptr=g32.data_ptr())
+    h = _desc(s, N.DS_F16, ptr=x.data_ptr())
+    f = _desc(s, N.DS_F32, ptr=g32.data_ptr())
     ws = torch.zeros(1 << 22, dtype=torch.uint8)
     assert lib.ds_attn_bwd(h, h, h, h, h, 0.0, f, f, f, ws.data_ptr(), ws.numel(), None) == N.DS_ERR_CUDA
     d = torch.ones(1)
