@@ -53,11 +53,8 @@ PROTOTYPES = {
     "ds_profile_collect": (_i, [C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "ds_debug_set_trace": (_i, [_vp, _i]),
     "ds_debug_set_gemm_variant": (_i, [_i]),
-    "ds_debug_set_simmat_max_kb": (_i, [_i]),
     "ds_debug_set_simmat_blocked": (_i, [_i]),
     "ds_debug_set_attn_mc": (_i, [_i]),
-    "ds_debug_set_attn_grid": (_i, [_i]),
-    "ds_debug_set_attn_l2_promotion": (_i, [_i]),
     "ds_attn_fwd": (_i, [Tensor4, Tensor4, Tensor4, _f, Tensor4, _vp, _sz, _vp]),
     "ds_attn_fwd_workspace_bytes": (_sz, [Tensor4, Tensor4]),
     "ds_attn_bwd": (_i, [Tensor4, Tensor4, Tensor4, Tensor4, Tensor4, _f, Tensor4, Tensor4, Tensor4, _vp, _sz, _vp]),
@@ -104,10 +101,6 @@ def load() -> C.CDLL:
             fn.argtypes = args
         if lib.ds_abi_version() != 1:
             raise RuntimeError(f"ABI mismatch: library reports version {lib.ds_abi_version()}, binding expects 1")
-        # A/B switches for whole-process runs (bench.py under tools/gpu_ab.sh): DIFFSIM_B200_DEBUG="gemm_variant=0,simmat_max_kb=128"
-        for item in filter(None, os.environ.get("DIFFSIM_B200_DEBUG", "").split(",")):
-            key, _, val = item.partition("=")
-            getattr(lib, "ds_debug_set_" + key.strip())(int(val))
         _lib = lib
         return lib
 

@@ -59,9 +59,6 @@ constexpr int kTmemS = 0;        // S_A: columns [0,128), S_B: [128,256); P of t
                                  // overwrites the first 16 of its own 32 S columns
 constexpr int kTmemO = 256;      // O: [256, 256 + D_PAD)
 constexpr int kTmemOs = 416;     // O_self, packed 16-bit: [416, 416 + D_PAD/2)
-#ifndef DS_POLY_STRIDE
-#define DS_POLY_STRIDE -1    // -1: per head dim (AttnCfg::POLY_STRIDE); >= 0 forces one value for every head dim (A/B builds)
-#endif
 constexpr int kTmemL = 496;      // softmax denominators l = P . 1 (a 16-column MMA against a constant ones tile): [496,512)
 
 template <int D>
@@ -71,7 +68,7 @@ struct AttnCfg : AttnTile<D> {
   // (0: none).  With head dims <= 80 an item carries at most half the tensor work of D = 160 but the same 32 768
   // exponentials, and long-kv streams of such items are MUFU-bound: measured +13% on SDXL (2,20,1024,64) / (2,10,4096,64),
   // +6% on SD-1.5 up1 / up2, neutral on DiT-XL/2, and -4% at D = 160 (profiles/r1z_poly_shapes.txt).
-  static constexpr int POLY_STRIDE = DS_POLY_STRIDE >= 0 ? DS_POLY_STRIDE : (D <= 80 ? 3 : 0);
+  static constexpr int POLY_STRIDE = D <= 80 ? 3 : 0;
   static constexpr int Q_SUB_BYTES = kBlockQ * Tile::SUB_BYTES;
   static constexpr int Q_BYTES = Tile::NSUB * Q_SUB_BYTES;
   static constexpr int KV_SUB_BYTES = kHalfKV * Tile::SUB_BYTES;
@@ -394,9 +391,6 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         const uint32_t d_tmem = tmem_base + kTmemS + h * kHalfKV;
 #pragma unroll
         for (int kc = 0; kc < C::D_PAD / 16; ++kc) {
-#if defined(DS_ABLATE) && (DS_ABLATE & 1)
-          if (kc >= C::D_PAD / 32) break;   // ABLATION: half of the QK MMAs
-#endif
           const int sub = kc / C::CPS, off = (kc % C::CPS) * 32;
           umma_f16_ss(d_tmem, q_desc0 + (uint64_t)((sub * C::Q_SUB_BYTES + off) >> 4),
                       k_desc + (uint64_t)((sub * C::KV_SUB_BYTES + off) >> 4), idesc_qk, kc > 0 ? 1u : 0u);
@@ -441,11 +435,7 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         // uniform-datapath instructions per step, about as long as the tensor core needs for the step itself
         if (ksteps == kHalfKV / 16) {
 #pragma unroll
-#if defined(DS_ABLATE) && (DS_ABLATE & 8)
-          for (int ks = 0; ks < kHalfKV / 32; ++ks) pv_step(ks);   // ABLATION: half of the PV MMAs
-#else
           for (int ks = 0; ks < kHalfKV / 16; ++ks) pv_step(ks);
-#endif
         } else {
 #pragma unroll 1
           for (int ks = 0; ks < ksteps; ++ks) pv_step(ks);
@@ -503,17 +493,9 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         mbar_wait(&s_full[h], (h ? cntB : cntA) & 1);
         DS_TRACE_EV(32 + h);
         tc_fence_after_sync();
-#if defined(DS_ABLATE) && (DS_ABLATE & 256)
-        mbar_arrive(&p_full[h]);   // ABLATION: P is declared ready at once -- the MMA side never waits for the softmax
-#endif
         uint32_t v[32];
-#if defined(DS_ABLATE) && (DS_ABLATE & 16)
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = __float_as_uint((float)((w + j + lane) & 15));   // ABLATION: S is not read
-#else
         tmem_ld_x32(s_col + h * kHalfKV, v);   // also when nv == 0: stale columns, never used
         tmem_wait_ld();
-#endif
         DS_TRACE_EV(48 + h);
         // ragged tail (rare): columns past the kv length hold stale data, possibly NaN -- overwrite them with -inf once,
         // so that the common path below carries no per-column selects (-inf is neutral for the maximum and
@@ -540,13 +522,9 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         float* mx = sMax + (w & 1) * 512;
         mx[qtr * 128 + row] = m;
         DS_TRACE_EV(34 + h);
-#if defined(DS_ABLATE) && (DS_ABLATE & 64)
-        const float Mh = m;   // ABLATION: no exchange of the row maximum
-#else
         named_bar_sync(1 + quad, 128);   // the four warps of this TMEM quadrant (= of this scheduler) hold the row
         DS_TRACE_EV(36 + h);
         const float Mh = fmaxf(fmaxf(mx[row], mx[128 + row]), fmaxf(mx[256 + row], mx[384 + row]));
-#endif
         // Lazy running maximum: the first half of the item fixes the row's reference m_run; a later half keeps it and
         // simply lets p = exp2(s - m_run) grow -- up to 2^14 for fp16 P, 2^30 for bf16 -- which 16-bit P and the fp32
         // accumulators hold without loss (the offset cancels in O / l).  Only beyond that does the reference move, which
@@ -591,34 +569,21 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
             // the MUFU pipe (16 ex2 / clk / SM) is what bounds this phase: every kPolyStride-th pair is evaluated on the
             // FMA pipe instead
             constexpr int kPolyStride = C::POLY_STRIDE;
-#if defined(DS_ABLATE) && (DS_ABLATE & 2)
-            e0 = x0; e1 = x1;   // ABLATION: no exponentials
-#else
             if (kPolyStride > 0 && ((j >> 1) % (kPolyStride > 0 ? kPolyStride : 1)) == 0) {
               exp2_poly_f2(x0, x1, e0, e1);
             } else {
               e0 = fast_exp2(x0);
               e1 = fast_exp2(x1);
             }
-#endif
             pk[j >> 1] = pack2<kBf16>(e0, e1);
           }
-#if defined(DS_ABLATE) && (DS_ABLATE & 32)
-          uint32_t x = 0;   // ABLATION: P is not written
-#pragma unroll
-          for (int j = 0; j < 16; ++j) x ^= pk[j];
-          if (x == 0x12345678u) tmem_st_x16(s_col + h * kHalfKV, pk);
-#else
           tmem_st_x16(s_col + h * kHalfKV, pk);
-#endif
         }
         DS_TRACE_EV(44 + h);
         tmem_wait_st();
         DS_TRACE_EV(46 + h);
         tc_fence_before_sync();
-#if !(defined(DS_ABLATE) && (DS_ABLATE & 256))
         mbar_arrive(&p_full[h]);
-#endif
         DS_TRACE_EV(38 + h);
         if (h) ++cntB; else ++cntA;
       }
@@ -716,11 +681,7 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         } else if constexpr (MODE == ATTN_MODE_COS) {
           // unnormalised: dot = inv_l * sum o s, |Oc|^2 = inv_l^2 * sum o^2 (applied once per row below)
 #pragma unroll
-#if defined(DS_ABLATE) && (DS_ABLATE & 4)
-          for (int j = 0; j < 1; ++j) {   // ABLATION: 1/8 of the epilogue arithmetic
-#else
           for (int j = 0; j < 8; ++j) {
-#endif
             const float2 sv = unpack2<kBf16>(os[cur][j]);
             const uint64_t o2 = f2_pack_u(v[cur][2 * j], v[cur][2 * j + 1]);
             acc01 = f2_fma(o2, f2_pack(sv.x, sv.y), acc01);
@@ -956,16 +917,9 @@ __global__ void matrix_setup_kernel(int64_t n_rows, int64_t n_cols, int chunks, 
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-// ds_debug_set_attn_l2_promotion: L2 fetch granularity of K1's Q / K / V boxes (0 / 64 / 128 / 256 bytes).  A box row is one
-// head's D elements (80-320 bytes) out of a (B, S, H*D) memory row whose other heads are needed much later (streams are
-// head-major): with 256-byte promotion every miss dragged the neighbouring heads' bytes in from DRAM -- 17.1 MB per triplet
-// against 11.8 MB algorithmic at D = 160, 2.9x at DiT's 144-byte rows.  64 bytes: +3% sustained, +5% DiT (gpurun_out/r2bc).
-int g_attn_l2_promotion = 64;
-
 // ds_debug_set_attn_mc: -1 automatic (the N x N matrix only: +2-3% there, -1% sustained and +16% DRAM reads on pair / triplet
 // lists, profiles/r2_attn_experiments.txt section 8), 0 off, 1 on wherever the q tile count is even
 static int g_attn_mc = -1;
-static int g_attn_grid = 0;   // ds_debug_set_attn_grid: > 0 caps K1's persistent grid (load experiments); 0 = one CTA per SM
 static unsigned long long* g_trace_ptr = nullptr;
 static int g_trace_cap = 0;
 
@@ -1044,7 +998,6 @@ static int launch_attn_d(AttnLaunch a, cudaStream_t st) {
   a.p.cycles = g_trace_ptr ? g_trace_ptr + (size_t)8 * g_trace_cap : nullptr;
   int grid = sm_count();
   if (n_streams < grid) grid = (int)n_streams;
-  if (g_attn_grid > 0 && g_attn_grid < grid) grid = g_attn_grid;
   if (grid <= 0) return DS_OK;
   // K/V multicast over CTA pairs needs the two q tiles of a pair to exist (q tile is the fastest stream index, so CTAs
   // 2c and 2c + 1 hold q tiles 2j and 2j + 1 of the same (group, b, h) when n_qt and the grid are even)
@@ -1110,16 +1063,6 @@ int ds_debug_set_trace(void* dev_buf, int cap) {
 #else
   return 0;
 #endif
-}
-
-int ds_debug_set_attn_l2_promotion(int bytes) {
-  if (bytes == 0 || bytes == 64 || bytes == 128 || bytes == 256) ds::g_attn_l2_promotion = bytes;
-  return ds::g_attn_l2_promotion;
-}
-
-int ds_debug_set_attn_grid(int ctas) {
-  if (ctas >= 0) ds::g_attn_grid = ctas;
-  return ds::g_attn_grid;
 }
 
 int ds_debug_set_attn_mc(int mode) {

@@ -87,7 +87,11 @@ inline ds_tensor5 lift(const ds_tensor4& t) {
   return r;
 }
 
-extern int g_attn_l2_promotion;   // ds_debug_set_attn_l2_promotion
+// L2 fetch granularity of the Q / K / V boxes.  A box row is one head's D elements (80-320 bytes) out of a (B, S, H*D)
+// memory row whose other heads are needed much later (streams are head-major): with 256-byte promotion every miss dragged
+// the neighbouring heads' bytes in from DRAM -- 17.1 MB per triplet against 11.8 MB algorithmic at D = 160, 2.9x at DiT's
+// 144-byte rows.  64 bytes: +3% sustained, +5% DiT (profiles/r2bc_attn_l2_promotion_ab.txt).
+constexpr int kAttnL2PromotionBytes = 64;
 
 // TMA map of a validated operand: boxes of rows x subw elements, each box row one swizzle span of subw * 2 bytes
 inline int make_map(CUtensorMap* m, const ds_tensor5& t, int subw, int rows) {
@@ -98,7 +102,7 @@ inline int make_map(CUtensorMap* m, const ds_tensor5& t, int subw, int rows) {
   auto st = [&](int i) -> uint64_t { return (uint64_t)(t.size[i] > 1 ? t.stride[i] : 8) * 2; };
   uint64_t strides[4] = {st(3), st(2), st(1), st(0)};
   uint32_t box[5] = {(uint32_t)subw, (uint32_t)rows, 1, 1, 1};
-  return encode_tensor_map(m, t.dtype, 5, t.ptr, dims, strides, box, subw * 2, g_attn_l2_promotion);
+  return encode_tensor_map(m, t.dtype, 5, t.ptr, dims, strides, box, subw * 2, kAttnL2PromotionBytes);
 }
 
 }  // namespace ds

@@ -551,7 +551,7 @@ static int launch_gemm_tn(const void* a, int64_t M, int64_t lda, const void* b, 
     GemmOutMaps om;
     memset(&om, 0, sizeof(om));
     p.tma_store = 0;
-    if (EPI == GEMM_EPI_16 && g_gemm_tma_store && p.cols_per_out % 64 == 0) {
+    if (EPI == GEMM_EPI_16 && p.cols_per_out % 64 == 0) {
       const int n_t = (int)(N / p.cols_per_out);
       p.tma_store = 1;
       for (int t = 0; t < n_t && t < 3; ++t) {

@@ -10,7 +10,6 @@
 namespace ds {
 
 int g_gemm_variant = -1;
-int g_gemm_tma_store = 1;
 
 
 static thread_local char g_err[512] = "";
@@ -251,18 +250,8 @@ int ds_profile_collect(float* total_ms, int* launches) {
 }
 
 int ds_debug_set_gemm_variant(int variant) {
-  // variants -1 / 0 / 2; adding 16 to 0 or 2 (or passing -17 for "automatic") turns the TMA-store epilogue off
-  if (variant == -17) {
-    ds::g_gemm_variant = -1;
-    ds::g_gemm_tma_store = 0;
-  } else if (variant >= 16) {
-    ds::g_gemm_variant = variant - 16;
-    ds::g_gemm_tma_store = 0;
-  } else {
-    ds::g_gemm_variant = variant;
-    ds::g_gemm_tma_store = 1;
-  }
-  return 0;
+  if (variant == -1 || variant == 0 || variant == 2) ds::g_gemm_variant = variant;
+  return ds::g_gemm_variant;
 }
 
 int ds_twoafc(const float* ab, const float* ac, int64_t n, int mode, int32_t* counts, uint8_t* flags,

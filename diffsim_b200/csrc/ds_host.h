@@ -41,10 +41,9 @@ int encode_tensor_map(CUtensorMap* out, int dtype, int rank, const void* base, c
 void profile_begin(cudaStream_t st);
 void profile_end(cudaStream_t st);
 
-// simple bump allocator over the caller's workspace
-extern int g_gemm_tma_store; // ds_debug_set_gemm_variant(variant | 16): bit 4 set = epilogue WITHOUT TMA stores (A/B)
 extern int g_gemm_variant;   // ds_debug_set_gemm_variant: -1 automatic, 0 1-CTA GEMM kernel only, 2 CTA-pair kernel always
 
+// simple bump allocator over the caller's workspace
 struct Workspace {
   char* base;
   size_t size;

@@ -66,9 +66,7 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 // the time limit passes: without it a waiting warp re-issues the try_wait every few dozen clocks -- 41% of all
 // instructions the v6 attention kernel executed were such spins, paid for in issue slots and, under the power cap,
 // in SM clock.
-#ifndef DS_TRYWAIT_HINT_NS
-#define DS_TRYWAIT_HINT_NS 0x989680
-#endif
+constexpr uint32_t kTryWaitHintNs = 10000000;   // 10 ms
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -78,7 +76,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       "selp.u32 %0, 1, 0, p;\n\t"
       "}\n"
       : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)DS_TRYWAIT_HINT_NS)
+      : "r"(smem_u32(bar)), "r"(parity), "r"(kTryWaitHintNs)
       : "memory");
   return ok != 0;
 }
@@ -97,21 +95,6 @@ __device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// try_wait without a suspend-time hint
-__device__ __forceinline__ bool mbar_try_wait_nohint(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-
 #ifndef DS_WATCHDOG_NS
 #define DS_WATCHDOG_NS 4000000000ull  // 4 s: a stuck pipeline traps instead of hanging the GPU
 #endif
@@ -121,12 +104,6 @@ __device__ __forceinline__ bool mbar_try_wait_nohint(uint64_t* bar, uint32_t par
 // role, and these kernels live or die by their instruction-cache footprint.  A stuck pipeline traps after 2^10 failed
 // try_waits (each may suspend for the hint time: seconds in total); build with -DDS_WATCHDOG_VERBOSE to have it say where.
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-#ifdef DS_FASTWAIT
-  // A try_wait WITHOUT the suspend hint returns ~30 clocks after issue when the phase has already completed (the hinted
-  // form costs ~100-130 even then, profiles/r2p_wait_costs.txt) -- but under the board power cap the extra probe cost 4% of
-  // the sustained rate of the attention kernel (profiles/r2s_power_bisect.txt): off.
-  if (mbar_try_wait_nohint(bar, parity)) return;
-#endif
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
     if (++spins == (1u << 10)) {

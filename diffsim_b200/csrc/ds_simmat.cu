@@ -151,7 +151,6 @@ __global__ void simmat_finish_kernel(const float* __restrict__ part, int splits,
   if (sym && c != r) C[(size_t)c * ldc + r] = (float)out;
 }
 
-static int g_simmat_max_kb = 256;   // ds_debug_set_simmat_max_kb (A/B)
 static int g_simmat_blocked = -1;   // ds_debug_set_simmat_blocked: -1 automatic, 0 never, 1 whenever the pair kernel runs
 
 struct SimmatPlan {
@@ -180,7 +179,7 @@ static SimmatPlan simmat_plan(int64_t n_rows, int64_t n_cols, int64_t L, bool sy
   // accuracy: the tensor core adds each K = 16 MMA into the fp32 accumulator with truncation, a bias that grows with the
   // length of the chain (measured on 655 360-long unit-cosine rows: 2.1e-3 at 20 480 MMAs per partial, 5e-4 at 1 100);
   // a partial therefore never covers more than kMaxKbPerSplit k blocks (1024 MMAs); the partials are added in double
-  const int kMaxKbPerSplit = g_simmat_max_kb;
+  constexpr int kMaxKbPerSplit = 256;
   const int min_s = (p.kb_total + kMaxKbPerSplit - 1) / kMaxKbPerSplit;
   int max_s = p.kb_total / 8;
   if (max_s > 64) max_s = 64;
@@ -232,11 +231,6 @@ extern "C" {
 int ds_debug_set_simmat_blocked(int mode) {
   if (mode >= -1 && mode <= 1) ds::g_simmat_blocked = mode;
   return ds::g_simmat_blocked;
-}
-
-int ds_debug_set_simmat_max_kb(int kb) {
-  if (kb >= 8) ds::g_simmat_max_kb = kb;
-  return ds::g_simmat_max_kb;
 }
 
 size_t ds_simmat_workspace_bytes(int64_t n_rows, int64_t n_cols, int64_t L) {

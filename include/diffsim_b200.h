@@ -89,27 +89,19 @@ int ds_profile_collect(float* total_ms, int* launches);
  * clocks CTA 0 spent in the last attention launch in word [8 x cap].  Returns 1 if tracing is compiled in, else 0.
  */
 int ds_debug_set_trace(void* dev_buf, int cap);
-/* Debug / A-B only: GEMM kernel behind ds_qkv_project and ds_simmat: -1 automatic (default), 0 the 1-CTA 128x256 kernel
- * only, 2 the CTA-pair (cta_group::2, 256x256) kernel always.  Adding 16 to 0 / 2 (or passing -17 for automatic) selects
- * the epilogue without TMA stores. */
+/*
+ * Test hooks: each forces one side of an automatic kernel choice, so that tests can compare both sides bitwise.  -1
+ * restores the automatic choice (the default); any other value not listed is ignored.  Each returns the value in force.
+ */
+/* GEMM kernel behind ds_qkv_project and ds_simmat: 0 the 1-CTA 128x256 kernel only, 2 the CTA-pair (cta_group::2,
+ * 256x256) kernel always. */
 int ds_debug_set_gemm_variant(int variant);
-/* Debug / A-B only: longest k range (in 64-element blocks, >= 8) one fp32 partial of ds_simmat may cover (default 256).
- * Shorter ranges mean more partials (HBM traffic) but a smaller L2 working set and a shorter truncating accumulation
- * chain.  Returns the value in force. */
-int ds_debug_set_simmat_max_kb(int kb);
-/* Debug / A-B only: K1's K/V multicast over CTA pairs (clusters of two CTAs on the q tiles 2j, 2j + 1 of one (group, b, h),
- * every K/V tile read from L2 once for both): -1 automatic (default: ds_aas_matrix only, where it measures +2-3%), 0 off,
- * 1 on in every call whose q tile count is even.  Returns the value in force. */
+/* K1's K/V multicast over CTA pairs (clusters of two CTAs on the q tiles 2j, 2j + 1 of one (group, b, h), every K/V tile
+ * read from L2 once for both; automatic: ds_aas_matrix only, where it measures +2-3%): 0 off, 1 on in every call whose
+ * q tile count is even. */
 int ds_debug_set_attn_mc(int mode);
-/* Debug / A-B only: granularity (0, 64, 128 or 256 bytes) at which the L2 fetches a missing row piece of K1's Q / K / V TMA
- * boxes from DRAM.  Returns the value in force. */
-int ds_debug_set_attn_l2_promotion(int bytes);
-/* Debug / experiments only: cap K1's persistent grid at `ctas` CTAs (0 = default, one CTA per SM) -- how the clocks per item
- * depend on how loaded the chip is.  Returns the value in force. */
-int ds_debug_set_attn_grid(int ctas);
-/* Debug / A-B only: whether ds_simmat's statistics pass also writes k-blocked operand copies for the CTA-pair GEMM:
- * -1 automatic (default: when the operands exceed 512 MB), 0 never, 1 whenever the pair kernel runs.  Returns the value
- * in force. */
+/* Whether ds_simmat's statistics pass also writes k-blocked operand copies for the CTA-pair GEMM (automatic: when an
+ * operand reaches 1.5 GB): 0 never, 1 whenever the pair kernel runs. */
 int ds_debug_set_simmat_blocked(int mode);
 
 /* ---- K1: attention ------------------------------------------------------ */

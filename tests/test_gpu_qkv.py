@@ -60,6 +60,33 @@ def test_dit_packed_projection_with_bias_and_ragged_rows():
     assert qkv[0].stride()[-1] == 1
 
 
+@pytest.mark.parametrize("rows,c_in,n_out", [(1000, 1280, 3840), (512, 320, 960), (777, 64, 192), (4096, 1152, 3456),
+                                             (5000, 640, 1920), (4096, 512, 3000)])
+def test_one_cta_and_cta_pair_gemm_kernels_are_bitwise_equal(rows, c_in, n_out):
+    """The 1-CTA (128 x 256) and CTA-pair (256 x 256) GEMM kernels accumulate every output over k in the same order, so
+    the projection is bitwise the same whichever serves it.  The last shape's 1000 columns per output are not a multiple of 64: the pair
+    kernel then writes 16-bit outputs without TMA stores."""
+    dev = _cuda()
+    from diffsim_b200 import _native, ops
+
+    lib = _native.load()
+    g = torch.Generator().manual_seed(rows + c_in)
+    h = torch.randn(rows, c_in, generator=g).half()
+    w = (torch.randn(n_out, c_in, generator=g) / c_in ** 0.5).half()
+    b = torch.randn(n_out, generator=g).half()
+    outs = {}
+    try:
+        for variant in (0, 2):
+            assert lib.ds_debug_set_gemm_variant(variant) == variant
+            outs[variant] = ops.qkv_project(h.to(dev), w.to(dev), b.to(dev), 3)
+    finally:
+        lib.ds_debug_set_gemm_variant(-1)
+    for one_cta, pair in zip(outs[0], outs[2]):
+        assert torch.equal(one_cta, pair)
+    for got, ref in zip(outs[2], O.project_qkv(h, w, b)):
+        _ulp_close(got, ref, torch.float16)
+
+
 def test_projection_writes_straight_into_a_cache_and_scores_match():
     dev = _cuda()
     from diffsim_b200 import scoring, synth

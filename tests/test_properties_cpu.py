@@ -64,29 +64,8 @@ def test_oracle_invariants(seed, S, D, c):
     assert torch.allclose(O.attention(qa, kb, vb), O.attention(qa, kb, vb, scale=D ** -0.5), rtol=1e-12, atol=1e-14)
 
 
-def test_debug_env_switches_are_applied_at_load(monkeypatch):
-    """DIFFSIM_B200_DEBUG='key=value,...' calls ds_debug_set_<key>(value) when the library is loaded (A/B runs of bench.py)."""
-    import importlib
-
-    from diffsim_b200 import _native
-
-    if not os.path.exists(_native.LIB_PATH):
-        pytest.skip("library not built")
-    monkeypatch.setenv("DIFFSIM_B200_DEBUG", "simmat_max_kb=128")
-    fresh = importlib.reload(_native)
-    try:
-        lib = fresh.load()
-        assert lib.ds_debug_set_simmat_max_kb(0) == 128       # values < 8 are ignored: returns the value in force
-        monkeypatch.setenv("DIFFSIM_B200_DEBUG", "no_such_switch=1")
-        with pytest.raises(AttributeError):
-            importlib.reload(fresh).load()
-    finally:
-        monkeypatch.delenv("DIFFSIM_B200_DEBUG", raising=False)
-        importlib.reload(_native).load().ds_debug_set_simmat_max_kb(256)
-
-
-def test_debug_switches_validate_their_argument_and_report_the_value_in_force():
-    """The A/B switches of include/diffsim_b200.h only store a validated value (no device work): out-of-range arguments are
+def test_kernel_choice_hooks_validate_their_argument_and_report_the_value_in_force():
+    """The test hooks of include/diffsim_b200.h only store a validated value (no device work): out-of-range arguments are
     ignored and every call returns what is in force -- which is how the GPU tests restore the defaults."""
     from diffsim_b200 import _native
 
@@ -98,11 +77,11 @@ def test_debug_switches_validate_their_argument_and_report_the_value_in_force():
         assert lib.ds_debug_set_attn_mc(1) == 1 and lib.ds_debug_set_attn_mc(7) == 1 and lib.ds_debug_set_attn_mc(0) == 0
         assert lib.ds_debug_set_simmat_blocked(-1) == -1
         assert lib.ds_debug_set_simmat_blocked(1) == 1 and lib.ds_debug_set_simmat_blocked(5) == 1
-        assert lib.ds_debug_set_attn_l2_promotion(64) == 64       # the default
-        assert lib.ds_debug_set_attn_l2_promotion(100) == 64 and lib.ds_debug_set_attn_l2_promotion(256) == 256
-        assert lib.ds_debug_set_attn_grid(0) == 0 and lib.ds_debug_set_attn_grid(-3) == 0 and lib.ds_debug_set_attn_grid(8) == 8
+        assert lib.ds_debug_set_gemm_variant(-1) == -1           # default: pairs when the 256 x 256 tiles fill the clusters
+        assert lib.ds_debug_set_gemm_variant(2) == 2 and lib.ds_debug_set_gemm_variant(1) == 2
+        assert lib.ds_debug_set_gemm_variant(18) == 2 and lib.ds_debug_set_gemm_variant(-17) == 2
+        assert lib.ds_debug_set_gemm_variant(0) == 0
     finally:
         lib.ds_debug_set_attn_mc(-1)
         lib.ds_debug_set_simmat_blocked(-1)
-        lib.ds_debug_set_attn_l2_promotion(64)
-        lib.ds_debug_set_attn_grid(0)
+        lib.ds_debug_set_gemm_variant(-1)

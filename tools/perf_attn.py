@@ -17,9 +17,7 @@ def child():
     trips = torch.arange(3 * T, dtype=torch.int32, device="cuda").view(T, 3)
     cyc = torch.zeros(8 * 4 + 1, dtype=torch.int64, device="cuda")
     lib = N.load()
-    grid = int(os.environ.get("PERF_GRID", "148"))
-    if grid != 148:
-        lib.ds_debug_set_attn_grid(grid)
+    grid = torch.cuda.get_device_properties(0).multi_processor_count   # K1 runs one persistent CTA per SM
     out = []
     for name, fn, attn in (("pairs", lambda: ops.aas_pairs(q, k, v, pairs, "cosine"), 4 * pairs.shape[0]),
                            ("triplets", lambda: ops.aas_triplets(q, k, v, trips, "cosine"), 7 * T)):

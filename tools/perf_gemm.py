@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""A/B of the GEMM kernels behind K3 / K4 (ds_debug_set_gemm_variant: 0 = 1-CTA 128x256, 2 = CTA pairs 256x256 with the
-TMA-store epilogue, 18 = CTA pairs with the LSU epilogue):
-results must agree, then throughput on the QKV-projection and similarity-matrix shapes."""
+"""A/B of the GEMM kernels behind K3 / K4 (ds_debug_set_gemm_variant: 0 = 1-CTA 128x256, 2 = CTA pairs 256x256):
+how far apart their similarity matrices are, then throughput on the QKV-projection and similarity-matrix shapes.
+tests/test_gpu_qkv.py checks that both give bitwise the same projections."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -20,21 +20,8 @@ def timeit(fn, iters=10, warmup=3):
     return e0.elapsed_time(e1) / iters
 
 
-# ---- correctness: pair kernel vs 1-CTA kernel vs torch
+# ---- similarity matrix: pair kernel vs 1-CTA kernel
 g = torch.Generator(device="cuda").manual_seed(1)
-for rows, cin, nout in ((1000, 1280, 3840), (512, 320, 960), (777, 64, 192), (4096, 1152, 3456), (5000, 640, 1920)):
-    h = torch.randn(rows, cin, generator=g, device="cuda").half()
-    w = (torch.randn(nout, cin, generator=g, device="cuda") / cin ** 0.5).half()
-    b = torch.randn(nout, generator=g, device="cuda").half()
-    outs = {}
-    for var in (0, 2, 18):
-        lib.ds_debug_set_gemm_variant(var)
-        outs[var] = torch.cat(ops.qkv_project(h, w, b, 3), dim=-1)
-    ref = (h.float() @ w.float().t() + b.float())
-    e0 = (outs[0].float() - ref).abs().max().item()
-    e2 = (outs[2].float() - ref).abs().max().item()
-    print(f"[check qkv {rows}x{cin}->{nout}] 1cta==pair(tma store) {torch.equal(outs[0], outs[2])} pair(lsu)==pair(tma) "
-          f"{torch.equal(outs[18], outs[2])} err1cta={e0:.2e} errpair={e2:.2e}", flush=True)
 for n, L in ((600, 4096), (1000, 2048), (2032, 1024)):
     f = (torch.randn(n, L, generator=g, device="cuda") * 0.8 + 0.1).half()
     f2 = f.clone()
@@ -54,7 +41,7 @@ for n_img in (96, 768):
     outs = [torch.empty(n_img, 2, 256, 1280, dtype=torch.float16, device="cuda") for _ in range(3)]
     fl = 2 * n_img * 512 * 1280 * 3840
     line = f"[K4 {n_img} images]"
-    for var in (0, 18, 2, 0, 18, 2):
+    for var in (0, 2, 0, 2):
         lib.ds_debug_set_gemm_variant(var)
         ms = timeit(lambda: ops.qkv_project(hid, w, None, 3, out=outs))
         line += f" variant {var}: {ms:.3f} ms {fl / ms / 1e9:.0f} TFLOP/s |"

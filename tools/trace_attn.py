@@ -14,8 +14,6 @@ pairs = torch.tensor([(3 * t, 3 * t + 1) for t in range(n_img // 3)] + [(3 * t, 
                      dtype=torch.int32, device="cuda")
 buf = torch.zeros(8 * CAP, dtype=torch.int64, device="cuda")
 lib = N.load()
-if os.environ.get("TR_GRID"):
-    lib.ds_debug_set_attn_grid(int(os.environ["TR_GRID"]))
 ops.aas_pairs(q, k, v, pairs, "cosine")
 torch.cuda.synchronize()
 on = lib.ds_debug_set_trace(buf.data_ptr(), CAP)
