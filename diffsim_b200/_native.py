@@ -75,6 +75,9 @@ PROTOTYPES = {
     "ds_simmat": (_i, [_vp, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _vp, _i64, _vp, _sz, _vp]),
     "ds_simmat_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "ds_qkv_project": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _i64, _i64, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), _i, _vp]),
+    "ds_qkv_project_bwd": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, C.POINTER(C.c_void_p), C.POINTER(C.c_int64),
+                                _vp, _i64, _vp, _i64, _vp, _i, _vp, _sz, _vp]),
+    "ds_qkv_project_bwd_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64]),
     "ds_twoafc": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp]),
 }
 

@@ -1,7 +1,8 @@
 // Shared tcgen05 GEMM core:  C[M,N] = A[M,K] . B[N,K]^T   (both operands K-major 16-bit, fp32 accumulation in TMEM).
 //
 // Used by K3 (N x N similarity matrix: fp32 split-K partials, ds_simmat.cu) and K4 (QKV projection of the hooked
-// attention layer: 16-bit outputs scattered into the Q / K / V caches, ds_qkv.cu).
+// attention layer: 16-bit outputs scattered into the Q / K / V caches, ds_qkv.cu).  K4's backward products take MN-major
+// operands through the kernels at the end of this file (gemm_bwd_kernel / gemm2_bwd_kernel).
 //
 // Persistent, warp-specialised, one CTA per SM:
 //   warp 0      TMA producer   ring of kGemmStages x (A 128x64 + B 256x64) 128B-swizzled tiles
@@ -591,6 +592,340 @@ static int launch_gemm_tn(const void* a, int64_t M, int64_t lda, const void* b, 
   } else {
     DS_CUDA_TRY(cudaFuncSetAttribute(gemm_tn_kernel<EPI, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGSmemBytes));
     gemm_tn_kernel<EPI, false><<<grid, kGThreads, kGSmemBytes, st>>>(map_a, map_b, p);
+  }
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Backward products of a projection Y = X W^T whose output columns are split over n_seg tensors of seg_len columns each
+// (K4's q / k / v, or one packed tensor).  dY arrives as those separate tensors and is read in place, one tensor map per
+// tensor with its own row stride; a k block (dX) or an M tile (dW) never mixes two tensors, so seg_len need only be a
+// multiple of 8: the tail of a tensor's last block is zero-filled by TMA.
+//
+//   GEMM_BWD_DX  dX[rows, C_in]  = sum_t dY_t W_t       A = dY_t  K-major (as stored), B = W_t [seg_len, C_in] MN-major
+//                                                       K = n_seg x seg_len, blocked per tensor: kb -> (t, local kb)
+//   GEMM_BWD_DW  dW_t[seg_len, C_in] = dY_t^T X         A = dY_t  MN-major,            B = X [rows, C_in]      MN-major
+//                                                       M = n_seg x seg_len, tiled per tensor:   tm -> (t, local tm)
+//
+// An MN-major tile is stored as MN / 64 swizzled sub-tiles of 64 k rows x 128 bytes (one 64 x 64 TMA box each, as K1 loads
+// V for P V); its descriptor has LBO = the sub-tile pitch, SBO = 8 rows, and a K step of 16 rows = 2048 bytes.  Both the
+// 1-CTA and the CTA-pair kernel are built on one body; the accumulators always leave as fp32 split-K partials
+// part[split][M][N] (GEMM_EPI_F32), which a finishing kernel adds in split order and rounds once.
+// ---------------------------------------------------------------------------------------------------------------------
+enum : int { GEMM_BWD_DX = 0, GEMM_BWD_DW = 1 };
+
+struct GemmBwdMaps {
+  CUtensorMap a[3];   // per tensor: dY_t
+  CUtensorMap b[3];   // dX: per tensor W_t; dW: X in b[0]
+};
+
+constexpr int kGSubBytes = 64 * kGBK * 2;   // 8 KB: one 64 (MN) x 64 (K) sub-tile of an MN-major operand
+
+template <bool kPair>
+__device__ __forceinline__ void gemm_bwd_tma(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
+  if constexpr (kPair) tma_load_2d_2cta(dst, m, bar, c0, c1);
+  else tma_load_2d(dst, m, bar, c0, c1);
+}
+
+template <int OP, bool kPair>
+__device__ __forceinline__ void gemm_bwd_body(const GemmBwdMaps& maps, const GemmParams& p, int seg_len, int seg_blocks) {
+  constexpr int STAGES = kPair ? kG2Stages : kGStages;
+  constexpr int STAGE_BYTES = kPair ? kG2StageBytes : kGStageBytes;
+  constexpr int BM = kPair ? kG2BM : kGBM;           // output rows per work unit (the pair's tile spans both CTAs)
+  constexpr int B_SUBS = (kPair ? kGBN / 2 : kGBN) / 64;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)STAGES * STAGE_BYTES);
+  uint64_t* full = bars;
+  uint64_t* empty = bars + STAGES;
+  uint64_t* acc_full = bars + 2 * STAGES;        // [2]
+  uint64_t* acc_empty = bars + 2 * STAGES + 2;   // [2]: one elected lane per epilogue warp (of both CTAs of a pair)
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
+  uint8_t* epi_stage = reinterpret_cast<uint8_t*>(bars) + (kPair ? 1024 : 256);   // 4 x 4 KB, as the forward kernels
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t rank = kPair ? cluster_ctarank() : 0u;
+  const bool leader = rank == 0;
+  if (warp == 0 && lane == 0) {
+    for (int t = 0; t < 3; ++t) {
+      tma_prefetch_desc(&maps.a[t]);
+      tma_prefetch_desc(&maps.b[t]);
+    }
+  }
+  if (warp == 1 && lane == 0) {
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    for (int b = 0; b < 2; ++b) {
+      mbar_init(&acc_full[b], 1);
+      mbar_init(&acc_empty[b], kPair ? 8 : 4);
+    }
+    fence_mbar_init();
+  }
+  if (warp == 1) {
+    if constexpr (kPair) {
+      tmem_alloc_2cta(tmem_slot, 512);
+      tmem_relinquish_2cta();
+    } else {
+      tmem_alloc(tmem_slot, 512);
+      tmem_relinquish();
+    }
+  }
+  tc_fence_before_sync();
+  if constexpr (kPair) cluster_sync_all();
+  else __syncthreads();
+  tc_fence_after_sync();
+  const uint32_t tmem_base = *tmem_slot;
+
+  const int tiles = p.tiles_used;
+  const int n_units = tiles * p.splits;
+  const int unit0 = kPair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
+  const int unit_step = kPair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+
+  if (warp == 0) {
+    if (elect_one()) {
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int u = unit0; u < n_units; u += unit_step) {
+        const int split = u / tiles, tile = u - split * tiles;
+        int tm, tn;
+        gemm_decode_tile(p, tile, tm, tn, BM);
+        const int kb0 = split * p.kb_per_split, kb1 = min(p.kb_total, kb0 + p.kb_per_split);
+        const int n_base = tn * kGBN + (int)rank * (kGBN / 2);
+        for (int kb = kb0; kb < kb1; ++kb) {
+          mbar_wait(&empty[stage], phase ^ 1);
+          uint8_t* a = smem + (size_t)stage * STAGE_BYTES;
+          uint8_t* b = a + kGABytes;
+          if (leader) mbar_arrive_expect_tx(&full[stage], kPair ? 2 * STAGE_BYTES : STAGE_BYTES);
+          if constexpr (OP == GEMM_BWD_DX) {
+            const int t = kb / seg_blocks, k0 = (kb - t * seg_blocks) * kGBK;
+            gemm_bwd_tma<kPair>(a, &maps.a[t], &full[stage], k0, tm * BM + (int)rank * kGBM);
+#pragma unroll
+            for (int s = 0; s < B_SUBS; ++s) gemm_bwd_tma<kPair>(b + s * kGSubBytes, &maps.b[t], &full[stage], n_base + s * 64, k0);
+          } else {
+            const int t = tm / seg_blocks, m0 = (tm - t * seg_blocks) * BM + (int)rank * kGBM;
+#pragma unroll
+            for (int s = 0; s < kGBM / 64; ++s) gemm_bwd_tma<kPair>(a + s * kGSubBytes, &maps.a[t], &full[stage], m0 + s * 64, kb * kGBK);
+#pragma unroll
+            for (int s = 0; s < B_SUBS; ++s) gemm_bwd_tma<kPair>(b + s * kGSubBytes, &maps.b[0], &full[stage], n_base + s * 64, kb * kGBK);
+          }
+          if (++stage == STAGES) {
+            stage = 0;
+            phase ^= 1;
+          }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (leader && elect_one()) {
+      int stage = 0;
+      uint32_t phase = 0, n_local = 0;
+      for (int u = unit0; u < n_units; u += unit_step, ++n_local) {
+        const int split = u / tiles;
+        const int kb0 = split * p.kb_per_split, kb1 = min(p.kb_total, kb0 + p.kb_per_split);
+        const uint32_t buf = n_local & 1u;
+        mbar_wait(&acc_empty[buf], ((n_local >> 1) & 1u) ^ 1u);
+        tc_fence_after_sync();
+        const uint32_t d_tmem = tmem_base + buf * kGBN;
+        for (int kb = kb0; kb < kb1; ++kb) {
+          mbar_wait(&full[stage], phase);
+          tc_fence_after_sync();
+          const uint32_t a_addr = smem_u32(smem + (size_t)stage * STAGE_BYTES);
+          // K-major: +32 bytes per K = 16 step inside the swizzle atom; MN-major: +16 rows of 128 bytes
+          const uint64_t a_desc = OP == GEMM_BWD_DX ? umma_smem_desc(a_addr, 16, 1024, UMMA_SW128)
+                                                    : umma_smem_desc(a_addr, kGSubBytes, 1024, UMMA_SW128);
+          const uint64_t b_desc = umma_smem_desc(a_addr + kGABytes, kGSubBytes, 1024, UMMA_SW128);
+          constexpr uint64_t A_STEP = OP == GEMM_BWD_DX ? 2 : 128, B_STEP = 128;
+#pragma unroll
+          for (int k = 0; k < kGBK / 16; ++k) {
+            const uint32_t acc = (kb > kb0 || k > 0) ? 1u : 0u;
+            if constexpr (kPair) umma_f16_ss_2cta(d_tmem, a_desc + A_STEP * k, b_desc + B_STEP * k, p.idesc2, acc);
+            else umma_f16_ss(d_tmem, a_desc + A_STEP * k, b_desc + B_STEP * k, p.idesc, acc);
+          }
+          if constexpr (kPair) umma_commit_2cta(&empty[stage]);
+          else umma_commit(&empty[stage]);
+          if (++stage == STAGES) {
+            stage = 0;
+            phase ^= 1;
+          }
+        }
+        if constexpr (kPair) umma_commit_2cta(&acc_full[buf]);
+        else umma_commit(&acc_full[buf]);
+      }
+    }
+  } else {
+    const int quad = warp & 3;
+    uint32_t n_local = 0;
+    uint8_t* stage_patch = epi_stage + (warp - 2) * kGEpiStageBytes;
+    for (int u = unit0; u < n_units; u += unit_step, ++n_local) {
+      const int split = u / tiles, tile = u - split * tiles;
+      int tm, tn;
+      gemm_decode_tile(p, tile, tm, tn, BM);
+      const uint32_t buf = n_local & 1u;
+      mbar_wait(&acc_full[buf], (n_local >> 1) & 1u);
+      tc_fence_after_sync();
+      const uint32_t t_addr = tmem_base + ((uint32_t)(quad * 32) << 16) + buf * kGBN;
+      const int r0 = (int)rank * kGBM + quad * 32;
+      if constexpr (OP == GEMM_BWD_DX) {
+        gemm_epilogue_rows<GEMM_EPI_F32, false>(p, t_addr, tm * BM + r0, tn * kGBN, split, stage_patch, lane);
+      } else {
+        // rows of tensor t: partial rows [t * seg_len, (t + 1) * seg_len)
+        const int t = tm / seg_blocks;
+        GemmParams q = p;
+        q.M = seg_len;
+        q.part = p.part + (size_t)t * seg_len * p.N;
+        gemm_epilogue_rows<GEMM_EPI_F32, false>(q, t_addr, (tm - t * seg_blocks) * BM + r0, tn * kGBN, split, stage_patch, lane);
+      }
+      tc_fence_before_sync();
+      __syncwarp();
+      if (lane == 0) {
+        if constexpr (kPair) mbar_arrive_leader(&acc_empty[buf]);
+        else mbar_arrive(&acc_empty[buf]);
+      }
+    }
+  }
+  tc_fence_before_sync();
+  if constexpr (kPair) {
+    cluster_sync_all();   // the peer may still be reading this CTA's B half / signalling its barriers
+    if (warp == 1) tmem_dealloc_2cta(tmem_base, 512);
+  } else {
+    __syncthreads();
+    if (warp == 1) tmem_dealloc(tmem_base, 512);
+  }
+}
+
+template <int OP>
+__global__ void __launch_bounds__(kGThreads, 1)
+gemm_bwd_kernel(const __grid_constant__ GemmBwdMaps maps, const GemmParams p, int seg_len, int seg_blocks) {
+  gemm_bwd_body<OP, false>(maps, p, seg_len, seg_blocks);
+}
+
+template <int OP>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGThreads, 1)
+gemm2_bwd_kernel(const __grid_constant__ GemmBwdMaps maps, const GemmParams p, int seg_len, int seg_blocks) {
+  gemm_bwd_body<OP, true>(maps, p, seg_len, seg_blocks);
+}
+
+// Split-K policy of the backward products: no partial longer than K3's 256 k blocks (the tensor core's truncating fp32
+// adds bias longer chains), then the smallest split count whose work units fill the persistent grid's waves to >= 95%
+// (each split keeping >= 4 k blocks, at most 16 splits beyond the minimum); the fullest of those if none reaches 95%.
+static int gemm_bwd_splits(int64_t tiles, int kb_total, int units_per_wave) {
+  constexpr int kMaxKbPerSplit = 256;
+  const int min_s = (kb_total + kMaxKbPerSplit - 1) / kMaxKbPerSplit;
+  int max_s = min_s + 16;
+  if (max_s > kb_total / 4) max_s = kb_total / 4;
+  if (max_s < min_s) max_s = min_s;
+  int best_s = min_s;
+  double best_eff = 0.0;
+  for (int s = min_s; s <= max_s; ++s) {
+    const int kps = (kb_total + s - 1) / s;
+    const int real_s = (kb_total + kps - 1) / kps;
+    const int64_t units = tiles * real_s;
+    const int64_t waves = (units + units_per_wave - 1) / units_per_wave;
+    const double eff = (double)units / (double)(waves * units_per_wave);
+    if (eff > best_eff + 1e-9) {
+      best_eff = eff;
+      best_s = real_s;
+    }
+    if (eff >= 0.95) break;
+  }
+  return best_s;
+}
+
+// Geometry of one backward product: M x N output, kb_total k blocks, tile and split counts for the chosen kernel
+struct GemmBwdPlan {
+  int pair;
+  int tiles_m, tiles_n, kb_total, splits, kb_per_split;
+  int seg_blocks;   // dX: k blocks per tensor; dW: M tiles per tensor
+};
+
+// n_seg tensors of seg_len columns; rows of the projection input; c_in its channels.  pair: -1 automatic, else 0 / 1.
+static GemmBwdPlan gemm_bwd_plan(int op, int64_t rows, int64_t c_in, int n_seg, int64_t seg_len, int pair) {
+  GemmBwdPlan g;
+  const int64_t M = op == GEMM_BWD_DX ? rows : (int64_t)n_seg * seg_len;
+  const int64_t seg_kb = (seg_len + kGBK - 1) / kGBK;
+  const int64_t kb = op == GEMM_BWD_DX ? n_seg * seg_kb : (rows + kGBK - 1) / kGBK;
+  g.pair = pair >= 0 ? pair : gemm_use_pair(M, c_in, 1, -1) ? 1 : 0;
+  const int bm = g.pair ? kG2BM : kGBM;
+  g.seg_blocks = op == GEMM_BWD_DX ? (int)seg_kb : (int)((seg_len + bm - 1) / bm);
+  g.tiles_m = op == GEMM_BWD_DX ? (int)((rows + bm - 1) / bm) : n_seg * g.seg_blocks;
+  g.tiles_n = (int)((c_in + kGBN - 1) / kGBN);
+  g.kb_total = (int)kb;
+  // the split count is planned on the pair kernel's 256 x 256 tiles and clusters whichever kernel runs, so that both give
+  // the same partials and hence bitwise the same result
+  int sms = sm_count();
+  if (sms <= 0) sms = 148;
+  const int64_t tiles2 = (op == GEMM_BWD_DX ? (rows + kG2BM - 1) / kG2BM : n_seg * ((seg_len + kG2BM - 1) / kG2BM)) * g.tiles_n;
+  g.splits = gemm_bwd_splits(tiles2, g.kb_total, sms / 2);
+  g.kb_per_split = (g.kb_total + g.splits - 1) / g.splits;
+  g.splits = (g.kb_total + g.kb_per_split - 1) / g.kb_per_split;
+  return g;
+}
+
+// One backward product into fp32 partials part[split][M][N] (M = rows for dX, n_seg * seg_len for dW; N = c_in).
+// dy[t]: [rows, seg_len] with row stride ld_dy[t]; w: [n_seg * seg_len, c_in] (ldw); x: [rows, c_in] (ldx).
+template <int OP>
+static int launch_gemm_bwd(const GemmBwdPlan& g, const void* const* dy, const int64_t* ld_dy, int n_seg, int64_t seg_len,
+                           const void* w, int64_t ldw, const void* x, int64_t ldx, int64_t rows, int64_t c_in, int dtype,
+                           float* part, cudaStream_t st) {
+  GemmBwdMaps maps;
+  memset(&maps, 0, sizeof(maps));
+  int rc;
+  for (int t = 0; t < n_seg; ++t) {
+    uint64_t dims[2] = {(uint64_t)seg_len, (uint64_t)rows};
+    uint64_t str[1] = {(uint64_t)ld_dy[t] * 2};
+    // dX: K-major boxes of 64 k x 128 rows; dW: MN-major boxes of 64 (MN) x 64 k
+    uint32_t box[2] = {(uint32_t)kGBK, OP == GEMM_BWD_DX ? (uint32_t)kGBM : (uint32_t)kGBK};
+    if ((rc = encode_tensor_map(&maps.a[t], dtype, 2, dy[t], dims, str, box, 128)) != DS_OK) return rc;
+    if (OP == GEMM_BWD_DX) {
+      uint64_t dw[2] = {(uint64_t)c_in, (uint64_t)seg_len};
+      uint64_t sw[1] = {(uint64_t)ldw * 2};
+      uint32_t bw[2] = {64u, (uint32_t)kGBK};
+      const void* wt = static_cast<const uint16_t*>(w) + (size_t)t * seg_len * ldw;
+      if ((rc = encode_tensor_map(&maps.b[t], dtype, 2, wt, dw, sw, bw, 128)) != DS_OK) return rc;
+    }
+  }
+  if (OP == GEMM_BWD_DW) {
+    uint64_t dx[2] = {(uint64_t)c_in, (uint64_t)rows};
+    uint64_t sx[1] = {(uint64_t)ldx * 2};
+    uint32_t bx[2] = {64u, (uint32_t)kGBK};
+    if ((rc = encode_tensor_map(&maps.b[0], dtype, 2, x, dx, sx, bx, 128)) != DS_OK) return rc;
+  }
+  for (int t = n_seg; t < 3; ++t) {   // unused slots repeat a valid map (prefetched, never loaded)
+    maps.a[t] = maps.a[0];
+    maps.b[t] = maps.b[0];
+  }
+  if (OP == GEMM_BWD_DW)
+    for (int t = 1; t < 3; ++t) maps.b[t] = maps.b[0];
+  GemmParams p = {};
+  p.M = (int)(OP == GEMM_BWD_DX ? rows : n_seg * seg_len);
+  p.N = (int)c_in;
+  p.tiles_m = g.tiles_m;
+  p.tiles_n = g.tiles_n;
+  p.kb_total = g.kb_total;
+  p.splits = g.splits;
+  p.kb_per_split = g.kb_per_split;
+  p.tiles_used = g.tiles_m * g.tiles_n;
+  p.part = part;
+  p.part_split_stride = (int64_t)p.M * p.N;
+  const uint32_t fmt = dtype == DS_BF16 ? 1u : 0u, a_mn = OP == GEMM_BWD_DX ? 0u : 1u;
+  const int64_t units = (int64_t)p.tiles_used * p.splits;
+  if (units <= 0) return DS_OK;
+  if (units > INT32_MAX) return fail(DS_ERR_INVALID, "gemm: too many work units");
+  if (g.pair) {
+    p.idesc2 = umma_idesc_f16(fmt, kG2BM, kGBN, a_mn, 1);
+    int clusters = sm_count() / 2;
+    if (units < clusters) clusters = (int)units;
+    DS_CUDA_TRY(cudaFuncSetAttribute(gemm2_bwd_kernel<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kG2SmemBytes));
+    gemm2_bwd_kernel<OP><<<2 * clusters, kGThreads, kG2SmemBytes, st>>>(maps, p, (int)seg_len, g.seg_blocks);
+  } else {
+    p.idesc = umma_idesc_f16(fmt, kGBM, kGBN, a_mn, 1);
+    int grid = sm_count();
+    if (units < grid) grid = (int)units;
+    DS_CUDA_TRY(cudaFuncSetAttribute(gemm_bwd_kernel<OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGSmemBytes));
+    gemm_bwd_kernel<OP><<<grid, kGThreads, kGSmemBytes, st>>>(maps, p, (int)seg_len, g.seg_blocks);
   }
   DS_CUDA_TRY(cudaGetLastError());
   return DS_OK;

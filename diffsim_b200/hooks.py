@@ -67,6 +67,8 @@ def project_qkv(attn, hidden_states: torch.Tensor, encoder_hidden_states: Option
 
     Self-attention on CUDA: one ds_qkv_project call on the stacked weight [W_q; W_k; W_v] (K4) instead of three
     nn.Linear; `out` = three pre-allocated (B,S,H*D) tensors (e.g. a slot of a QKVCache) receives the result in place.
+    The fused projection is differentiable: with grad recorded, hidden_states and the to_q / to_k / to_v weights and
+    biases get their gradients (ds_qkv_project_bwd).  A capture with `out` is forward-only, like the cache scorers.
     already_normed: the caller (a processor) has applied attn.spatial_norm(hidden_states, temb) itself -- a pre-hook has no
     temb and cannot."""
     if getattr(attn, "spatial_norm", None) is not None and not already_normed:
@@ -79,7 +81,13 @@ def project_qkv(attn, hidden_states: torch.Tensor, encoder_hidden_states: Option
         hidden_states = attn.group_norm(hidden_states.transpose(1, 2)).transpose(1, 2)
     if encoder_hidden_states is None and fused_qkv and _can_fuse(attn, hidden_states):
         weight, bias = _stacked_qkv_weight(attn)
-        query, key, value = ops.qkv_project(hidden_states, weight, bias, 3, out=out)
+        if out is None:
+            # differentiable in hidden_states and in the three modules' weights and biases (not in the cached stack)
+            lins = (attn.to_q, attn.to_k, attn.to_v)
+            query, key, value = ops.qkv_project_stacked(hidden_states, weight, bias, 3, [m.weight for m in lins],
+                                                        [m.bias for m in lins])
+        else:
+            query, key, value = ops.qkv_project(hidden_states, weight, bias, 3, out=out)
         return split_heads(query, attn.heads), split_heads(key, attn.heads), split_heads(value, attn.heads)
     query = attn.to_q(hidden_states)
     if encoder_hidden_states is None:
@@ -121,7 +129,7 @@ def make_dit_pre_hook(early_exit: bool = False, fused_qkv: bool = True):
         lin = module.qkv
         if (fused_qkv and x.is_cuda and x.dtype in (torch.float16, torch.bfloat16) and type(lin) is torch.nn.Linear
                 and lin.weight.dtype == x.dtype and C % 8 == 0 and lin.out_features % 8 == 0):
-            packed = ops.qkv_project(x, lin.weight.detach(), None if lin.bias is None else lin.bias.detach(), 1)[0]
+            packed = ops.qkv_project(x, lin.weight, lin.bias, 1)[0]   # differentiable in x, weight and bias
         else:
             packed = lin(x)
         qkv = packed.reshape(B, N, 3, module.num_heads, module.head_dim).permute(2, 0, 3, 1, 4)

@@ -363,7 +363,29 @@ def qkv_project(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch
     The capture step of the reference on the hook's input: attn.to_q / to_k / to_v (diffsim/hacked_attn.py:61-69,
     weight = the three nn.Linear weights stacked along dim 0) or DiT's fused module.qkv (diffsim/diffsim_dit.py:21,
     n_outputs = 1: one packed (..., 3C) tensor).  fp32 accumulation on tcgen05, one rounding to the input dtype.
-    `out`: optional pre-allocated outputs (row stride may exceed the column count, e.g. slices of a cache)."""
+    `out`: optional pre-allocated outputs (row stride may exceed the column count, e.g. slices of a cache).
+    Differentiable in hidden, weight and bias (qkv_project_bwd) when one of them requires grad and `out` is not given;
+    the outputs are bitwise the same either way.  A call with `out` (a capture into a cache) is forward-only."""
+    if out is None and wants_grad(hidden, weight, *(() if bias is None else (bias,))):
+        return _QKVProjectFn.apply(n_outputs, 0, hidden, weight, bias)
+    return _qkv_project(hidden, weight, bias, n_outputs, out)
+
+
+def qkv_project_stacked(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], n_outputs: int,
+                        weights: Sequence[torch.Tensor], biases: Sequence[Optional[torch.Tensor]]) -> Tuple[torch.Tensor, ...]:
+    """qkv_project on a stacked weight (and bias) built from the equal-sized row blocks `weights` (and `biases`, None
+    where a block has none), e.g. a cached [W_q; W_k; W_v] of three nn.Linear modules.  The product runs once on the
+    stack; when grad is recorded, the gradients of its row blocks go to `weights` / `biases`, which are the graph's
+    inputs (the stack itself receives none)."""
+    if len(weights) != len(biases):
+        raise RuntimeError("weights and biases must have one entry per row block")
+    if wants_grad(hidden, *weights, *[b for b in biases if b is not None]):
+        return _QKVProjectFn.apply(n_outputs, len(weights), hidden, weight.detach(),
+                                   None if bias is None else bias.detach(), *weights, *biases)
+    return _qkv_project(hidden, weight, bias, n_outputs)
+
+
+def _qkv_project(hidden, weight, bias=None, n_outputs=3, out=None) -> Tuple[torch.Tensor, ...]:
     import ctypes as C
 
     dev = _need_cuda(hidden, weight)
@@ -395,6 +417,74 @@ def qkv_project(hidden: torch.Tensor, weight: torch.Tensor, bias: Optional[torch
     _call("ds_qkv_project", dev, h2.data_ptr(), rows, h2.stride(0), c_in, weight.data_ptr(), weight.stride(0),
           bias.data_ptr() if bias is not None else None, n_out, cols, ptrs, lds, _dtype_code(hidden), launches=1)
     return tuple(out)
+
+
+def _rows_tma(t: torch.Tensor, rows: int, cols: int) -> torch.Tensor:
+    # (rows, cols) view of a 16-bit gradient the library reads by TMA (unit column stride, 16-byte aligned base and rows)
+    t2 = t.reshape(rows, cols)
+    ok = t2.stride(1) == 1 and t2.data_ptr() % 16 == 0 and (rows == 1 or (t2.stride(0) >= cols and t2.stride(0) % 8 == 0))
+    return t2 if ok else t2.contiguous()
+
+
+def qkv_project_bwd(hidden: torch.Tensor, weight: torch.Tensor, dys: Sequence[torch.Tensor], need_hidden: bool = True,
+                    need_weight: bool = True, need_bias: bool = False):
+    """Gradients (dhidden, dweight, dbias) of qkv_project(hidden, weight, bias, len(dys)) for the output gradients dys,
+    each None where not wanted (and then not computed): dY W, dY^T hidden and the column sums of dY, where dY is the
+    dys side by side.  In the input dtype, as an fp16 / bf16 nn.Linear backward returns them: fp32 accumulation, one
+    rounding; deterministic (split-K partials added in a fixed order, no atomics).  The dys are read in place."""
+    import ctypes as C
+
+    dev = _need_cuda(hidden, weight, *dys)
+    c_in = hidden.shape[-1]
+    n_out, n_t = weight.shape[0], len(dys)
+    if weight.dim() != 2 or weight.shape[1] != c_in or weight.stride(1) != 1 or hidden.dtype != weight.dtype:
+        raise RuntimeError(f"weight must be (n_out, {c_in}) with contiguous rows, of hidden's dtype")
+    if n_t < 1 or n_out % n_t:
+        raise RuntimeError("n_out must be a multiple of the number of output gradients")
+    cols = n_out // n_t
+    rows = hidden.numel() // c_in
+    dx = torch.empty(hidden.shape, dtype=hidden.dtype, device=dev) if need_hidden else None
+    dw = torch.empty((n_out, c_in), dtype=hidden.dtype, device=dev) if need_weight else None
+    db = torch.empty(n_out, dtype=hidden.dtype, device=dev) if need_bias else None
+    if rows == 0:   # nothing to add up: the weight and bias gradients are zero, the input gradient is empty
+        return dx, None if dw is None else dw.zero_(), None if db is None else db.zero_()
+    if dx is None and dw is None and db is None:
+        return dx, dw, db
+    d2 = [_rows_tma(d.to(hidden.dtype), rows, cols) for d in dys]
+    h2 = hidden.reshape(rows, c_in) if need_weight else None
+    if h2 is not None and h2.stride(1) != 1:
+        h2 = h2.contiguous()
+    ptrs = (C.c_void_p * n_t)(*[d.data_ptr() for d in d2])
+    lds = (C.c_int64 * n_t)(*[d.stride(0) if rows > 1 else cols for d in d2])
+    _call("ds_qkv_project_bwd", dev, None if h2 is None else h2.data_ptr(), rows, c_in if h2 is None else h2.stride(0),
+          c_in, weight.data_ptr(), weight.stride(0), n_out, cols, ptrs, lds, None if dx is None else dx.data_ptr(), c_in,
+          None if dw is None else dw.data_ptr(), c_in, None if db is None else db.data_ptr(), _dtype_code(hidden),
+          ws_query=(rows, c_in, n_out, cols), slot="bwd",
+          launches=2 * sum(g is not None for g in (dx, dw, db)))  # per wanted gradient: product or column sums + finish
+    return dx, dw, db
+
+
+class _QKVProjectFn(torch.autograd.Function):
+    """qkv_project with the K4 backward; saves only the inputs.  The product runs on (weight, bias); with n_parts > 0 the
+    gradients of their n_parts row blocks go to the trailing inputs (n_parts weights, then n_parts biases or None)."""
+
+    @staticmethod
+    def forward(ctx, n_outputs, n_parts, hidden, weight, bias, *parts):
+        ctx.save_for_backward(hidden, weight)
+        ctx.n_outputs, ctx.n_parts = n_outputs, n_parts
+        return _qkv_project(hidden, weight, bias, n_outputs)
+
+    @staticmethod
+    def backward(ctx, *dys):
+        hidden, weight = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        n = ctx.n_parts
+        w_need, b_need = need[5:5 + n], need[5 + n:]
+        dx, dw, db = qkv_project_bwd(hidden, weight, dys, need[2], need[3] or any(w_need), need[4] or any(b_need))
+        blk = weight.shape[0] // n if n else 0
+        w_parts = [dw[i * blk:(i + 1) * blk] if w_need[i] else None for i in range(n)]
+        b_parts = [db[i * blk:(i + 1) * blk] if b_need[i] else None for i in range(n)]
+        return (None, None, dx, dw if need[3] else None, db if need[4] else None, *w_parts, *b_parts)
 
 
 # --------------------------------------------------------------------------------------

@@ -66,7 +66,7 @@ def _simmat(rows, cols=None, similarity="cosine"):
 
 
 def _qkv_project(hidden, weight, bias=None, n_outputs=3) -> List[torch.Tensor]:
-    return list(ops.qkv_project(hidden, weight, bias, n_outputs))
+    return list(ops._qkv_project(hidden, weight, bias, n_outputs))   # forward only: no autograd registered
 
 
 for _name, _fn in (("attn_fwd", _attn_fwd), ("aas_score", _aas_score), ("aas_pairs", _aas_pairs),

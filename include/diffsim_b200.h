@@ -93,8 +93,8 @@ int ds_debug_set_trace(void* dev_buf, int cap);
  * Test hooks: each forces one side of an automatic kernel choice, so that tests can compare both sides bitwise.  -1
  * restores the automatic choice (the default); any other value not listed is ignored.  Each returns the value in force.
  */
-/* GEMM kernel behind ds_qkv_project and ds_simmat: 0 the 1-CTA 128x256 kernel only, 2 the CTA-pair (cta_group::2,
- * 256x256) kernel always. */
+/* GEMM kernel behind ds_qkv_project, both products of ds_qkv_project_bwd and ds_simmat: 0 the 1-CTA 128x256 kernel only,
+ * 2 the CTA-pair (cta_group::2, 256x256) kernel always. */
 int ds_debug_set_gemm_variant(int variant);
 /* K1's K/V multicast over CTA pairs (clusters of two CTAs on the q tiles 2j, 2j + 1 of one (group, b, h), every K/V tile
  * read from L2 once for both; automatic: ds_aas_matrix only, where it measures +2-3%): 0 off, 1 on in every call whose
@@ -272,6 +272,22 @@ int ds_qkv_project(const void* hidden, int64_t n_rows, int64_t ld_hidden, int64_
                    const void* weight, int64_t ld_weight, const void* bias,
                    int64_t n_out, int64_t cols_per_out,
                    void* const* out, const int64_t* ld_out, int dtype, void* stream);
+
+/*
+ * Backward of ds_qkv_project for the gradient dy of its outputs (the same hidden / weight / n_out / cols_per_out):
+ *   dhidden = dY . weight  [n_rows, c_in]    dweight = dY^T . hidden  [n_out, c_in]    dbias = sum over rows of dY  [n_out]
+ * where dY[r, n] = dy[n / cols_per_out][r, n % cols_per_out]: n_out / cols_per_out tensors of n_rows x cols_per_out,
+ * row stride ld_dy[.] elements, read in place.  Each of dhidden (row stride ld_dhidden), dweight (ld_dweight) and dbias
+ * may be null: not wanted, not computed; hidden may be null when dweight is, weight when dhidden is.  Outputs are of
+ * `dtype`, written (not added into): fp32 accumulation, split-K partials added in a fixed order, one rounding --
+ * bitwise reproducible, no atomics.  Launches: 2 per wanted output (product or column sums, then its finish).
+ */
+size_t ds_qkv_project_bwd_workspace_bytes(int64_t n_rows, int64_t c_in, int64_t n_out, int64_t cols_per_out);
+int ds_qkv_project_bwd(const void* hidden, int64_t n_rows, int64_t ld_hidden, int64_t c_in,
+                       const void* weight, int64_t ld_weight, int64_t n_out, int64_t cols_per_out,
+                       const void* const* dy, const int64_t* ld_dy,
+                       void* dhidden, int64_t ld_dhidden, void* dweight, int64_t ld_dweight, void* dbias,
+                       int dtype, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- decisions ---------------------------------------------------------- */
 
