@@ -62,6 +62,14 @@ PROTOTYPES = {
     "ds_aas_dir_bwd": (_i, [Tensor4, Tensor4, Tensor4, Tensor4, Tensor4, _f, _i, _vp, Tensor4, Tensor4, Tensor4, Tensor4,
                             Tensor4, _vp, _sz, _vp]),
     "ds_aas_dir_bwd_workspace_bytes": (_sz, [Tensor4, Tensor4]),
+    "ds_aas_groups_bwd": (_i, [Tensor5, Tensor5, Tensor5, Tensor5, Tensor5, _vp, _vp, _i64, _vp, _i64, _f, _i, _vp, Tensor5,
+                               Tensor5, Tensor5, Tensor5, Tensor5, _vp, _sz, _vp]),
+    "ds_aas_groups_bwd_workspace_bytes": (_sz, [Tensor5, Tensor5, _i64, _i64]),
+    "ds_aas_pairs_bwd": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, Tensor5, Tensor5, Tensor5, _vp, _sz, _vp]),
+    "ds_aas_pairs_bwd_workspace_bytes": (_sz, [Tensor5, _i64]),
+    "ds_aas_triplets_bwd": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, _vp, Tensor5, Tensor5, Tensor5, _vp, _sz,
+                                 _vp]),
+    "ds_aas_triplets_bwd_workspace_bytes": (_sz, [Tensor5, _i64]),
     "ds_aas_groups": (_i, [Tensor5, Tensor5, Tensor5, Tensor5, Tensor5, _vp, _vp, _i64, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),
     "ds_aas_groups_workspace_bytes": (_sz, [Tensor5, _i64, _i64]),
     "ds_aas_pairs": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),

@@ -45,7 +45,9 @@
 
 namespace ds {
 
-enum : int { ATTN_MODE_COS = 0, ATTN_MODE_MSE = 1, ATTN_MODE_STORE = 2 };
+// LIST: the store form of a grouped work list (the recompute of the AAS backward): every item's O is written, rounded as in
+// STORE, to output slot g (the self item of group g) or n_groups + t (entry t) of a contiguous (slot, B, H, Sq, D) stack
+enum : int { ATTN_MODE_COS = 0, ATTN_MODE_MSE = 1, ATTN_MODE_STORE = 2, ATTN_MODE_LIST = 3 };
 
 constexpr int kAttnThreads = 832;   // 26 warps: producer, MMA, 8 epilogue, 16 softmax
 constexpr int kWarpProducer = 0;
@@ -121,7 +123,7 @@ struct AttnParams {
 
 // One kv group of one item of one stream, as every warp role enumerates them (identically).
 struct GroupInfo {
-  int b, h, qt, bh, qi;     // stream
+  int b, h, qt, bh, qi, g;  // stream
   int img, entry;           // item: kv image, index into kv_idx / part (cross items)
   int kv0, rowsA, rowsB;    // group: first kv row, valid rows of the two halves
   bool self, first_of_stream, last_of_stream, first_of_item, last_of_item;
@@ -140,6 +142,7 @@ __device__ __forceinline__ void for_each_group(const AttnParams& p, F&& f) {
     G.qt = (int)(st - r * (uint32_t)p.n_qt);
     G.bh = (int)(r / (uint32_t)p.n_groups);
     const int g = (int)(r - (uint32_t)G.bh * (uint32_t)p.n_groups);
+    G.g = g;
     G.b = G.bh / p.H;
     G.h = G.bh - G.b * p.H;
     // the work list lives in global memory and every role walks it between barriers the compiler cannot move loads
@@ -628,7 +631,12 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
       if constexpr (MODE == ATTN_MODE_STORE)
         out_row = static_cast<uint8_t*>(p.out) + 2 * ((int64_t)G.b * p.out_sb + (int64_t)G.h * p.out_sh +
                                                      (int64_t)(G.qt * kBlockQ + row) * p.out_ss + c_base * 16);
-      const bool cross = (MODE != ATTN_MODE_STORE) && !G.self;
+      if constexpr (MODE == ATTN_MODE_LIST) {
+        const int64_t slot = G.self ? G.g : p.n_groups + G.entry;   // contiguous slots: slot stride B * out_sb
+        out_row = static_cast<uint8_t*>(p.out) + 2 * ((slot * p.B + G.b) * p.out_sb + (int64_t)G.h * p.out_sh +
+                                                     (int64_t)(G.qt * kBlockQ + row) * p.out_ss + c_base * 16);
+      }
+      const bool cross = (MODE < ATTN_MODE_STORE) && !G.self;
       constexpr int NC = NC0;                 // trip count of the unrolled loop; the second half may own one chunk less
       const int nc_mine = dh ? NC_ALL - NC0 : NC0;
       // software pipeline over the 16-column chunks of O: the TMEM loads of chunk c+1 are in flight while chunk c is
@@ -648,7 +656,7 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
           tc_fence_before_sync();
           mbar_arrive(o_empty);
         }
-        if constexpr (MODE == ATTN_MODE_STORE) {
+        if constexpr (MODE >= ATTN_MODE_STORE) {
           uint32_t pk[8];
 #pragma unroll
           for (int j = 0; j < 8; ++j)
@@ -703,7 +711,7 @@ aas_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         }
         if (c + 1 < nc_mine) tmem_wait_ld();
       }
-      if constexpr (MODE != ATTN_MODE_STORE) {
+      if constexpr (MODE < ATTN_MODE_STORE) {
         if (G.self) tmem_wait_st();
         float r0, r1;   // cross: (dot, |Oc|^2) or (sq, 0); self: (|Os|^2, 0)
         if (G.self) {
@@ -977,6 +985,7 @@ static int launch_attn_mode(const AttnLaunch& a, int grid, const CUtensorMap& mq
   switch (a.mode) {
     case ATTN_MODE_COS: return launch_attn_one<D, kBf16, ATTN_MODE_COS>(a, grid, mq, mks, mvs, mk, mv, st);
     case ATTN_MODE_MSE: return launch_attn_one<D, kBf16, ATTN_MODE_MSE>(a, grid, mq, mks, mvs, mk, mv, st);
+    case ATTN_MODE_LIST: return launch_attn_one<D, kBf16, ATTN_MODE_LIST>(a, grid, mq, mks, mvs, mk, mv, st);
     default: return launch_attn_one<D, kBf16, ATTN_MODE_STORE>(a, grid, mq, mks, mvs, mk, mv, st);
   }
 }
@@ -1049,6 +1058,66 @@ static int prepare(AttnLaunch& a, float scale, const char* who) {
   const float sc = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
   a.p.scale_log2 = sc * 1.4426950408889634f;
   return DS_OK;
+}
+
+int check_group_operands(const ds_tensor5& q, const ds_tensor5& k_self, const ds_tensor5& v_self, const ds_tensor5& k,
+                         const ds_tensor5& v, const char* who) {
+  AttnLaunch a;
+  a.q = q;
+  a.ks = k_self;
+  a.vs = v_self;
+  a.k = k;
+  a.v = v;
+  return prepare(a, 0.f, who);
+}
+
+int launch_validate_groups(const int32_t* group_q, int64_t n_groups, const int32_t* kv_idx, int64_t n_entries,
+                           int64_t nq_images, int64_t nk_images, int32_t* bad, cudaStream_t st) {
+  const int64_t nv = n_groups > n_entries ? n_groups : n_entries;
+  validate_groups_kernel<<<(unsigned)((nv + 255) / 256), 256, 0, st>>>(group_q, n_groups, kv_idx, n_entries, nq_images,
+                                                                       nk_images, bad);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
+int launch_pairs_setup(const int32_t* pair_idx, int64_t n_pairs, int32_t* group_q, int32_t* group_off, int32_t* kv_idx,
+                       cudaStream_t st) {
+  pairs_setup_kernel<<<(unsigned)((2 * n_pairs + 1 + 255) / 256), 256, 0, st>>>(pair_idx, n_pairs, group_q, group_off, kv_idx);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
+int launch_triplets_setup(const int32_t* trip_idx, int64_t n_triplets, int32_t* group_q, int32_t* group_off,
+                          int32_t* kv_idx, cudaStream_t st) {
+  triplets_setup_kernel<<<(unsigned)((n_triplets + 1 + 255) / 256), 256, 0, st>>>(trip_idx, n_triplets, group_q, group_off,
+                                                                                kv_idx);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
+int attn_list_store(const ds_tensor5& q, const ds_tensor5& k_self, const ds_tensor5& v_self, const ds_tensor5& k,
+                    const ds_tensor5& v, const int32_t* group_q, const int32_t* group_off, int64_t n_groups,
+                    const int32_t* kv_idx, float scale, void* out, const char* who, cudaStream_t st) {
+  AttnLaunch a;
+  a.q = q;
+  a.ks = k_self;
+  a.vs = v_self;
+  a.k = k;
+  a.v = v;
+  int rc = prepare(a, scale, who);
+  if (rc != DS_OK) return rc;
+  a.p.group_q = group_q;
+  a.p.group_off = group_off;
+  a.p.kv_idx = kv_idx;
+  a.p.n_groups = (int)n_groups;
+  a.p.self_first = 1;
+  a.mode = ATTN_MODE_LIST;
+  a.p.part = nullptr;
+  a.p.out = out;
+  a.p.out_ss = q.size[4];
+  a.p.out_sh = q.size[3] * q.size[4];
+  a.p.out_sb = q.size[2] * a.p.out_sh;
+  return launch_attn(a, who, st);
 }
 
 }  // namespace ds

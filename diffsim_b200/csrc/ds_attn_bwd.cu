@@ -71,10 +71,10 @@ struct Params {
 // rows x D_PAD tile of a (B, H, S, D) tensor, as K1 loads it: NSUB swizzled sub-tiles of SUBW columns
 template <int D>
 __device__ __forceinline__ void load_tile(uint8_t* dst, const CUtensorMap* m, uint64_t* bar, int rows, int row0, int h,
-                                          int b) {
+                                          int b, int img = 0) {
   using C = Cfg<D>;
 #pragma unroll
-  for (int s = 0; s < C::NSUB; ++s) tma_load_5d(dst + s * rows * C::SUB_BYTES, m, bar, s * C::SUBW, row0, h, b, 0);
+  for (int s = 0; s < C::NSUB; ++s) tma_load_5d(dst + s * rows * C::SUB_BYTES, m, bar, s * C::SUBW, row0, h, b, img);
 }
 
 // D[tmem] (+)= A B^T over the head dim, both operands K-major tiles (K1's Q K^T form).  a_rows / b_rows: rows of the
@@ -447,8 +447,8 @@ constexpr int kRedBlocks = 256, kRedThreads = 256;
 
 // per-block (dot(X,Y), |X|^2, |Y|^2) over n contiguous elements, fixed split (deterministic)
 template <bool kBf16>
-__global__ void sim_partials_kernel(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2,
-                                    float* __restrict__ part) {
+__device__ __forceinline__ void sim_partials(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2,
+                                             float* __restrict__ part) {
   float d = 0.f, xx = 0.f, yy = 0.f;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n2; i += (int64_t)gridDim.x * blockDim.x) {
     const float2 a = unpack2<kBf16>(x[i]), c = unpack2<kBf16>(y[i]);
@@ -474,11 +474,16 @@ __global__ void sim_partials_kernel(const uint32_t* __restrict__ x, const uint32
   }
 }
 
+template <bool kBf16>
+__global__ void sim_partials_kernel(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2,
+                                    float* __restrict__ part) {
+  sim_partials<kBf16>(x, y, n2, part);
+}
+
 // coef = {gradient factor of X, of Y, k_X, k_Y}: dX = coef[0] (Y - k_X X), dY = coef[1] (X - k_Y Y) for the cosine
 // (torch's per-norm max(|.|, 1e-8) clamp: a clamped norm contributes no k term); dX = -dY = coef[0] (X - Y) for MSE
-__global__ void sim_coef_kernel(const float* __restrict__ part, int mode, double E, const float* __restrict__ d_dir,
-                                float* __restrict__ coef) {
-  if (threadIdx.x != 0) return;
+__device__ __forceinline__ void sim_coef(const float* __restrict__ part, int mode, double E, const float* __restrict__ d_dir,
+                                         float* __restrict__ coef) {
   const float g = *d_dir;
   if (mode == DS_SIM_MSE) {
     const float c = (float)(2.0 * (double)g / E);
@@ -502,10 +507,16 @@ __global__ void sim_coef_kernel(const float* __restrict__ part, int mode, double
   coef[3] = ny > 1e-8 ? (float)(cos * cx / cy) : 0.f;
 }
 
+__global__ void sim_coef_kernel(const float* __restrict__ part, int mode, double E, const float* __restrict__ d_dir,
+                                float* __restrict__ coef) {
+  if (threadIdx.x != 0) return;
+  sim_coef(part, mode, E, d_dir, coef);
+}
+
 // the O(1) factors of dX and dY, rounded to the input dtype (the dO operands of the two attention backwards)
 template <bool kBf16>
-__global__ void sim_factor_kernel(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2, int mode,
-                                  const float* __restrict__ coef, uint32_t* __restrict__ fx, uint32_t* __restrict__ fy) {
+__device__ __forceinline__ void sim_factor(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2, int mode,
+                                           const float* __restrict__ coef, uint32_t* __restrict__ fx, uint32_t* __restrict__ fy) {
   const float kx = coef[2], ky = coef[3];
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n2; i += (int64_t)gridDim.x * blockDim.x) {
     const float2 a = unpack2<kBf16>(x[i]), c = unpack2<kBf16>(y[i]);
@@ -515,6 +526,562 @@ __global__ void sim_factor_kernel(const uint32_t* __restrict__ x, const uint32_t
     } else {
       fx[i] = pack2<kBf16>(c.x - kx * a.x, c.y - kx * a.y);
       fy[i] = pack2<kBf16>(a.x - ky * c.x, a.y - ky * c.y);
+    }
+  }
+}
+
+template <bool kBf16>
+__global__ void sim_factor_kernel(const uint32_t* __restrict__ x, const uint32_t* __restrict__ y, int64_t n2, int mode,
+                                  const float* __restrict__ coef, uint32_t* __restrict__ fx, uint32_t* __restrict__ fy) {
+  sim_factor<kBf16>(x, y, n2, mode, coef, fx, fy);
+}
+
+// ---------------------------------------------------------------------------
+// grouped similarity gradient (ds_aas_groups_bwd): the backward of a whole ds_aas_groups work list
+// ---------------------------------------------------------------------------
+// Entry t of group g contributes two TERMS: tau = 2t (cross: Attn(Q_i, K_j, V_j), dO = fx_t) and tau = 2t + 1 (self:
+// Attn(Q_i, K_i, V_i), dO = fy_t).  Every gradient row receives its terms in ascending tau -- the order of one
+// ds_aas_dir_bwd call per entry -- with the same arithmetic, so the result is bitwise that of the per-entry loop.
+
+// entry -> group (binary search over group_off), and bad[0] = 1 unless group_off is 0 = off[0] <= ... <= off[G] = E
+__global__ void entry_group_kernel(const int32_t* __restrict__ group_off, int64_t n_groups, int64_t n_entries,
+                                   int32_t* __restrict__ entry_group, int32_t* __restrict__ bad) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i < n_groups && (group_off[i] > group_off[i + 1] || (i == 0 && group_off[0] != 0) ||
+                       (i == n_groups - 1 && group_off[n_groups] != n_entries)))
+    atomicExch(bad, 1);
+  if (i < n_entries) {
+    int64_t lo = 0, hi = n_groups - 1;   // last g with group_off[g] <= i
+    while (lo < hi) {
+      const int64_t mid = (lo + hi + 1) >> 1;
+      if (group_off[mid] <= i) lo = mid;
+      else hi = mid - 1;
+    }
+    entry_group[i] = (int32_t)lo;
+  }
+}
+
+// One contribution-list family: every term goes to one list, keyed by the gradient image it adds into; lists are ordered
+// by key and hold their terms in ascending tau.  Family 0: dQ, key = the query image.  Family 1: dK / dV, key = the kv
+// image of a cross term and the query image of a self term, offset by n_kbuf when dk_self is not dk (separate buffers).
+struct ListFamily {
+  int32_t* cnt;        // [n_keys] scratch
+  int32_t* n_lists;    // [1]
+  int32_t* list_key;   // [<= n_terms]
+  int32_t* list_off;   // [<= n_terms + 1]
+  int32_t* terms;      // [n_terms]
+  int64_t n_keys;
+};
+
+struct ListBuild {
+  const int32_t* group_q;
+  const int32_t* kv_idx;
+  const int32_t* entry_group;
+  const int32_t* bad;
+  int64_t n_terms;
+  int n_kbuf;   // dK / dV self-term key offset (0: dk_self is dk)
+  ListFamily fam[2];
+};
+
+__device__ __forceinline__ int term_key(const ListBuild& b, int family, int64_t tau) {
+  const int64_t t = tau >> 1;
+  const bool self = tau & 1;
+  const int qi = b.group_q[b.entry_group[t]];
+  if (family == 0) return qi;
+  return self ? b.n_kbuf + qi : b.kv_idx[t];
+}
+
+// exclusive block scan of two counters over kListThreads threads; returns the block totals
+constexpr int kListThreads = 1024;
+__device__ __forceinline__ int2 block_scan2(int a, int c, int& ea, int& ec, int2* s_warp) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  int ia = a, ic = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int ua = __shfl_up_sync(0xffffffffu, ia, o), uc = __shfl_up_sync(0xffffffffu, ic, o);
+    if (lane >= o) {
+      ia += ua;
+      ic += uc;
+    }
+  }
+  if (lane == 31) s_warp[w] = make_int2(ia, ic);
+  __syncthreads();
+  if (w == 0) {
+    int2 v = s_warp[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int ua = __shfl_up_sync(0xffffffffu, v.x, o), uc = __shfl_up_sync(0xffffffffu, v.y, o);
+      if (lane >= o) {
+        v.x += ua;
+        v.y += uc;
+      }
+    }
+    s_warp[lane] = v;   // inclusive warp prefixes
+  }
+  __syncthreads();
+  const int2 before = w > 0 ? s_warp[w - 1] : make_int2(0, 0);
+  ea = before.x + ia - a;
+  ec = before.y + ic - c;
+  const int2 tot = s_warp[31];
+  __syncthreads();
+  return tot;
+}
+
+// block f builds family f: a stable counting sort of the terms by key (deterministic: integer counts only)
+__global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBuild b) {
+  const int f = blockIdx.x;
+  const ListFamily& L = b.fam[f];
+  __shared__ int2 s_warp[32];
+  __shared__ int s_key[kListThreads];
+  if (*b.bad) {   // an index is out of range: no lists, no gradient work (the gradients become NaN)
+    if (threadIdx.x == 0) *L.n_lists = 0;
+    return;
+  }
+  for (int64_t k = threadIdx.x; k < L.n_keys; k += kListThreads) L.cnt[k] = 0;
+  __syncthreads();
+  for (int64_t tau = threadIdx.x; tau < b.n_terms; tau += kListThreads) atomicAdd(&L.cnt[term_key(b, f, tau)], 1);
+  __syncthreads();
+  int n_lists = 0, n_seen = 0;   // running totals over the key chunks
+  for (int64_t k0 = 0; k0 < L.n_keys; k0 += kListThreads) {
+    const int64_t k = k0 + threadIdx.x;
+    const int c = k < L.n_keys ? L.cnt[k] : 0;
+    int el, ec;
+    const int2 tot = block_scan2(c > 0 ? 1 : 0, c, el, ec, s_warp);
+    if (c > 0) {
+      L.list_key[n_lists + el] = (int32_t)k;
+      L.list_off[n_lists + el] = n_seen + ec;
+    }
+    if (k < L.n_keys) L.cnt[k] = n_seen + ec;   // first slot of key k's terms
+    n_lists += tot.x;
+    n_seen += tot.y;
+  }
+  if (threadIdx.x == 0) {
+    *L.n_lists = n_lists;
+    L.list_off[n_lists] = n_seen;
+  }
+  __syncthreads();
+  for (int64_t t0 = 0; t0 < b.n_terms; t0 += kListThreads) {
+    const int64_t tau = t0 + threadIdx.x;
+    const int key = tau < b.n_terms ? term_key(b, f, tau) : -1;
+    s_key[threadIdx.x] = key;
+    __syncthreads();
+    if (tau < b.n_terms) {
+      int r = 0;   // earlier terms of this chunk with the same key
+      for (int j = 0; j < (int)threadIdx.x; ++j) r += s_key[j] == key;
+      L.terms[L.cnt[key] + r] = (int32_t)tau;
+    }
+    __syncthreads();
+    if (tau < b.n_terms) atomicAdd(&L.cnt[key], 1);
+    __syncthreads();
+  }
+}
+
+// per entry: (dot, |X|^2, |Y|^2) partials, coefficients and factors exactly as for one ds_aas_dir_bwd call
+template <bool kBf16>
+__global__ void sim_partials_list_kernel(const uint32_t* __restrict__ o, int64_t n2, int n_groups, int64_t n_entries,
+                                         const int32_t* __restrict__ entry_group, float* __restrict__ part) {
+  for (int64_t t = blockIdx.y; t < n_entries; t += gridDim.y) {
+    sim_partials<kBf16>(o + (n_groups + t) * n2, o + entry_group[t] * n2, n2, part + t * (kRedBlocks * 3));
+    __syncthreads();
+  }
+}
+
+__global__ void sim_coef_list_kernel(const float* __restrict__ part, int64_t n_entries, int mode, double E,
+                                     const float* __restrict__ d_dir, float* __restrict__ coef) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t < n_entries) sim_coef(part + t * (kRedBlocks * 3), mode, E, d_dir + t, coef + 4 * t);
+}
+
+template <bool kBf16>
+__global__ void sim_factor_list_kernel(const uint32_t* __restrict__ o, int64_t n2, int n_groups, int64_t n_entries,
+                                       const int32_t* __restrict__ entry_group, int mode, const float* __restrict__ coef,
+                                       uint32_t* __restrict__ f) {
+  for (int64_t t = blockIdx.y; t < n_entries; t += gridDim.y)
+    sim_factor<kBf16>(o + (n_groups + t) * n2, o + entry_group[t] * n2, n2, mode, coef + 4 * t, f + 2 * t * n2,
+                      f + (2 * t + 1) * n2);
+}
+
+struct GradT {   // an fp32 (N, B, H, S, D) gradient
+  float* ptr;
+  int64_t sn, sb, sh, ss;
+};
+
+struct ListParams {
+  int B, H, Sq, Skv, n_qt, n_kt;
+  float scale, scale_log2;
+  int n_groups;
+  const int32_t* group_q;
+  const int32_t* kv_idx;
+  const int32_t* entry_group;
+  const int32_t* n_lists;    // device count of the family's lists (the grid covers an upper bound)
+  const int32_t* list_key;
+  const int32_t* list_off;
+  const int32_t* terms;
+  int n_kbuf;                // dK / dV keys >= n_kbuf address (dk_self, dv_self) at image key - n_kbuf
+  const void* o;             // Y_g at slot g, X_t at slot n_groups + t: contiguous (B, H, Sq, D) images
+  const void* f;             // fx_t at slot 2t, fy_t at slot 2t + 1 (= tau)
+  int64_t img;               // B H Sq D: slot stride of o and f
+  float* lse;                // [tau][B H][n_qt 128]
+  float* delta;
+  const float* coef;         // [t][4]: factor of the cross term at 4t, of the self term at 4t + 1
+  GradT dq, dk, dv, dks, dvs;
+};
+
+// attn_bwd_dq_kernel over a list: one CTA per (query image, b, h, 128-row q tile), the steps of that kernel once per
+// term, dQ drained (x the term's coefficient) into the fp32 rows before the next term
+template <int D, bool kBf16>
+__global__ void __launch_bounds__(kThreads, 1)
+attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
+                        const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
+                        const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
+                        const ListParams p) {
+  using C = Cfg<D>;
+  const int per_list = p.B * p.H * p.n_qt;
+  const int li = blockIdx.x / per_list;
+  if (li >= *p.n_lists) return;
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint8_t* sQ = smem;
+  uint8_t* sDO = sQ + C::TILE_BYTES;
+  uint8_t* sK = sDO + C::TILE_BYTES;
+  uint8_t* sV = sK + C::TILE_BYTES;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + C::TILE_BYTES);
+  uint64_t* q_bar = bars;
+  uint64_t* kv_bar = bars + 1;
+  uint64_t* mma_bar = bars + 2;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
+
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const int rest = blockIdx.x - li * per_list;
+  const int bh = rest / p.n_qt, qt = rest - bh * p.n_qt;
+  const int b = bh / p.H, h = bh - b * p.H;
+  const int grow = qt * kTile + tid;
+  const bool row_ok = grow < p.Sq;
+  const int qi = p.list_key[li];
+  const int i0 = p.list_off[li], i1 = p.list_off[li + 1];
+
+  if (tid == 0) {
+    mbar_init(q_bar, 1);
+    mbar_init(kv_bar, 1);
+    mbar_init(mma_bar, 1);
+    fence_mbar_init();
+    tma_prefetch_desc(&map_q);
+    tma_prefetch_desc(&map_k);
+    tma_prefetch_desc(&map_v);
+    tma_prefetch_desc(&map_ks);
+    tma_prefetch_desc(&map_vs);
+    tma_prefetch_desc(&map_do);
+  }
+  if (warp == 0) {
+    tmem_alloc(tmem_slot, 512);
+    tmem_relinquish();
+  }
+  sync_all_tc();
+  const uint32_t tmem = *tmem_slot;
+  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
+  constexpr uint32_t kS = 0, kDP = 128, kDQ = 256;
+  const uint32_t fmt = kBf16 ? 1u : 0u;
+  const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, kTile, 0, 0);
+  const uint32_t idesc_dq = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
+  const float sl2 = p.scale_log2;
+  const int64_t row_off = ((int64_t)b * p.H + h) * p.Sq * D + (int64_t)grow * D;   // in a contiguous (B, H, Sq, D) image
+  float* dq_row = p.dq.ptr + qi * p.dq.sn + b * p.dq.sb + h * p.dq.sh + (int64_t)grow * p.dq.ss;
+  uint32_t q_ph = 0, kv_ph = 0, mma_ph = 0;
+
+  for (int i = i0; i < i1; ++i) {
+    const int tau = p.terms[i], t = tau >> 1;
+    const bool self = tau & 1;
+    const int kv_img = self ? qi : p.kv_idx[t];
+    const CUtensorMap* mk = self ? &map_ks : &map_k;
+    const CUtensorMap* mv = self ? &map_vs : &map_v;
+    const int64_t o_slot = self ? p.entry_group[t] : p.n_groups + t;
+    if (tid == 0) {
+      mbar_arrive_expect_tx(q_bar, 2 * C::TILE_BYTES);
+      load_tile<D>(sQ, &map_q, q_bar, kTile, qt * kTile, h, b, qi);
+      load_tile<D>(sDO, &map_do, q_bar, kTile, qt * kTile, h, b, tau);
+    }
+    __syncwarp();
+    float delta = 0.f;
+    if (row_ok)
+      delta = row_dot<kBf16>(static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
+                             static_cast<const uint16_t*>(p.f) + tau * p.img + row_off, D);
+    mbar_wait(q_bar, q_ph);
+    q_ph ^= 1;
+
+    // ---- pass 1: log-sum-exp of every row (log2 domain)
+    float m = -INFINITY, l = 0.f;
+    for (int kt = 0; kt < p.n_kt; ++kt) {
+      if (tid == 0) {
+        mbar_arrive_expect_tx(kv_bar, C::TILE_BYTES);
+        load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
+      }
+      __syncwarp();
+      mbar_wait(kv_bar, kv_ph);
+      kv_ph ^= 1;
+      if (tid == 0) {
+        tc_fence_after_sync();
+        mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+      const int nv = p.Skv - kt * kTile;
+#pragma unroll 1
+      for (int c = 0; c < kTile / 32; ++c) {
+        uint32_t v[32];
+        tmem_ld_x32(lane_t + kS + c * 32, v);
+        tmem_wait_ld();
+        float mx = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          if (c * 32 + j >= nv) v[j] = 0xff800000u;
+          mx = fmaxf(mx, __uint_as_float(v[j]));
+        }
+        if (mx == -INFINITY) continue;
+        const float mn = fmaxf(m, mx);
+        float s = 0.f;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) s += fast_exp2((__uint_as_float(v[j]) - mn) * sl2);
+        l = l * fast_exp2((m - mn) * sl2) + s;
+        m = mn;
+      }
+      sync_all_tc();
+    }
+    const float lse2 = m * sl2 + __log2f(l);
+    {
+      const size_t k = ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
+      p.lse[k] = lse2;
+      p.delta[k] = delta;
+    }
+
+    // ---- pass 2: dQ
+    for (int kt = 0; kt < p.n_kt; ++kt) {
+      if (tid == 0) {
+        mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
+        load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
+        load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
+      }
+      __syncwarp();
+      mbar_wait(kv_bar, kv_ph);
+      kv_ph ^= 1;
+      if (tid == 0) {
+        tc_fence_after_sync();
+        mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);
+        mma_ss_kmajor<D>(tmem + kDP, sDO, kTile, sV, kTile, idesc_s);
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+      const int nv = p.Skv - kt * kTile;
+#pragma unroll 1
+      for (int c = 0; c < kTile / 32; ++c) {
+        uint32_t s[32], dp[32], pk[16];
+        tmem_ld_x32(lane_t + kS + c * 32, s);
+        tmem_ld_x32(lane_t + kDP + c * 32, dp);
+        tmem_wait_ld();
+#pragma unroll
+        for (int j = 0; j < 32; j += 2) {
+          float ds[2];
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const float pr = (c * 32 + j + e < nv) ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -lse2)) : 0.f;
+            ds[e] = pr * (__uint_as_float(dp[j + e]) - delta);
+          }
+          pk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
+        }
+        tmem_st_x16(lane_t + kS + c * 32, pk);
+      }
+      tmem_wait_st();
+      sync_all_tc();
+      if (tid == 0) {
+        mma_ts_mnmajor<D>(tmem + kDQ, tmem + kS, sK, kTile, idesc_dq, kt > 0);
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+    }
+
+    const float fq = p.scale * p.coef[4 * t + (self ? 1 : 0)];
+    add_row_out<D>(lane_t + kDQ, fq, dq_row, row_ok);
+    sync_all_tc();   // dQ read out (and Q / dO free) before the next term
+  }
+  if (warp == 0) tmem_dealloc(tmem, 512);
+}
+
+// attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), the steps of that kernel once per term
+template <int D, bool kBf16>
+__global__ void __launch_bounds__(kThreads, 1)
+attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
+                         const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
+                         const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
+                         const ListParams p) {
+  using C = Cfg<D>;
+  constexpr int BQ = C::BQ;
+  const int per_list = p.B * p.H * p.n_kt;
+  const int li = blockIdx.x / per_list;
+  if (li >= *p.n_lists) return;
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint8_t* sK = smem;
+  uint8_t* sV = sK + C::TILE_BYTES;
+  uint8_t* sQ = sV + C::TILE_BYTES;
+  uint8_t* sDO = sQ + C::QB_BYTES;
+  float* sLse = reinterpret_cast<float*>(sDO + C::QB_BYTES);
+  float* sDelta = sLse + BQ;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sDelta + BQ);
+  uint64_t* kv_bar = bars;
+  uint64_t* q_bar = bars + 1;
+  uint64_t* mma_bar = bars + 2;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
+
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const int rest = blockIdx.x - li * per_list;
+  const int bh = rest / p.n_kt, kt = rest - bh * p.n_kt;
+  const int b = bh / p.H, h = bh - b * p.H;
+  const int krow = kt * kTile + tid;
+  const bool row_ok = krow < p.Skv;
+  int img = p.list_key[li];
+  GradT gk = p.dk, gv = p.dv;
+  if (img >= p.n_kbuf && p.n_kbuf > 0) {
+    img -= p.n_kbuf;
+    gk = p.dks;
+    gv = p.dvs;
+  }
+  const int i0 = p.list_off[li], i1 = p.list_off[li + 1];
+
+  if (tid == 0) {
+    mbar_init(kv_bar, 1);
+    mbar_init(q_bar, 1);
+    mbar_init(mma_bar, 1);
+    fence_mbar_init();
+    tma_prefetch_desc(&map_q);
+    tma_prefetch_desc(&map_k);
+    tma_prefetch_desc(&map_v);
+    tma_prefetch_desc(&map_ks);
+    tma_prefetch_desc(&map_vs);
+    tma_prefetch_desc(&map_do);
+  }
+  if (warp == 0) {
+    tmem_alloc(tmem_slot, 512);
+    tmem_relinquish();
+  }
+  sync_all_tc();
+  const uint32_t tmem = *tmem_slot;
+  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
+  constexpr uint32_t kST = 0, kDPT = BQ, kDV = 2 * BQ, kDK = 2 * BQ + C::D_PAD;
+  const uint32_t fmt = kBf16 ? 1u : 0u;
+  const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, BQ, 0, 0);
+  const uint32_t idesc_o = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
+  const float sl2 = p.scale_log2;
+  const int n_qb = (p.Sq + BQ - 1) / BQ;
+  float* dv_row = gv.ptr + img * gv.sn + b * gv.sb + h * gv.sh + (int64_t)krow * gv.ss;
+  float* dk_row = gk.ptr + img * gk.sn + b * gk.sb + h * gk.sh + (int64_t)krow * gk.ss;
+  uint32_t kv_ph = 0, q_ph = 0, mma_ph = 0;
+
+  for (int i = i0; i < i1; ++i) {
+    const int tau = p.terms[i], t = tau >> 1;
+    const bool self = tau & 1;
+    const int qi = p.group_q[p.entry_group[t]];
+    if (tid == 0) {
+      mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
+      load_tile<D>(sK, self ? &map_ks : &map_k, kv_bar, kTile, kt * kTile, h, b, img);
+      load_tile<D>(sV, self ? &map_vs : &map_v, kv_bar, kTile, kt * kTile, h, b, img);
+    }
+    __syncwarp();
+    const float* lse_bh = p.lse + ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile);
+    const float* delta_bh = p.delta + ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile);
+    mbar_wait(kv_bar, kv_ph);
+    kv_ph ^= 1;
+    for (int qb = 0; qb < n_qb; ++qb) {
+      if (tid == 0) {
+        mbar_arrive_expect_tx(q_bar, 2 * C::QB_BYTES);
+        load_tile<D>(sQ, &map_q, q_bar, BQ, qb * BQ, h, b, qi);
+        load_tile<D>(sDO, &map_do, q_bar, BQ, qb * BQ, h, b, tau);
+      }
+      __syncwarp();
+      if (tid < BQ) {
+        sLse[tid] = lse_bh[qb * BQ + tid];
+        sDelta[tid] = delta_bh[qb * BQ + tid];
+      }
+      mbar_wait(q_bar, q_ph);
+      q_ph ^= 1;
+      if (tid == 0) {
+        tc_fence_after_sync();
+        mma_ss_kmajor<D>(tmem + kST, sK, kTile, sQ, BQ, idesc_s);
+        mma_ss_kmajor<D>(tmem + kDPT, sV, kTile, sDO, BQ, idesc_s);
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      __syncthreads();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+      const int nq = p.Sq - qb * BQ;
+#pragma unroll 1
+      for (int c = 0; c < BQ / 32; ++c) {
+        uint32_t s[32], dp[32], pk[16], dk[16];
+        tmem_ld_x32(lane_t + kST + c * 32, s);
+        tmem_ld_x32(lane_t + kDPT + c * 32, dp);
+        tmem_wait_ld();
+#pragma unroll
+        for (int j = 0; j < 32; j += 2) {
+          float pr[2], ds[2];
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const int q = c * 32 + j + e;
+            pr[e] = q < nq ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -sLse[q])) : 0.f;
+            ds[e] = pr[e] * (__uint_as_float(dp[j + e]) - sDelta[q]);
+          }
+          pk[j >> 1] = pack2<kBf16>(pr[0], pr[1]);
+          dk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
+        }
+        tmem_st_x16(lane_t + kST + c * 32, pk);
+        tmem_st_x16(lane_t + kDPT + c * 32, dk);
+      }
+      tmem_wait_st();
+      sync_all_tc();
+      if (tid == 0) {
+        mma_ts_mnmajor<D>(tmem + kDV, tmem + kST, sDO, BQ, idesc_o, qb > 0);
+        mma_ts_mnmajor<D>(tmem + kDK, tmem + kDPT, sQ, BQ, idesc_o, qb > 0);
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+      __syncthreads();
+    }
+    const float g = p.coef[4 * t + (self ? 1 : 0)];
+    add_row_out<D>(lane_t + kDV, g, dv_row, row_ok);
+    add_row_out<D>(lane_t + kDK, g * p.scale, dk_row, row_ok);
+    sync_all_tc();   // dK / dV read out (and K / V free) before the next term
+  }
+  if (warp == 0) tmem_dealloc(tmem, 512);
+}
+
+// every element of the five gradients := NaN when bad[0] is set (an image index of the list was out of range)
+struct NanFill {
+  float* ptr[5];
+  int64_t size[5][5];
+  int64_t stride[5][5];
+};
+
+__global__ void nan_fill_kernel(const NanFill f, const int32_t* __restrict__ bad) {
+  if (!*bad) return;
+  for (int k = 0; k < 5; ++k) {
+    const int64_t* sz = f.size[k];
+    const int64_t n = sz[0] * sz[1] * sz[2] * sz[3] * sz[4];
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+      int64_t r = i, off = 0;
+      for (int d = 4; d >= 0; --d) {
+        off += (r % sz[d]) * f.stride[k][d];
+        r /= sz[d];
+      }
+      f.ptr[k][off] = __int_as_float(0x7fc00000);
     }
   }
 }
@@ -620,6 +1187,114 @@ static ds_tensor4 contiguous_like(const ds_tensor4& t, void* ptr) {
   return r;
 }
 
+// ---- grouped similarity gradient: host side
+
+static int check_grad5(const ds_tensor5& g, const ds_tensor5& like, const char* who, const char* name) {
+  if (!g.ptr) return fail(DS_ERR_INVALID, "%s: %s: null pointer", who, name);
+  if (g.dtype != DS_F32) return fail(DS_ERR_INVALID, "%s: %s: gradients are float32", who, name);
+  for (int i = 0; i < 5; ++i)
+    if (g.size[i] != like.size[i]) return fail(DS_ERR_INVALID, "%s: %s: shape must match its input", who, name);
+  if (g.stride[4] != 1) return fail(DS_ERR_INVALID, "%s: %s: innermost stride must be 1", who, name);
+  if ((uintptr_t)g.ptr & 3) return fail(DS_ERR_INVALID, "%s: %s: base pointer must be 4-byte aligned", who, name);
+  for (int i = 0; i < 4; ++i)
+    if (g.size[i] > 1 && g.stride[i] <= 0) return fail(DS_ERR_INVALID, "%s: %s: stride[%d] must be positive", who, name, i);
+  return DS_OK;
+}
+
+static bool same_tensor(const ds_tensor5& a, const ds_tensor5& b) {
+  if (a.ptr != b.ptr || a.dtype != b.dtype) return false;
+  for (int i = 0; i < 5; ++i)
+    if (a.size[i] != b.size[i] || (a.size[i] > 1 && a.stride[i] != b.stride[i])) return false;
+  return true;
+}
+
+// the address ranges of two fp32 tensors with positive strides intersect
+static bool extents_meet(const ds_tensor5& a, const ds_tensor5& b) {
+  auto end = [](const ds_tensor5& t) {
+    int64_t e = 1;
+    for (int i = 0; i < 5; ++i) e += (t.size[i] - 1) * t.stride[i];
+    return static_cast<const char*>(t.ptr) + 4 * e;
+  };
+  const char* a0 = static_cast<const char*>(a.ptr);
+  const char* b0 = static_cast<const char*>(b.ptr);
+  return a0 < end(b) && b0 < end(a);
+}
+
+// workspace layout of ds_aas_groups_bwd (the size query runs it on a dummy base)
+struct GroupsBwdWs {
+  void* o;                 // (n_groups + n_entries) attention outputs, 16-bit
+  void* f;                 // 2 n_entries dO factors, 16-bit
+  float* part;             // [n_entries][kRedBlocks][3]
+  float* coef;             // [n_entries][4]
+  float* lse;              // [2 n_entries][B H][n_qt 128]
+  float* delta;
+  int32_t* entry_group;    // [n_entries]
+  int32_t* bad;
+  ListFamily fam[2];
+};
+
+static bool groups_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor5& k, int64_t G, int64_t E,
+                              GroupsBwdWs* L) {
+  const int64_t img = q.size[1] * q.size[2] * q.size[3] * q.size[4];
+  const int64_t n_qt = (q.size[3] + kTile - 1) / kTile;
+  const size_t stats = (size_t)(2 * E) * q.size[1] * q.size[2] * n_qt * kTile * sizeof(float);
+  const int64_t nt = 2 * E;
+  L->o = w.take((size_t)(G + E) * img * 2);
+  L->f = w.take((size_t)nt * img * 2);
+  L->part = static_cast<float*>(w.take((size_t)E * kRedBlocks * 3 * sizeof(float)));
+  L->coef = static_cast<float*>(w.take((size_t)E * 4 * sizeof(float)));
+  L->lse = static_cast<float*>(w.take(stats));
+  L->delta = static_cast<float*>(w.take(stats));
+  L->entry_group = static_cast<int32_t*>(w.take((size_t)E * 4));
+  L->bad = static_cast<int32_t*>(w.take(4));
+  bool ok = L->o && L->f && L->part && L->coef && L->lse && L->delta && L->entry_group && L->bad;
+  const int64_t n_keys[2] = {q.size[0], k.size[0] + q.size[0]};
+  for (int i = 0; i < 2; ++i) {
+    ListFamily& F = L->fam[i];
+    F.n_keys = n_keys[i];
+    F.cnt = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
+    F.n_lists = static_cast<int32_t*>(w.take(4));
+    F.list_key = static_cast<int32_t*>(w.take((size_t)nt * 4));
+    F.list_off = static_cast<int32_t*>(w.take((size_t)(nt + 1) * 4));
+    F.terms = static_cast<int32_t*>(w.take((size_t)nt * 4));
+    ok = ok && F.cnt && F.n_lists && F.list_key && F.list_off && F.terms;
+  }
+  return ok;
+}
+
+static GradT grad_t(const ds_tensor5& g) {
+  return GradT{static_cast<float*>(g.ptr), g.stride[0], g.stride[1], g.stride[2], g.stride[3]};
+}
+
+template <int D, bool kBf16>
+static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
+                               const ds_tensor5& v, const ds_tensor5& F, ListParams p, int64_t grid_q, int64_t grid_kv,
+                               const GroupsBwdWs& L, cudaStream_t st) {
+  using C = Cfg<D>;
+  CUtensorMap mq, mk, mv, mks, mvs, mdo, mqb, mdob;
+  int rc;
+  if ((rc = make_map(&mq, q, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mk, k, C::SUBW, kTile)) != DS_OK ||
+      (rc = make_map(&mv, v, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mks, ks, C::SUBW, kTile)) != DS_OK ||
+      (rc = make_map(&mvs, vs, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mdo, F, C::SUBW, kTile)) != DS_OK ||
+      (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, F, C::SUBW, C::BQ)) != DS_OK)
+    return rc;
+  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_list_kernel<D, kBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::DQ_SMEM));
+  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dkv_list_kernel<D, kBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::DKV_SMEM));
+  p.n_lists = L.fam[0].n_lists;
+  p.list_key = L.fam[0].list_key;
+  p.list_off = L.fam[0].list_off;
+  p.terms = L.fam[0].terms;
+  attn_bwd_dq_list_kernel<D, kBf16><<<(unsigned)grid_q, kThreads, C::DQ_SMEM, st>>>(mq, mk, mv, mks, mvs, mdo, p);
+  DS_CUDA_TRY(cudaGetLastError());
+  p.n_lists = L.fam[1].n_lists;
+  p.list_key = L.fam[1].list_key;
+  p.list_off = L.fam[1].list_off;
+  p.terms = L.fam[1].terms;
+  attn_bwd_dkv_list_kernel<D, kBf16><<<(unsigned)grid_kv, kThreads, C::DKV_SMEM, st>>>(mqb, mk, mv, mks, mvs, mdob, p);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
 }  // namespace bwd
 }  // namespace ds
 
@@ -712,6 +1387,266 @@ int ds_aas_dir_bwd(ds_tensor4 q_i, ds_tensor4 k_i, ds_tensor4 v_i, ds_tensor4 k_
   if ((rc = launch_bwd(cross, who, st)) != DS_OK) return rc;
   BwdArgs self{q_i, k_i, v_i, Y, contiguous_like(q_i, fy), dq_i, dk_i, dv_i, scale, coef + 1, lse, delta};
   return launch_bwd(self, who, st);
+}
+
+}  // extern "C"
+
+namespace ds {
+namespace bwd {
+
+__global__ void pairs_ddir_kernel(const float* __restrict__ d_scores, int64_t n, float* __restrict__ d_dir) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i < n) d_dir[2 * i] = d_dir[2 * i + 1] = d_scores[i] * 0.5f;   // score = (dir[2p] + dir[2p + 1]) / 2
+}
+
+// entries 4t .. 4t + 3 = ref->left, ref->right, left->ref, right->ref; ab = (dir[4t] + dir[4t + 2]) / 2, ac likewise
+__global__ void triplets_ddir_kernel(const float* __restrict__ d_ab, const float* __restrict__ d_ac, int64_t n,
+                                     float* __restrict__ d_dir) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i < n) {
+    d_dir[4 * i] = d_dir[4 * i + 2] = d_ab[i] * 0.5f;
+    d_dir[4 * i + 1] = d_dir[4 * i + 3] = d_ac[i] * 0.5f;
+  }
+}
+
+// every argument of a grouped backward except the work list itself; *aliased: dk_self is dk and dv_self is dv
+static int groups_bwd_check(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
+                            const ds_tensor5& v, int mode, const float* d, const ds_tensor5& dq, const ds_tensor5& dks,
+                            const ds_tensor5& dvs, const ds_tensor5& dk, const ds_tensor5& dv, const char* who,
+                            bool* aliased) {
+  int rc;
+  if (mode != DS_SIM_COSINE && mode != DS_SIM_MSE) return fail(DS_ERR_INVALID, "%s: bad mode %d", who, mode);
+  if (!d) return fail(DS_ERR_INVALID, "%s: score gradient: null pointer", who);
+  if ((rc = check_group_operands(q, ks, vs, k, v, who)) != DS_OK) return rc;
+  if ((rc = check_grad5(dq, q, who, "dq")) != DS_OK || (rc = check_grad5(dks, ks, who, "dk_self")) != DS_OK ||
+      (rc = check_grad5(dvs, vs, who, "dv_self")) != DS_OK || (rc = check_grad5(dk, k, who, "dk")) != DS_OK ||
+      (rc = check_grad5(dv, v, who, "dv")) != DS_OK)
+    return rc;
+  const bool ak = same_tensor(dks, dk), av = same_tensor(dvs, dv);
+  if (ak != av) return fail(DS_ERR_INVALID, "%s: dk_self / dk and dv_self / dv must both be the same tensor or both be separate", who);
+  if (!ak && (extents_meet(dks, dk) || extents_meet(dvs, dv)))
+    return fail(DS_ERR_INVALID, "%s: dk_self / dk (dv_self / dv) must be the same tensor or not overlap", who);
+  *aliased = ak;
+  return DS_OK;
+}
+
+// the device work of ds_aas_groups_bwd on a checked call whose work list (and d_dir) is on the device
+static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
+                             const ds_tensor5& v, const int32_t* group_q, const int32_t* group_off, int64_t G,
+                             const int32_t* kv_idx, int64_t E, float scale, int mode, const float* d_dir,
+                             const ds_tensor5& dq, const ds_tensor5& dks, const ds_tensor5& dvs, const ds_tensor5& dk,
+                             const ds_tensor5& dv, bool aliased, const GroupsBwdWs& L, const char* who, cudaStream_t st) {
+  int rc;
+  const int D = (int)q.size[4];
+  const int64_t img = q.size[1] * q.size[2] * q.size[3] * D, n2 = img / 2;
+  const bool bf = q.dtype == DS_BF16;
+  ListParams p;
+  p.B = (int)q.size[1];
+  p.H = (int)q.size[2];
+  p.Sq = (int)q.size[3];
+  p.Skv = (int)k.size[3];
+  p.n_qt = (p.Sq + kTile - 1) / kTile;
+  p.n_kt = (p.Skv + kTile - 1) / kTile;
+  p.scale = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
+  p.scale_log2 = p.scale * 1.4426950408889634f;
+  const int64_t bh = (int64_t)p.B * p.H;
+  const int64_t nl_q = std::min<int64_t>(q.size[0], G);
+  const int64_t nl_kv = aliased ? std::min<int64_t>(k.size[0], G + E) : nl_q + std::min<int64_t>(k.size[0], E);
+  const int64_t grid_q = nl_q * bh * p.n_qt, grid_kv = nl_kv * bh * p.n_kt;
+  if (grid_q >= INT32_MAX || grid_kv >= INT32_MAX) return fail(DS_ERR_INVALID, "%s: too many tiles: split the work list", who);
+
+  DS_CUDA_TRY(cudaMemsetAsync(L.bad, 0, sizeof(int32_t), st));
+  if ((rc = launch_validate_groups(group_q, G, kv_idx, E, q.size[0], k.size[0], L.bad, st)) != DS_OK) return rc;
+  entry_group_kernel<<<(unsigned)((std::max(G, E) + 255) / 256), 256, 0, st>>>(group_off, G, E, L.entry_group, L.bad);
+  DS_CUDA_TRY(cudaGetLastError());
+  ListBuild lb;
+  lb.group_q = group_q;
+  lb.kv_idx = kv_idx;
+  lb.entry_group = L.entry_group;
+  lb.bad = L.bad;
+  lb.n_terms = 2 * E;
+  lb.n_kbuf = aliased ? 0 : (int)k.size[0];
+  lb.fam[0] = L.fam[0];
+  lb.fam[1] = L.fam[1];
+  lb.fam[1].n_keys = aliased ? k.size[0] : k.size[0] + q.size[0];
+  build_lists_kernel<<<2, kListThreads, 0, st>>>(lb);
+  DS_CUDA_TRY(cudaGetLastError());
+  // X_t and Y_g, rounded to the input dtype as ds_attn_fwd rounds them
+  if ((rc = attn_list_store(q, ks, vs, k, v, group_q, group_off, G, kv_idx, scale, L.o, who, st)) != DS_OK) return rc;
+  const uint32_t* ou = static_cast<const uint32_t*>(L.o);
+  const unsigned ey = (unsigned)std::min<int64_t>(E, 65535);
+  if (bf) sim_partials_list_kernel<true><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)G, E, L.entry_group, L.part);
+  else sim_partials_list_kernel<false><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)G, E, L.entry_group, L.part);
+  DS_CUDA_TRY(cudaGetLastError());
+  sim_coef_list_kernel<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(L.part, E, mode, (double)img, d_dir, L.coef);
+  DS_CUDA_TRY(cudaGetLastError());
+  const unsigned fb = (unsigned)std::min<int64_t>((n2 + 255) / 256, 4 * (int64_t)sm_count());
+  uint32_t* fu = static_cast<uint32_t*>(L.f);
+  if (bf) sim_factor_list_kernel<true><<<dim3(fb, ey), 256, 0, st>>>(ou, n2, (int)G, E, L.entry_group, mode, L.coef, fu);
+  else sim_factor_list_kernel<false><<<dim3(fb, ey), 256, 0, st>>>(ou, n2, (int)G, E, L.entry_group, mode, L.coef, fu);
+  DS_CUDA_TRY(cudaGetLastError());
+
+  p.n_groups = (int)G;
+  p.group_q = group_q;
+  p.kv_idx = kv_idx;
+  p.entry_group = L.entry_group;
+  p.n_kbuf = lb.n_kbuf;
+  p.o = L.o;
+  p.f = L.f;
+  p.img = img;
+  p.lse = L.lse;
+  p.delta = L.delta;
+  p.coef = L.coef;
+  p.dq = grad_t(dq);
+  p.dk = grad_t(dk);
+  p.dv = grad_t(dv);
+  p.dks = grad_t(dks);
+  p.dvs = grad_t(dvs);
+  ds_tensor5 F = q;   // the factors as a (2 n_entries, B, H, Sq, D) contiguous stack
+  F.ptr = L.f;
+  F.size[0] = 2 * E;
+  F.stride[4] = 1;
+  F.stride[3] = D;
+  F.stride[2] = q.size[3] * D;
+  F.stride[1] = q.size[2] * F.stride[2];
+  F.stride[0] = q.size[1] * F.stride[1];
+  rc = with_head_dim(D, who, [&](auto d) {
+    return with_dtype(q.dtype, [&](auto b) {
+      return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value>(q, ks, vs, k, v, F, p, grid_q, grid_kv, L, st);
+    });
+  });
+  if (rc != DS_OK) return rc;
+  NanFill nf;
+  const ds_tensor5* gs[5] = {&dq, &dks, &dvs, &dk, &dv};
+  for (int i = 0; i < 5; ++i) {
+    nf.ptr[i] = static_cast<float*>(gs[i]->ptr);
+    for (int j = 0; j < 5; ++j) {
+      nf.size[i][j] = gs[i]->size[j];
+      nf.stride[i][j] = gs[i]->stride[j];
+    }
+  }
+  nan_fill_kernel<<<4 * sm_count(), 256, 0, st>>>(nf, L.bad);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
+}
+
+static Workspace size_query() { return Workspace(reinterpret_cast<void*>(4096), SIZE_MAX / 4); }
+
+}  // namespace bwd
+}  // namespace ds
+
+extern "C" {
+
+size_t ds_aas_groups_bwd_workspace_bytes(ds_tensor5 q, ds_tensor5 k, int64_t n_groups, int64_t n_entries) {
+  using namespace ds::bwd;
+  if (n_groups <= 0 || n_entries <= 0) return 256;
+  ds::Workspace w = size_query();
+  GroupsBwdWs L;
+  groups_bwd_layout(w, q, k, n_groups, n_entries, &L);
+  return w.off + 256;
+}
+
+int ds_aas_groups_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5 k, ds_tensor5 v,
+                      const int32_t* group_q, const int32_t* group_off, int64_t n_groups, const int32_t* kv_idx,
+                      int64_t n_entries, float scale, int mode, const float* d_dir, ds_tensor5 dq, ds_tensor5 dk_self,
+                      ds_tensor5 dv_self, ds_tensor5 dk, ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream) {
+  using namespace ds;
+  using namespace ds::bwd;
+  const char* who = "ds_aas_groups_bwd";
+  if (n_groups < 0 || n_entries < 0) return fail(DS_ERR_INVALID, "%s: negative counts", who);
+  if (n_groups == 0 || n_entries == 0) return DS_OK;
+  if (!group_q || !group_off || !kv_idx) return fail(DS_ERR_INVALID, "%s: work list: null pointer", who);
+  if (n_groups > INT32_MAX / 4 || n_entries > INT32_MAX / 4) return fail(DS_ERR_INVALID, "%s: work list too long", who);
+  bool aliased;
+  int rc = groups_bwd_check(q, k_self, v_self, k, v, mode, d_dir, dq, dk_self, dv_self, dk, dv, who, &aliased);
+  if (rc != DS_OK) return rc;
+  Workspace w(ws, ws_bytes);
+  GroupsBwdWs L;
+  if (!groups_bwd_layout(w, q, k, n_groups, n_entries, &L))
+    return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes,
+                ds_aas_groups_bwd_workspace_bytes(q, k, n_groups, n_entries));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
+  return groups_bwd_launch(q, k_self, v_self, k, v, group_q, group_off, n_groups, kv_idx, n_entries, scale, mode, d_dir,
+                           dq, dk_self, dv_self, dk, dv, aliased, L, who, static_cast<cudaStream_t>(stream));
+}
+
+size_t ds_aas_pairs_bwd_workspace_bytes(ds_tensor5 q, int64_t n_pairs) {
+  using namespace ds;
+  if (n_pairs <= 0) return 256;
+  const size_t lists = 2 * align_up((size_t)(2 * n_pairs) * 4, 256) + align_up((size_t)(2 * n_pairs + 1) * 4, 256) +
+                       align_up((size_t)(2 * n_pairs) * 4, 256);   // group_q, kv_idx, group_off, d_dir
+  return lists + ds_aas_groups_bwd_workspace_bytes(q, q, 2 * n_pairs, 2 * n_pairs) + 256;
+}
+
+int ds_aas_pairs_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t* pair_idx, int64_t n_pairs, float scale,
+                     int mode, const float* d_scores, ds_tensor5 dq, ds_tensor5 dk, ds_tensor5 dv, void* ws,
+                     size_t ws_bytes, void* stream) {
+  using namespace ds;
+  using namespace ds::bwd;
+  const char* who = "ds_aas_pairs_bwd";
+  if (n_pairs < 0) return fail(DS_ERR_INVALID, "%s: negative n_pairs", who);
+  if (n_pairs == 0) return DS_OK;
+  if (!pair_idx) return fail(DS_ERR_INVALID, "%s: pair_idx: null pointer", who);
+  if (n_pairs > INT32_MAX / 8) return fail(DS_ERR_INVALID, "%s: too many pairs", who);
+  bool aliased;
+  int rc = groups_bwd_check(q, k, v, k, v, mode, d_scores, dq, dk, dv, dk, dv, who, &aliased);
+  if (rc != DS_OK) return rc;
+  const int64_t G = 2 * n_pairs;
+  Workspace w(ws, ws_bytes);
+  int32_t* gq = static_cast<int32_t*>(w.take((size_t)G * 4));
+  int32_t* kv = static_cast<int32_t*>(w.take((size_t)G * 4));
+  int32_t* go = static_cast<int32_t*>(w.take((size_t)(G + 1) * 4));
+  float* d_dir = static_cast<float*>(w.take((size_t)G * 4));
+  GroupsBwdWs L;
+  if (!gq || !kv || !go || !d_dir || !groups_bwd_layout(w, q, k, G, G, &L))
+    return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes,
+                ds_aas_pairs_bwd_workspace_bytes(q, n_pairs));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = launch_pairs_setup(pair_idx, n_pairs, gq, go, kv, st)) != DS_OK) return rc;
+  pairs_ddir_kernel<<<(unsigned)((n_pairs + 255) / 256), 256, 0, st>>>(d_scores, n_pairs, d_dir);
+  DS_CUDA_TRY(cudaGetLastError());
+  return groups_bwd_launch(q, k, v, k, v, gq, go, G, kv, G, scale, mode, d_dir, dq, dk, dv, dk, dv, aliased, L, who, st);
+}
+
+size_t ds_aas_triplets_bwd_workspace_bytes(ds_tensor5 q, int64_t n_triplets) {
+  using namespace ds;
+  if (n_triplets <= 0) return 256;
+  const size_t lists = align_up((size_t)(3 * n_triplets) * 4, 256) + align_up((size_t)(3 * n_triplets + 1) * 4, 256) +
+                       2 * align_up((size_t)(4 * n_triplets) * 4, 256);   // group_q, group_off, kv_idx, d_dir
+  return lists + ds_aas_groups_bwd_workspace_bytes(q, q, 3 * n_triplets, 4 * n_triplets) + 256;
+}
+
+int ds_aas_triplets_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t* trip_idx, int64_t n_triplets,
+                        float scale, int mode, const float* d_ab, const float* d_ac, ds_tensor5 dq, ds_tensor5 dk,
+                        ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream) {
+  using namespace ds;
+  using namespace ds::bwd;
+  const char* who = "ds_aas_triplets_bwd";
+  if (n_triplets < 0) return fail(DS_ERR_INVALID, "%s: negative n_triplets", who);
+  if (n_triplets == 0) return DS_OK;
+  if (!trip_idx) return fail(DS_ERR_INVALID, "%s: trip_idx: null pointer", who);
+  if (!d_ab || !d_ac) return fail(DS_ERR_INVALID, "%s: d_ab / d_ac: null pointer", who);
+  if (n_triplets > INT32_MAX / 16) return fail(DS_ERR_INVALID, "%s: too many triplets", who);
+  bool aliased;
+  int rc = groups_bwd_check(q, k, v, k, v, mode, d_ab, dq, dk, dv, dk, dv, who, &aliased);
+  if (rc != DS_OK) return rc;
+  const int64_t G = 3 * n_triplets, T = 4 * n_triplets;
+  Workspace w(ws, ws_bytes);
+  int32_t* gq = static_cast<int32_t*>(w.take((size_t)G * 4));
+  int32_t* go = static_cast<int32_t*>(w.take((size_t)(G + 1) * 4));
+  int32_t* kv = static_cast<int32_t*>(w.take((size_t)T * 4));
+  float* d_dir = static_cast<float*>(w.take((size_t)T * 4));
+  GroupsBwdWs L;
+  if (!gq || !go || !kv || !d_dir || !groups_bwd_layout(w, q, k, G, T, &L))
+    return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes,
+                ds_aas_triplets_bwd_workspace_bytes(q, n_triplets));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = launch_triplets_setup(trip_idx, n_triplets, gq, go, kv, st)) != DS_OK) return rc;
+  triplets_ddir_kernel<<<(unsigned)((n_triplets + 255) / 256), 256, 0, st>>>(d_ab, d_ac, n_triplets, d_dir);
+  DS_CUDA_TRY(cudaGetLastError());
+  return groups_bwd_launch(q, k, v, k, v, gq, go, G, kv, T, scale, mode, d_dir, dq, dk, dv, dk, dv, aliased, L, who, st);
 }
 
 }  // extern "C"

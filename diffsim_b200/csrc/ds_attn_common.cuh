@@ -105,4 +105,22 @@ inline int make_map(CUtensorMap* m, const ds_tensor5& t, int subw, int rows) {
   return encode_tensor_map(m, t.dtype, 5, t.ptr, dims, strides, box, subw * 2, kAttnL2PromotionBytes);
 }
 
+// Grouped work lists (ds_attn.cu), for the AAS backward (ds_attn_bwd.cu):
+// the argument checks of ds_aas_groups' five operands (no device work)
+int check_group_operands(const ds_tensor5& q, const ds_tensor5& k_self, const ds_tensor5& v_self, const ds_tensor5& k,
+                         const ds_tensor5& v, const char* who);
+// bad[0] = 1 when an image index of the list is out of range (bad[0] must be zeroed first)
+int launch_validate_groups(const int32_t* group_q, int64_t n_groups, const int32_t* kv_idx, int64_t n_entries,
+                           int64_t nq_images, int64_t nk_images, int32_t* bad, cudaStream_t st);
+// the work lists of ds_aas_pairs / ds_aas_triplets (pairs_setup_kernel, triplets_setup_kernel)
+int launch_pairs_setup(const int32_t* pair_idx, int64_t n_pairs, int32_t* group_q, int32_t* group_off, int32_t* kv_idx,
+                       cudaStream_t st);
+int launch_triplets_setup(const int32_t* trip_idx, int64_t n_triplets, int32_t* group_q, int32_t* group_off,
+                          int32_t* kv_idx, cudaStream_t st);
+// one K1 launch storing Y_g = Attn(Q_i, K_i, V_i) at slot g and X_t = Attn(Q_i, K_j, V_j) at slot n_groups + t of `out`, a
+// contiguous (n_groups + n_entries, B, H, Sq, D) stack of q's dtype, rounded exactly as ds_attn_fwd rounds its output
+int attn_list_store(const ds_tensor5& q, const ds_tensor5& k_self, const ds_tensor5& v_self, const ds_tensor5& k,
+                    const ds_tensor5& v, const int32_t* group_q, const int32_t* group_off, int64_t n_groups,
+                    const int32_t* kv_idx, float scale, void* out, const char* who, cudaStream_t st);
+
 }  // namespace ds

@@ -241,7 +241,16 @@ def pair_dirs(qa, ka, va, qb, kb, vb, similarity="cosine", scale: Optional[float
 def aas_groups(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                group_q, group_off, kv_idx, similarity="cosine", scale: Optional[float] = None) -> torch.Tensor:
     """Directional AAS similarities for grouped (query image, kv image list) work -- see ds_aas_groups.
-    q/k_self/v_self: (Nq,B,H,S,D); k/v: (Nk,B,H,S,D).  Returns float32 [n_entries]."""
+    q/k_self/v_self: (Nq,B,H,S,D); k/v: (Nk,B,H,S,D).  Returns float32 [n_entries].  Differentiable in the five
+    caches (aas_groups_bwd) when one of them requires grad; the values are the same either way."""
+    if wants_grad(q, k_self, v_self, k, v):
+        dev = _need_cuda(q)
+        return _AASGroupsFn.apply(similarity, scale, _i32(group_q, dev), _i32(group_off, dev), _i32(kv_idx, dev), q,
+                                  k_self, v_self, k, v)
+    return _aas_groups(q, k_self, v_self, k, v, group_q, group_off, kv_idx, similarity, scale)
+
+
+def _aas_groups(q, k_self, v_self, k, v, group_q, group_off, kv_idx, similarity="cosine", scale=None) -> torch.Tensor:
     dev = _need_cuda(q, k_self, v_self, k, v)
     gq, go, kv = _i32(group_q, dev), _i32(group_off, dev), _i32(kv_idx, dev)
     n_groups, n_entries = gq.numel(), kv.numel()
@@ -258,7 +267,14 @@ def aas_groups(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: t
 def aas_pairs(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, pair_idx, similarity="cosine",
               scale: Optional[float] = None) -> torch.Tensor:
     """score[p] = (dir(a->b) + dir(b->a)) / 2 for pair_idx[p] = (a, b): the value DiffSim.diffsim returns
-    (diffsim/diffsim.py:177-197).  q,k,v: (N,B,H,S,D) caches.  Returns float32 [P]."""
+    (diffsim/diffsim.py:177-197).  q,k,v: (N,B,H,S,D) caches.  Returns float32 [P].  Differentiable in the caches
+    (aas_pairs_bwd) when one of them requires grad; the values are the same either way."""
+    if wants_grad(q, k, v):
+        return _AASPairsFn.apply(similarity, scale, _i32(pair_idx, _need_cuda(q)).reshape(-1, 2), q, k, v)
+    return _aas_pairs(q, k, v, pair_idx, similarity, scale)
+
+
+def _aas_pairs(q, k, v, pair_idx, similarity="cosine", scale=None) -> torch.Tensor:
     dev = _need_cuda(q, k, v)
     pairs = _i32(pair_idx, dev).reshape(-1, 2)
     P = pairs.shape[0]
@@ -273,7 +289,16 @@ def aas_triplets(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, trip_idx, si
                  scale: Optional[float] = None, round_scores: bool = False, want_flags: bool = True):
     """2AFC triplets (ref, left, right) as the benchmark drivers score them (cute_main.py:111-132,196-205):
     returns (ab, ac, counts, flags) on the device: ab = diffsim(ref,left), ac = diffsim(ref,right) (float32 [T]),
-    counts int32[2] = {correct, correct_2x}, flags uint8[T].  One library call, no host sync."""
+    counts int32[2] = {correct, correct_2x}, flags uint8[T].  One library call, no host sync.  ab and ac are
+    differentiable in the caches (aas_triplets_bwd) when one of them requires grad (the rounding of round_scores passes
+    straight through); counts and flags are not.  The values are the same either way."""
+    if wants_grad(q, k, v):
+        trips = _i32(trip_idx, _need_cuda(q)).reshape(-1, 3)
+        return _AASTripletsFn.apply(similarity, scale, round_scores, want_flags, trips, q, k, v)
+    return _aas_triplets(q, k, v, trip_idx, similarity, scale, round_scores, want_flags)
+
+
+def _aas_triplets(q, k, v, trip_idx, similarity="cosine", scale=None, round_scores=False, want_flags=True):
     dev = _need_cuda(q, k, v)
     trips = _i32(trip_idx, dev).reshape(-1, 3)
     T = trips.shape[0]
@@ -287,6 +312,155 @@ def aas_triplets(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, trip_idx, si
           counts.data_ptr(), flags.data_ptr() if want_flags else None, ws_query=(q5, T),
           launches=5)  # setup + index validation + attention + finish + combine/decide
     return ab, ac, counts, flags
+
+
+# Cap on the workspace of one grouped-backward library call: longer lists are cut into chunks of whole groups (pairs,
+# triplets), issued in list order.  Every gradient row still receives its terms in entry order, so chunking keeps the
+# bitwise contract of ds_aas_groups_bwd.  About 4 MB per entry at the SD-1.5 up0 shape (2, 8, 256, 160).
+GROUPS_BWD_WORKSPACE_CAP = 1 << 30
+
+
+def _grad_buffers(ts, grads):
+    """float32 zeros with the strides of each input where it is dense (a head-split view of a (N,B,S,H*D) cache gets its
+    gradient in that memory layout), or the caller's `grads` to add into; a repeated input shares one buffer."""
+    if grads is not None:
+        return _grads_like(ts, grads)
+    out = []
+    for t in ts:
+        same = [o for o, u in zip(out, ts) if u is t]
+        out.append(same[0] if same else torch.zeros_like(t, dtype=torch.float32))
+    return tuple(out)
+
+
+def _chunks(n: int, ws_bytes) -> list:
+    """[(i0, i1)] cutting n units into runs whose workspace ws_bytes(i1 - i0) stays under GROUPS_BWD_WORKSPACE_CAP."""
+    per = max(1, GROUPS_BWD_WORKSPACE_CAP // max(1, ws_bytes(1)))
+    return [(i, min(n, i + per)) for i in range(0, n, per)]
+
+
+def aas_groups_bwd(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
+                   group_q, group_off, kv_idx, d_dir: torch.Tensor, similarity="cosine", scale: Optional[float] = None,
+                   grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
+    """float32 gradients (dq, dk_self, dv_self, dk, dv) of aas_groups for dL/ddir = d_dir (n_entries values on the device),
+    bitwise those of one aas_dir_bwd call per entry in list order (ds_aas_groups_bwd).  When k_self is k (v_self is v)
+    the gradient is one buffer: dk_self is dk.  grads: optional float32 tensors to add into (dk_self is dk allowed)."""
+    dev = _need_cuda(q, k_self, v_self, k, v, d_dir)
+    gq, go, kv = _i32(group_q, dev), _i32(group_off, dev), _i32(kv_idx, dev)
+    n_groups, n_entries = gq.numel(), kv.numel()
+    if go.numel() != n_groups + 1:
+        raise RuntimeError("group_off must have n_groups + 1 entries")
+    g = d_dir.detach().reshape(-1).to(torch.float32).contiguous()
+    if g.numel() != n_entries:
+        raise RuntimeError("d_dir must have one value per entry")
+    out = _grad_buffers((q, k_self, v_self, k, v), grads)
+    if n_groups == 0 or n_entries == 0:
+        return out
+    lib = N.load()
+    q5, k5 = _desc(q, 5), _desc(k, 5)
+    args = (q5, _desc(k_self, 5), _desc(v_self, 5), k5, _desc(v, 5))
+    gdesc = [_desc(t, 5) for t in out]
+    if lib.ds_aas_groups_bwd_workspace_bytes(q5, k5, n_groups, n_entries) <= GROUPS_BWD_WORKSPACE_CAP:
+        spans = [(0, n_groups)]
+    else:   # cut into runs of whole groups (needs the group offsets on the host)
+        off = go.tolist()
+        spans, g0 = [], 0
+        for g1 in range(1, n_groups + 1):
+            if g1 > g0 + 1 and lib.ds_aas_groups_bwd_workspace_bytes(q5, k5, g1 - g0, off[g1] - off[g0]) > GROUPS_BWD_WORKSPACE_CAP:
+                spans.append((g0, g1 - 1))
+                g0 = g1 - 1
+        spans.append((g0, n_groups))
+        go = go.cpu()
+    for g0, g1 in spans:
+        e0, e1 = (0, n_entries) if len(spans) == 1 else (int(go[g0]), int(go[g1]))
+        off = go if len(spans) == 1 else (go[g0:g1 + 1] - e0).to(dev)
+        _call("ds_aas_groups_bwd", dev, *args, gq[g0:].data_ptr(), off.data_ptr(), g1 - g0, kv[e0:].data_ptr(), e1 - e0,
+              _scale_arg(scale), _mode(similarity), g[e0:].data_ptr(), *gdesc, ws_query=(q5, k5, g1 - g0, e1 - e0),
+              slot="bwd", launches=10)  # validation + entry groups + lists + recompute + partials + coefficients
+        #                                  + factors + dQ + dK/dV + NaN fill
+    return out
+
+
+def aas_pairs_bwd(q, k, v, pair_idx, d_scores, similarity="cosine", scale=None, grads=None) -> Tuple[torch.Tensor, ...]:
+    """float32 gradients (dq, dk, dv) of aas_pairs for dL/dscore = d_scores (ds_aas_pairs_bwd: aas_groups_bwd of the
+    pairs' work list), added into `grads` when given."""
+    dev = _need_cuda(q, k, v, d_scores)
+    pairs = _i32(pair_idx, dev).reshape(-1, 2)
+    g = d_scores.detach().reshape(-1).to(torch.float32).contiguous()
+    if g.numel() != pairs.shape[0]:
+        raise RuntimeError("d_scores must have one value per pair")
+    out = _grad_buffers((q, k, v), grads)
+    lib, q5 = N.load(), _desc(q, 5)
+    args, gdesc = (q5, _desc(k, 5), _desc(v, 5)), [_desc(t, 5) for t in out]
+    for p0, p1 in _chunks(pairs.shape[0], lambda n: lib.ds_aas_pairs_bwd_workspace_bytes(q5, n)):
+        _call("ds_aas_pairs_bwd", dev, *args, pairs[p0:].data_ptr(), p1 - p0, _scale_arg(scale), _mode(similarity),
+              g[p0:].data_ptr(), *gdesc, ws_query=(q5, p1 - p0), slot="bwd", launches=12)  # setup + d_dir + groups_bwd
+    return out
+
+
+def aas_triplets_bwd(q, k, v, trip_idx, d_ab, d_ac, similarity="cosine", scale=None, grads=None) -> Tuple[torch.Tensor, ...]:
+    """float32 gradients (dq, dk, dv) of the (ab, ac) of aas_triplets for dL/dab = d_ab and dL/dac = d_ac (either may
+    be None: zero) -- ds_aas_triplets_bwd -- added into `grads` when given."""
+    dev = _need_cuda(q, k, v)
+    trips = _i32(trip_idx, dev).reshape(-1, 3)
+    T = trips.shape[0]
+    zero = torch.zeros(T, dtype=torch.float32, device=dev)
+    gab = zero if d_ab is None else d_ab.detach().reshape(-1).to(torch.float32).contiguous()
+    gac = zero if d_ac is None else d_ac.detach().reshape(-1).to(torch.float32).contiguous()
+    if gab.numel() != T or gac.numel() != T:
+        raise RuntimeError("d_ab and d_ac must have one value per triplet")
+    out = _grad_buffers((q, k, v), grads)
+    lib, q5 = N.load(), _desc(q, 5)
+    args, gdesc = (q5, _desc(k, 5), _desc(v, 5)), [_desc(t, 5) for t in out]
+    for t0, t1 in _chunks(T, lambda n: lib.ds_aas_triplets_bwd_workspace_bytes(q5, n)):
+        _call("ds_aas_triplets_bwd", dev, *args, trips[t0:].data_ptr(), t1 - t0, _scale_arg(scale), _mode(similarity),
+              gab[t0:].data_ptr(), gac[t0:].data_ptr(), *gdesc, ws_query=(q5, t1 - t0), slot="bwd",
+              launches=12)  # setup + d_dir + groups_bwd
+    return out
+
+
+class _AASGroupsFn(torch.autograd.Function):
+    """aas_groups with the grouped K5 backward; saves only the caches and the index tensors."""
+
+    @staticmethod
+    def forward(ctx, similarity, scale, gq, go, kv, q, k_self, v_self, k, v):
+        ctx.save_for_backward(gq, go, kv, q, k_self, v_self, k, v)
+        ctx.similarity, ctx.scale = similarity, scale
+        return _aas_groups(q, k_self, v_self, k, v, gq, go, kv, similarity, scale)
+
+    @staticmethod
+    def backward(ctx, d_dir):
+        gq, go, kv, q, ks, vs, k, v = ctx.saved_tensors
+        dq, dks, dvs, dk, dv = aas_groups_bwd(q, ks, vs, k, v, gq, go, kv, d_dir, ctx.similarity, ctx.scale)
+        # one buffer for a repeated input holds the gradient once: hand it to one of the two slots only
+        return (None,) * 5 + (dq, None if dks is dk else dks, None if dvs is dv else dvs, dk, dv)
+
+
+class _AASPairsFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, similarity, scale, pairs, q, k, v):
+        ctx.save_for_backward(pairs, q, k, v)
+        ctx.similarity, ctx.scale = similarity, scale
+        return _aas_pairs(q, k, v, pairs, similarity, scale)
+
+    @staticmethod
+    def backward(ctx, d_scores):
+        pairs, q, k, v = ctx.saved_tensors
+        return (None,) * 3 + aas_pairs_bwd(q, k, v, pairs, d_scores, ctx.similarity, ctx.scale)
+
+
+class _AASTripletsFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, similarity, scale, round_scores, want_flags, trips, q, k, v):
+        ctx.save_for_backward(trips, q, k, v)
+        ctx.similarity, ctx.scale = similarity, scale
+        ab, ac, counts, flags = _aas_triplets(q, k, v, trips, similarity, scale, round_scores, want_flags)
+        ctx.mark_non_differentiable(*[t for t in (counts, flags) if t is not None])
+        return ab, ac, counts, flags
+
+    @staticmethod
+    def backward(ctx, d_ab, d_ac, _counts, _flags):
+        trips, q, k, v = ctx.saved_tensors
+        return (None,) * 5 + aas_triplets_bwd(q, k, v, trips, d_ab, d_ac, ctx.similarity, ctx.scale)
 
 
 def aas_matrix(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,

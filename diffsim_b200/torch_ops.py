@@ -46,11 +46,11 @@ def _aas_score(qa, ka, va, qb, kb, vb, similarity="cosine", scale=0.0):
 
 
 def _aas_pairs(q, k, v, pair_idx, similarity="cosine", scale=0.0):
-    return ops.aas_pairs(q, k, v, pair_idx, similarity, scale)
+    return ops._aas_pairs(q, k, v, pair_idx, similarity, scale)   # forward only: no autograd registered
 
 
 def _aas_triplets(q, k, v, trip_idx, similarity="cosine", scale=0.0, round_scores=False):
-    return ops.aas_triplets(q, k, v, trip_idx, similarity, scale, round_scores)
+    return ops._aas_triplets(q, k, v, trip_idx, similarity, scale, round_scores)   # forward only
 
 
 def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=0.0):

@@ -221,6 +221,47 @@ int ds_aas_dir_bwd(ds_tensor4 q_i, ds_tensor4 k_i, ds_tensor4 v_i, ds_tensor4 k_
                    void* ws, size_t ws_bytes, void* stream);
 size_t ds_aas_dir_bwd_workspace_bytes(ds_tensor4 q_i, ds_tensor4 k_j);
 
+/*
+ * Backward of ds_aas_groups (the directional similarities dir[t] of a whole work list) for d_dir = dL/ddir, float[n_entries]
+ * on the device.  Same arguments as ds_aas_groups; the five FLOAT32 (N,B,H,S,D) gradients (of q, k_self, v_self, k, v;
+ * any strides with a unit innermost one) are ADDED INTO.  dk_self / dk, and dv_self / dv, are either the same tensor
+ * (same pointer, sizes and strides: the pairs / triplets case, where k_self is k) or have disjoint address ranges.
+ *
+ * Bitwise contract: the buffers end up exactly as after one ds_aas_dir_bwd call per entry, t = 0 .. n_entries - 1 in order,
+ * on the slices (q, k_self, v_self)[group_q[g(t)]], (k, v)[kv_idx[t]], d_dir + t and the matching gradient slices: every
+ * gradient row receives its terms in that order (entry, then cross term before self term) with the same arithmetic.
+ * One K1 launch recomputes every X_t and Y_g; one dQ launch (a CTA per query image, b, h and 128-row q tile) and one dK/dV
+ * launch (per kv image, b, h, 128-row kv tile) walk contribution lists built on the device.  No float atomics, no host
+ * synchronisation.  An out-of-range image index fills every gradient buffer of the call with NaN.  Workspace: about
+ * (3 n_entries + n_groups) x B H S D x 2 bytes.
+ */
+int ds_aas_groups_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5 k, ds_tensor5 v,
+                      const int32_t* group_q, const int32_t* group_off, int64_t n_groups,
+                      const int32_t* kv_idx, int64_t n_entries, float scale, int mode,
+                      const float* d_dir,
+                      ds_tensor5 dq, ds_tensor5 dk_self, ds_tensor5 dv_self, ds_tensor5 dk, ds_tensor5 dv,
+                      void* ws, size_t ws_bytes, void* stream);
+size_t ds_aas_groups_bwd_workspace_bytes(ds_tensor5 q, ds_tensor5 k, int64_t n_groups, int64_t n_entries);
+
+/*
+ * Backward of ds_aas_pairs for d_scores = dL/dscore (float[n_pairs] on the device): ds_aas_groups_bwd on the pairs'
+ * work list with d_dir[2p] = d_dir[2p+1] = d_scores[p] / 2.  dq, dk, dv: FLOAT32 gradients of q, k, v, added into.
+ */
+int ds_aas_pairs_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t* pair_idx, int64_t n_pairs,
+                     float scale, int mode, const float* d_scores,
+                     ds_tensor5 dq, ds_tensor5 dk, ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream);
+size_t ds_aas_pairs_bwd_workspace_bytes(ds_tensor5 q, int64_t n_pairs);
+
+/*
+ * Backward of the scores ab, ac of ds_aas_triplets (without DS_OPT_ROUND_SCORES; with it, the rounding passes straight
+ * through) for d_ab, d_ac (float[n_triplets] each, on the device): entries 4t .. 4t+3 of the triplets' work list are
+ * ref->left, ref->right, left->ref, right->ref, so d_dir = (d_ab, d_ac, d_ab, d_ac)[t] / 2.
+ */
+int ds_aas_triplets_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t* trip_idx, int64_t n_triplets,
+                        float scale, int mode, const float* d_ab, const float* d_ac,
+                        ds_tensor5 dq, ds_tensor5 dk, ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream);
+size_t ds_aas_triplets_bwd_workspace_bytes(ds_tensor5 q, int64_t n_triplets);
+
 /* ---- K2: similarity reductions ----------------------------------------- */
 
 /*
