@@ -70,6 +70,9 @@ PROTOTYPES = {
     "ds_aas_triplets_bwd": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, _vp, Tensor5, Tensor5, Tensor5, _vp, _sz,
                                  _vp]),
     "ds_aas_triplets_bwd_workspace_bytes": (_sz, [Tensor5, _i64]),
+    "ds_aas_matrix_bwd": (_i, [Tensor5, Tensor5, Tensor5, Tensor5, Tensor5, _f, _i, _vp, _i64, Tensor5, Tensor5, Tensor5,
+                               Tensor5, Tensor5, _vp, _sz, _vp]),
+    "ds_aas_matrix_bwd_workspace_bytes": (_sz, [Tensor5, Tensor5]),
     "ds_aas_groups": (_i, [Tensor5, Tensor5, Tensor5, Tensor5, Tensor5, _vp, _vp, _i64, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),
     "ds_aas_groups_workspace_bytes": (_sz, [Tensor5, _i64, _i64]),
     "ds_aas_pairs": (_i, [Tensor5, Tensor5, Tensor5, _vp, _i64, _f, _i, _vp, _vp, _sz, _vp]),

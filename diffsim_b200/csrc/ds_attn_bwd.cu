@@ -26,6 +26,7 @@
 // Algorithmic work per attention backward: 10 B H Sq Skv D flops (QK^T recompute, dP, dV, dK, dQ); this implementation
 // issues 12 (the LSE pass recomputes QK^T once more).
 #include <algorithm>
+#include <type_traits>
 
 #include "ds_attn_common.cuh"
 
@@ -583,6 +584,21 @@ struct ListBuild {
   ListFamily fam[2];
 };
 
+// ds_aas_matrix_bwd: the row-major matrix list (group r = row r, n_cols entries), with ONE self term per row -- the folded
+// one, at tau = 2t + 1 of the row's last entry t, so that it follows the row's cross terms
+struct FoldListBuild : ListBuild {
+  int n_cols;
+};
+
+template <bool kFold>
+using ListBuildT = std::conditional_t<kFold, FoldListBuild, ListBuild>;
+
+template <bool kFold>
+__device__ __forceinline__ bool term_live(const ListBuildT<kFold>& b, int64_t tau) {
+  if constexpr (kFold) return !(tau & 1) || ((tau >> 1) + 1) % b.n_cols == 0;
+  else return true;
+}
+
 __device__ __forceinline__ int term_key(const ListBuild& b, int family, int64_t tau) {
   const int64_t t = tau >> 1;
   const bool self = tau & 1;
@@ -627,8 +643,9 @@ __device__ __forceinline__ int2 block_scan2(int a, int c, int& ea, int& ec, int2
   return tot;
 }
 
-// block f builds family f: a stable counting sort of the terms by key (deterministic: integer counts only)
-__global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBuild b) {
+// block f builds family f: a stable counting sort of the live terms by key (deterministic: integer counts only)
+template <bool kFold>
+__global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBuildT<kFold> b) {
   const int f = blockIdx.x;
   const ListFamily& L = b.fam[f];
   __shared__ int2 s_warp[32];
@@ -639,7 +656,8 @@ __global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBui
   }
   for (int64_t k = threadIdx.x; k < L.n_keys; k += kListThreads) L.cnt[k] = 0;
   __syncthreads();
-  for (int64_t tau = threadIdx.x; tau < b.n_terms; tau += kListThreads) atomicAdd(&L.cnt[term_key(b, f, tau)], 1);
+  for (int64_t tau = threadIdx.x; tau < b.n_terms; tau += kListThreads)
+    if (term_live<kFold>(b, tau)) atomicAdd(&L.cnt[term_key(b, f, tau)], 1);
   __syncthreads();
   int n_lists = 0, n_seen = 0;   // running totals over the key chunks
   for (int64_t k0 = 0; k0 < L.n_keys; k0 += kListThreads) {
@@ -662,16 +680,17 @@ __global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBui
   __syncthreads();
   for (int64_t t0 = 0; t0 < b.n_terms; t0 += kListThreads) {
     const int64_t tau = t0 + threadIdx.x;
-    const int key = tau < b.n_terms ? term_key(b, f, tau) : -1;
+    const bool live = tau < b.n_terms && term_live<kFold>(b, tau);
+    const int key = live ? term_key(b, f, tau) : -1;
     s_key[threadIdx.x] = key;
     __syncthreads();
-    if (tau < b.n_terms) {
+    if (live) {
       int r = 0;   // earlier terms of this chunk with the same key
       for (int j = 0; j < (int)threadIdx.x; ++j) r += s_key[j] == key;
       L.terms[L.cnt[key] + r] = (int32_t)tau;
     }
     __syncthreads();
-    if (tau < b.n_terms) atomicAdd(&L.cnt[key], 1);
+    if (live) atomicAdd(&L.cnt[key], 1);
     __syncthreads();
   }
 }
@@ -701,6 +720,96 @@ __global__ void sim_factor_list_kernel(const uint32_t* __restrict__ o, int64_t n
                       f + (2 * t + 1) * n2);
 }
 
+// ---------------------------------------------------------------------------
+// matrix similarity gradient (ds_aas_matrix_bwd): the grouped backward of the row-major matrix list, with each row's
+// self terms folded into one.  The attention backward is linear in dO and so is delta = rowsum(dO o O): the Nc self terms
+// of row r (O = Y_r, dO = coef_self_rc fy_rc) are ONE term with dO = F_r = sum_c coef_self_rc fy_rc.
+// ---------------------------------------------------------------------------
+// the row-major list (group r = row r: entries t = r n_cols + c, kv image c), entry -> row, and d_dir[t] = d_Dm[r, c]
+__global__ void matrix_bwd_setup_kernel(int64_t n_rows, int64_t n_cols, const float* __restrict__ d_Dm, int64_t ldd,
+                                        int32_t* __restrict__ group_q, int32_t* __restrict__ group_off,
+                                        int32_t* __restrict__ kv_idx, int32_t* __restrict__ entry_group,
+                                        float* __restrict__ d_dir) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i < n_rows * n_cols) {
+    const int64_t r = i / n_cols, c = i - r * n_cols;
+    kv_idx[i] = (int32_t)c;
+    entry_group[i] = (int32_t)r;
+    d_dir[i] = d_Dm[r * ldd + c];
+  }
+  if (i <= n_rows) group_off[i] = (int32_t)(i * n_cols);
+  if (i < n_rows) group_q[i] = (int32_t)i;
+}
+
+// per row r and element pair: fx_t of every entry t = (r, c) as sim_factor rounds it, and the fp32 fold
+// F_r = sum over ascending c of coef[4t + 1] fy_t, fy_t unrounded (F32 [r][n2]); row_max[r] (zeroed before): max |F_r|
+// as float bits (non-negative floats order as integers, so the integer atomic is order-independent)
+template <bool kBf16>
+__global__ void matrix_fold_kernel(const uint32_t* __restrict__ o, int64_t n2, int n_rows, int n_cols, int mode,
+                                   const float* __restrict__ coef, uint32_t* __restrict__ fx, float2* __restrict__ F32,
+                                   int32_t* __restrict__ row_max) {
+  __shared__ float s_max[kRedThreads / 32];
+  for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+    const uint32_t* y = o + (int64_t)r * n2;
+    float mx = 0.f;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n2; i += (int64_t)gridDim.x * blockDim.x) {
+      const float2 c = unpack2<kBf16>(y[i]);
+      float fx0 = 0.f, fx1 = 0.f;
+      for (int col = 0; col < n_cols; ++col) {
+        const int64_t t = (int64_t)r * n_cols + col;
+        const float* cf = coef + 4 * t;
+        const float2 a = unpack2<kBf16>(o[(n_rows + t) * n2 + i]);
+        float fy0, fy1;
+        if (mode == DS_SIM_MSE) {
+          fx[t * n2 + i] = pack2<kBf16>(a.x - c.x, a.y - c.y);
+          fy0 = c.x - a.x;
+          fy1 = c.y - a.y;
+        } else {
+          const float kx = cf[2], ky = cf[3];
+          fx[t * n2 + i] = pack2<kBf16>(c.x - kx * a.x, c.y - kx * a.y);
+          fy0 = a.x - ky * c.x;
+          fy1 = a.y - ky * c.y;
+        }
+        fx0 = fmaf(cf[1], fy0, fx0);
+        fx1 = fmaf(cf[1], fy1, fx1);
+      }
+      F32[(int64_t)r * n2 + i] = make_float2(fx0, fx1);
+      mx = fmaxf(mx, fmaxf(fabsf(fx0), fabsf(fx1)));
+    }
+#pragma unroll
+    for (int o2 = 16; o2 > 0; o2 >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o2));
+    if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int w = 1; w < kRedThreads / 32; ++w) mx = fmaxf(mx, s_max[w]);
+      atomicMax(row_max + r, __float_as_int(mx));
+    }
+    __syncthreads();
+  }
+}
+
+// F_r rounded ONCE to the input dtype after a power-of-two scale 2^-e that puts max |F_r| in [0.5, 1): at SD-1.5 up0 the
+// elements of F_r fall below fp16's normal range.  fold_scale[r] = 2^e, the coefficient of the folded self term.
+template <bool kBf16>
+__global__ void matrix_fold_round_kernel(const float2* __restrict__ F32, int64_t n2, int n_rows,
+                                         const int32_t* __restrict__ row_max, uint32_t* __restrict__ F16,
+                                         float* __restrict__ fold_scale) {
+  for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+    const float m = __int_as_float(row_max[r]);
+    int e = 0;
+    if (m > 0.f && m <= 3.402823466e38f) {
+      frexpf(m, &e);
+      e = min(max(e, -126), 127);
+    }
+    const float inv = ldexpf(1.f, -e);
+    if (blockIdx.x == 0 && threadIdx.x == 0) fold_scale[r] = ldexpf(1.f, e);
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n2; i += (int64_t)gridDim.x * blockDim.x) {
+      const float2 v = F32[(int64_t)r * n2 + i];
+      F16[(int64_t)r * n2 + i] = pack2<kBf16>(v.x * inv, v.y * inv);
+    }
+  }
+}
+
 struct GradT {   // an fp32 (N, B, H, S, D) gradient
   float* ptr;
   int64_t sn, sb, sh, ss;
@@ -727,14 +836,24 @@ struct ListParams {
   GradT dq, dk, dv, dks, dvs;
 };
 
+// ds_aas_matrix_bwd (kFold): the self term of row r is the folded one.  Its dO factor and its LSE / delta rows sit at
+// slot n_entries + r, a cross term's at slot t (instead of tau); its coefficient is fold_scale[r].
+struct FoldListParams : ListParams {
+  int64_t n_entries;
+  const float* fold_scale;
+};
+
+template <bool kFold>
+using ListParamsT = std::conditional_t<kFold, FoldListParams, ListParams>;
+
 // attn_bwd_dq_kernel over a list: one CTA per (query image, b, h, 128-row q tile), the steps of that kernel once per
 // term, dQ drained (x the term's coefficient) into the fp32 rows before the next term
-template <int D, bool kBf16>
+template <int D, bool kBf16, bool kFold>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                         const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
                         const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
-                        const ListParams p) {
+                        const ListParamsT<kFold> p) {
   using C = Cfg<D>;
   const int per_list = p.B * p.H * p.n_qt;
   const int li = blockIdx.x / per_list;
@@ -794,16 +913,18 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
     const CUtensorMap* mk = self ? &map_ks : &map_k;
     const CUtensorMap* mv = self ? &map_vs : &map_v;
     const int64_t o_slot = self ? p.entry_group[t] : p.n_groups + t;
+    int slot = tau;   // of the dO factor and of the LSE / delta rows
+    if constexpr (kFold) slot = self ? (int)p.n_entries + p.entry_group[t] : t;
     if (tid == 0) {
       mbar_arrive_expect_tx(q_bar, 2 * C::TILE_BYTES);
       load_tile<D>(sQ, &map_q, q_bar, kTile, qt * kTile, h, b, qi);
-      load_tile<D>(sDO, &map_do, q_bar, kTile, qt * kTile, h, b, tau);
+      load_tile<D>(sDO, &map_do, q_bar, kTile, qt * kTile, h, b, slot);
     }
     __syncwarp();
     float delta = 0.f;
     if (row_ok)
       delta = row_dot<kBf16>(static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
-                             static_cast<const uint16_t*>(p.f) + tau * p.img + row_off, D);
+                             static_cast<const uint16_t*>(p.f) + slot * p.img + row_off, D);
     mbar_wait(q_bar, q_ph);
     q_ph ^= 1;
 
@@ -850,7 +971,7 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
     }
     const float lse2 = m * sl2 + __log2f(l);
     {
-      const size_t k = ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
+      const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
       p.lse[k] = lse2;
       p.delta[k] = delta;
     }
@@ -906,7 +1027,9 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
       tc_fence_after_sync();
     }
 
-    const float fq = p.scale * p.coef[4 * t + (self ? 1 : 0)];
+    float fq;
+    if constexpr (kFold) fq = p.scale * (self ? p.fold_scale[p.entry_group[t]] : p.coef[4 * t]);
+    else fq = p.scale * p.coef[4 * t + (self ? 1 : 0)];
     add_row_out<D>(lane_t + kDQ, fq, dq_row, row_ok);
     sync_all_tc();   // dQ read out (and Q / dO free) before the next term
   }
@@ -914,12 +1037,12 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
 }
 
 // attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), the steps of that kernel once per term
-template <int D, bool kBf16>
+template <int D, bool kBf16, bool kFold>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                          const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
                          const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
-                         const ListParams p) {
+                         const ListParamsT<kFold> p) {
   using C = Cfg<D>;
   constexpr int BQ = C::BQ;
   const int per_list = p.B * p.H * p.n_kt;
@@ -986,21 +1109,23 @@ attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
     const int tau = p.terms[i], t = tau >> 1;
     const bool self = tau & 1;
     const int qi = p.group_q[p.entry_group[t]];
+    int slot = tau;   // of the dO factor and of the LSE / delta rows
+    if constexpr (kFold) slot = self ? (int)p.n_entries + p.entry_group[t] : t;
     if (tid == 0) {
       mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
       load_tile<D>(sK, self ? &map_ks : &map_k, kv_bar, kTile, kt * kTile, h, b, img);
       load_tile<D>(sV, self ? &map_vs : &map_v, kv_bar, kTile, kt * kTile, h, b, img);
     }
     __syncwarp();
-    const float* lse_bh = p.lse + ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile);
-    const float* delta_bh = p.delta + ((size_t)tau * (p.B * p.H) + bh) * (p.n_qt * kTile);
+    const float* lse_bh = p.lse + ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
+    const float* delta_bh = p.delta + ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
     mbar_wait(kv_bar, kv_ph);
     kv_ph ^= 1;
     for (int qb = 0; qb < n_qb; ++qb) {
       if (tid == 0) {
         mbar_arrive_expect_tx(q_bar, 2 * C::QB_BYTES);
         load_tile<D>(sQ, &map_q, q_bar, BQ, qb * BQ, h, b, qi);
-        load_tile<D>(sDO, &map_do, q_bar, BQ, qb * BQ, h, b, tau);
+        load_tile<D>(sDO, &map_do, q_bar, BQ, qb * BQ, h, b, slot);
       }
       __syncwarp();
       if (tid < BQ) {
@@ -1055,7 +1180,9 @@ attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
       tc_fence_after_sync();
       __syncthreads();
     }
-    const float g = p.coef[4 * t + (self ? 1 : 0)];
+    float g;
+    if constexpr (kFold) g = self ? p.fold_scale[p.entry_group[t]] : p.coef[4 * t];
+    else g = p.coef[4 * t + (self ? 1 : 0)];
     add_row_out<D>(lane_t + kDV, g, dv_row, row_ok);
     add_row_out<D>(lane_t + kDK, g * p.scale, dk_row, row_ok);
     sync_all_tc();   // dK / dV read out (and K / V free) before the next term
@@ -1266,10 +1393,10 @@ static GradT grad_t(const ds_tensor5& g) {
   return GradT{static_cast<float*>(g.ptr), g.stride[0], g.stride[1], g.stride[2], g.stride[3]};
 }
 
-template <int D, bool kBf16>
+template <int D, bool kBf16, bool kFold>
 static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
-                               const ds_tensor5& v, const ds_tensor5& F, ListParams p, int64_t grid_q, int64_t grid_kv,
-                               const GroupsBwdWs& L, cudaStream_t st) {
+                               const ds_tensor5& v, const ds_tensor5& F, ListParamsT<kFold> p, int64_t grid_q,
+                               int64_t grid_kv, const ListFamily* fam, cudaStream_t st) {
   using C = Cfg<D>;
   CUtensorMap mq, mk, mv, mks, mvs, mdo, mqb, mdob;
   int rc;
@@ -1278,21 +1405,68 @@ static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const 
       (rc = make_map(&mvs, vs, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mdo, F, C::SUBW, kTile)) != DS_OK ||
       (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, F, C::SUBW, C::BQ)) != DS_OK)
     return rc;
-  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_list_kernel<D, kBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::DQ_SMEM));
-  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dkv_list_kernel<D, kBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::DKV_SMEM));
-  p.n_lists = L.fam[0].n_lists;
-  p.list_key = L.fam[0].list_key;
-  p.list_off = L.fam[0].list_off;
-  p.terms = L.fam[0].terms;
-  attn_bwd_dq_list_kernel<D, kBf16><<<(unsigned)grid_q, kThreads, C::DQ_SMEM, st>>>(mq, mk, mv, mks, mvs, mdo, p);
+  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_list_kernel<D, kBf16, kFold>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   C::DQ_SMEM));
+  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dkv_list_kernel<D, kBf16, kFold>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   C::DKV_SMEM));
+  p.n_lists = fam[0].n_lists;
+  p.list_key = fam[0].list_key;
+  p.list_off = fam[0].list_off;
+  p.terms = fam[0].terms;
+  attn_bwd_dq_list_kernel<D, kBf16, kFold><<<(unsigned)grid_q, kThreads, C::DQ_SMEM, st>>>(mq, mk, mv, mks, mvs, mdo, p);
   DS_CUDA_TRY(cudaGetLastError());
-  p.n_lists = L.fam[1].n_lists;
-  p.list_key = L.fam[1].list_key;
-  p.list_off = L.fam[1].list_off;
-  p.terms = L.fam[1].terms;
-  attn_bwd_dkv_list_kernel<D, kBf16><<<(unsigned)grid_kv, kThreads, C::DKV_SMEM, st>>>(mqb, mk, mv, mks, mvs, mdob, p);
+  p.n_lists = fam[1].n_lists;
+  p.list_key = fam[1].list_key;
+  p.list_off = fam[1].list_off;
+  p.terms = fam[1].terms;
+  attn_bwd_dkv_list_kernel<D, kBf16, kFold><<<(unsigned)grid_kv, kThreads, C::DKV_SMEM, st>>>(mqb, mk, mv, mks, mvs, mdob, p);
   DS_CUDA_TRY(cudaGetLastError());
   return DS_OK;
+}
+
+// the factors of a list backward as a contiguous (n_slots, B, H, Sq, D) stack of q's dtype at ptr
+static ds_tensor5 factor_stack(const ds_tensor5& q, void* ptr, int64_t n_slots) {
+  ds_tensor5 F = q;
+  F.ptr = ptr;
+  F.size[0] = n_slots;
+  F.stride[4] = 1;
+  F.stride[3] = q.size[4];
+  F.stride[2] = q.size[3] * q.size[4];
+  F.stride[1] = q.size[2] * F.stride[2];
+  F.stride[0] = q.size[1] * F.stride[1];
+  return F;
+}
+
+// ListParams of a checked list backward: shapes, grids (false: too many tiles) and everything but the lists
+static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, int64_t G, int64_t E, int n_kbuf,
+                        bool aliased, ListParams* p, int64_t* grid_q, int64_t* grid_kv) {
+  const int D = (int)q.size[4];
+  p->B = (int)q.size[1];
+  p->H = (int)q.size[2];
+  p->Sq = (int)q.size[3];
+  p->Skv = (int)k.size[3];
+  p->n_qt = (p->Sq + kTile - 1) / kTile;
+  p->n_kt = (p->Skv + kTile - 1) / kTile;
+  p->scale = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
+  p->scale_log2 = p->scale * 1.4426950408889634f;
+  p->n_groups = (int)G;
+  p->n_kbuf = n_kbuf;
+  p->img = q.size[1] * q.size[2] * q.size[3] * D;
+  const int64_t bh = (int64_t)p->B * p->H;
+  const int64_t nl_q = std::min<int64_t>(q.size[0], G);
+  const int64_t nl_kv = aliased ? std::min<int64_t>(k.size[0], G + E) : nl_q + std::min<int64_t>(k.size[0], E);
+  *grid_q = nl_q * bh * p->n_qt;
+  *grid_kv = nl_kv * bh * p->n_kt;
+  return *grid_q < INT32_MAX && *grid_kv < INT32_MAX;
+}
+
+static void set_grads(ListParams* p, const ds_tensor5& dq, const ds_tensor5& dks, const ds_tensor5& dvs,
+                      const ds_tensor5& dk, const ds_tensor5& dv) {
+  p->dq = grad_t(dq);
+  p->dk = grad_t(dk);
+  p->dv = grad_t(dv);
+  p->dks = grad_t(dks);
+  p->dvs = grad_t(dvs);
 }
 
 }  // namespace bwd
@@ -1438,22 +1612,12 @@ static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds
                              const ds_tensor5& dv, bool aliased, const GroupsBwdWs& L, const char* who, cudaStream_t st) {
   int rc;
   const int D = (int)q.size[4];
-  const int64_t img = q.size[1] * q.size[2] * q.size[3] * D, n2 = img / 2;
   const bool bf = q.dtype == DS_BF16;
   ListParams p;
-  p.B = (int)q.size[1];
-  p.H = (int)q.size[2];
-  p.Sq = (int)q.size[3];
-  p.Skv = (int)k.size[3];
-  p.n_qt = (p.Sq + kTile - 1) / kTile;
-  p.n_kt = (p.Skv + kTile - 1) / kTile;
-  p.scale = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
-  p.scale_log2 = p.scale * 1.4426950408889634f;
-  const int64_t bh = (int64_t)p.B * p.H;
-  const int64_t nl_q = std::min<int64_t>(q.size[0], G);
-  const int64_t nl_kv = aliased ? std::min<int64_t>(k.size[0], G + E) : nl_q + std::min<int64_t>(k.size[0], E);
-  const int64_t grid_q = nl_q * bh * p.n_qt, grid_kv = nl_kv * bh * p.n_kt;
-  if (grid_q >= INT32_MAX || grid_kv >= INT32_MAX) return fail(DS_ERR_INVALID, "%s: too many tiles: split the work list", who);
+  int64_t grid_q, grid_kv;
+  if (!list_params(q, k, scale, G, E, aliased ? 0 : (int)k.size[0], aliased, &p, &grid_q, &grid_kv))
+    return fail(DS_ERR_INVALID, "%s: too many tiles: split the work list", who);
+  const int64_t img = p.img, n2 = img / 2;
 
   DS_CUDA_TRY(cudaMemsetAsync(L.bad, 0, sizeof(int32_t), st));
   if ((rc = launch_validate_groups(group_q, G, kv_idx, E, q.size[0], k.size[0], L.bad, st)) != DS_OK) return rc;
@@ -1465,11 +1629,11 @@ static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds
   lb.entry_group = L.entry_group;
   lb.bad = L.bad;
   lb.n_terms = 2 * E;
-  lb.n_kbuf = aliased ? 0 : (int)k.size[0];
+  lb.n_kbuf = p.n_kbuf;
   lb.fam[0] = L.fam[0];
   lb.fam[1] = L.fam[1];
   lb.fam[1].n_keys = aliased ? k.size[0] : k.size[0] + q.size[0];
-  build_lists_kernel<<<2, kListThreads, 0, st>>>(lb);
+  build_lists_kernel<false><<<2, kListThreads, 0, st>>>(lb);
   DS_CUDA_TRY(cudaGetLastError());
   // X_t and Y_g, rounded to the input dtype as ds_attn_fwd rounds them
   if ((rc = attn_list_store(q, ks, vs, k, v, group_q, group_off, G, kv_idx, scale, L.o, who, st)) != DS_OK) return rc;
@@ -1486,33 +1650,20 @@ static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds
   else sim_factor_list_kernel<false><<<dim3(fb, ey), 256, 0, st>>>(ou, n2, (int)G, E, L.entry_group, mode, L.coef, fu);
   DS_CUDA_TRY(cudaGetLastError());
 
-  p.n_groups = (int)G;
   p.group_q = group_q;
   p.kv_idx = kv_idx;
   p.entry_group = L.entry_group;
-  p.n_kbuf = lb.n_kbuf;
   p.o = L.o;
   p.f = L.f;
-  p.img = img;
   p.lse = L.lse;
   p.delta = L.delta;
   p.coef = L.coef;
-  p.dq = grad_t(dq);
-  p.dk = grad_t(dk);
-  p.dv = grad_t(dv);
-  p.dks = grad_t(dks);
-  p.dvs = grad_t(dvs);
-  ds_tensor5 F = q;   // the factors as a (2 n_entries, B, H, Sq, D) contiguous stack
-  F.ptr = L.f;
-  F.size[0] = 2 * E;
-  F.stride[4] = 1;
-  F.stride[3] = D;
-  F.stride[2] = q.size[3] * D;
-  F.stride[1] = q.size[2] * F.stride[2];
-  F.stride[0] = q.size[1] * F.stride[1];
+  set_grads(&p, dq, dks, dvs, dk, dv);
+  const ds_tensor5 F = factor_stack(q, L.f, 2 * E);
   rc = with_head_dim(D, who, [&](auto d) {
     return with_dtype(q.dtype, [&](auto b) {
-      return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value>(q, ks, vs, k, v, F, p, grid_q, grid_kv, L, st);
+      return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value, false>(q, ks, vs, k, v, F, p, grid_q, grid_kv,
+                                                                                L.fam, st);
     });
   });
   if (rc != DS_OK) return rc;
@@ -1647,6 +1798,168 @@ int ds_aas_triplets_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t*
   triplets_ddir_kernel<<<(unsigned)((n_triplets + 255) / 256), 256, 0, st>>>(d_ab, d_ac, n_triplets, d_dir);
   DS_CUDA_TRY(cudaGetLastError());
   return groups_bwd_launch(q, k, v, k, v, gq, go, G, kv, T, scale, mode, d_dir, dq, dk, dv, dk, dv, aliased, L, who, st);
+}
+
+}  // extern "C"
+
+namespace ds {
+namespace bwd {
+
+// workspace layout of ds_aas_matrix_bwd (the size query runs it on a dummy base).  E = n_rows n_cols entries.
+struct MatrixBwdWs {
+  void* o;                 // (n_rows + E) attention outputs, 16-bit: Y_r at slot r, X_t at n_rows + t
+  void* f;                 // (E + n_rows) dO factors, 16-bit: fx_t at slot t, the folded F_r at E + r
+  float* fold32;           // [n_rows] fp32 F_r images
+  float* part;             // [E][kRedBlocks][3]
+  float* coef;             // [E][4]
+  float* lse;              // [E + n_rows][B H][n_qt 128]
+  float* delta;
+  float* fold_scale;       // [n_rows]
+  int32_t* row_max;        // [n_rows]
+  int32_t* group_q;        // [n_rows]
+  int32_t* group_off;      // [n_rows + 1]
+  int32_t* kv_idx;         // [E]
+  int32_t* entry_group;    // [E]
+  float* d_dir;            // [E]
+  int32_t* bad;
+  ListFamily fam[2];
+};
+
+static bool matrix_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor5& k, MatrixBwdWs* L) {
+  const int64_t R = q.size[0], Cn = k.size[0], E = R * Cn, nt = E + R;   // nt: live terms, E cross + R folded self
+  const int64_t img = q.size[1] * q.size[2] * q.size[3] * q.size[4];
+  const int64_t n_qt = (q.size[3] + kTile - 1) / kTile;
+  const size_t stats = (size_t)nt * q.size[1] * q.size[2] * n_qt * kTile * sizeof(float);
+  L->o = w.take((size_t)(R + E) * img * 2);
+  L->f = w.take((size_t)nt * img * 2);
+  L->fold32 = static_cast<float*>(w.take((size_t)R * img * sizeof(float)));
+  L->part = static_cast<float*>(w.take((size_t)E * kRedBlocks * 3 * sizeof(float)));
+  L->coef = static_cast<float*>(w.take((size_t)E * 4 * sizeof(float)));
+  L->lse = static_cast<float*>(w.take(stats));
+  L->delta = static_cast<float*>(w.take(stats));
+  L->fold_scale = static_cast<float*>(w.take((size_t)R * sizeof(float)));
+  L->row_max = static_cast<int32_t*>(w.take((size_t)R * 4));
+  L->group_q = static_cast<int32_t*>(w.take((size_t)R * 4));
+  L->group_off = static_cast<int32_t*>(w.take((size_t)(R + 1) * 4));
+  L->kv_idx = static_cast<int32_t*>(w.take((size_t)E * 4));
+  L->entry_group = static_cast<int32_t*>(w.take((size_t)E * 4));
+  L->d_dir = static_cast<float*>(w.take((size_t)E * sizeof(float)));
+  L->bad = static_cast<int32_t*>(w.take(4));
+  bool ok = L->o && L->f && L->fold32 && L->part && L->coef && L->lse && L->delta && L->fold_scale && L->row_max &&
+            L->group_q && L->group_off && L->kv_idx && L->entry_group && L->d_dir && L->bad;
+  const int64_t n_keys[2] = {R, Cn + R};
+  for (int i = 0; i < 2; ++i) {
+    ListFamily& F = L->fam[i];
+    F.n_keys = n_keys[i];
+    F.cnt = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
+    F.n_lists = static_cast<int32_t*>(w.take(4));
+    F.list_key = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
+    F.list_off = static_cast<int32_t*>(w.take((size_t)(n_keys[i] + 1) * 4));
+    F.terms = static_cast<int32_t*>(w.take((size_t)nt * 4));
+    ok = ok && F.cnt && F.n_lists && F.list_key && F.list_off && F.terms;
+  }
+  return ok;
+}
+
+}  // namespace bwd
+}  // namespace ds
+
+extern "C" {
+
+size_t ds_aas_matrix_bwd_workspace_bytes(ds_tensor5 q, ds_tensor5 k) {
+  using namespace ds::bwd;
+  if (q.size[0] <= 0 || k.size[0] <= 0) return 256;
+  ds::Workspace w = size_query();
+  MatrixBwdWs L;
+  matrix_bwd_layout(w, q, k, &L);
+  return w.off + 256;
+}
+
+int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5 k, ds_tensor5 v, float scale,
+                      int mode, const float* d_Dm, int64_t ldd, ds_tensor5 dq, ds_tensor5 dk_self, ds_tensor5 dv_self,
+                      ds_tensor5 dk, ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream) {
+  using namespace ds;
+  using namespace ds::bwd;
+  const char* who = "ds_aas_matrix_bwd";
+  const int64_t R = q.size[0], Cn = k.size[0], E = R * Cn;
+  if (R <= 0 || Cn <= 0) return fail(DS_ERR_INVALID, "%s: empty image set", who);
+  if (ldd < Cn) return fail(DS_ERR_INVALID, "%s: ldd < columns", who);
+  // the term index 2t + 1 of the lists is an int32
+  if (E > INT32_MAX / 4) return fail(DS_ERR_INVALID, "%s: more than 2^29 entries; split the rows", who);
+  bool aliased;
+  int rc = groups_bwd_check(q, k_self, v_self, k, v, mode, d_Dm, dq, dk_self, dv_self, dk, dv, who, &aliased);
+  if (rc != DS_OK) return rc;
+  ListParamsT<true> p;
+  int64_t grid_q, grid_kv;
+  if (!list_params(q, k, scale, R, E, aliased ? 0 : (int)Cn, aliased, &p, &grid_q, &grid_kv))
+    return fail(DS_ERR_INVALID, "%s: too many tiles: split the rows", who);
+  Workspace w(ws, ws_bytes);
+  MatrixBwdWs L;
+  if (!matrix_bwd_layout(w, q, k, &L))
+    return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes,
+                ds_aas_matrix_bwd_workspace_bytes(q, k));
+  if ((rc = ds_device_ok()) != DS_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t n2 = p.img / 2;
+  const bool bf = q.dtype == DS_BF16;
+
+  DS_CUDA_TRY(cudaMemsetAsync(L.bad, 0, sizeof(int32_t), st));
+  DS_CUDA_TRY(cudaMemsetAsync(L.row_max, 0, (size_t)R * 4, st));
+  matrix_bwd_setup_kernel<<<(unsigned)((E + 256) / 256), 256, 0, st>>>(R, Cn, d_Dm, ldd, L.group_q, L.group_off, L.kv_idx,
+                                                                      L.entry_group, L.d_dir);
+  DS_CUDA_TRY(cudaGetLastError());
+  ListBuildT<true> lb;
+  lb.group_q = L.group_q;
+  lb.kv_idx = L.kv_idx;
+  lb.entry_group = L.entry_group;
+  lb.bad = L.bad;
+  lb.n_terms = 2 * E;
+  lb.n_kbuf = p.n_kbuf;
+  lb.fam[0] = L.fam[0];
+  lb.fam[1] = L.fam[1];
+  lb.fam[1].n_keys = aliased ? Cn : Cn + R;
+  lb.n_cols = (int)Cn;
+  build_lists_kernel<true><<<2, kListThreads, 0, st>>>(lb);
+  DS_CUDA_TRY(cudaGetLastError());
+  // X_t and Y_r, rounded to the input dtype as ds_attn_fwd rounds them
+  if ((rc = attn_list_store(q, k_self, v_self, k, v, L.group_q, L.group_off, R, L.kv_idx, scale, L.o, who, st)) != DS_OK)
+    return rc;
+  const uint32_t* ou = static_cast<const uint32_t*>(L.o);
+  const unsigned ey = (unsigned)std::min<int64_t>(E, 65535), ry = (unsigned)std::min<int64_t>(R, 65535);
+  if (bf) sim_partials_list_kernel<true><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)R, E, L.entry_group, L.part);
+  else sim_partials_list_kernel<false><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)R, E, L.entry_group, L.part);
+  DS_CUDA_TRY(cudaGetLastError());
+  sim_coef_list_kernel<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(L.part, E, mode, (double)p.img, L.d_dir, L.coef);
+  DS_CUDA_TRY(cudaGetLastError());
+  const unsigned fb = (unsigned)std::min<int64_t>((n2 + 255) / 256, 4 * (int64_t)sm_count());
+  uint32_t* fu = static_cast<uint32_t*>(L.f);
+  float2* f32 = reinterpret_cast<float2*>(L.fold32);
+  if (bf) matrix_fold_kernel<true><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+  else matrix_fold_kernel<false><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+  DS_CUDA_TRY(cudaGetLastError());
+  uint32_t* f16 = fu + E * n2;
+  if (bf) matrix_fold_round_kernel<true><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
+  else matrix_fold_round_kernel<false><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
+  DS_CUDA_TRY(cudaGetLastError());
+
+  p.group_q = L.group_q;
+  p.kv_idx = L.kv_idx;
+  p.entry_group = L.entry_group;
+  p.o = L.o;
+  p.f = L.f;
+  p.lse = L.lse;
+  p.delta = L.delta;
+  p.coef = L.coef;
+  p.n_entries = E;
+  p.fold_scale = L.fold_scale;
+  set_grads(&p, dq, dk_self, dv_self, dk, dv);
+  const ds_tensor5 F = factor_stack(q, L.f, E + R);
+  return with_head_dim(q.size[4], who, [&](auto d) {
+    return with_dtype(q.dtype, [&](auto b) {
+      return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value, true>(q, k_self, v_self, k, v, F, p, grid_q,
+                                                                               grid_kv, L.fam, st);
+    });
+  });
 }
 
 }  // extern "C"

@@ -418,6 +418,80 @@ def aas_triplets_bwd(q, k, v, trip_idx, d_ab, d_ac, similarity="cosine", scale=N
     return out
 
 
+def _matrix_spans(nr: int, nc: int, ws_bytes) -> list:
+    """[((r0, r1), (c0, c1))] cutting an nr x nc matrix backward into calls whose workspace ws_bytes(rows, cols) stays under
+    GROUPS_BWD_WORKSPACE_CAP: blocks of whole rows, in order, and column blocks only when one row does not fit."""
+    cap = GROUPS_BWD_WORKSPACE_CAP
+    if ws_bytes(nr, nc) <= cap:
+        return [((0, nr), (0, nc))]
+    if ws_bytes(1, nc) <= cap:
+        per = 1
+        while per < nr and ws_bytes(per + 1, nc) <= cap:
+            per += 1
+        return [((r, min(nr, r + per)), (0, nc)) for r in range(0, nr, per)]
+    per = 1
+    while per < nc and ws_bytes(1, per + 1) <= cap:
+        per += 1
+    return [((r, r + 1), (c, min(nc, c + per))) for r in range(nr) for c in range(0, nc, per)]
+
+
+def aas_matrix_bwd(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
+                   d_Dm: torch.Tensor, similarity="cosine", scale: Optional[float] = None,
+                   grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
+    """float32 gradients (dq, dk_self, dv_self, dk, dv) of aas_matrix for dL/dDm = d_Dm ([Nr, Nc] on the device) --
+    ds_aas_matrix_bwd: the grouped backward of the row-major list with each row's self terms folded into one.  When
+    k_self is k (v_self is v) the gradient is one buffer.  grads: optional float32 tensors to add into.
+
+    A matrix whose workspace would exceed GROUPS_BWD_WORKSPACE_CAP is cut into blocks of whole rows (columns only when
+    one row does not fit; each column block then folds its own self term).  Row blocks are bitwise one call when the
+    self gradients are separate buffers; with one shared buffer a block's self terms are added after the block."""
+    dev = _need_cuda(q, k_self, v_self, k, v, d_Dm)
+    nr, nc = q.shape[0], k.shape[0]
+    g = d_Dm.detach().to(torch.float32)
+    if g.shape != (nr, nc):
+        raise RuntimeError(f"d_Dm must have shape ({nr}, {nc}), got {tuple(g.shape)}")
+    if (nc > 1 and g.stride(1) != 1) or (nr > 1 and g.stride(0) < nc):
+        g = g.contiguous()
+    ldd = g.stride(0) if nr > 1 else nc
+    out = _grad_buffers((q, k_self, v_self, k, v), grads)
+    dq, dks, dvs, dk, dv = out
+    lib = N.load()
+    ws = lambda r, c: lib.ds_aas_matrix_bwd_workspace_bytes(_desc(q[:r], 5), _desc(k[:c], 5))  # noqa: E731
+    spans = _matrix_spans(nr, nc, ws)
+    shared = dks is dk or dvs is dv
+    for (r0, r1), (c0, c1) in spans:
+        rows = (q[r0:r1], k_self[r0:r1], v_self[r0:r1])
+        cols = (k[c0:c1], v[c0:c1])
+        gks, gvs = dks[r0:r1], dvs[r0:r1]
+        if shared and len(spans) > 1:   # the C call takes one shared buffer whole, not a block of it
+            gks, gvs = torch.zeros_like(gks), torch.zeros_like(gvs)
+        q5, k5 = _desc(rows[0], 5), _desc(cols[0], 5)
+        _call("ds_aas_matrix_bwd", dev, q5, _desc(rows[1], 5), _desc(rows[2], 5), k5, _desc(cols[1], 5), _scale_arg(scale),
+              _mode(similarity), g[r0:, c0:].data_ptr(), ldd, _desc(dq[r0:r1], 5), _desc(gks, 5), _desc(gvs, 5),
+              _desc(dk[c0:c1], 5), _desc(dv[c0:c1], 5), ws_query=(q5, k5), slot="bwd",
+              launches=9)  # setup + lists + recompute + partials + coefficients + fold + fold rounding + dQ + dK/dV
+        if shared and len(spans) > 1:
+            dks[r0:r1] += gks
+            dvs[r0:r1] += gvs
+    return out
+
+
+class _AASMatrixFn(torch.autograd.Function):
+    """aas_matrix with the folded grouped K5 backward; saves only the caches."""
+
+    @staticmethod
+    def forward(ctx, similarity, scale, q, k_self, v_self, k, v):
+        ctx.save_for_backward(q, k_self, v_self, k, v)
+        ctx.similarity, ctx.scale = similarity, scale
+        return _aas_matrix(q, k_self, v_self, k, v, similarity, scale)
+
+    @staticmethod
+    def backward(ctx, d_Dm):
+        q, ks, vs, k, v = ctx.saved_tensors
+        dq, dks, dvs, dk, dv = aas_matrix_bwd(q, ks, vs, k, v, d_Dm, ctx.similarity, ctx.scale)
+        return (None,) * 2 + (dq, None if dks is dk else dks, None if dvs is dv else dvs, dk, dv)
+
+
 class _AASGroupsFn(torch.autograd.Function):
     """aas_groups with the grouped K5 backward; saves only the caches and the index tensors."""
 
@@ -466,7 +540,14 @@ class _AASTripletsFn(torch.autograd.Function):
 def aas_matrix(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                similarity="cosine", scale: Optional[float] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Directional matrix Dm[r,c] = dir(row image r -> column image c); rows (q,k_self,v_self): (Nr,...),
-    columns (k,v): (Nc,...).  Returns float32 [Nr,Nc]."""
+    columns (k,v): (Nc,...).  Returns float32 [Nr,Nc].  Differentiable in the five caches (aas_matrix_bwd) when one of
+    them requires grad and `out` is not given; the values are the same either way."""
+    if out is None and wants_grad(q, k_self, v_self, k, v):
+        return _AASMatrixFn.apply(similarity, scale, q, k_self, v_self, k, v)
+    return _aas_matrix(q, k_self, v_self, k, v, similarity, scale, out)
+
+
+def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=None, out=None) -> torch.Tensor:
     dev = _need_cuda(q, k_self, v_self, k, v)
     nr, nc = q.shape[0], k.shape[0]
     if out is None:

@@ -212,10 +212,12 @@ def row_block(n: int, rank: int, world: int) -> Tuple[int, int]:
 
 
 def aas_matrix_local(rows: QKVCache, cols: QKVCache, similarity: str = "cosine", scale: Optional[float] = None):
-    """Directional block Dm[rows, all columns] on this device."""
+    """Directional block Dm[rows, all columns] on this device; differentiable in the caches (ops.aas_matrix) when one
+    of them requires grad."""
     return ops.aas_matrix(rows.q, rows.k, rows.v, cols.k, cols.v, similarity, scale)
 
 
+@torch.no_grad()
 def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optional[float] = None, group=None,
                        gather_to_all: bool = True, timings: Optional[dict] = None) -> torch.Tensor:
     """All-pairs directional matrix with the images row-block sharded over the ranks of `group`.
@@ -227,6 +229,8 @@ def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optio
     Dm[own rows, :] and the row blocks are gathered at the end.  Per-element arithmetic does not depend on the
     sharding or on how the columns are cut into calls, so the result is bit-identical to the single-device matrix.
     `timings` (optional dict) receives CUDA events: 'start', 'own_done', 'exchange_done', 'block_done', 'end'.
+    Forward only: the peers' K and V arrive through all_gather, so a graph built here would silently lack their
+    gradients; the blocks run without one.
     """
     import torch.distributed as dist
 

@@ -54,7 +54,7 @@ def _aas_triplets(q, k, v, trip_idx, similarity="cosine", scale=0.0, round_score
 
 
 def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=0.0):
-    return ops.aas_matrix(q, k_self, v_self, k, v, similarity, scale)
+    return ops._aas_matrix(q, k_self, v_self, k, v, similarity, scale)   # forward only
 
 
 def _pair_reduce(x, y, similarity="cosine"):

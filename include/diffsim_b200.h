@@ -262,6 +262,28 @@ int ds_aas_triplets_bwd(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t*
                         ds_tensor5 dq, ds_tensor5 dk, ds_tensor5 dv, void* ws, size_t ws_bytes, void* stream);
 size_t ds_aas_triplets_bwd_workspace_bytes(ds_tensor5 q, int64_t n_triplets);
 
+/*
+ * Backward of ds_aas_matrix for d_Dm[r*ldd + c] = dL/dDm[r, c] (float, Nr rows of Nc values, on the device; read there,
+ * no host synchronisation).  Same operands as ds_aas_matrix; the five FLOAT32 (N,B,H,S,D) gradients (of q, k_self,
+ * v_self, k, v; any strides with a unit innermost one) are ADDED INTO, with the aliasing rule of ds_aas_groups_bwd:
+ * dk_self / dk (dv_self / dv) are the same tensor or have disjoint address ranges.
+ *
+ * It is the grouped backward of the row-major matrix list (group r = row r, entries (r, c) for c = 0 .. Nc-1), except
+ * that the Nc self terms of row r -- Attn(q_r, k_self_r, v_self_r) with dO = coef_self_rc fy_rc -- are FOLDED into one
+ * attention backward with dO = F_r = sum_c coef_self_rc fy_rc (fp32, ascending c, fy unrounded), rounded once to the input
+ * dtype after a per-row power-of-two scale: Nr Nc + Nr attention backwards instead of 2 Nr Nc.
+ * Term order of every gradient row: ascending row r, the cross terms of row r in ascending column, then the folded self
+ * term of row r.  So dk and dv, when they are not dk_self and dv_self, are bitwise those of ds_aas_groups_bwd on the
+ * row-major list.  No float atomics: repeated calls are bitwise equal.  At most 2^29 entries (the lists' term index is an
+ * int32).  Workspace: per entry about 2 x B H S D x 2 bytes (X, fx) plus 3 KB of partials; per row about B H S D x 8
+ * bytes (Y, F_r in 16 and 32 bits); LSE and delta for every entry and row.
+ */
+int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5 k, ds_tensor5 v,
+                      float scale, int mode, const float* d_Dm, int64_t ldd,
+                      ds_tensor5 dq, ds_tensor5 dk_self, ds_tensor5 dv_self, ds_tensor5 dk, ds_tensor5 dv,
+                      void* ws, size_t ws_bytes, void* stream);
+size_t ds_aas_matrix_bwd_workspace_bytes(ds_tensor5 q, ds_tensor5 k);
+
 /* ---- K2: similarity reductions ----------------------------------------- */
 
 /*
