@@ -14,6 +14,11 @@
 //                  dV += P^T dO, dK += dS^T Q (TS)
 //                BQ = 128 while 2 x 128 + 2 x D_PAD TMEM columns fit in 512; at D = 160 (576 columns) BQ = 64 (448).
 //
+// Each kernel exists in two forms that run the same per-term body (dq_term, dkv_term) and the same prologue: the single
+// kernels run it once, for ds_attn_bwd and ds_aas_dir_bwd; the list kernels run it once per term of a device-built
+// contribution list, for ds_aas_groups_bwd and ds_aas_matrix_bwd.  They differ only in where a term's operands, LSE /
+// delta rows and coefficient are found, so the list backwards are bitwise a sequence of single ones by construction.
+//
 // Operand forms are exactly K1's (ds_attn.cu): 128B / 64B-swizzled TMA tiles of D_PAD columns, K-major for the SS
 // products and MN-major for the B operand of the TS products.  One thread issues TMA and MMA; the four warps of the CTA
 // own the 128 TMEM lanes (one row each) for the elementwise work.  The phases of an iteration are serialised (load,
@@ -42,8 +47,10 @@ struct Cfg : AttnTile<D> {   // K1's operand tiles
   static constexpr int BQ = (2 * 128 + 2 * Tile::D_PAD <= 512) ? 128 : 64;   // q rows per dK/dV step
   static constexpr int TILE_BYTES = Tile::NSUB * kTile * Tile::SUB_BYTES;      // 128-row tile
   static constexpr int QB_BYTES = Tile::NSUB * BQ * Tile::SUB_BYTES;           // BQ-row tile
-  static constexpr int DQ_SMEM = 4 * TILE_BYTES + 1024;                        // Q, dO, K, V + barriers
-  static constexpr int DKV_SMEM = 2 * TILE_BYTES + 2 * QB_BYTES + 2 * BQ * 4 + 1024;
+  static constexpr int DQ_BARS = 4 * TILE_BYTES;                               // after Q, dO, K, V
+  static constexpr int DKV_BARS = 2 * TILE_BYTES + 2 * QB_BYTES + 2 * BQ * 4;  // after K, V, Q, dO, LSE, delta
+  static constexpr int DQ_SMEM = DQ_BARS + 1024;
+  static constexpr int DKV_SMEM = DKV_BARS + 1024;
   static_assert(256 + Tile::D_PAD <= 512, "dQ TMEM budget");
   static_assert(2 * BQ + 2 * Tile::D_PAD <= 512, "dK/dV TMEM budget");
   static_assert(DQ_SMEM <= 232448 && DKV_SMEM <= 232448, "shared memory");
@@ -51,9 +58,13 @@ struct Cfg : AttnTile<D> {   // K1's operand tiles
                 "swizzle atoms need 1024-byte tiles");
 };
 
-struct Params {
+// the shape of one attention backward, common to the single (Params) and list (ListParams) kernels
+struct Shape {
   int B, H, Sq, Skv, n_qt, n_kt;
   float scale, scale_log2;
+};
+
+struct Params : Shape {
   const void* o;      // forward output (16-bit), for delta
   int64_t o_sb, o_sh, o_ss;
   const void* dout;   // (scaled-down) output gradient (16-bit)
@@ -149,73 +160,72 @@ __device__ __forceinline__ void add_row_out(uint32_t taddr, float f, float* out,
   }
 }
 
-template <int D, bool kBf16>
-__global__ void __launch_bounds__(kThreads, 1)
-attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                   const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_do, const Params p) {
-  using C = Cfg<D>;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sQ = smem;
-  uint8_t* sDO = sQ + C::TILE_BYTES;
-  uint8_t* sK = sDO + C::TILE_BYTES;
-  uint8_t* sV = sK + C::TILE_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + C::TILE_BYTES);
-  uint64_t* q_bar = bars;
-  uint64_t* kv_bar = bars + 1;
-  uint64_t* mma_bar = bars + 2;
+// the start of every K5 kernel: its three barriers at bars[0 .. 2], the prefetch of its tensor maps, and all 512 TMEM
+// columns (one CTA per SM); returns the TMEM base address
+template <class... Maps>
+__device__ __forceinline__ uint32_t kernel_prologue(uint64_t* bars, const Maps*... maps) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const int bh = blockIdx.x / p.n_qt, qt = blockIdx.x - bh * p.n_qt;
-  const int b = bh / p.H, h = bh - b * p.H;
-  const int grow = qt * kTile + tid;
-  const bool row_ok = grow < p.Sq;
-
-  if (tid == 0) {
-    mbar_init(q_bar, 1);
-    mbar_init(kv_bar, 1);
-    mbar_init(mma_bar, 1);
+  if (threadIdx.x == 0) {
+    mbar_init(bars, 1);
+    mbar_init(bars + 1, 1);
+    mbar_init(bars + 2, 1);
     fence_mbar_init();
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    tma_prefetch_desc(&map_do);
+    (tma_prefetch_desc(maps), ...);
   }
-  if (warp == 0) {
+  if (threadIdx.x < 32) {
     tmem_alloc(tmem_slot, 512);
     tmem_relinquish();
   }
   sync_all_tc();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
+  return *tmem_slot;
+}
+
+// One term of a dQ kernel, on the 128-row q tile qt of (b, h): the Q and dO tiles (images q_img of mq and do_img of
+// mdo), delta = rowsum(dO o O) from this thread's 16-bit rows o_row and do_row, the LSE pass and the dS / dQ pass over
+// the kv tiles of image kv_img of mk and mv.  LSE and delta go to *lse and *delta_out, dQ x scale coef is added into
+// dq_row.
+// The barrier phases carry over to the next term.
+template <int D, bool kBf16>
+__device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shape& p, int b, int h, int qt,
+                                        const CUtensorMap* mq, int q_img, const CUtensorMap* mdo, int do_img,
+                                        const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, const void* o_row,
+                                        const void* do_row, float* lse, float* delta_out, float coef, float* dq_row,
+                                        uint32_t& q_ph, uint32_t& kv_ph, uint32_t& mma_ph) {
+  using C = Cfg<D>;
+  uint8_t* sQ = smem;
+  uint8_t* sDO = sQ + C::TILE_BYTES;
+  uint8_t* sK = sDO + C::TILE_BYTES;
+  uint8_t* sV = sK + C::TILE_BYTES;
+  uint64_t* q_bar = reinterpret_cast<uint64_t*>(smem + C::DQ_BARS);
+  uint64_t* kv_bar = q_bar + 1;
+  uint64_t* mma_bar = q_bar + 2;
+  const int tid = threadIdx.x;
+  const uint32_t lane_t = tmem + ((uint32_t)((tid >> 5) * 32) << 16);
+  const bool row_ok = qt * kTile + tid < p.Sq;
   constexpr uint32_t kS = 0, kDP = 128, kDQ = 256;
   const uint32_t fmt = kBf16 ? 1u : 0u;
   const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, kTile, 0, 0);
   const uint32_t idesc_dq = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
+  const float sl2 = p.scale_log2;
 
   if (tid == 0) {
     mbar_arrive_expect_tx(q_bar, 2 * C::TILE_BYTES);
-    load_tile<D>(sQ, &map_q, q_bar, kTile, qt * kTile, h, b);
-    load_tile<D>(sDO, &map_do, q_bar, kTile, qt * kTile, h, b);
+    load_tile<D>(sQ, mq, q_bar, kTile, qt * kTile, h, b, q_img);
+    load_tile<D>(sDO, mdo, q_bar, kTile, qt * kTile, h, b, do_img);
   }
   __syncwarp();
   // delta = rowsum(dO o O) in fp32 (while the tiles land)
   float delta = 0.f;
-  if (row_ok) {
-    const uint8_t* o = static_cast<const uint8_t*>(p.o) + 2 * (b * p.o_sb + h * p.o_sh + grow * p.o_ss);
-    const uint8_t* g = static_cast<const uint8_t*>(p.dout) + 2 * (b * p.do_sb + h * p.do_sh + grow * p.do_ss);
-    delta = row_dot<kBf16>(o, g, D);
-  }
-  const float sl2 = p.scale_log2;
-  uint32_t kv_ph = 0, mma_ph = 0;
-  mbar_wait(q_bar, 0);
+  if (row_ok) delta = row_dot<kBf16>(o_row, do_row, D);
+  mbar_wait(q_bar, q_ph);
+  q_ph ^= 1;
 
   // ---- pass 1: log-sum-exp of every row (log2 domain)
   float m = -INFINITY, l = 0.f;
   for (int kt = 0; kt < p.n_kt; ++kt) {
     if (tid == 0) {
       mbar_arrive_expect_tx(kv_bar, C::TILE_BYTES);
-      load_tile<D>(sK, &map_k, kv_bar, kTile, kt * kTile, h, b);
+      load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
     }
     __syncwarp();
     mbar_wait(kv_bar, kv_ph);
@@ -252,18 +262,15 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     sync_all_tc();   // S read out before the next tile's MMA overwrites it
   }
   const float lse2 = m * sl2 + __log2f(l);
-  {
-    const size_t i = (size_t)bh * (p.n_qt * kTile) + grow;
-    p.lse[i] = lse2;
-    p.delta[i] = delta;
-  }
+  *lse = lse2;
+  *delta_out = delta;
 
   // ---- pass 2: dQ
   for (int kt = 0; kt < p.n_kt; ++kt) {
     if (tid == 0) {
       mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
-      load_tile<D>(sK, &map_k, kv_bar, kTile, kt * kTile, h, b);
-      load_tile<D>(sV, &map_v, kv_bar, kTile, kt * kTile, h, b);
+      load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
+      load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
     }
     __syncwarp();
     mbar_wait(kv_bar, kv_ph);
@@ -309,81 +316,59 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     tc_fence_after_sync();
   }
 
-  const float f = p.scale * (p.coef ? *p.coef : 1.0f);
-  add_row_out<D>(lane_t + kDQ, f, p.dq + b * p.dq_sb + h * p.dq_sh + (int64_t)grow * p.dq_ss, row_ok);
-  sync_all_tc();
-  if (warp == 0) tmem_dealloc(tmem, 512);
+  add_row_out<D>(lane_t + kDQ, p.scale * coef, dq_row, row_ok);
+  sync_all_tc();   // dQ read out (and Q / dO free) before the next term
 }
 
+// One term of a dK/dV kernel, on the 128-row kv tile kt of (b, h): the K and V tiles (image kv_img of mk and mv), then
+// per block of BQ q rows the Q and dO tiles (images q_img of mq and do_img of mdo) with their LSE and delta, read from
+// the term's (b, h) rows lse and delta.  dV x coef is added into dv_row, dK x coef scale into dk_row.  The barrier
+// phases carry over to the next term.
 template <int D, bool kBf16>
-__global__ void __launch_bounds__(kThreads, 1)
-attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                    const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_do, const Params p) {
+__device__ __forceinline__ void dkv_term(uint8_t* smem, uint32_t tmem, const Shape& p, int b, int h, int kt,
+                                         const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, const CUtensorMap* mq,
+                                         int q_img, const CUtensorMap* mdo, int do_img, const float* lse,
+                                         const float* delta, float coef, float* dv_row, float* dk_row, uint32_t& kv_ph,
+                                         uint32_t& q_ph, uint32_t& mma_ph) {
   using C = Cfg<D>;
   constexpr int BQ = C::BQ;
-  extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* sK = smem;
   uint8_t* sV = sK + C::TILE_BYTES;
   uint8_t* sQ = sV + C::TILE_BYTES;
   uint8_t* sDO = sQ + C::QB_BYTES;
   float* sLse = reinterpret_cast<float*>(sDO + C::QB_BYTES);
   float* sDelta = sLse + BQ;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sDelta + BQ);
-  uint64_t* kv_bar = bars;
-  uint64_t* q_bar = bars + 1;
-  uint64_t* mma_bar = bars + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const int bh = blockIdx.x / p.n_kt, kt = blockIdx.x - bh * p.n_kt;
-  const int b = bh / p.H, h = bh - b * p.H;
-  const int krow = kt * kTile + tid;
-  const bool row_ok = krow < p.Skv;
-
-  if (tid == 0) {
-    mbar_init(kv_bar, 1);
-    mbar_init(q_bar, 1);
-    mbar_init(mma_bar, 1);
-    fence_mbar_init();
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    tma_prefetch_desc(&map_do);
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  sync_all_tc();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
+  uint64_t* kv_bar = reinterpret_cast<uint64_t*>(smem + C::DKV_BARS);
+  uint64_t* q_bar = kv_bar + 1;
+  uint64_t* mma_bar = kv_bar + 2;
+  const int tid = threadIdx.x;
+  const uint32_t lane_t = tmem + ((uint32_t)((tid >> 5) * 32) << 16);
+  const bool row_ok = kt * kTile + tid < p.Skv;
   constexpr uint32_t kST = 0, kDPT = BQ, kDV = 2 * BQ, kDK = 2 * BQ + C::D_PAD;
   const uint32_t fmt = kBf16 ? 1u : 0u;
   const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, BQ, 0, 0);
   const uint32_t idesc_o = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
+  const float sl2 = p.scale_log2;
+  const int n_qb = (p.Sq + BQ - 1) / BQ;
 
   if (tid == 0) {
     mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
-    load_tile<D>(sK, &map_k, kv_bar, kTile, kt * kTile, h, b);
-    load_tile<D>(sV, &map_v, kv_bar, kTile, kt * kTile, h, b);
+    load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
+    load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
   }
   __syncwarp();
-  const float sl2 = p.scale_log2;
-  const int n_qb = (p.Sq + BQ - 1) / BQ;
-  const float* lse_bh = p.lse + (size_t)bh * (p.n_qt * kTile);
-  const float* delta_bh = p.delta + (size_t)bh * (p.n_qt * kTile);
-  uint32_t q_ph = 0, mma_ph = 0;
-  mbar_wait(kv_bar, 0);
+  mbar_wait(kv_bar, kv_ph);
+  kv_ph ^= 1;
   for (int qb = 0; qb < n_qb; ++qb) {
     if (tid == 0) {
       mbar_arrive_expect_tx(q_bar, 2 * C::QB_BYTES);
-      load_tile<D>(sQ, &map_q, q_bar, BQ, qb * BQ, h, b);
-      load_tile<D>(sDO, &map_do, q_bar, BQ, qb * BQ, h, b);
+      load_tile<D>(sQ, mq, q_bar, BQ, qb * BQ, h, b, q_img);
+      load_tile<D>(sDO, mdo, q_bar, BQ, qb * BQ, h, b, do_img);
     }
     __syncwarp();
     if (tid < BQ) {
-      sLse[tid] = lse_bh[qb * BQ + tid];
-      sDelta[tid] = delta_bh[qb * BQ + tid];
+      sLse[tid] = lse[qb * BQ + tid];
+      sDelta[tid] = delta[qb * BQ + tid];
     }
     mbar_wait(q_bar, q_ph);
     q_ph ^= 1;
@@ -434,11 +419,49 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
     __syncthreads();
   }
 
-  const float g = p.coef ? *p.coef : 1.0f;
-  add_row_out<D>(lane_t + kDV, g, p.dv + b * p.dv_sb + h * p.dv_sh + (int64_t)krow * p.dv_ss, row_ok);
-  add_row_out<D>(lane_t + kDK, g * p.scale, p.dk + b * p.dk_sb + h * p.dk_sh + (int64_t)krow * p.dk_ss, row_ok);
-  sync_all_tc();
-  if (warp == 0) tmem_dealloc(tmem, 512);
+  add_row_out<D>(lane_t + kDV, coef, dv_row, row_ok);
+  add_row_out<D>(lane_t + kDK, coef * p.scale, dk_row, row_ok);
+  sync_all_tc();   // dK / dV read out (and K / V free) before the next term
+}
+
+// one CTA per (b, h, 128-row q tile)
+template <int D, bool kBf16>
+__global__ void __launch_bounds__(kThreads, 1)
+attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
+                   const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_do, const Params p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  const uint32_t tmem =
+      kernel_prologue(reinterpret_cast<uint64_t*>(smem + Cfg<D>::DQ_BARS), &map_q, &map_k, &map_v, &map_do);
+  const int bh = blockIdx.x / p.n_qt, qt = blockIdx.x - bh * p.n_qt;
+  const int b = bh / p.H, h = bh - b * p.H;
+  const int grow = qt * kTile + threadIdx.x;
+  const uint8_t* o = static_cast<const uint8_t*>(p.o) + 2 * (b * p.o_sb + h * p.o_sh + grow * p.o_ss);
+  const uint8_t* g = static_cast<const uint8_t*>(p.dout) + 2 * (b * p.do_sb + h * p.do_sh + grow * p.do_ss);
+  const size_t i = (size_t)bh * (p.n_qt * kTile) + grow;
+  uint32_t q_ph = 0, kv_ph = 0, mma_ph = 0;
+  dq_term<D, kBf16>(smem, tmem, p, b, h, qt, &map_q, 0, &map_do, 0, &map_k, &map_v, 0, o, g, p.lse + i, p.delta + i,
+                    p.coef ? *p.coef : 1.0f, p.dq + b * p.dq_sb + h * p.dq_sh + (int64_t)grow * p.dq_ss, q_ph, kv_ph,
+                    mma_ph);
+  if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
+}
+
+// one CTA per (b, h, 128-row kv tile)
+template <int D, bool kBf16>
+__global__ void __launch_bounds__(kThreads, 1)
+attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
+                    const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_do, const Params p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  const uint32_t tmem =
+      kernel_prologue(reinterpret_cast<uint64_t*>(smem + Cfg<D>::DKV_BARS), &map_q, &map_k, &map_v, &map_do);
+  const int bh = blockIdx.x / p.n_kt, kt = blockIdx.x - bh * p.n_kt;
+  const int b = bh / p.H, h = bh - b * p.H;
+  const int krow = kt * kTile + threadIdx.x;
+  const size_t i = (size_t)bh * (p.n_qt * kTile);
+  uint32_t kv_ph = 0, q_ph = 0, mma_ph = 0;
+  dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, &map_k, &map_v, 0, &map_q, 0, &map_do, 0, p.lse + i, p.delta + i,
+                     p.coef ? *p.coef : 1.0f, p.dv + b * p.dv_sb + h * p.dv_sh + (int64_t)krow * p.dv_ss,
+                     p.dk + b * p.dk_sb + h * p.dk_sh + (int64_t)krow * p.dk_ss, kv_ph, q_ph, mma_ph);
+  if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
 // ---------------------------------------------------------------------------
@@ -815,9 +838,7 @@ struct GradT {   // an fp32 (N, B, H, S, D) gradient
   int64_t sn, sb, sh, ss;
 };
 
-struct ListParams {
-  int B, H, Sq, Skv, n_qt, n_kt;
-  float scale, scale_log2;
+struct ListParams : Shape {
   int n_groups;
   const int32_t* group_q;
   const int32_t* kv_idx;
@@ -846,62 +867,40 @@ struct FoldListParams : ListParams {
 template <bool kFold>
 using ListParamsT = std::conditional_t<kFold, FoldListParams, ListParams>;
 
-// attn_bwd_dq_kernel over a list: one CTA per (query image, b, h, 128-row q tile), the steps of that kernel once per
-// term, dQ drained (x the term's coefficient) into the fp32 rows before the next term
+// term tau = 2t (+ 1 for the self term) of a list: the slot of its dO factor and of its LSE / delta rows, and its
+// coefficient
+template <bool kFold>
+__device__ __forceinline__ float term_coef(const ListParamsT<kFold>& p, int tau, int& slot) {
+  const int t = tau >> 1;
+  const bool self = tau & 1;
+  if constexpr (kFold) {
+    slot = self ? (int)p.n_entries + p.entry_group[t] : t;
+    return self ? p.fold_scale[p.entry_group[t]] : p.coef[4 * t];
+  }
+  slot = tau;
+  return p.coef[4 * t + (self ? 1 : 0)];
+}
+
+// attn_bwd_dq_kernel over a list: one CTA per (query image, b, h, 128-row q tile), one dQ term per list entry, each
+// drained (x its coefficient) into the fp32 rows before the next
 template <int D, bool kBf16, bool kFold>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                         const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
                         const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
                         const ListParamsT<kFold> p) {
-  using C = Cfg<D>;
   const int per_list = p.B * p.H * p.n_qt;
   const int li = blockIdx.x / per_list;
   if (li >= *p.n_lists) return;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sQ = smem;
-  uint8_t* sDO = sQ + C::TILE_BYTES;
-  uint8_t* sK = sDO + C::TILE_BYTES;
-  uint8_t* sV = sK + C::TILE_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + C::TILE_BYTES);
-  uint64_t* q_bar = bars;
-  uint64_t* kv_bar = bars + 1;
-  uint64_t* mma_bar = bars + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const int tid = threadIdx.x, warp = tid >> 5;
+  const uint32_t tmem = kernel_prologue(reinterpret_cast<uint64_t*>(smem + Cfg<D>::DQ_BARS), &map_q, &map_k, &map_v,
+                                        &map_ks, &map_vs, &map_do);
   const int rest = blockIdx.x - li * per_list;
   const int bh = rest / p.n_qt, qt = rest - bh * p.n_qt;
   const int b = bh / p.H, h = bh - b * p.H;
-  const int grow = qt * kTile + tid;
-  const bool row_ok = grow < p.Sq;
+  const int grow = qt * kTile + threadIdx.x;
   const int qi = p.list_key[li];
   const int i0 = p.list_off[li], i1 = p.list_off[li + 1];
-
-  if (tid == 0) {
-    mbar_init(q_bar, 1);
-    mbar_init(kv_bar, 1);
-    mbar_init(mma_bar, 1);
-    fence_mbar_init();
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    tma_prefetch_desc(&map_ks);
-    tma_prefetch_desc(&map_vs);
-    tma_prefetch_desc(&map_do);
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  sync_all_tc();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
-  constexpr uint32_t kS = 0, kDP = 128, kDQ = 256;
-  const uint32_t fmt = kBf16 ? 1u : 0u;
-  const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, kTile, 0, 0);
-  const uint32_t idesc_dq = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
-  const float sl2 = p.scale_log2;
   const int64_t row_off = ((int64_t)b * p.H + h) * p.Sq * D + (int64_t)grow * D;   // in a contiguous (B, H, Sq, D) image
   float* dq_row = p.dq.ptr + qi * p.dq.sn + b * p.dq.sb + h * p.dq.sh + (int64_t)grow * p.dq.ss;
   uint32_t q_ph = 0, kv_ph = 0, mma_ph = 0;
@@ -909,164 +908,36 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
   for (int i = i0; i < i1; ++i) {
     const int tau = p.terms[i], t = tau >> 1;
     const bool self = tau & 1;
-    const int kv_img = self ? qi : p.kv_idx[t];
-    const CUtensorMap* mk = self ? &map_ks : &map_k;
-    const CUtensorMap* mv = self ? &map_vs : &map_v;
     const int64_t o_slot = self ? p.entry_group[t] : p.n_groups + t;
-    int slot = tau;   // of the dO factor and of the LSE / delta rows
-    if constexpr (kFold) slot = self ? (int)p.n_entries + p.entry_group[t] : t;
-    if (tid == 0) {
-      mbar_arrive_expect_tx(q_bar, 2 * C::TILE_BYTES);
-      load_tile<D>(sQ, &map_q, q_bar, kTile, qt * kTile, h, b, qi);
-      load_tile<D>(sDO, &map_do, q_bar, kTile, qt * kTile, h, b, slot);
-    }
-    __syncwarp();
-    float delta = 0.f;
-    if (row_ok)
-      delta = row_dot<kBf16>(static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
-                             static_cast<const uint16_t*>(p.f) + slot * p.img + row_off, D);
-    mbar_wait(q_bar, q_ph);
-    q_ph ^= 1;
-
-    // ---- pass 1: log-sum-exp of every row (log2 domain)
-    float m = -INFINITY, l = 0.f;
-    for (int kt = 0; kt < p.n_kt; ++kt) {
-      if (tid == 0) {
-        mbar_arrive_expect_tx(kv_bar, C::TILE_BYTES);
-        load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
-      }
-      __syncwarp();
-      mbar_wait(kv_bar, kv_ph);
-      kv_ph ^= 1;
-      if (tid == 0) {
-        tc_fence_after_sync();
-        mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);
-        umma_commit(mma_bar);
-      }
-      __syncwarp();
-      mbar_wait(mma_bar, mma_ph);
-      mma_ph ^= 1;
-      tc_fence_after_sync();
-      const int nv = p.Skv - kt * kTile;
-#pragma unroll 1
-      for (int c = 0; c < kTile / 32; ++c) {
-        uint32_t v[32];
-        tmem_ld_x32(lane_t + kS + c * 32, v);
-        tmem_wait_ld();
-        float mx = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          if (c * 32 + j >= nv) v[j] = 0xff800000u;
-          mx = fmaxf(mx, __uint_as_float(v[j]));
-        }
-        if (mx == -INFINITY) continue;
-        const float mn = fmaxf(m, mx);
-        float s = 0.f;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) s += fast_exp2((__uint_as_float(v[j]) - mn) * sl2);
-        l = l * fast_exp2((m - mn) * sl2) + s;
-        m = mn;
-      }
-      sync_all_tc();
-    }
-    const float lse2 = m * sl2 + __log2f(l);
-    {
-      const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
-      p.lse[k] = lse2;
-      p.delta[k] = delta;
-    }
-
-    // ---- pass 2: dQ
-    for (int kt = 0; kt < p.n_kt; ++kt) {
-      if (tid == 0) {
-        mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
-        load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
-        load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
-      }
-      __syncwarp();
-      mbar_wait(kv_bar, kv_ph);
-      kv_ph ^= 1;
-      if (tid == 0) {
-        tc_fence_after_sync();
-        mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);
-        mma_ss_kmajor<D>(tmem + kDP, sDO, kTile, sV, kTile, idesc_s);
-        umma_commit(mma_bar);
-      }
-      __syncwarp();
-      mbar_wait(mma_bar, mma_ph);
-      mma_ph ^= 1;
-      tc_fence_after_sync();
-      const int nv = p.Skv - kt * kTile;
-#pragma unroll 1
-      for (int c = 0; c < kTile / 32; ++c) {
-        uint32_t s[32], dp[32], pk[16];
-        tmem_ld_x32(lane_t + kS + c * 32, s);
-        tmem_ld_x32(lane_t + kDP + c * 32, dp);
-        tmem_wait_ld();
-#pragma unroll
-        for (int j = 0; j < 32; j += 2) {
-          float ds[2];
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const float pr = (c * 32 + j + e < nv) ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -lse2)) : 0.f;
-            ds[e] = pr * (__uint_as_float(dp[j + e]) - delta);
-          }
-          pk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
-        }
-        tmem_st_x16(lane_t + kS + c * 32, pk);
-      }
-      tmem_wait_st();
-      sync_all_tc();
-      if (tid == 0) {
-        mma_ts_mnmajor<D>(tmem + kDQ, tmem + kS, sK, kTile, idesc_dq, kt > 0);
-        umma_commit(mma_bar);
-      }
-      __syncwarp();
-      mbar_wait(mma_bar, mma_ph);
-      mma_ph ^= 1;
-      tc_fence_after_sync();
-    }
-
-    float fq;
-    if constexpr (kFold) fq = p.scale * (self ? p.fold_scale[p.entry_group[t]] : p.coef[4 * t]);
-    else fq = p.scale * p.coef[4 * t + (self ? 1 : 0)];
-    add_row_out<D>(lane_t + kDQ, fq, dq_row, row_ok);
-    sync_all_tc();   // dQ read out (and Q / dO free) before the next term
+    int slot;
+    const float coef = term_coef<kFold>(p, tau, slot);
+    const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
+    dq_term<D, kBf16>(smem, tmem, p, b, h, qt, &map_q, qi, &map_do, slot, self ? &map_ks : &map_k,
+                      self ? &map_vs : &map_v, self ? qi : p.kv_idx[t],
+                      static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
+                      static_cast<const uint16_t*>(p.f) + slot * p.img + row_off, p.lse + k, p.delta + k, coef, dq_row,
+                      q_ph, kv_ph, mma_ph);
   }
-  if (warp == 0) tmem_dealloc(tmem, 512);
+  if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
-// attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), the steps of that kernel once per term
+// attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), one dK/dV term per list entry
 template <int D, bool kBf16, bool kFold>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                          const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
                          const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
                          const ListParamsT<kFold> p) {
-  using C = Cfg<D>;
-  constexpr int BQ = C::BQ;
   const int per_list = p.B * p.H * p.n_kt;
   const int li = blockIdx.x / per_list;
   if (li >= *p.n_lists) return;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sK = smem;
-  uint8_t* sV = sK + C::TILE_BYTES;
-  uint8_t* sQ = sV + C::TILE_BYTES;
-  uint8_t* sDO = sQ + C::QB_BYTES;
-  float* sLse = reinterpret_cast<float*>(sDO + C::QB_BYTES);
-  float* sDelta = sLse + BQ;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sDelta + BQ);
-  uint64_t* kv_bar = bars;
-  uint64_t* q_bar = bars + 1;
-  uint64_t* mma_bar = bars + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const int tid = threadIdx.x, warp = tid >> 5;
+  const uint32_t tmem = kernel_prologue(reinterpret_cast<uint64_t*>(smem + Cfg<D>::DKV_BARS), &map_q, &map_k, &map_v,
+                                        &map_ks, &map_vs, &map_do);
   const int rest = blockIdx.x - li * per_list;
   const int bh = rest / p.n_kt, kt = rest - bh * p.n_kt;
   const int b = bh / p.H, h = bh - b * p.H;
-  const int krow = kt * kTile + tid;
-  const bool row_ok = krow < p.Skv;
+  const int krow = kt * kTile + threadIdx.x;
   int img = p.list_key[li];
   GradT gk = p.dk, gv = p.dv;
   if (img >= p.n_kbuf && p.n_kbuf > 0) {
@@ -1075,32 +946,6 @@ attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
     gv = p.dvs;
   }
   const int i0 = p.list_off[li], i1 = p.list_off[li + 1];
-
-  if (tid == 0) {
-    mbar_init(kv_bar, 1);
-    mbar_init(q_bar, 1);
-    mbar_init(mma_bar, 1);
-    fence_mbar_init();
-    tma_prefetch_desc(&map_q);
-    tma_prefetch_desc(&map_k);
-    tma_prefetch_desc(&map_v);
-    tma_prefetch_desc(&map_ks);
-    tma_prefetch_desc(&map_vs);
-    tma_prefetch_desc(&map_do);
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  sync_all_tc();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t lane_t = tmem + ((uint32_t)(warp * 32) << 16);
-  constexpr uint32_t kST = 0, kDPT = BQ, kDV = 2 * BQ, kDK = 2 * BQ + C::D_PAD;
-  const uint32_t fmt = kBf16 ? 1u : 0u;
-  const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, BQ, 0, 0);
-  const uint32_t idesc_o = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
-  const float sl2 = p.scale_log2;
-  const int n_qb = (p.Sq + BQ - 1) / BQ;
   float* dv_row = gv.ptr + img * gv.sn + b * gv.sb + h * gv.sh + (int64_t)krow * gv.ss;
   float* dk_row = gk.ptr + img * gk.sn + b * gk.sb + h * gk.sh + (int64_t)krow * gk.ss;
   uint32_t kv_ph = 0, q_ph = 0, mma_ph = 0;
@@ -1108,86 +953,14 @@ attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
   for (int i = i0; i < i1; ++i) {
     const int tau = p.terms[i], t = tau >> 1;
     const bool self = tau & 1;
-    const int qi = p.group_q[p.entry_group[t]];
-    int slot = tau;   // of the dO factor and of the LSE / delta rows
-    if constexpr (kFold) slot = self ? (int)p.n_entries + p.entry_group[t] : t;
-    if (tid == 0) {
-      mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
-      load_tile<D>(sK, self ? &map_ks : &map_k, kv_bar, kTile, kt * kTile, h, b, img);
-      load_tile<D>(sV, self ? &map_vs : &map_v, kv_bar, kTile, kt * kTile, h, b, img);
-    }
-    __syncwarp();
-    const float* lse_bh = p.lse + ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
-    const float* delta_bh = p.delta + ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
-    mbar_wait(kv_bar, kv_ph);
-    kv_ph ^= 1;
-    for (int qb = 0; qb < n_qb; ++qb) {
-      if (tid == 0) {
-        mbar_arrive_expect_tx(q_bar, 2 * C::QB_BYTES);
-        load_tile<D>(sQ, &map_q, q_bar, BQ, qb * BQ, h, b, qi);
-        load_tile<D>(sDO, &map_do, q_bar, BQ, qb * BQ, h, b, slot);
-      }
-      __syncwarp();
-      if (tid < BQ) {
-        sLse[tid] = lse_bh[qb * BQ + tid];
-        sDelta[tid] = delta_bh[qb * BQ + tid];
-      }
-      mbar_wait(q_bar, q_ph);
-      q_ph ^= 1;
-      if (tid == 0) {
-        tc_fence_after_sync();
-        mma_ss_kmajor<D>(tmem + kST, sK, kTile, sQ, BQ, idesc_s);
-        mma_ss_kmajor<D>(tmem + kDPT, sV, kTile, sDO, BQ, idesc_s);
-        umma_commit(mma_bar);
-      }
-      __syncwarp();
-      __syncthreads();
-      mbar_wait(mma_bar, mma_ph);
-      mma_ph ^= 1;
-      tc_fence_after_sync();
-      const int nq = p.Sq - qb * BQ;
-#pragma unroll 1
-      for (int c = 0; c < BQ / 32; ++c) {
-        uint32_t s[32], dp[32], pk[16], dk[16];
-        tmem_ld_x32(lane_t + kST + c * 32, s);
-        tmem_ld_x32(lane_t + kDPT + c * 32, dp);
-        tmem_wait_ld();
-#pragma unroll
-        for (int j = 0; j < 32; j += 2) {
-          float pr[2], ds[2];
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const int q = c * 32 + j + e;
-            pr[e] = q < nq ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -sLse[q])) : 0.f;
-            ds[e] = pr[e] * (__uint_as_float(dp[j + e]) - sDelta[q]);
-          }
-          pk[j >> 1] = pack2<kBf16>(pr[0], pr[1]);
-          dk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
-        }
-        tmem_st_x16(lane_t + kST + c * 32, pk);
-        tmem_st_x16(lane_t + kDPT + c * 32, dk);
-      }
-      tmem_wait_st();
-      sync_all_tc();
-      if (tid == 0) {
-        mma_ts_mnmajor<D>(tmem + kDV, tmem + kST, sDO, BQ, idesc_o, qb > 0);
-        mma_ts_mnmajor<D>(tmem + kDK, tmem + kDPT, sQ, BQ, idesc_o, qb > 0);
-        umma_commit(mma_bar);
-      }
-      __syncwarp();
-      mbar_wait(mma_bar, mma_ph);
-      mma_ph ^= 1;
-      tc_fence_after_sync();
-      __syncthreads();
-    }
-    float g;
-    if constexpr (kFold) g = self ? p.fold_scale[p.entry_group[t]] : p.coef[4 * t];
-    else g = p.coef[4 * t + (self ? 1 : 0)];
-    add_row_out<D>(lane_t + kDV, g, dv_row, row_ok);
-    add_row_out<D>(lane_t + kDK, g * p.scale, dk_row, row_ok);
-    sync_all_tc();   // dK / dV read out (and K / V free) before the next term
+    int slot;
+    const float coef = term_coef<kFold>(p, tau, slot);
+    const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
+    dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, self ? &map_ks : &map_k, self ? &map_vs : &map_v, img, &map_q,
+                       p.group_q[p.entry_group[t]], &map_do, slot, p.lse + k, p.delta + k, coef, dv_row, dk_row, kv_ph,
+                       q_ph, mma_ph);
   }
-  if (warp == 0) tmem_dealloc(tmem, 512);
+  if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
 // every element of the five gradients := NaN when bad[0] is set (an image index of the list was out of range)
@@ -1247,6 +1020,18 @@ static size_t stats_bytes(const ds_tensor4& q) {
   return 2 * align_up((size_t)(q.size[0] * q.size[1] * n_qt * kTile) * sizeof(float), 256);
 }
 
+// the Shape of the backward of q (., B, H, Sq, D) against k (., B, H, Skv, D)
+static void set_shape(Shape* s, const ds_tensor5& q, const ds_tensor5& k, float scale) {
+  s->B = (int)q.size[1];
+  s->H = (int)q.size[2];
+  s->Sq = (int)q.size[3];
+  s->Skv = (int)k.size[3];
+  s->n_qt = (s->Sq + kTile - 1) / kTile;
+  s->n_kt = (s->Skv + kTile - 1) / kTile;
+  s->scale = scale > 0.f ? scale : 1.0f / sqrtf((float)q.size[4]);
+  s->scale_log2 = s->scale * 1.4426950408889634f;
+}
+
 struct BwdArgs {
   ds_tensor4 q, k, v, out, dout, dq, dk, dv;
   float scale;
@@ -1260,20 +1045,13 @@ static int launch_bwd_t(const BwdArgs& a, cudaStream_t st) {
   using C = Cfg<D>;
   CUtensorMap mq, mk, mv, mdo, mqb, mdob;
   int rc;
-  const ds_tensor5 q = lift(a.q), dout = lift(a.dout);
-  if ((rc = make_map(&mq, q, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mk, lift(a.k), C::SUBW, kTile)) != DS_OK ||
+  const ds_tensor5 q = lift(a.q), k = lift(a.k), dout = lift(a.dout);
+  if ((rc = make_map(&mq, q, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mk, k, C::SUBW, kTile)) != DS_OK ||
       (rc = make_map(&mv, lift(a.v), C::SUBW, kTile)) != DS_OK || (rc = make_map(&mdo, dout, C::SUBW, kTile)) != DS_OK ||
       (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, dout, C::SUBW, C::BQ)) != DS_OK)
     return rc;
   Params p;
-  p.B = (int)a.q.size[0];
-  p.H = (int)a.q.size[1];
-  p.Sq = (int)a.q.size[2];
-  p.Skv = (int)a.k.size[2];
-  p.n_qt = (p.Sq + kTile - 1) / kTile;
-  p.n_kt = (p.Skv + kTile - 1) / kTile;
-  p.scale = a.scale > 0.f ? a.scale : 1.0f / sqrtf((float)D);
-  p.scale_log2 = p.scale * 1.4426950408889634f;
+  set_shape(&p, q, k, a.scale);
   p.o = a.out.ptr;
   p.o_sb = a.out.stride[0], p.o_sh = a.out.stride[1], p.o_ss = a.out.stride[2];
   p.dout = a.dout.ptr;
@@ -1347,7 +1125,7 @@ static bool extents_meet(const ds_tensor5& a, const ds_tensor5& b) {
   return a0 < end(b) && b0 < end(a);
 }
 
-// workspace layout of ds_aas_groups_bwd (the size query runs it on a dummy base)
+// workspace layout of ds_aas_groups_bwd (the size query runs it on a dummy base); ds_aas_matrix_bwd's extends it
 struct GroupsBwdWs {
   void* o;                 // (n_groups + n_entries) attention outputs, 16-bit
   void* f;                 // 2 n_entries dO factors, 16-bit
@@ -1359,6 +1137,17 @@ struct GroupsBwdWs {
   int32_t* bad;
   ListFamily fam[2];
 };
+
+// a contribution-list family of n_keys keys, at most max_lists lists and n_terms terms
+static bool take_family(Workspace& w, ListFamily* F, int64_t n_keys, int64_t max_lists, int64_t n_terms) {
+  F->n_keys = n_keys;
+  F->cnt = static_cast<int32_t*>(w.take((size_t)n_keys * 4));
+  F->n_lists = static_cast<int32_t*>(w.take(4));
+  F->list_key = static_cast<int32_t*>(w.take((size_t)max_lists * 4));
+  F->list_off = static_cast<int32_t*>(w.take((size_t)(max_lists + 1) * 4));
+  F->terms = static_cast<int32_t*>(w.take((size_t)n_terms * 4));
+  return F->cnt && F->n_lists && F->list_key && F->list_off && F->terms;
+}
 
 static bool groups_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor5& k, int64_t G, int64_t E,
                               GroupsBwdWs* L) {
@@ -1374,19 +1163,9 @@ static bool groups_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor
   L->delta = static_cast<float*>(w.take(stats));
   L->entry_group = static_cast<int32_t*>(w.take((size_t)E * 4));
   L->bad = static_cast<int32_t*>(w.take(4));
-  bool ok = L->o && L->f && L->part && L->coef && L->lse && L->delta && L->entry_group && L->bad;
-  const int64_t n_keys[2] = {q.size[0], k.size[0] + q.size[0]};
-  for (int i = 0; i < 2; ++i) {
-    ListFamily& F = L->fam[i];
-    F.n_keys = n_keys[i];
-    F.cnt = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
-    F.n_lists = static_cast<int32_t*>(w.take(4));
-    F.list_key = static_cast<int32_t*>(w.take((size_t)nt * 4));
-    F.list_off = static_cast<int32_t*>(w.take((size_t)(nt + 1) * 4));
-    F.terms = static_cast<int32_t*>(w.take((size_t)nt * 4));
-    ok = ok && F.cnt && F.n_lists && F.list_key && F.list_off && F.terms;
-  }
-  return ok;
+  const bool ok = L->o && L->f && L->part && L->coef && L->lse && L->delta && L->entry_group && L->bad;
+  return ok && take_family(w, &L->fam[0], q.size[0], nt, nt) &&
+         take_family(w, &L->fam[1], k.size[0] + q.size[0], nt, nt);
 }
 
 static GradT grad_t(const ds_tensor5& g) {
@@ -1437,21 +1216,13 @@ static ds_tensor5 factor_stack(const ds_tensor5& q, void* ptr, int64_t n_slots) 
   return F;
 }
 
-// ListParams of a checked list backward: shapes, grids (false: too many tiles) and everything but the lists
-static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, int64_t G, int64_t E, int n_kbuf,
-                        bool aliased, ListParams* p, int64_t* grid_q, int64_t* grid_kv) {
-  const int D = (int)q.size[4];
-  p->B = (int)q.size[1];
-  p->H = (int)q.size[2];
-  p->Sq = (int)q.size[3];
-  p->Skv = (int)k.size[3];
-  p->n_qt = (p->Sq + kTile - 1) / kTile;
-  p->n_kt = (p->Skv + kTile - 1) / kTile;
-  p->scale = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
-  p->scale_log2 = p->scale * 1.4426950408889634f;
+// ListParams of a checked list backward: shapes, grids (false: too many tiles) and everything but the pointers
+static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, int64_t G, int64_t E, bool aliased,
+                        ListParams* p, int64_t* grid_q, int64_t* grid_kv) {
+  set_shape(p, q, k, scale);
   p->n_groups = (int)G;
-  p->n_kbuf = n_kbuf;
-  p->img = q.size[1] * q.size[2] * q.size[3] * D;
+  p->n_kbuf = aliased ? 0 : (int)k.size[0];
+  p->img = q.size[1] * q.size[2] * q.size[3] * q.size[4];
   const int64_t bh = (int64_t)p->B * p->H;
   const int64_t nl_q = std::min<int64_t>(q.size[0], G);
   const int64_t nl_kv = aliased ? std::min<int64_t>(k.size[0], G + E) : nl_q + std::min<int64_t>(k.size[0], E);
@@ -1460,13 +1231,55 @@ static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, i
   return *grid_q < INT32_MAX && *grid_kv < INT32_MAX;
 }
 
-static void set_grads(ListParams* p, const ds_tensor5& dq, const ds_tensor5& dks, const ds_tensor5& dvs,
-                      const ds_tensor5& dk, const ds_tensor5& dv) {
+// the pointers of a ListParams: the work list, the workspace and the five gradients
+static void set_pointers(ListParams* p, const int32_t* group_q, const int32_t* kv_idx, const GroupsBwdWs& L,
+                         const ds_tensor5& dq, const ds_tensor5& dks, const ds_tensor5& dvs, const ds_tensor5& dk,
+                         const ds_tensor5& dv) {
+  p->group_q = group_q;
+  p->kv_idx = kv_idx;
+  p->entry_group = L.entry_group;
+  p->o = L.o;
+  p->f = L.f;
+  p->lse = L.lse;
+  p->delta = L.delta;
+  p->coef = L.coef;
   p->dq = grad_t(dq);
   p->dk = grad_t(dk);
   p->dv = grad_t(dv);
   p->dks = grad_t(dks);
   p->dvs = grad_t(dvs);
+}
+
+// the input of build_lists_kernel for the E entries of a list backward (the matrix adds n_cols); aliased: one dk / dv
+// buffer, whose self terms share the kv images' keys
+static void set_list_build(ListBuild* lb, const int32_t* group_q, const int32_t* kv_idx, int64_t E,
+                           const ds_tensor5& q, const ds_tensor5& k, bool aliased, const ListParams& p,
+                           const GroupsBwdWs& L) {
+  lb->group_q = group_q;
+  lb->kv_idx = kv_idx;
+  lb->entry_group = L.entry_group;
+  lb->bad = L.bad;
+  lb->n_terms = 2 * E;
+  lb->n_kbuf = p.n_kbuf;
+  lb->fam[0] = L.fam[0];
+  lb->fam[1] = L.fam[1];
+  lb->fam[1].n_keys = aliased ? k.size[0] : k.size[0] + q.size[0];
+}
+
+// per entry of a list backward: the (dot, |X|^2, |Y|^2) partials of X_t and Y_{group(t)} and the coefficients from
+// d_dir[t], exactly as one ds_aas_dir_bwd call computes them
+static int launch_list_coefs(const ds_tensor5& q, const ListParams& p, int64_t E, int mode, const float* d_dir,
+                             const GroupsBwdWs& L, cudaStream_t st) {
+  const uint32_t* ou = static_cast<const uint32_t*>(L.o);
+  const int64_t n2 = p.img / 2;
+  const dim3 grid(kRedBlocks, (unsigned)std::min<int64_t>(E, 65535));
+  const bool bf = q.dtype == DS_BF16;
+  if (bf) sim_partials_list_kernel<true><<<grid, kRedThreads, 0, st>>>(ou, n2, p.n_groups, E, L.entry_group, L.part);
+  else sim_partials_list_kernel<false><<<grid, kRedThreads, 0, st>>>(ou, n2, p.n_groups, E, L.entry_group, L.part);
+  DS_CUDA_TRY(cudaGetLastError());
+  sim_coef_list_kernel<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(L.part, E, mode, (double)p.img, d_dir, L.coef);
+  DS_CUDA_TRY(cudaGetLastError());
+  return DS_OK;
 }
 
 }  // namespace bwd
@@ -1611,56 +1424,35 @@ static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds
                              const ds_tensor5& dq, const ds_tensor5& dks, const ds_tensor5& dvs, const ds_tensor5& dk,
                              const ds_tensor5& dv, bool aliased, const GroupsBwdWs& L, const char* who, cudaStream_t st) {
   int rc;
-  const int D = (int)q.size[4];
-  const bool bf = q.dtype == DS_BF16;
   ListParams p;
   int64_t grid_q, grid_kv;
-  if (!list_params(q, k, scale, G, E, aliased ? 0 : (int)k.size[0], aliased, &p, &grid_q, &grid_kv))
+  if (!list_params(q, k, scale, G, E, aliased, &p, &grid_q, &grid_kv))
     return fail(DS_ERR_INVALID, "%s: too many tiles: split the work list", who);
-  const int64_t img = p.img, n2 = img / 2;
+  set_pointers(&p, group_q, kv_idx, L, dq, dks, dvs, dk, dv);
+  const int64_t n2 = p.img / 2;
+  const bool bf = q.dtype == DS_BF16;
 
   DS_CUDA_TRY(cudaMemsetAsync(L.bad, 0, sizeof(int32_t), st));
   if ((rc = launch_validate_groups(group_q, G, kv_idx, E, q.size[0], k.size[0], L.bad, st)) != DS_OK) return rc;
   entry_group_kernel<<<(unsigned)((std::max(G, E) + 255) / 256), 256, 0, st>>>(group_off, G, E, L.entry_group, L.bad);
   DS_CUDA_TRY(cudaGetLastError());
   ListBuild lb;
-  lb.group_q = group_q;
-  lb.kv_idx = kv_idx;
-  lb.entry_group = L.entry_group;
-  lb.bad = L.bad;
-  lb.n_terms = 2 * E;
-  lb.n_kbuf = p.n_kbuf;
-  lb.fam[0] = L.fam[0];
-  lb.fam[1] = L.fam[1];
-  lb.fam[1].n_keys = aliased ? k.size[0] : k.size[0] + q.size[0];
+  set_list_build(&lb, group_q, kv_idx, E, q, k, aliased, p, L);
   build_lists_kernel<false><<<2, kListThreads, 0, st>>>(lb);
   DS_CUDA_TRY(cudaGetLastError());
   // X_t and Y_g, rounded to the input dtype as ds_attn_fwd rounds them
   if ((rc = attn_list_store(q, ks, vs, k, v, group_q, group_off, G, kv_idx, scale, L.o, who, st)) != DS_OK) return rc;
+  if ((rc = launch_list_coefs(q, p, E, mode, d_dir, L, st)) != DS_OK) return rc;
   const uint32_t* ou = static_cast<const uint32_t*>(L.o);
   const unsigned ey = (unsigned)std::min<int64_t>(E, 65535);
-  if (bf) sim_partials_list_kernel<true><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)G, E, L.entry_group, L.part);
-  else sim_partials_list_kernel<false><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)G, E, L.entry_group, L.part);
-  DS_CUDA_TRY(cudaGetLastError());
-  sim_coef_list_kernel<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(L.part, E, mode, (double)img, d_dir, L.coef);
-  DS_CUDA_TRY(cudaGetLastError());
   const unsigned fb = (unsigned)std::min<int64_t>((n2 + 255) / 256, 4 * (int64_t)sm_count());
   uint32_t* fu = static_cast<uint32_t*>(L.f);
   if (bf) sim_factor_list_kernel<true><<<dim3(fb, ey), 256, 0, st>>>(ou, n2, (int)G, E, L.entry_group, mode, L.coef, fu);
   else sim_factor_list_kernel<false><<<dim3(fb, ey), 256, 0, st>>>(ou, n2, (int)G, E, L.entry_group, mode, L.coef, fu);
   DS_CUDA_TRY(cudaGetLastError());
 
-  p.group_q = group_q;
-  p.kv_idx = kv_idx;
-  p.entry_group = L.entry_group;
-  p.o = L.o;
-  p.f = L.f;
-  p.lse = L.lse;
-  p.delta = L.delta;
-  p.coef = L.coef;
-  set_grads(&p, dq, dks, dvs, dk, dv);
   const ds_tensor5 F = factor_stack(q, L.f, 2 * E);
-  rc = with_head_dim(D, who, [&](auto d) {
+  rc = with_head_dim(q.size[4], who, [&](auto d) {
     return with_dtype(q.dtype, [&](auto b) {
       return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value, false>(q, ks, vs, k, v, F, p, grid_q, grid_kv,
                                                                                 L.fam, st);
@@ -1806,23 +1598,16 @@ namespace ds {
 namespace bwd {
 
 // workspace layout of ds_aas_matrix_bwd (the size query runs it on a dummy base).  E = n_rows n_cols entries.
-struct MatrixBwdWs {
-  void* o;                 // (n_rows + E) attention outputs, 16-bit: Y_r at slot r, X_t at n_rows + t
-  void* f;                 // (E + n_rows) dO factors, 16-bit: fx_t at slot t, the folded F_r at E + r
+// The buffers of the grouped backward, with n_rows groups: o holds Y_r at slot r and X_t at n_rows + t; f, lse and delta
+// have E + n_rows slots, fx_t at slot t and the folded F_r at E + r.
+struct MatrixBwdWs : GroupsBwdWs {
   float* fold32;           // [n_rows] fp32 F_r images
-  float* part;             // [E][kRedBlocks][3]
-  float* coef;             // [E][4]
-  float* lse;              // [E + n_rows][B H][n_qt 128]
-  float* delta;
   float* fold_scale;       // [n_rows]
   int32_t* row_max;        // [n_rows]
   int32_t* group_q;        // [n_rows]
   int32_t* group_off;      // [n_rows + 1]
   int32_t* kv_idx;         // [E]
-  int32_t* entry_group;    // [E]
   float* d_dir;            // [E]
-  int32_t* bad;
-  ListFamily fam[2];
 };
 
 static bool matrix_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor5& k, MatrixBwdWs* L) {
@@ -1845,20 +1630,9 @@ static bool matrix_bwd_layout(Workspace& w, const ds_tensor5& q, const ds_tensor
   L->entry_group = static_cast<int32_t*>(w.take((size_t)E * 4));
   L->d_dir = static_cast<float*>(w.take((size_t)E * sizeof(float)));
   L->bad = static_cast<int32_t*>(w.take(4));
-  bool ok = L->o && L->f && L->fold32 && L->part && L->coef && L->lse && L->delta && L->fold_scale && L->row_max &&
-            L->group_q && L->group_off && L->kv_idx && L->entry_group && L->d_dir && L->bad;
-  const int64_t n_keys[2] = {R, Cn + R};
-  for (int i = 0; i < 2; ++i) {
-    ListFamily& F = L->fam[i];
-    F.n_keys = n_keys[i];
-    F.cnt = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
-    F.n_lists = static_cast<int32_t*>(w.take(4));
-    F.list_key = static_cast<int32_t*>(w.take((size_t)n_keys[i] * 4));
-    F.list_off = static_cast<int32_t*>(w.take((size_t)(n_keys[i] + 1) * 4));
-    F.terms = static_cast<int32_t*>(w.take((size_t)nt * 4));
-    ok = ok && F.cnt && F.n_lists && F.list_key && F.list_off && F.terms;
-  }
-  return ok;
+  const bool ok = L->o && L->f && L->fold32 && L->part && L->coef && L->lse && L->delta && L->fold_scale &&
+                  L->row_max && L->group_q && L->group_off && L->kv_idx && L->entry_group && L->d_dir && L->bad;
+  return ok && take_family(w, &L->fam[0], R, R, nt) && take_family(w, &L->fam[1], Cn + R, Cn + R, nt);
 }
 
 }  // namespace bwd
@@ -1891,7 +1665,7 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   if (rc != DS_OK) return rc;
   ListParamsT<true> p;
   int64_t grid_q, grid_kv;
-  if (!list_params(q, k, scale, R, E, aliased ? 0 : (int)Cn, aliased, &p, &grid_q, &grid_kv))
+  if (!list_params(q, k, scale, R, E, aliased, &p, &grid_q, &grid_kv))
     return fail(DS_ERR_INVALID, "%s: too many tiles: split the rows", who);
   Workspace w(ws, ws_bytes);
   MatrixBwdWs L;
@@ -1899,6 +1673,9 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
     return fail(DS_ERR_WORKSPACE, "%s: workspace too small (%zu given, need %zu)", who, ws_bytes,
                 ds_aas_matrix_bwd_workspace_bytes(q, k));
   if ((rc = ds_device_ok()) != DS_OK) return rc;
+  set_pointers(&p, L.group_q, L.kv_idx, L, dq, dk_self, dv_self, dk, dv);
+  p.n_entries = E;
+  p.fold_scale = L.fold_scale;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t n2 = p.img / 2;
   const bool bf = q.dtype == DS_BF16;
@@ -1909,28 +1686,16 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
                                                                       L.entry_group, L.d_dir);
   DS_CUDA_TRY(cudaGetLastError());
   ListBuildT<true> lb;
-  lb.group_q = L.group_q;
-  lb.kv_idx = L.kv_idx;
-  lb.entry_group = L.entry_group;
-  lb.bad = L.bad;
-  lb.n_terms = 2 * E;
-  lb.n_kbuf = p.n_kbuf;
-  lb.fam[0] = L.fam[0];
-  lb.fam[1] = L.fam[1];
-  lb.fam[1].n_keys = aliased ? Cn : Cn + R;
+  set_list_build(&lb, L.group_q, L.kv_idx, E, q, k, aliased, p, L);
   lb.n_cols = (int)Cn;
   build_lists_kernel<true><<<2, kListThreads, 0, st>>>(lb);
   DS_CUDA_TRY(cudaGetLastError());
   // X_t and Y_r, rounded to the input dtype as ds_attn_fwd rounds them
   if ((rc = attn_list_store(q, k_self, v_self, k, v, L.group_q, L.group_off, R, L.kv_idx, scale, L.o, who, st)) != DS_OK)
     return rc;
+  if ((rc = launch_list_coefs(q, p, E, mode, L.d_dir, L, st)) != DS_OK) return rc;
   const uint32_t* ou = static_cast<const uint32_t*>(L.o);
-  const unsigned ey = (unsigned)std::min<int64_t>(E, 65535), ry = (unsigned)std::min<int64_t>(R, 65535);
-  if (bf) sim_partials_list_kernel<true><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)R, E, L.entry_group, L.part);
-  else sim_partials_list_kernel<false><<<dim3(kRedBlocks, ey), kRedThreads, 0, st>>>(ou, n2, (int)R, E, L.entry_group, L.part);
-  DS_CUDA_TRY(cudaGetLastError());
-  sim_coef_list_kernel<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(L.part, E, mode, (double)p.img, L.d_dir, L.coef);
-  DS_CUDA_TRY(cudaGetLastError());
+  const unsigned ry = (unsigned)std::min<int64_t>(R, 65535);
   const unsigned fb = (unsigned)std::min<int64_t>((n2 + 255) / 256, 4 * (int64_t)sm_count());
   uint32_t* fu = static_cast<uint32_t*>(L.f);
   float2* f32 = reinterpret_cast<float2*>(L.fold32);
@@ -1942,17 +1707,6 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   else matrix_fold_round_kernel<false><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
   DS_CUDA_TRY(cudaGetLastError());
 
-  p.group_q = L.group_q;
-  p.kv_idx = L.kv_idx;
-  p.entry_group = L.entry_group;
-  p.o = L.o;
-  p.f = L.f;
-  p.lse = L.lse;
-  p.delta = L.delta;
-  p.coef = L.coef;
-  p.n_entries = E;
-  p.fold_scale = L.fold_scale;
-  set_grads(&p, dq, dk_self, dv_self, dk, dv);
   const ds_tensor5 F = factor_stack(q, L.f, E + R);
   return with_head_dim(q.size[4], who, [&](auto d) {
     return with_dtype(q.dtype, [&](auto b) {
