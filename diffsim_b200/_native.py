@@ -83,6 +83,8 @@ PROTOTYPES = {
     "ds_aas_matrix_workspace_bytes": (_sz, [Tensor5, Tensor5]),
     "ds_pair_reduce": (_i, [_vp, _vp, _i64, _i64, _i64, _i64, _i, _i, _vp, _vp, _sz, _vp]),
     "ds_pair_reduce_workspace_bytes": (_sz, [_i64, _i64]),
+    "ds_pair_reduce_bwd": (_i, [_vp, _vp, _i64, _i64, _i64, _i64, _i, _i, _vp, _vp, _i64, _vp, _i64, _vp, _sz, _vp]),
+    "ds_pair_reduce_bwd_workspace_bytes": (_sz, [_i64, _i64]),
     "ds_simmat": (_i, [_vp, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _vp, _i64, _vp, _sz, _vp]),
     "ds_simmat_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "ds_qkv_project": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _i64, _i64, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), _i, _vp]),

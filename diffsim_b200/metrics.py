@@ -13,6 +13,9 @@ tensors its model returned, and replaces the torch arithmetic that follows with 
     ffa_similarity     metrics/foreground_feature_averaging.py:90   cosine of two masked-mean embeddings -> K2
     all_pairs          N x N form of feature_score / diffeats_score                            -> K3
 
+Every score but ffa_similarity (a Python float, as in the reference) and all_pairs is differentiable in its tensor
+inputs: the attention (K5), projection (K4) and reduction (K2) backwards run when an input requires grad.
+
 The backbones themselves (CLIP, DINOv2, VGG, CarveKit) are out of scope; none is installed offline.
 """
 from __future__ import annotations
@@ -52,8 +55,12 @@ def attention_calc(q, k, v, scale: Optional[float], hidden_size_shape: Sequence[
     B, H, S, D = q.shape
     if (B, S, H * D) != (bsz, tgt_len, embed_dim):
         raise RuntimeError(f"hidden_size_shape {tuple(hidden_size_shape)} does not match q {tuple(q.shape)}")
-    merged = torch.empty((B, S, H, D), dtype=q.dtype, device=q.device)
-    ops.attn_fwd(q, k, v, scale, out=merged.permute(0, 2, 1, 3))
+    if ops.wants_grad(q, k, v):
+        # the differentiable attention allocates its (B,H,S,D) output over (B,S,H*D) memory: merging heads is a view
+        merged = ops.attn_fwd(q, k, v, scale).permute(0, 2, 1, 3)
+    else:
+        merged = torch.empty((B, S, H, D), dtype=q.dtype, device=q.device)
+        ops.attn_fwd(q, k, v, scale, out=merged.permute(0, 2, 1, 3))
     (out,) = ops.qkv_project(merged.view(B, S, H * D), out_proj_weight, out_proj_bias, n_outputs=1)
     return out
 

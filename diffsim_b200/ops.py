@@ -564,23 +564,82 @@ def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=None, out=No
 def pair_reduce(x: torch.Tensor, y: torch.Tensor, similarity="cosine") -> torch.Tensor:
     """sim(x[p], y[p]) over the flattened trailing dims, for every leading row p.  x, y: (P, ...) tensors whose rows
     are contiguous.  Replaces F.cosine_similarity on flattened tensors / F.mse_loss / min-max + cosine
-    (diffsim/diffsim.py:182-195, metrics/diffeats.py:136-140,202-205).  Returns float32 [P]."""
+    (diffsim/diffsim.py:182-195, metrics/diffeats.py:136-140,202-205).  Returns float32 [P].  Differentiable in x and
+    y (pair_reduce_bwd) when one of them requires grad; the values are the same either way."""
+    if wants_grad(x, y):
+        return _PairReduceFn.apply(similarity, x, y)
+    return _pair_reduce(x, y, similarity)
+
+
+def _rows(x: torch.Tensor, y: torch.Tensor):
+    """(x, y) as (P, E) views with unit column stride, copied only when the flattened rows are not contiguous."""
+    P = x.shape[0]
+    x2, y2 = x.reshape(P, -1), y.reshape(P, -1)
+    if x2.stride(1) != 1:
+        x2 = x2.contiguous()
+    if y2.stride(1) != 1:
+        y2 = y2.contiguous()
+    return x2, y2
+
+
+def _row_stride(t: torch.Tensor) -> int:
+    return t.stride(0) if t.shape[0] > 1 else t.shape[1]
+
+
+def _pair_reduce(x, y, similarity="cosine") -> torch.Tensor:
     dev = _need_cuda(x, y)
     if x.shape != y.shape or x.dtype != y.dtype:
         raise RuntimeError("x and y must have the same shape and dtype")
     P = x.shape[0]
     if P == 0:
         return torch.empty(0, dtype=torch.float32, device=dev)
-    x2, y2 = x.reshape(P, -1), y.reshape(P, -1)
-    if x2.stride(1) != 1:
-        x2 = x2.contiguous()
-    if y2.stride(1) != 1:
-        y2 = y2.contiguous()
+    x2, y2 = _rows(x, y)
     E = x2.shape[1]
     out = torch.empty(P, dtype=torch.float32, device=dev)
-    _call("ds_pair_reduce", dev, x2.data_ptr(), y2.data_ptr(), P, E, x2.stride(0) if P > 1 else E,
-          y2.stride(0) if P > 1 else E, _dtype_code(x2), _mode(similarity), out.data_ptr(), ws_query=(P, E), launches=1)
+    _call("ds_pair_reduce", dev, x2.data_ptr(), y2.data_ptr(), P, E, _row_stride(x2), _row_stride(y2), _dtype_code(x2),
+          _mode(similarity), out.data_ptr(), ws_query=(P, E), launches=1)
     return out
+
+
+def pair_reduce_bwd(x: torch.Tensor, y: torch.Tensor, d_out: torch.Tensor, similarity="cosine", need_x: bool = True,
+                    need_y: bool = True) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """float32 gradients (dx, dy) of pair_reduce(x, y, similarity) for dL/dout = d_out (P values on the device), in
+    the shapes of x and y, None where not asked for (and then not computed) -- ds_pair_reduce_bwd: the float64 autograd
+    gradients of the reference's expressions, deterministic (no atomics)."""
+    dev = _need_cuda(x, y, d_out)
+    if x.shape != y.shape or x.dtype != y.dtype:
+        raise RuntimeError("x and y must have the same shape and dtype")
+    P = x.shape[0]
+    g = d_out.detach().reshape(-1).to(torch.float32).contiguous()
+    if g.numel() != P:
+        raise RuntimeError("d_out must have one value per row")
+    dx = torch.empty(x.shape, dtype=torch.float32, device=dev) if need_x else None
+    dy = torch.empty(y.shape, dtype=torch.float32, device=dev) if need_y else None
+    if P == 0 or (dx is None and dy is None):
+        return dx, dy
+    x2, y2 = _rows(x, y)
+    E = x2.shape[1]
+    mode = _mode(similarity)
+    _call("ds_pair_reduce_bwd", dev, x2.data_ptr(), y2.data_ptr(), P, E, _row_stride(x2), _row_stride(y2),
+          _dtype_code(x2), mode, g.data_ptr(), None if dx is None else dx.data_ptr(), E,
+          None if dy is None else dy.data_ptr(), E, ws_query=(P, E), slot="bwd",
+          launches=1 if mode == N.DS_SIM_MSE else 2)  # (statistics +) gradient pass
+    return dx, dy
+
+
+class _PairReduceFn(torch.autograd.Function):
+    """pair_reduce with the K2 backward; saves only x and y (the backward recomputes the row statistics)."""
+
+    @staticmethod
+    def forward(ctx, similarity, x, y):
+        ctx.save_for_backward(x, y)
+        ctx.similarity = similarity
+        return _pair_reduce(x, y, similarity)
+
+    @staticmethod
+    def backward(ctx, d_out):
+        x, y = ctx.saved_tensors
+        return (None,) + pair_reduce_bwd(x, y, d_out, ctx.similarity, ctx.needs_input_grad[1], ctx.needs_input_grad[2])
 
 
 # --------------------------------------------------------------------------------------

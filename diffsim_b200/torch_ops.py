@@ -58,7 +58,7 @@ def _aas_matrix(q, k_self, v_self, k, v, similarity="cosine", scale=0.0):
 
 
 def _pair_reduce(x, y, similarity="cosine"):
-    return ops.pair_reduce(x, y, similarity)
+    return ops._pair_reduce(x, y, similarity)   # forward only: no autograd registered
 
 
 def _simmat(rows, cols=None, similarity="cosine"):

@@ -300,6 +300,29 @@ int ds_pair_reduce(const void* x, const void* y, int64_t n_pairs, int64_t E,
                    float* out, void* ws, size_t ws_bytes, void* stream);
 size_t ds_pair_reduce_workspace_bytes(int64_t n_pairs, int64_t E);
 
+/*
+ * Backward of ds_pair_reduce: for row p with g = d_out[p] (float[n_pairs] on the device, no host sync), the gradients
+ * of out[p] that float64 torch autograd gives on the same inputs:
+ *   cosine  s = x.y / (nx ny), n = max(|.|, 1e-8):  dx = g (y / (nx ny) - s x / (nx |x|)), the second term 0 when
+ *           |x| = 0 (torch clamps the norm without a gradient); dy symmetric.
+ *   mse     dx = 2 g (x - y) / E,  dy = -dx.
+ *   minmax  x^ = (x - m) / (M - m) with the row's min m and max M, G = dcos/dx^ by the cosine rule:
+ *           dx = g (G / (M - m) + [x = m] S_m / n_m + [x = M] S_M / n_M),
+ *           S_m = sum G (x^ - 1) / (M - m), S_M = -sum G x^ / (M - m), n_m / n_M the numbers of elements equal to m / M
+ *           (t.min() / t.max() split the gradient evenly among ties); dy symmetric.  A constant row (M = m) has a NaN
+ *           score and gets NaN gradients in that row only.
+ * x, y, n_pairs, E, strides, dtype and mode as for ds_pair_reduce.  dx, dy: float[n_pairs, E] with row strides
+ * dx_stride, dy_stride (>= E) elements, written (not added into); either may be null (not computed), and both null is
+ * DS_OK and does nothing.  Launches: a counter memset, a statistics pass (the forward's reduction plus min / max tie
+ * counts) and one elementwise gradient pass; mse runs the gradient pass only.  No float atomics: repeated calls are
+ * bitwise equal.
+ */
+size_t ds_pair_reduce_bwd_workspace_bytes(int64_t n_pairs, int64_t E);
+int ds_pair_reduce_bwd(const void* x, const void* y, int64_t n_pairs, int64_t E, int64_t x_stride, int64_t y_stride,
+                       int dtype, int mode, const float* d_out,
+                       float* dx, int64_t dx_stride, float* dy, int64_t dy_stride,
+                       void* ws, size_t ws_bytes, void* stream);
+
 /* ---- K3: N x N similarity matrix of feature vectors --------------------- */
 
 /*
