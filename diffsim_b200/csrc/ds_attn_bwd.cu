@@ -183,9 +183,10 @@ __device__ __forceinline__ uint32_t kernel_prologue(uint64_t* bars, const Maps*.
 // One term of a dQ kernel, on the 128-row q tile qt of (b, h): the Q and dO tiles (images q_img of mq and do_img of
 // mdo), delta = rowsum(dO o O) from this thread's 16-bit rows o_row and do_row, the LSE pass and the dS / dQ pass over
 // the kv tiles of image kv_img of mk and mv.  LSE and delta go to *lse and *delta_out, dQ x scale coef is added into
-// dq_row.
+// dq_row.  kStats: the statistics only -- LSE and delta are written, there is no dS / dQ pass and no drain (dq_row is
+// not read).
 // The barrier phases carry over to the next term.
-template <int D, bool kBf16>
+template <int D, bool kBf16, bool kStats = false>
 __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shape& p, int b, int h, int qt,
                                         const CUtensorMap* mq, int q_img, const CUtensorMap* mdo, int do_img,
                                         const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, const void* o_row,
@@ -264,60 +265,62 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
   const float lse2 = m * sl2 + __log2f(l);
   *lse = lse2;
   *delta_out = delta;
-
-  // ---- pass 2: dQ
-  for (int kt = 0; kt < p.n_kt; ++kt) {
-    if (tid == 0) {
-      mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
-      load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
-      load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
-    }
-    __syncwarp();
-    mbar_wait(kv_bar, kv_ph);
-    kv_ph ^= 1;
-    if (tid == 0) {
-      tc_fence_after_sync();
-      mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);    // S = Q K^T
-      mma_ss_kmajor<D>(tmem + kDP, sDO, kTile, sV, kTile, idesc_s);  // dP = dO V^T
-      umma_commit(mma_bar);
-    }
-    __syncwarp();
-    mbar_wait(mma_bar, mma_ph);
-    mma_ph ^= 1;
-    tc_fence_after_sync();
-    const int nv = p.Skv - kt * kTile;
-#pragma unroll 1
-    for (int c = 0; c < kTile / 32; ++c) {
-      uint32_t s[32], dp[32], pk[16];
-      tmem_ld_x32(lane_t + kS + c * 32, s);
-      tmem_ld_x32(lane_t + kDP + c * 32, dp);
-      tmem_wait_ld();
-#pragma unroll
-      for (int j = 0; j < 32; j += 2) {
-        float ds[2];
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-          const float pr = (c * 32 + j + e < nv) ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -lse2)) : 0.f;
-          ds[e] = pr * (__uint_as_float(dp[j + e]) - delta);
-        }
-        pk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
+  // kStats: the last tile's sync_all_tc has freed S, Q and dO for the next term
+  if constexpr (!kStats) {
+    // ---- pass 2: dQ
+    for (int kt = 0; kt < p.n_kt; ++kt) {
+      if (tid == 0) {
+        mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
+        load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
+        load_tile<D>(sV, mv, kv_bar, kTile, kt * kTile, h, b, kv_img);
       }
-      tmem_st_x16(lane_t + kS + c * 32, pk);   // dS over the first 16 of the 32 S columns just read
+      __syncwarp();
+      mbar_wait(kv_bar, kv_ph);
+      kv_ph ^= 1;
+      if (tid == 0) {
+        tc_fence_after_sync();
+        mma_ss_kmajor<D>(tmem + kS, sQ, kTile, sK, kTile, idesc_s);    // S = Q K^T
+        mma_ss_kmajor<D>(tmem + kDP, sDO, kTile, sV, kTile, idesc_s);  // dP = dO V^T
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);
+      mma_ph ^= 1;
+      tc_fence_after_sync();
+      const int nv = p.Skv - kt * kTile;
+#pragma unroll 1
+      for (int c = 0; c < kTile / 32; ++c) {
+        uint32_t s[32], dp[32], pk[16];
+        tmem_ld_x32(lane_t + kS + c * 32, s);
+        tmem_ld_x32(lane_t + kDP + c * 32, dp);
+        tmem_wait_ld();
+#pragma unroll
+        for (int j = 0; j < 32; j += 2) {
+          float ds[2];
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const float pr = (c * 32 + j + e < nv) ? fast_exp2(fmaf(__uint_as_float(s[j + e]), sl2, -lse2)) : 0.f;
+            ds[e] = pr * (__uint_as_float(dp[j + e]) - delta);
+          }
+          pk[j >> 1] = pack2<kBf16>(ds[0], ds[1]);
+        }
+        tmem_st_x16(lane_t + kS + c * 32, pk);   // dS over the first 16 of the 32 S columns just read
+      }
+      tmem_wait_st();
+      sync_all_tc();
+      if (tid == 0) {
+        mma_ts_mnmajor<D>(tmem + kDQ, tmem + kS, sK, kTile, idesc_dq, kt > 0);   // dQ += dS K
+        umma_commit(mma_bar);
+      }
+      __syncwarp();
+      mbar_wait(mma_bar, mma_ph);   // K / V buffers and the S columns are free again
+      mma_ph ^= 1;
+      tc_fence_after_sync();
     }
-    tmem_wait_st();
-    sync_all_tc();
-    if (tid == 0) {
-      mma_ts_mnmajor<D>(tmem + kDQ, tmem + kS, sK, kTile, idesc_dq, kt > 0);   // dQ += dS K
-      umma_commit(mma_bar);
-    }
-    __syncwarp();
-    mbar_wait(mma_bar, mma_ph);   // K / V buffers and the S columns are free again
-    mma_ph ^= 1;
-    tc_fence_after_sync();
-  }
 
-  add_row_out<D>(lane_t + kDQ, p.scale * coef, dq_row, row_ok);
-  sync_all_tc();   // dQ read out (and Q / dO free) before the next term
+    add_row_out<D>(lane_t + kDQ, p.scale * coef, dq_row, row_ok);
+    sync_all_tc();   // dQ read out (and Q / dO free) before the next term
+  }
 }
 
 // One term of a dK/dV kernel, on the 128-row kv tile kt of (b, h): the K and V tiles (image kv_img of mk and mv), then
@@ -608,18 +611,26 @@ struct ListBuild {
 };
 
 // ds_aas_matrix_bwd: the row-major matrix list (group r = row r, n_cols entries), with ONE self term per row -- the folded
-// one, at tau = 2t + 1 of the row's last entry t, so that it follows the row's cross terms
+// one, at tau = 2t + 1 of the row's last entry t, so that it follows the row's cross terms.  rows: the row terms are
+// wanted (dQ of every term, dK / dV of the folded self terms); cols: the column terms (dK / dV of the cross terms).
+// Without rows no self term is live; without cols the dK / dV family holds the self terms only.  The dQ family keeps
+// the cross terms either way: without rows it drives the statistics-only dQ kernel.
 struct FoldListBuild : ListBuild {
   int n_cols;
+  bool rows, cols;
 };
 
 template <bool kFold>
 using ListBuildT = std::conditional_t<kFold, FoldListBuild, ListBuild>;
 
 template <bool kFold>
-__device__ __forceinline__ bool term_live(const ListBuildT<kFold>& b, int64_t tau) {
-  if constexpr (kFold) return !(tau & 1) || ((tau >> 1) + 1) % b.n_cols == 0;
-  else return true;
+__device__ __forceinline__ bool term_live(const ListBuildT<kFold>& b, int family, int64_t tau) {
+  if constexpr (kFold) {
+    if (tau & 1) return b.rows && ((tau >> 1) + 1) % b.n_cols == 0;
+    return family == 0 || b.cols;
+  } else {
+    return true;
+  }
 }
 
 __device__ __forceinline__ int term_key(const ListBuild& b, int family, int64_t tau) {
@@ -680,7 +691,7 @@ __global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBui
   for (int64_t k = threadIdx.x; k < L.n_keys; k += kListThreads) L.cnt[k] = 0;
   __syncthreads();
   for (int64_t tau = threadIdx.x; tau < b.n_terms; tau += kListThreads)
-    if (term_live<kFold>(b, tau)) atomicAdd(&L.cnt[term_key(b, f, tau)], 1);
+    if (term_live<kFold>(b, f, tau)) atomicAdd(&L.cnt[term_key(b, f, tau)], 1);
   __syncthreads();
   int n_lists = 0, n_seen = 0;   // running totals over the key chunks
   for (int64_t k0 = 0; k0 < L.n_keys; k0 += kListThreads) {
@@ -703,7 +714,7 @@ __global__ void __launch_bounds__(kListThreads) build_lists_kernel(const ListBui
   __syncthreads();
   for (int64_t t0 = 0; t0 < b.n_terms; t0 += kListThreads) {
     const int64_t tau = t0 + threadIdx.x;
-    const bool live = tau < b.n_terms && term_live<kFold>(b, tau);
+    const bool live = tau < b.n_terms && term_live<kFold>(b, f, tau);
     const int key = live ? term_key(b, f, tau) : -1;
     s_key[threadIdx.x] = key;
     __syncthreads();
@@ -766,8 +777,9 @@ __global__ void matrix_bwd_setup_kernel(int64_t n_rows, int64_t n_cols, const fl
 
 // per row r and element pair: fx_t of every entry t = (r, c) as sim_factor rounds it, and the fp32 fold
 // F_r = sum over ascending c of coef[4t + 1] fy_t, fy_t unrounded (F32 [r][n2]); row_max[r] (zeroed before): max |F_r|
-// as float bits (non-negative floats order as integers, so the integer atomic is order-independent)
-template <bool kBf16>
+// as float bits (non-negative floats order as integers, so the integer atomic is order-independent).
+// kSum = false: fx_t only, for a call without the row terms (no fold, F32 and row_max are not touched).
+template <bool kBf16, bool kSum = true>
 __global__ void matrix_fold_kernel(const uint32_t* __restrict__ o, int64_t n2, int n_rows, int n_cols, int mode,
                                    const float* __restrict__ coef, uint32_t* __restrict__ fx, float2* __restrict__ F32,
                                    int32_t* __restrict__ row_max) {
@@ -793,21 +805,27 @@ __global__ void matrix_fold_kernel(const uint32_t* __restrict__ o, int64_t n2, i
           fy0 = a.x - ky * c.x;
           fy1 = a.y - ky * c.y;
         }
-        fx0 = fmaf(cf[1], fy0, fx0);
-        fx1 = fmaf(cf[1], fy1, fx1);
+        if constexpr (kSum) {
+          fx0 = fmaf(cf[1], fy0, fx0);
+          fx1 = fmaf(cf[1], fy1, fx1);
+        }
       }
-      F32[(int64_t)r * n2 + i] = make_float2(fx0, fx1);
-      mx = fmaxf(mx, fmaxf(fabsf(fx0), fabsf(fx1)));
+      if constexpr (kSum) {
+        F32[(int64_t)r * n2 + i] = make_float2(fx0, fx1);
+        mx = fmaxf(mx, fmaxf(fabsf(fx0), fabsf(fx1)));
+      }
     }
+    if constexpr (kSum) {
 #pragma unroll
-    for (int o2 = 16; o2 > 0; o2 >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o2));
-    if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = mx;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      for (int w = 1; w < kRedThreads / 32; ++w) mx = fmaxf(mx, s_max[w]);
-      atomicMax(row_max + r, __float_as_int(mx));
+      for (int o2 = 16; o2 > 0; o2 >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o2));
+      if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = mx;
+      __syncthreads();
+      if (threadIdx.x == 0) {
+        for (int w = 1; w < kRedThreads / 32; ++w) mx = fmaxf(mx, s_max[w]);
+        atomicMax(row_max + r, __float_as_int(mx));
+      }
+      __syncthreads();
     }
-    __syncthreads();
   }
 }
 
@@ -882,8 +900,9 @@ __device__ __forceinline__ float term_coef(const ListParamsT<kFold>& p, int tau,
 }
 
 // attn_bwd_dq_kernel over a list: one CTA per (query image, b, h, 128-row q tile), one dQ term per list entry, each
-// drained (x its coefficient) into the fp32 rows before the next
-template <int D, bool kBf16, bool kFold>
+// drained (x its coefficient) into the fp32 rows before the next.  kStats: only every term's LSE and delta (dq_term's
+// statistics-only form), for a dK/dV list that runs without the dQ gradient.
+template <int D, bool kBf16, bool kFold, bool kStats = false>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                         const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
@@ -912,7 +931,7 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
     int slot;
     const float coef = term_coef<kFold>(p, tau, slot);
     const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
-    dq_term<D, kBf16>(smem, tmem, p, b, h, qt, &map_q, qi, &map_do, slot, self ? &map_ks : &map_k,
+    dq_term<D, kBf16, kStats>(smem, tmem, p, b, h, qt, &map_q, qi, &map_do, slot, self ? &map_ks : &map_k,
                       self ? &map_vs : &map_v, self ? qi : p.kv_idx[t],
                       static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
                       static_cast<const uint16_t*>(p.f) + slot * p.img + row_off, p.lse + k, p.delta + k, coef, dq_row,
@@ -1172,7 +1191,8 @@ static GradT grad_t(const ds_tensor5& g) {
   return GradT{static_cast<float*>(g.ptr), g.stride[0], g.stride[1], g.stride[2], g.stride[3]};
 }
 
-template <int D, bool kBf16, bool kFold>
+// the dQ and dK/dV list kernels of a list backward; kStats: the dQ kernel in its statistics-only form
+template <int D, bool kBf16, bool kFold, bool kStats = false>
 static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
                                const ds_tensor5& v, const ds_tensor5& F, ListParamsT<kFold> p, int64_t grid_q,
                                int64_t grid_kv, const ListFamily* fam, cudaStream_t st) {
@@ -1184,7 +1204,7 @@ static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const 
       (rc = make_map(&mvs, vs, C::SUBW, kTile)) != DS_OK || (rc = make_map(&mdo, F, C::SUBW, kTile)) != DS_OK ||
       (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, F, C::SUBW, C::BQ)) != DS_OK)
     return rc;
-  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_list_kernel<D, kBf16, kFold>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_list_kernel<D, kBf16, kFold, kStats>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    C::DQ_SMEM));
   DS_CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dkv_list_kernel<D, kBf16, kFold>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    C::DKV_SMEM));
@@ -1192,7 +1212,8 @@ static int launch_groups_bwd_t(const ds_tensor5& q, const ds_tensor5& ks, const 
   p.list_key = fam[0].list_key;
   p.list_off = fam[0].list_off;
   p.terms = fam[0].terms;
-  attn_bwd_dq_list_kernel<D, kBf16, kFold><<<(unsigned)grid_q, kThreads, C::DQ_SMEM, st>>>(mq, mk, mv, mks, mvs, mdo, p);
+  attn_bwd_dq_list_kernel<D, kBf16, kFold, kStats><<<(unsigned)grid_q, kThreads, C::DQ_SMEM, st>>>(mq, mk, mv, mks, mvs, mdo,
+                                                                                                 p);
   DS_CUDA_TRY(cudaGetLastError());
   p.n_lists = fam[1].n_lists;
   p.list_key = fam[1].list_key;
@@ -1396,19 +1417,22 @@ __global__ void triplets_ddir_kernel(const float* __restrict__ d_ab, const float
   }
 }
 
-// every argument of a grouped backward except the work list itself; *aliased: dk_self is dk and dv_self is dv
+// every argument of a grouped backward except the work list itself; *aliased: dk_self is dk and dv_self is dv.
+// rows / cols: the gradient families (dq, dk_self, dv_self) / (dk, dv) are given; a missing family is not checked.
 static int groups_bwd_check(const ds_tensor5& q, const ds_tensor5& ks, const ds_tensor5& vs, const ds_tensor5& k,
                             const ds_tensor5& v, int mode, const float* d, const ds_tensor5& dq, const ds_tensor5& dks,
                             const ds_tensor5& dvs, const ds_tensor5& dk, const ds_tensor5& dv, const char* who,
-                            bool* aliased) {
+                            bool* aliased, bool rows = true, bool cols = true) {
   int rc;
   if (mode != DS_SIM_COSINE && mode != DS_SIM_MSE) return fail(DS_ERR_INVALID, "%s: bad mode %d", who, mode);
   if (!d) return fail(DS_ERR_INVALID, "%s: score gradient: null pointer", who);
   if ((rc = check_group_operands(q, ks, vs, k, v, who)) != DS_OK) return rc;
-  if ((rc = check_grad5(dq, q, who, "dq")) != DS_OK || (rc = check_grad5(dks, ks, who, "dk_self")) != DS_OK ||
-      (rc = check_grad5(dvs, vs, who, "dv_self")) != DS_OK || (rc = check_grad5(dk, k, who, "dk")) != DS_OK ||
-      (rc = check_grad5(dv, v, who, "dv")) != DS_OK)
+  if (rows && ((rc = check_grad5(dq, q, who, "dq")) != DS_OK || (rc = check_grad5(dks, ks, who, "dk_self")) != DS_OK ||
+               (rc = check_grad5(dvs, vs, who, "dv_self")) != DS_OK))
     return rc;
+  if (cols && ((rc = check_grad5(dk, k, who, "dk")) != DS_OK || (rc = check_grad5(dv, v, who, "dv")) != DS_OK)) return rc;
+  *aliased = false;
+  if (!rows || !cols) return DS_OK;
   const bool ak = same_tensor(dks, dk), av = same_tensor(dvs, dv);
   if (ak != av) return fail(DS_ERR_INVALID, "%s: dk_self / dk and dv_self / dv must both be the same tensor or both be separate", who);
   if (!ak && (extents_meet(dks, dk) || extents_meet(dvs, dv)))
@@ -1660,13 +1684,25 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   if (ldd < Cn) return fail(DS_ERR_INVALID, "%s: ldd < columns", who);
   // the term index 2t + 1 of the lists is an int32
   if (E > INT32_MAX / 4) return fail(DS_ERR_INVALID, "%s: more than 2^29 entries; split the rows", who);
+  // the two gradient families: row terms (dq, dk_self, dv_self) and column terms (dk, dv), each given whole or null
+  const bool rows = dq.ptr || dk_self.ptr || dv_self.ptr, cols = dk.ptr || dv.ptr;
+  const bool all_rows = dq.ptr && dk_self.ptr && dv_self.ptr, all_cols = dk.ptr && dv.ptr;
+  if ((!all_rows || !all_cols) && ((dk_self.ptr && dk_self.ptr == dk.ptr) || (dv_self.ptr && dv_self.ptr == dv.ptr)))
+    return fail(DS_ERR_INVALID, "%s: dk_self / dk (dv_self / dv) may be one tensor only when all five gradients are given",
+                who);
+  if (rows && !all_rows)
+    return fail(DS_ERR_INVALID, "%s: dq, dk_self and dv_self must be all given or all null (no row terms)", who);
+  if (cols && !all_cols) return fail(DS_ERR_INVALID, "%s: dk and dv must be both given or both null (no column terms)", who);
+  if (!rows && !cols) return fail(DS_ERR_INVALID, "%s: all five gradients are null", who);
   bool aliased;
-  int rc = groups_bwd_check(q, k_self, v_self, k, v, mode, d_Dm, dq, dk_self, dv_self, dk, dv, who, &aliased);
+  int rc = groups_bwd_check(q, k_self, v_self, k, v, mode, d_Dm, dq, dk_self, dv_self, dk, dv, who, &aliased, rows, cols);
   if (rc != DS_OK) return rc;
   ListParamsT<true> p;
   int64_t grid_q, grid_kv;
   if (!list_params(q, k, scale, R, E, aliased, &p, &grid_q, &grid_kv))
     return fail(DS_ERR_INVALID, "%s: too many tiles: split the rows", who);
+  if (!rows || !cols)   // one family: the dK/dV lists are those of the columns only, or of the rows' self terms only
+    grid_kv = (rows ? R : Cn) * p.B * p.H * p.n_kt;
   Workspace w(ws, ws_bytes);
   MatrixBwdWs L;
   if (!matrix_bwd_layout(w, q, k, &L))
@@ -1681,13 +1717,15 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   const bool bf = q.dtype == DS_BF16;
 
   DS_CUDA_TRY(cudaMemsetAsync(L.bad, 0, sizeof(int32_t), st));
-  DS_CUDA_TRY(cudaMemsetAsync(L.row_max, 0, (size_t)R * 4, st));
+  if (rows) DS_CUDA_TRY(cudaMemsetAsync(L.row_max, 0, (size_t)R * 4, st));
   matrix_bwd_setup_kernel<<<(unsigned)((E + 256) / 256), 256, 0, st>>>(R, Cn, d_Dm, ldd, L.group_q, L.group_off, L.kv_idx,
                                                                       L.entry_group, L.d_dir);
   DS_CUDA_TRY(cudaGetLastError());
   ListBuildT<true> lb;
   set_list_build(&lb, L.group_q, L.kv_idx, E, q, k, aliased, p, L);
   lb.n_cols = (int)Cn;
+  lb.rows = rows;
+  lb.cols = cols;
   build_lists_kernel<true><<<2, kListThreads, 0, st>>>(lb);
   DS_CUDA_TRY(cudaGetLastError());
   // X_t and Y_r, rounded to the input dtype as ds_attn_fwd rounds them
@@ -1699,19 +1737,28 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   const unsigned fb = (unsigned)std::min<int64_t>((n2 + 255) / 256, 4 * (int64_t)sm_count());
   uint32_t* fu = static_cast<uint32_t*>(L.f);
   float2* f32 = reinterpret_cast<float2*>(L.fold32);
-  if (bf) matrix_fold_kernel<true><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
-  else matrix_fold_kernel<false><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
-  DS_CUDA_TRY(cudaGetLastError());
-  uint32_t* f16 = fu + E * n2;
-  if (bf) matrix_fold_round_kernel<true><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
-  else matrix_fold_round_kernel<false><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
-  DS_CUDA_TRY(cudaGetLastError());
+  if (!rows) {   // fx_t only: no self term is folded
+    if (bf) matrix_fold_kernel<true, false><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+    else matrix_fold_kernel<false, false><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+    DS_CUDA_TRY(cudaGetLastError());
+  } else {
+    if (bf) matrix_fold_kernel<true><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+    else matrix_fold_kernel<false><<<dim3(fb, ry), kRedThreads, 0, st>>>(ou, n2, (int)R, (int)Cn, mode, L.coef, fu, f32, L.row_max);
+    DS_CUDA_TRY(cudaGetLastError());
+    uint32_t* f16 = fu + E * n2;
+    if (bf) matrix_fold_round_kernel<true><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
+    else matrix_fold_round_kernel<false><<<dim3(fb, ry), 256, 0, st>>>(f32, n2, (int)R, L.row_max, f16, L.fold_scale);
+    DS_CUDA_TRY(cudaGetLastError());
+  }
 
   const ds_tensor5 F = factor_stack(q, L.f, E + R);
   return with_head_dim(q.size[4], who, [&](auto d) {
     return with_dtype(q.dtype, [&](auto b) {
-      return launch_groups_bwd_t<decltype(d)::value, decltype(b)::value, true>(q, k_self, v_self, k, v, F, p, grid_q,
-                                                                               grid_kv, L.fam, st);
+      constexpr int kD = decltype(d)::value;
+      constexpr bool kB = decltype(b)::value;
+      // without the row terms the dQ kernel only writes the cross terms' LSE and delta for the dK/dV kernel
+      return rows ? launch_groups_bwd_t<kD, kB, true>(q, k_self, v_self, k, v, F, p, grid_q, grid_kv, L.fam, st)
+                  : launch_groups_bwd_t<kD, kB, true, true>(q, k_self, v_self, k, v, F, p, grid_q, grid_kv, L.fam, st);
     });
   });
 }

@@ -437,14 +437,23 @@ def _matrix_spans(nr: int, nc: int, ws_bytes) -> list:
 
 def aas_matrix_bwd(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                    d_Dm: torch.Tensor, similarity="cosine", scale: Optional[float] = None,
-                   grads: Optional[Sequence[torch.Tensor]] = None) -> Tuple[torch.Tensor, ...]:
+                   grads: Optional[Sequence[torch.Tensor]] = None, need_rows: bool = True,
+                   need_cols: bool = True) -> Tuple[Optional[torch.Tensor], ...]:
     """float32 gradients (dq, dk_self, dv_self, dk, dv) of aas_matrix for dL/dDm = d_Dm ([Nr, Nc] on the device) --
     ds_aas_matrix_bwd: the grouped backward of the row-major list with each row's self terms folded into one.  When
-    k_self is k (v_self is v) the gradient is one buffer.  grads: optional float32 tensors to add into.
+    k_self is k (v_self is v) the gradient is one buffer.  grads: optional float32 tensors to add into (None in the
+    places of a family that is not asked for).
+
+    need_rows / need_cols select the two gradient families: the row terms (dq, dk_self, dv_self) and the column terms
+    (dk, dv); a family not asked for is returned as None and not computed.  Each family alone is bitwise what the full
+    call gives it when dk_self / dv_self are separate buffers, so the gradients of a set of images can be formed from
+    its rows against all columns (need_cols=False) and all rows against its columns (need_rows=False).
 
     A matrix whose workspace would exceed GROUPS_BWD_WORKSPACE_CAP is cut into blocks of whole rows (columns only when
     one row does not fit; each column block then folds its own self term).  Row blocks are bitwise one call when the
     self gradients are separate buffers; with one shared buffer a block's self terms are added after the block."""
+    if not (need_rows or need_cols):
+        raise RuntimeError("aas_matrix_bwd: need_rows or need_cols must be set")
     dev = _need_cuda(q, k_self, v_self, k, v, d_Dm)
     nr, nc = q.shape[0], k.shape[0]
     g = d_Dm.detach().to(torch.float32)
@@ -453,26 +462,37 @@ def aas_matrix_bwd(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, 
     if (nc > 1 and g.stride(1) != 1) or (nr > 1 and g.stride(0) < nc):
         g = g.contiguous()
     ldd = g.stride(0) if nr > 1 else nc
-    out = _grad_buffers((q, k_self, v_self, k, v), grads)
+    if need_rows and need_cols:
+        out = _grad_buffers((q, k_self, v_self, k, v), grads)
+    else:   # one family: its buffers only (a skipped family's entries of grads are not used)
+        want = (need_rows,) * 3 + (need_cols,) * 2
+        ts = [t for t, w in zip((q, k_self, v_self, k, v), want) if w]
+        got = iter(_grad_buffers(ts, None if grads is None else [t for t, w in zip(grads, want) if w]))
+        out = tuple(next(got) if w else None for w in want)
     dq, dks, dvs, dk, dv = out
     lib = N.load()
     ws = lambda r, c: lib.ds_aas_matrix_bwd_workspace_bytes(_desc(q[:r], 5), _desc(k[:c], 5))  # noqa: E731
     spans = _matrix_spans(nr, nc, ws)
-    shared = dks is dk or dvs is dv
+    shared = need_rows and need_cols and (dks is dk or dvs is dv)
+    null = N.Tensor5()   # ptr 0: a family not asked for
+    part = lambda t, i0, i1: null if t is None else _desc(t[i0:i1], 5)  # noqa: E731
     for (r0, r1), (c0, c1) in spans:
         rows = (q[r0:r1], k_self[r0:r1], v_self[r0:r1])
         cols = (k[c0:c1], v[c0:c1])
-        gks, gvs = dks[r0:r1], dvs[r0:r1]
+        gks, gvs = part(dks, r0, r1), part(dvs, r0, r1)
         if shared and len(spans) > 1:   # the C call takes one shared buffer whole, not a block of it
-            gks, gvs = torch.zeros_like(gks), torch.zeros_like(gvs)
+            bks, bvs = torch.zeros_like(dks[r0:r1]), torch.zeros_like(dvs[r0:r1])
+            gks, gvs = _desc(bks, 5), _desc(bvs, 5)
         q5, k5 = _desc(rows[0], 5), _desc(cols[0], 5)
         _call("ds_aas_matrix_bwd", dev, q5, _desc(rows[1], 5), _desc(rows[2], 5), k5, _desc(cols[1], 5), _scale_arg(scale),
-              _mode(similarity), g[r0:, c0:].data_ptr(), ldd, _desc(dq[r0:r1], 5), _desc(gks, 5), _desc(gvs, 5),
-              _desc(dk[c0:c1], 5), _desc(dv[c0:c1], 5), ws_query=(q5, k5), slot="bwd",
-              launches=9)  # setup + lists + recompute + partials + coefficients + fold + fold rounding + dQ + dK/dV
+              _mode(similarity), g[r0:, c0:].data_ptr(), ldd, part(dq, r0, r1), gks, gvs, part(dk, c0, c1),
+              part(dv, c0, c1), ws_query=(q5, k5), slot="bwd",
+              # setup + lists + recompute + partials + coefficients + fold (+ fold rounding) + dQ (or statistics)
+              # + dK/dV; without the row terms nothing is folded, so there is no rounding
+              launches=9 if need_rows else 8)
         if shared and len(spans) > 1:
-            dks[r0:r1] += gks
-            dvs[r0:r1] += gvs
+            dks[r0:r1] += bks
+            dvs[r0:r1] += bvs
     return out
 
 

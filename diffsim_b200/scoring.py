@@ -217,7 +217,6 @@ def aas_matrix_local(rows: QKVCache, cols: QKVCache, similarity: str = "cosine",
     return ops.aas_matrix(rows.q, rows.k, rows.v, cols.k, cols.v, similarity, scale)
 
 
-@torch.no_grad()
 def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optional[float] = None, group=None,
                        gather_to_all: bool = True, timings: Optional[dict] = None) -> torch.Tensor:
     """All-pairs directional matrix with the images row-block sharded over the ranks of `group`.
@@ -229,9 +228,33 @@ def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optio
     Dm[own rows, :] and the row blocks are gathered at the end.  Per-element arithmetic does not depend on the
     sharding or on how the columns are cut into calls, so the result is bit-identical to the single-device matrix.
     `timings` (optional dict) receives CUDA events: 'start', 'own_done', 'exchange_done', 'block_done', 'end'.
-    Forward only: the peers' K and V arrive through all_gather, so a graph built here would silently lack their
-    gradients; the blocks run without one.
+
+    gather_to_all=False returns the rank's row block Dm[own rows, all columns], differentiable in local.q/k/v when
+    grad mode is on and one of them requires grad.  Its backward gathers the row blocks of dL/dDm and the Q, K, V of
+    every image, and computes the gradients of the rank's own images with two passes of the matrix backward: its rows
+    against all columns (dq, dk_self, dv_self) and all rows against its columns (dk, dv).  No gradient crosses ranks,
+    and every rank's gradients are bit for bit those of one device's ops.aas_matrix_bwd with separate self buffers.
+    Two requirements, as for DistributedDataParallel: every rank runs the backward (it holds collectives), and a
+    rank's loss depends on its own block only (a gradient reaching a peer's block through another path is lost).
+    gather_to_all=True is forward only: the gathered matrix has no graph.
     """
+    if not gather_to_all and ops.wants_grad(local.q, local.k, local.v):
+        return _ShardedMatrixFn.apply(similarity, scale, group, timings, local.q, local.k, local.v)
+    with torch.no_grad():
+        return _aas_matrix_sharded(local, similarity, scale, group, gather_to_all, timings)[0]
+
+
+def _shard_counts(n_local: int, group, dev) -> List[int]:
+    import torch.distributed as dist
+
+    n = torch.tensor([n_local], dtype=torch.int64, device=dev)
+    counts = [torch.zeros_like(n) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(counts, n, group=group)
+    return [int(c) for c in counts]
+
+
+def _aas_matrix_sharded(local: QKVCache, similarity, scale, group, gather_to_all, timings):
+    """(matrix or row block, image counts per rank) of aas_matrix_sharded, without a graph."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group)
@@ -239,10 +262,7 @@ def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optio
     _, km, vm = local.memory()
     dev = km.device
     B, H, S, D = local.shape
-    n_local = torch.tensor([km.shape[0]], dtype=torch.int64, device=dev)
-    counts = [torch.zeros_like(n_local) for _ in range(world)]
-    dist.all_gather(counts, n_local, group=group)
-    counts = [int(c) for c in counts]
+    counts = _shard_counts(km.shape[0], group, dev)
     nmax, n_total = max(counts), sum(counts)
     offs = [sum(counts[:r]) for r in range(world)]
 
@@ -252,18 +272,13 @@ def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optio
             ev.record()
             timings[name] = ev
 
-    def padded(mem):
-        if mem.shape[0] == nmax:
-            return mem.contiguous()
-        return torch.cat([mem, mem.new_zeros((nmax - mem.shape[0],) + tuple(mem.shape[1:]))], 0)
-
     mark("start")
     k_all = torch.empty((world, nmax, B, S, H * D), dtype=km.dtype, device=dev)
     v_all = torch.empty_like(k_all)
     pending = []
     if nmax > 0:
-        pending = [dist.all_gather_into_tensor(k_all.view(world * nmax, B, S, H * D), padded(km), group=group, async_op=True),
-                   dist.all_gather_into_tensor(v_all.view(world * nmax, B, S, H * D), padded(vm), group=group, async_op=True)]
+        pending = [dist.all_gather_into_tensor(k_all.view(world * nmax, B, S, H * D), _padded(km, nmax), group=group, async_op=True),
+                   dist.all_gather_into_tensor(v_all.view(world * nmax, B, S, H * D), _padded(vm, nmax), group=group, async_op=True)]
     block = torch.zeros((counts[rank], n_total), dtype=torch.float32 if dev.type == "cuda" else torch.float64, device=dev)
     if counts[rank] > 0:
         # own columns first: this work hides the exchange
@@ -282,20 +297,76 @@ def aas_matrix_sharded(local: QKVCache, similarity: str = "cosine", scale: Optio
     mark("block_done")
     if not gather_to_all:
         mark("end")
-        return block
-    pad = block
-    if block.shape[0] < nmax:
-        pad = torch.cat([block, block.new_zeros((nmax - block.shape[0], block.shape[1]))], 0)
-    out = torch.empty((world * nmax, n_total), dtype=block.dtype, device=dev)
-    if nmax > 0:
-        dist.all_gather_into_tensor(out, pad.contiguous(), group=group)
+        return block, counts
+    out = _all_gather_rows(block, counts, group)
     mark("end")
+    return out, counts
+
+
+def _padded(mem: torch.Tensor, n: int) -> torch.Tensor:
+    """mem (contiguous) with zero rows appended up to n rows: the equal-size piece of an all_gather_into_tensor."""
+    if mem.shape[0] == n:
+        return mem.contiguous()
+    return torch.cat([mem, mem.new_zeros((n - mem.shape[0],) + tuple(mem.shape[1:]))], 0)
+
+
+def _all_gather_rows(t: torch.Tensor, counts: List[int], group) -> torch.Tensor:
+    """The ranks' row blocks t (counts[r] rows on rank r) concatenated in rank order, on every rank."""
+    import torch.distributed as dist
+
+    nmax = max(counts)
+    out = torch.empty((len(counts) * nmax,) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+    if nmax > 0:
+        dist.all_gather_into_tensor(out, _padded(t, nmax), group=group)
+    if all(c == nmax for c in counts):
+        return out
     return torch.cat([out[r * nmax: r * nmax + c] for r, c in enumerate(counts)], 0)
+
+
+class _ShardedMatrixFn(torch.autograd.Function):
+    """aas_matrix_sharded's row block with the two-pass sharded matrix backward; saves only the local caches."""
+
+    @staticmethod
+    def forward(ctx, similarity, scale, group, timings, q, k, v):
+        block, counts = _aas_matrix_sharded(QKVCache(q, k, v), similarity, scale, group, False, timings)
+        ctx.save_for_backward(q, k, v)
+        ctx.similarity, ctx.scale, ctx.group, ctx.counts = similarity, scale, group, counts
+        return block
+
+    @staticmethod
+    def backward(ctx, d_block):
+        import torch.distributed as dist
+
+        q, k, v = ctx.saved_tensors
+        counts, group = ctx.counts, ctx.group
+        rank = dist.get_rank(group)
+        r0 = sum(counts[:rank])
+        r1 = r0 + counts[rank]
+        d_full = _all_gather_rows(d_block.contiguous(), counts, group)
+        n, B, H, S, D = q.shape
+        mems = [_all_gather_rows(m, counts, group) for m in QKVCache(q, k, v).memory()]
+        q_all, k_all, v_all = (m.view(m.shape[0], B, S, H, D).permute(0, 1, 3, 2, 4) for m in mems)
+        if r1 == r0:
+            return (None,) * 4 + tuple(torch.zeros_like(t, dtype=d_block.dtype) for t in (q, k, v))
+        dq, dks, dvs, dk, dv = _matrix_grad_block(q_all, k_all, v_all, r0, r1, d_full, ctx.similarity, ctx.scale)
+        return (None,) * 4 + (dq, dks + dk, dvs + dv)
 
 
 def _matrix_block(local: QKVCache, k_all: torch.Tensor, v_all: torch.Tensor, similarity, scale):
     """Hook for tests: the per-rank block computation (CUDA kernels)."""
     return ops.aas_matrix(local.q, local.k, local.v, k_all, v_all, similarity, scale)
+
+
+def _matrix_grad_block(q_all, k_all, v_all, r0: int, r1: int, d_full: torch.Tensor, similarity, scale):
+    """Hook for tests: the per-rank backward (CUDA kernels).  (dq, dk_self, dv_self, dk, dv) of sum(d_full * Dm) for
+    the images [r0, r1) of the global caches: the row pass (own rows against all columns) and the column pass (all
+    rows against own columns).  Each is bitwise the single-device aas_matrix_bwd's with separate self buffers."""
+    own = slice(r0, r1)
+    dq, dks, dvs, _, _ = ops.aas_matrix_bwd(q_all[own], k_all[own], v_all[own], k_all, v_all, d_full[own], similarity,
+                                            scale, need_cols=False)
+    _, _, _, dk, dv = ops.aas_matrix_bwd(q_all, k_all, v_all, k_all[own], v_all[own], d_full[:, own], similarity,
+                                         scale, need_rows=False)
+    return dq, dks, dvs, dk, dv
 
 
 def symmetrize(dm: torch.Tensor) -> torch.Tensor:

@@ -277,6 +277,16 @@ size_t ds_aas_triplets_bwd_workspace_bytes(ds_tensor5 q, int64_t n_triplets);
  * row-major list.  No float atomics: repeated calls are bitwise equal.  At most 2^29 entries (the lists' term index is an
  * int32).  Workspace: per entry about 2 x B H S D x 2 bytes (X, fx) plus 3 KB of partials; per row about B H S D x 8
  * bytes (Y, F_r in 16 and 32 bits); LSE and delta for every entry and row.
+ *
+ * Gradient families: the ROW terms (dq of every term; dk_self, dv_self of the folded self terms) and the COLUMN terms
+ * (dk, dv of the cross terms).  A family whose pointers are all null is not computed: (dq, dk_self, dv_self) all null, or
+ * (dk, dv) both null, not both.  A partly null family is DS_ERR_INVALID, and so is dk_self / dk (dv_self / dv) as one
+ * tensor unless all five are given.  Only the work of the given family runs: without the column terms the dK/dV kernel
+ * runs the folded self terms only; without the row terms nothing is folded, and the dQ kernel writes only the cross
+ * terms' LSE and delta.  Every per-term quantity depends only on its entry (r, c) and its row r, so each family alone is
+ * bitwise what the full call gives it with separate self buffers.  The rows [r0, r1) against all columns and all rows
+ * against the columns [c0, c1) thus give bitwise the full call's gradients of those images.  The workspace query is
+ * that of the full call (an upper bound).
  */
 int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_tensor5 k, ds_tensor5 v,
                       float scale, int mode, const float* d_Dm, int64_t ldd,
