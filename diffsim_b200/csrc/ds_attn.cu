@@ -92,7 +92,12 @@ struct AttnParams {
   const int32_t* kv_idx;     // [n_entries] kv image of each entry
   int n_groups;
   int self_first;            // 1: every group starts with the query image's own K/V (AAS)
-  int B, H, Sq, Skv;
+  int B, H, Sq, Skv;         // Skv: kv length of the cross items (k, v)
+  int Skv_self;              // kv length of the self item (k_self, v_self); independent of Sq and of Skv
+  // kv groups of a cross item / of the self item, and the valid rows of the two halves of their last group (set by the
+  // host: the walkers select them per item and divide nothing)
+  int n_grp, rowsA_last, rowsB_last;
+  int n_grp_self, rowsA_last_self, rowsB_last_self;
   int n_qt;                  // q tiles per (b,h)
   float scale_log2;          // softmax scale * log2(e)
   // AAS output: part[entry][bh * n_qt + qt] = (dot, |Oc|^2, |Os|^2, sum (Oc-Os)^2)
@@ -133,7 +138,6 @@ template <typename F>
 __device__ __forceinline__ void for_each_group(const AttnParams& p, F&& f) {
   const uint32_t BH = (uint32_t)(p.B * p.H);
   const uint32_t n_streams = (uint32_t)p.n_groups * BH * (uint32_t)p.n_qt;   // < 2^31, checked by the host
-  const int n_grp = (p.Skv + kGroupKV - 1) / kGroupKV;
   // stream -> (bh, group, q tile): q tile fastest so that neighbouring CTAs share K/V in L2.  32-bit arithmetic only:
   // this decode sits between two items on every role's critical path.
   for (uint32_t st = blockIdx.x; st < n_streams; st += gridDim.x) {
@@ -161,9 +165,11 @@ __device__ __forceinline__ void for_each_group(const AttnParams& p, F&& f) {
       G.entry = t0 + it - p.self_first;
       if (it + 1 < n_items) prefetch_l1(p.kv_idx + G.entry + 1);
       G.img = G.self ? G.qi : p.kv_idx[G.entry];
+      const int skv = G.self ? p.Skv_self : p.Skv;   // each item is cut by its own kv length
+      const int n_grp = G.self ? p.n_grp_self : p.n_grp;
       for (int gg = 0; gg < n_grp; ++gg) {
         G.kv0 = gg * kGroupKV;
-        const int rem = p.Skv - G.kv0;
+        const int rem = skv - G.kv0;
         G.rowsA = min(rem, kHalfKV);
         G.rowsB = max(0, min(rem - kHalfKV, kHalfKV));
         G.first_of_item = gg == 0;
@@ -188,9 +194,6 @@ template <typename F>
 __device__ __forceinline__ void for_each_group_lite(const AttnParams& p, F&& f) {
   const uint32_t nq = (uint32_t)p.n_qt, ng = (uint32_t)p.n_groups;
   const uint32_t n_streams = ng * (uint32_t)(p.B * p.H) * nq;   // < 2^31, checked by the host
-  const int n_grp = (p.Skv + kGroupKV - 1) / kGroupKV;
-  const int rem_last = p.Skv - (n_grp - 1) * kGroupKV;
-  const int rowsA_last = min(rem_last, kHalfKV), rowsB_last = max(0, min(rem_last - kHalfKV, kHalfKV));
   // stream st = (bh * n_groups + g) * n_qt + qt
   uint32_t qt = blockIdx.x % nq, g = (blockIdx.x / nq) % ng;
   const uint32_t d_qt = gridDim.x % nq, d_g = (gridDim.x / nq) % ng;
@@ -207,6 +210,10 @@ __device__ __forceinline__ void for_each_group_lite(const AttnParams& p, F&& f) 
     prefetch_l1(p.group_off + g);
     LiteGroup G;
     for (int it = 0; it < n_items; ++it) {
+      // each item by its own kv length: the self item is item 0 of a self_first stream
+      const bool self = it < p.self_first;
+      const int n_grp = self ? p.n_grp_self : p.n_grp;
+      const int rowsA_last = self ? p.rowsA_last_self : p.rowsA_last, rowsB_last = self ? p.rowsB_last_self : p.rowsB_last;
       for (int gg = 0; gg < n_grp; ++gg) {
         const bool last = gg == n_grp - 1;
         G.rowsA = last ? rowsA_last : kHalfKV;
@@ -1026,6 +1033,14 @@ static int launch_attn(const AttnLaunch& a, const char* who, cudaStream_t st) {
   return with_head_dim(a.q.size[4], who, [&](auto d) { return launch_attn_d<decltype(d)::value>(a, st); });
 }
 
+// kv groups of an item of skv rows and the valid rows of the two halves of its last group
+static void kv_split(int skv, int* n_grp, int* rowsA_last, int* rowsB_last) {
+  *n_grp = (skv + kGroupKV - 1) / kGroupKV;
+  const int rem = skv - (*n_grp - 1) * kGroupKV;
+  *rowsA_last = rem < kHalfKV ? rem : kHalfKV;
+  *rowsB_last = rem <= kHalfKV ? 0 : rem - kHalfKV;   // rem <= kGroupKV
+}
+
 // common validation of a (q, k_self, v_self, k, v) set, before any device work; fills the shape part of AttnParams
 static int prepare(AttnLaunch& a, float scale, const char* who) {
   const ds_tensor5* all[5] = {&a.q, &a.ks, &a.vs, &a.k, &a.v};
@@ -1041,19 +1056,23 @@ static int prepare(AttnLaunch& a, float scale, const char* who) {
     if (all[i]->size[1] != a.q.size[1] || all[i]->size[2] != a.q.size[2] || all[i]->size[4] != a.q.size[4])
       return fail(DS_ERR_INVALID, "%s: B, H and D must match across q, k, v", who);
   }
-  if (a.ks.size[3] != a.k.size[3] || a.vs.size[3] != a.k.size[3] || a.v.size[3] != a.k.size[3])
-    return fail(DS_ERR_INVALID, "%s: all key/value tensors must share the kv length", who);
+  // (k_self, v_self) share one kv length and (k, v) another; the two are independent of each other and of q's length
+  if (a.vs.size[3] != a.ks.size[3]) return fail(DS_ERR_INVALID, "%s: k_self and v_self must share the kv length", who);
+  if (a.v.size[3] != a.k.size[3]) return fail(DS_ERR_INVALID, "%s: k and v must share the kv length", who);
   if (a.ks.size[0] != a.q.size[0] || a.vs.size[0] != a.q.size[0])
     return fail(DS_ERR_INVALID, "%s: k_self / v_self must hold the same images as q", who);
   if (a.k.size[0] != a.v.size[0]) return fail(DS_ERR_INVALID, "%s: k and v must hold the same images", who);
-  const int64_t Skv = a.k.size[3];
-  if (Skv > INT32_MAX / 2) return fail(DS_ERR_INVALID, "%s: kv length too large", who);
+  const int64_t Skv = a.k.size[3], Skv_self = a.ks.size[3];
+  if (Skv > INT32_MAX / 2 || Skv_self > INT32_MAX / 2) return fail(DS_ERR_INVALID, "%s: kv length too large", who);
   const int64_t D = a.q.size[4];
   if ((rc = with_head_dim(D, who, [](auto) { return DS_OK; })) != DS_OK) return rc;
   a.p.B = (int)a.q.size[1];
   a.p.H = (int)a.q.size[2];
   a.p.Sq = (int)a.q.size[3];
   a.p.Skv = (int)Skv;
+  a.p.Skv_self = (int)Skv_self;
+  kv_split(a.p.Skv, &a.p.n_grp, &a.p.rowsA_last, &a.p.rowsB_last);
+  kv_split(a.p.Skv_self, &a.p.n_grp_self, &a.p.rowsA_last_self, &a.p.rowsB_last_self);
   a.p.n_qt = (int)((a.q.size[3] + kBlockQ - 1) / kBlockQ);
   const float sc = scale > 0.f ? scale : 1.0f / sqrtf((float)D);
   a.p.scale_log2 = sc * 1.4426950408889634f;
@@ -1325,6 +1344,7 @@ int ds_aas_triplets(ds_tensor5 q, ds_tensor5 k, ds_tensor5 v, const int32_t* tri
 static void matrix_plan(const ds_tensor5& q, const ds_tensor5& k, int64_t n_rows, int64_t n_cols, int* chunks, int64_t* chunk_cols) {
   const int64_t per_row = q.size[1] * q.size[2] * ((q.size[3] + ds::kBlockQ - 1) / ds::kBlockQ);
   // (1) L2 blocking: the K and V slices of one (b, h) of a chunk's columns should fill about a third of the 126 MB L2
+  //     (sized from the column K / V, whose kv length may differ from the rows' k_self / v_self)
   const int64_t slice_bytes = 2 * k.size[3] * k.size[4] * 2;
   int64_t cc = (40ll << 20) / (slice_bytes > 0 ? slice_bytes : 1);
   if (cc > n_cols) cc = n_cols;

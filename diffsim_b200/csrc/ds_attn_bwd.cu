@@ -58,9 +58,11 @@ struct Cfg : AttnTile<D> {   // K1's operand tiles
                 "swizzle atoms need 1024-byte tiles");
 };
 
-// the shape of one attention backward, common to the single (Params) and list (ListParams) kernels
+// the shape of one attention backward, common to the single (Params) and list (ListParams) kernels.  Skv / n_kt: kv
+// length and tiles of the cross terms (k, v), Skv_self / n_kt_self: of the self terms (k_self, v_self) of a list; the
+// single kernels have one kv length and set both alike.
 struct Shape {
-  int B, H, Sq, Skv, n_qt, n_kt;
+  int B, H, Sq, Skv, Skv_self, n_qt, n_kt, n_kt_self;
   float scale, scale_log2;
 };
 
@@ -182,16 +184,16 @@ __device__ __forceinline__ uint32_t kernel_prologue(uint64_t* bars, const Maps*.
 
 // One term of a dQ kernel, on the 128-row q tile qt of (b, h): the Q and dO tiles (images q_img of mq and do_img of
 // mdo), delta = rowsum(dO o O) from this thread's 16-bit rows o_row and do_row, the LSE pass and the dS / dQ pass over
-// the kv tiles of image kv_img of mk and mv.  LSE and delta go to *lse and *delta_out, dQ x scale coef is added into
-// dq_row.  kStats: the statistics only -- LSE and delta are written, there is no dS / dQ pass and no drain (dq_row is
-// not read).
+// the skv rows (the term's own kv length) of image kv_img of mk and mv.  LSE and delta go to *lse and *delta_out,
+// dQ x scale coef is added into dq_row.  kStats: the statistics only -- LSE and delta are written, there is no dS / dQ
+// pass and no drain (dq_row is not read).
 // The barrier phases carry over to the next term.
 template <int D, bool kBf16, bool kStats = false>
 __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shape& p, int b, int h, int qt,
                                         const CUtensorMap* mq, int q_img, const CUtensorMap* mdo, int do_img,
-                                        const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, const void* o_row,
-                                        const void* do_row, float* lse, float* delta_out, float coef, float* dq_row,
-                                        uint32_t& q_ph, uint32_t& kv_ph, uint32_t& mma_ph) {
+                                        const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, int skv,
+                                        const void* o_row, const void* do_row, float* lse, float* delta_out, float coef,
+                                        float* dq_row, uint32_t& q_ph, uint32_t& kv_ph, uint32_t& mma_ph) {
   using C = Cfg<D>;
   uint8_t* sQ = smem;
   uint8_t* sDO = sQ + C::TILE_BYTES;
@@ -208,6 +210,7 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
   const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, kTile, 0, 0);
   const uint32_t idesc_dq = umma_idesc_f16(fmt, kTile, C::D_PAD, 0, 1);
   const float sl2 = p.scale_log2;
+  const int n_kt = (skv + kTile - 1) / kTile;
 
   if (tid == 0) {
     mbar_arrive_expect_tx(q_bar, 2 * C::TILE_BYTES);
@@ -223,7 +226,7 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
 
   // ---- pass 1: log-sum-exp of every row (log2 domain)
   float m = -INFINITY, l = 0.f;
-  for (int kt = 0; kt < p.n_kt; ++kt) {
+  for (int kt = 0; kt < n_kt; ++kt) {
     if (tid == 0) {
       mbar_arrive_expect_tx(kv_bar, C::TILE_BYTES);
       load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
@@ -240,7 +243,7 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
     mbar_wait(mma_bar, mma_ph);
     mma_ph ^= 1;
     tc_fence_after_sync();
-    const int nv = p.Skv - kt * kTile;   // valid kv columns of this tile (>= 1)
+    const int nv = skv - kt * kTile;   // valid kv columns of this tile (>= 1)
 #pragma unroll 1
     for (int c = 0; c < kTile / 32; ++c) {
       uint32_t v[32];
@@ -268,7 +271,7 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
   // kStats: the last tile's sync_all_tc has freed S, Q and dO for the next term
   if constexpr (!kStats) {
     // ---- pass 2: dQ
-    for (int kt = 0; kt < p.n_kt; ++kt) {
+    for (int kt = 0; kt < n_kt; ++kt) {
       if (tid == 0) {
         mbar_arrive_expect_tx(kv_bar, 2 * C::TILE_BYTES);
         load_tile<D>(sK, mk, kv_bar, kTile, kt * kTile, h, b, kv_img);
@@ -287,7 +290,7 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
       mbar_wait(mma_bar, mma_ph);
       mma_ph ^= 1;
       tc_fence_after_sync();
-      const int nv = p.Skv - kt * kTile;
+      const int nv = skv - kt * kTile;
 #pragma unroll 1
       for (int c = 0; c < kTile / 32; ++c) {
         uint32_t s[32], dp[32], pk[16];
@@ -323,16 +326,16 @@ __device__ __forceinline__ void dq_term(uint8_t* smem, uint32_t tmem, const Shap
   }
 }
 
-// One term of a dK/dV kernel, on the 128-row kv tile kt of (b, h): the K and V tiles (image kv_img of mk and mv), then
-// per block of BQ q rows the Q and dO tiles (images q_img of mq and do_img of mdo) with their LSE and delta, read from
-// the term's (b, h) rows lse and delta.  dV x coef is added into dv_row, dK x coef scale into dk_row.  The barrier
-// phases carry over to the next term.
+// One term of a dK/dV kernel, on the 128-row kv tile kt (< the tiles of skv, the term's kv length) of (b, h): the K and
+// V tiles (image kv_img of mk and mv), then per block of BQ q rows the Q and dO tiles (images q_img of mq and do_img of
+// mdo) with their LSE and delta, read from the term's (b, h) rows lse and delta.  dV x coef is added into dv_row,
+// dK x coef scale into dk_row.  The barrier phases carry over to the next term.
 template <int D, bool kBf16>
 __device__ __forceinline__ void dkv_term(uint8_t* smem, uint32_t tmem, const Shape& p, int b, int h, int kt,
-                                         const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, const CUtensorMap* mq,
-                                         int q_img, const CUtensorMap* mdo, int do_img, const float* lse,
-                                         const float* delta, float coef, float* dv_row, float* dk_row, uint32_t& kv_ph,
-                                         uint32_t& q_ph, uint32_t& mma_ph) {
+                                         const CUtensorMap* mk, const CUtensorMap* mv, int kv_img, int skv,
+                                         const CUtensorMap* mq, int q_img, const CUtensorMap* mdo, int do_img,
+                                         const float* lse, const float* delta, float coef, float* dv_row, float* dk_row,
+                                         uint32_t& kv_ph, uint32_t& q_ph, uint32_t& mma_ph) {
   using C = Cfg<D>;
   constexpr int BQ = C::BQ;
   uint8_t* sK = smem;
@@ -346,7 +349,7 @@ __device__ __forceinline__ void dkv_term(uint8_t* smem, uint32_t tmem, const Sha
   uint64_t* mma_bar = kv_bar + 2;
   const int tid = threadIdx.x;
   const uint32_t lane_t = tmem + ((uint32_t)((tid >> 5) * 32) << 16);
-  const bool row_ok = kt * kTile + tid < p.Skv;
+  const bool row_ok = kt * kTile + tid < skv;
   constexpr uint32_t kST = 0, kDPT = BQ, kDV = 2 * BQ, kDK = 2 * BQ + C::D_PAD;
   const uint32_t fmt = kBf16 ? 1u : 0u;
   const uint32_t idesc_s = umma_idesc_f16(fmt, kTile, BQ, 0, 0);
@@ -442,9 +445,9 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
   const uint8_t* g = static_cast<const uint8_t*>(p.dout) + 2 * (b * p.do_sb + h * p.do_sh + grow * p.do_ss);
   const size_t i = (size_t)bh * (p.n_qt * kTile) + grow;
   uint32_t q_ph = 0, kv_ph = 0, mma_ph = 0;
-  dq_term<D, kBf16>(smem, tmem, p, b, h, qt, &map_q, 0, &map_do, 0, &map_k, &map_v, 0, o, g, p.lse + i, p.delta + i,
-                    p.coef ? *p.coef : 1.0f, p.dq + b * p.dq_sb + h * p.dq_sh + (int64_t)grow * p.dq_ss, q_ph, kv_ph,
-                    mma_ph);
+  dq_term<D, kBf16>(smem, tmem, p, b, h, qt, &map_q, 0, &map_do, 0, &map_k, &map_v, 0, p.Skv, o, g, p.lse + i,
+                    p.delta + i, p.coef ? *p.coef : 1.0f, p.dq + b * p.dq_sb + h * p.dq_sh + (int64_t)grow * p.dq_ss,
+                    q_ph, kv_ph, mma_ph);
   if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
@@ -461,7 +464,7 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
   const int krow = kt * kTile + threadIdx.x;
   const size_t i = (size_t)bh * (p.n_qt * kTile);
   uint32_t kv_ph = 0, q_ph = 0, mma_ph = 0;
-  dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, &map_k, &map_v, 0, &map_q, 0, &map_do, 0, p.lse + i, p.delta + i,
+  dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, &map_k, &map_v, 0, p.Skv, &map_q, 0, &map_do, 0, p.lse + i, p.delta + i,
                      p.coef ? *p.coef : 1.0f, p.dv + b * p.dv_sb + h * p.dv_sh + (int64_t)krow * p.dv_ss,
                      p.dk + b * p.dk_sb + h * p.dk_sh + (int64_t)krow * p.dk_ss, kv_ph, q_ph, mma_ph);
   if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
@@ -932,7 +935,7 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
     const float coef = term_coef<kFold>(p, tau, slot);
     const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile) + grow;
     dq_term<D, kBf16, kStats>(smem, tmem, p, b, h, qt, &map_q, qi, &map_do, slot, self ? &map_ks : &map_k,
-                      self ? &map_vs : &map_v, self ? qi : p.kv_idx[t],
+                      self ? &map_vs : &map_v, self ? qi : p.kv_idx[t], self ? p.Skv_self : p.Skv,
                       static_cast<const uint16_t*>(p.o) + o_slot * p.img + row_off,
                       static_cast<const uint16_t*>(p.f) + slot * p.img + row_off, p.lse + k, p.delta + k, coef, dq_row,
                       q_ph, kv_ph, mma_ph);
@@ -940,26 +943,32 @@ attn_bwd_dq_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_
   if (threadIdx.x < 32) tmem_dealloc(tmem, 512);
 }
 
-// attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), one dK/dV term per list entry
+// attn_bwd_dkv_kernel over a list: one CTA per (kv image, b, h, 128-row kv tile), one dK/dV term per list entry.  The
+// grid gives every list max(n_kt, n_kt_self) tiles per (b, h); the CTAs past the tiles of the list's own kv length (that
+// of k_self for a self-term list, of k otherwise) exit at once.  With separate self buffers (n_kbuf > 0) a list holds
+// terms of one kind only; with one shared buffer the two lengths are equal.
 template <int D, bool kBf16, bool kFold>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                          const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_ks,
                          const __grid_constant__ CUtensorMap map_vs, const __grid_constant__ CUtensorMap map_do,
                          const ListParamsT<kFold> p) {
-  const int per_list = p.B * p.H * p.n_kt;
+  const int n_kt = max(p.n_kt, p.n_kt_self);
+  const int per_list = p.B * p.H * n_kt;
   const int li = blockIdx.x / per_list;
   if (li >= *p.n_lists) return;
+  const int rest = blockIdx.x - li * per_list;
+  const int bh = rest / n_kt, kt = rest - bh * n_kt;
+  int img = p.list_key[li];
+  const bool self_list = img >= p.n_kbuf && p.n_kbuf > 0;
+  if (kt >= (self_list ? p.n_kt_self : p.n_kt)) return;
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t tmem = kernel_prologue(reinterpret_cast<uint64_t*>(smem + Cfg<D>::DKV_BARS), &map_q, &map_k, &map_v,
                                         &map_ks, &map_vs, &map_do);
-  const int rest = blockIdx.x - li * per_list;
-  const int bh = rest / p.n_kt, kt = rest - bh * p.n_kt;
   const int b = bh / p.H, h = bh - b * p.H;
   const int krow = kt * kTile + threadIdx.x;
-  int img = p.list_key[li];
   GradT gk = p.dk, gv = p.dv;
-  if (img >= p.n_kbuf && p.n_kbuf > 0) {
+  if (self_list) {
     img -= p.n_kbuf;
     gk = p.dks;
     gv = p.dvs;
@@ -975,7 +984,8 @@ attn_bwd_dkv_list_kernel(const __grid_constant__ CUtensorMap map_q, const __grid
     int slot;
     const float coef = term_coef<kFold>(p, tau, slot);
     const size_t k = ((size_t)slot * (p.B * p.H) + bh) * (p.n_qt * kTile);
-    dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, self ? &map_ks : &map_k, self ? &map_vs : &map_v, img, &map_q,
+    dkv_term<D, kBf16>(smem, tmem, p, b, h, kt, self ? &map_ks : &map_k, self ? &map_vs : &map_v, img,
+                       self ? p.Skv_self : p.Skv, &map_q,
                        p.group_q[p.entry_group[t]], &map_do, slot, p.lse + k, p.delta + k, coef, dv_row, dk_row, kv_ph,
                        q_ph, mma_ph);
   }
@@ -1039,14 +1049,17 @@ static size_t stats_bytes(const ds_tensor4& q) {
   return 2 * align_up((size_t)(q.size[0] * q.size[1] * n_qt * kTile) * sizeof(float), 256);
 }
 
-// the Shape of the backward of q (., B, H, Sq, D) against k (., B, H, Skv, D)
-static void set_shape(Shape* s, const ds_tensor5& q, const ds_tensor5& k, float scale) {
+// the Shape of the backward of q (., B, H, Sq, D) against k (., B, H, Skv, D) and, for the self terms of a list, k_self
+// (., B, H, Skv_self, D)
+static void set_shape(Shape* s, const ds_tensor5& q, const ds_tensor5& k, const ds_tensor5& ks, float scale) {
   s->B = (int)q.size[1];
   s->H = (int)q.size[2];
   s->Sq = (int)q.size[3];
   s->Skv = (int)k.size[3];
+  s->Skv_self = (int)ks.size[3];
   s->n_qt = (s->Sq + kTile - 1) / kTile;
   s->n_kt = (s->Skv + kTile - 1) / kTile;
+  s->n_kt_self = (s->Skv_self + kTile - 1) / kTile;
   s->scale = scale > 0.f ? scale : 1.0f / sqrtf((float)q.size[4]);
   s->scale_log2 = s->scale * 1.4426950408889634f;
 }
@@ -1070,7 +1083,7 @@ static int launch_bwd_t(const BwdArgs& a, cudaStream_t st) {
       (rc = make_map(&mqb, q, C::SUBW, C::BQ)) != DS_OK || (rc = make_map(&mdob, dout, C::SUBW, C::BQ)) != DS_OK)
     return rc;
   Params p;
-  set_shape(&p, q, k, a.scale);
+  set_shape(&p, q, k, k, a.scale);
   p.o = a.out.ptr;
   p.o_sb = a.out.stride[0], p.o_sh = a.out.stride[1], p.o_ss = a.out.stride[2];
   p.dout = a.dout.ptr;
@@ -1238,9 +1251,9 @@ static ds_tensor5 factor_stack(const ds_tensor5& q, void* ptr, int64_t n_slots) 
 }
 
 // ListParams of a checked list backward: shapes, grids (false: too many tiles) and everything but the pointers
-static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, int64_t G, int64_t E, bool aliased,
-                        ListParams* p, int64_t* grid_q, int64_t* grid_kv) {
-  set_shape(p, q, k, scale);
+static bool list_params(const ds_tensor5& q, const ds_tensor5& k, const ds_tensor5& ks, float scale, int64_t G,
+                        int64_t E, bool aliased, ListParams* p, int64_t* grid_q, int64_t* grid_kv) {
+  set_shape(p, q, k, ks, scale);
   p->n_groups = (int)G;
   p->n_kbuf = aliased ? 0 : (int)k.size[0];
   p->img = q.size[1] * q.size[2] * q.size[3] * q.size[4];
@@ -1248,7 +1261,7 @@ static bool list_params(const ds_tensor5& q, const ds_tensor5& k, float scale, i
   const int64_t nl_q = std::min<int64_t>(q.size[0], G);
   const int64_t nl_kv = aliased ? std::min<int64_t>(k.size[0], G + E) : nl_q + std::min<int64_t>(k.size[0], E);
   *grid_q = nl_q * bh * p->n_qt;
-  *grid_kv = nl_kv * bh * p->n_kt;
+  *grid_kv = nl_kv * bh * std::max(p->n_kt, p->n_kt_self);   // attn_bwd_dkv_list_kernel's grid
   return *grid_q < INT32_MAX && *grid_kv < INT32_MAX;
 }
 
@@ -1450,7 +1463,7 @@ static int groups_bwd_launch(const ds_tensor5& q, const ds_tensor5& ks, const ds
   int rc;
   ListParams p;
   int64_t grid_q, grid_kv;
-  if (!list_params(q, k, scale, G, E, aliased, &p, &grid_q, &grid_kv))
+  if (!list_params(q, k, ks, scale, G, E, aliased, &p, &grid_q, &grid_kv))
     return fail(DS_ERR_INVALID, "%s: too many tiles: split the work list", who);
   set_pointers(&p, group_q, kv_idx, L, dq, dks, dvs, dk, dv);
   const int64_t n2 = p.img / 2;
@@ -1699,10 +1712,10 @@ int ds_aas_matrix_bwd(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self, ds_ten
   if (rc != DS_OK) return rc;
   ListParamsT<true> p;
   int64_t grid_q, grid_kv;
-  if (!list_params(q, k, scale, R, E, aliased, &p, &grid_q, &grid_kv))
+  if (!list_params(q, k, k_self, scale, R, E, aliased, &p, &grid_q, &grid_kv))
     return fail(DS_ERR_INVALID, "%s: too many tiles: split the rows", who);
   if (!rows || !cols)   // one family: the dK/dV lists are those of the columns only, or of the rows' self terms only
-    grid_kv = (rows ? R : Cn) * p.B * p.H * p.n_kt;
+    grid_kv = (rows ? R : Cn) * p.B * p.H * std::max(p.n_kt, p.n_kt_self);
   Workspace w(ws, ws_bytes);
   MatrixBwdWs L;
   if (!matrix_bwd_layout(w, q, k, &L))

@@ -231,8 +231,10 @@ class _PairDirsFn(torch.autograd.Function):
 
 
 def pair_dirs(qa, ka, va, qb, kb, vb, similarity="cosine", scale: Optional[float] = None):
-    """(dir(a->b), dir(b->a)) of one image pair as float32 (1,) tensors -- two aas_groups launches.  Differentiable
-    (aas_dir_bwd) when an input requires grad; the values are the same either way."""
+    """(dir(a->b), dir(b->a)) of one image pair as float32 (1,) tensors -- two aas_groups launches.  The two images may
+    have different token counts (a (B,H,S_a,D) against a (B,H,S_b,D) capture): each direction's self attention runs
+    over the query image's own K/V and its cross attention over the other image's.  Differentiable (aas_dir_bwd) when
+    an input requires grad; the values are the same either way."""
     if wants_grad(qa, ka, va, qb, kb, vb):
         return _PairDirsFn.apply(similarity, scale, qa, ka, va, qb, kb, vb)
     return _pair_dirs(qa, ka, va, qb, kb, vb, similarity, scale)
@@ -241,7 +243,8 @@ def pair_dirs(qa, ka, va, qb, kb, vb, similarity="cosine", scale: Optional[float
 def aas_groups(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                group_q, group_off, kv_idx, similarity="cosine", scale: Optional[float] = None) -> torch.Tensor:
     """Directional AAS similarities for grouped (query image, kv image list) work -- see ds_aas_groups.
-    q/k_self/v_self: (Nq,B,H,S,D); k/v: (Nk,B,H,S,D).  Returns float32 [n_entries].  Differentiable in the five
+    q: (Nq,B,H,S_q,D), k_self/v_self: (Nq,B,H,S_self,D); k/v: (Nk,B,H,S_cross,D); the three lengths are independent
+    (for AAS S_self = S_q).  Returns float32 [n_entries].  Differentiable in the five
     caches (aas_groups_bwd) when one of them requires grad; the values are the same either way."""
     if wants_grad(q, k_self, v_self, k, v):
         dev = _need_cuda(q)
@@ -560,7 +563,8 @@ class _AASTripletsFn(torch.autograd.Function):
 def aas_matrix(q: torch.Tensor, k_self: torch.Tensor, v_self: torch.Tensor, k: torch.Tensor, v: torch.Tensor,
                similarity="cosine", scale: Optional[float] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Directional matrix Dm[r,c] = dir(row image r -> column image c); rows (q,k_self,v_self): (Nr,...),
-    columns (k,v): (Nc,...).  Returns float32 [Nr,Nc].  Differentiable in the five caches (aas_matrix_bwd) when one of
+    columns (k,v): (Nc,...); the columns' token count may differ from the rows' (captures at two resolutions, see
+    scoring.aas_scores_between).  Returns float32 [Nr,Nc].  Differentiable in the five caches (aas_matrix_bwd) when one of
     them requires grad and `out` is not given; the values are the same either way."""
     if out is None and wants_grad(q, k_self, v_self, k, v):
         return _AASMatrixFn.apply(similarity, scale, q, k_self, v_self, k, v)

@@ -369,6 +369,16 @@ def _matrix_grad_block(q_all, k_all, v_all, r0: int, r1: int, d_full: torch.Tens
     return dq, dks, dvs, dk, dv
 
 
+def aas_scores_between(a: QKVCache, b: QKVCache, similarity: str = "cosine", scale: Optional[float] = None) -> torch.Tensor:
+    """DiffSim scores [Na, Nb] between the images of two caches: (Dm(a->b) + Dm(b->a)^T) / 2, entry (i, j) the value of
+    DiffSim.diffsim(a_i, b_j).  The caches may hold different token counts (a query set and a gallery captured at two
+    image sizes); B, H, D and the dtype must match.  Differentiable in both caches (ops.aas_matrix) when one of them
+    requires grad."""
+    ab = ops.aas_matrix(a.q, a.k, a.v, b.k, b.v, similarity, scale)
+    ba = ops.aas_matrix(b.q, b.k, b.v, a.k, a.v, similarity, scale)
+    return (ab + ba.t()) * 0.5
+
+
 def symmetrize(dm: torch.Tensor) -> torch.Tensor:
     """S = (Dm + Dm^T)/2: DiffSim.diffsim(i, j) for every pair (diffsim/diffsim.py:197)."""
     return (dm + dm.t()) * 0.5

@@ -135,6 +135,12 @@ size_t ds_attn_fwd_workspace_bytes(ds_tensor4 q, ds_tensor4 k);
  *
  * (q, k_self, v_self) are indexed by group_q; (k, v) are indexed by kv_idx.
  * For ordinary pair scoring pass k_self = k and v_self = v.
+ * Lengths: (k_self, v_self) share one kv length S_self and (k, v) one kv
+ * length S_cross; both are independent of q's S_q (for AAS S_self is S_q, the
+ * query image's own token count, and S_cross that of the other images: two
+ * captures at different resolutions score against each other).  B, H, D and
+ * the dtype match across all five.  k_self / v_self (k / v) of different
+ * lengths are DS_ERR_INVALID.
  * mode: DS_SIM_COSINE | DS_SIM_MSE.   dir: float[n_entries].
  */
 int ds_aas_groups(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self,
@@ -181,7 +187,9 @@ size_t ds_aas_triplets_workspace_bytes(ds_tensor5 q, int64_t n_triplets);
  * ships the consumer of its output, retrieval_vis.py:57-68):
  *     Dm[r*ldd + c] = dir(row image r -> column image c)
  * rows: (q, k_self, v_self) of Nr images; columns: (k, v) of Nc images.
- * The symmetric score is S = (Dm + Dm^T)/2 over a square index set.
+ * The kv lengths of rows and columns may differ, as in ds_aas_groups.
+ * The symmetric score is S = (Dm + Dm^T)/2 over a square index set; between
+ * two image sets A and B it is (Dm(A->B) + Dm(B->A)^T)/2.
  * Row-block sharding over GPUs calls this with the local rows and all columns.
  */
 int ds_aas_matrix(ds_tensor5 q, ds_tensor5 k_self, ds_tensor5 v_self,
@@ -213,7 +221,8 @@ size_t ds_attn_bwd_workspace_bytes(ds_tensor4 q, ds_tensor4 k);
  * the rounding passed straight through.  d_dir: ONE float on the device (dL/ddir;
  * read there, no host synchronisation).  The five FLOAT32 gradients are added
  * into; they may alias (dk_i = dk_j when image i is image j).  dq_i receives
- * the cross term before the self term.
+ * the cross term before the self term.  k_i / v_i and k_j / v_j may have
+ * different kv lengths (each pair one length), independent of q_i's.
  */
 int ds_aas_dir_bwd(ds_tensor4 q_i, ds_tensor4 k_i, ds_tensor4 v_i, ds_tensor4 k_j, ds_tensor4 v_j,
                    float scale, int mode, const float* d_dir,
@@ -226,6 +235,8 @@ size_t ds_aas_dir_bwd_workspace_bytes(ds_tensor4 q_i, ds_tensor4 k_j);
  * on the device.  Same arguments as ds_aas_groups; the five FLOAT32 (N,B,H,S,D) gradients (of q, k_self, v_self, k, v;
  * any strides with a unit innermost one) are ADDED INTO.  dk_self / dk, and dv_self / dv, are either the same tensor
  * (same pointer, sizes and strides: the pairs / triplets case, where k_self is k) or have disjoint address ranges.
+ * The kv lengths follow ds_aas_groups: S_self for (k_self, v_self), S_cross for (k, v); every term walks its own length
+ * (shared gradient buffers imply S_self = S_cross).
  *
  * Bitwise contract: the buffers end up exactly as after one ds_aas_dir_bwd call per entry, t = 0 .. n_entries - 1 in order,
  * on the slices (q, k_self, v_self)[group_q[g(t)]], (k, v)[kv_idx[t]], d_dir + t and the matching gradient slices: every
@@ -266,7 +277,8 @@ size_t ds_aas_triplets_bwd_workspace_bytes(ds_tensor5 q, int64_t n_triplets);
  * Backward of ds_aas_matrix for d_Dm[r*ldd + c] = dL/dDm[r, c] (float, Nr rows of Nc values, on the device; read there,
  * no host synchronisation).  Same operands as ds_aas_matrix; the five FLOAT32 (N,B,H,S,D) gradients (of q, k_self,
  * v_self, k, v; any strides with a unit innermost one) are ADDED INTO, with the aliasing rule of ds_aas_groups_bwd:
- * dk_self / dk (dv_self / dv) are the same tensor or have disjoint address ranges.
+ * dk_self / dk (dv_self / dv) are the same tensor or have disjoint address ranges.  The rows' and the columns' kv
+ * lengths may differ, as in ds_aas_matrix.
  *
  * It is the grouped backward of the row-major matrix list (group r = row r, entries (r, c) for c = 0 .. Nc-1), except
  * that the Nc self terms of row r -- Attn(q_r, k_self_r, v_self_r) with dO = coef_self_rc fy_rc -- are FOLDED into one
