@@ -28,11 +28,12 @@
 // lives in TMEM as well.  Shared memory then carries only TMA writes + one read of K and V + two reads of Q.
 //
 // Softmax.  Online over 128-column halves with a LAZY running maximum: the first half of an item fixes the
-// reference maximum m of every row; a later half only moves m (and rescales O and the running sum) when some
-// row of the tile exceeds m by more than 2^8 -- otherwise p = exp2(s - m) is simply allowed to be as large as
-// 256, which 16-bit P and fp32 sums hold without loss.  The result is the exact softmax either way (any common
-// offset cancels in O / l).  The rare rescale is done by the first-quarter softmax warps themselves before they
-// release P, so the common path has no extra barrier and half A never waits for half B.
+// reference maximum m of every row; a later half only moves a row's m (and rescales its O and running sum) when the
+// half's maximum exceeds m by more than tau = 14 (fp16) or 30 (bf16) in log2 units -- otherwise p = exp2(s - m) is
+// simply allowed to grow up to 2^14 (fp16) or 2^30 (bf16), which 16-bit P and fp32 sums hold without loss.  The
+// result is the exact softmax either way (any common offset cancels in O / l).  The rare rescale is done by the
+// first-quarter softmax warps themselves before they release P, so the common path has no extra barrier and half A
+// never waits for half B.
 //
 // Pipeline.  The MMA warp issues, in this fixed order, PV_A(u), QK_A(u+1), PV_B(u), QK_B(u+1): tcgen05 ops of
 // one thread execute in issue order, so QK_A(u+1) may overwrite the columns PV_A(u) reads P from without any
